@@ -26,6 +26,11 @@
 `cpu_baseline`: the oracle (literal C port of the reference step) on all host cores, bounded sample.
 `--impl reference`: the CPU arm alone (the reference Java cannot run here: no JVM; the literal C port of oracle/ stands
            in, one single-threaded process per host core); its `config` says exactly what a "step" of that arm is.
+`--dump-outputs DIR`: after the timed steps, what the timed (device-resident) path computed in its last timed step is
+           written as DIR/<name>.npy in float32: configs 2 / 4 obs, reward, done of every env (what rlfc_env_step_device
+           hands its caller), configs 3 / 5 the fields ux, uy, p of the domain.  The inputs depend on the arguments only,
+           so two builds run with the same arguments can be compared array for array.  At most 64 MB in all: an array
+           over its share is replaced by a fixed sample of its elements (sorted unique flat indices drawn with seed 0).
 """
 from __future__ import annotations
 
@@ -51,6 +56,21 @@ UNIT = "env-steps/s"
 
 METRIC3 = "solver-steps/sec (single 2048x1024 BDIM domain)"
 UNIT3 = "solver-steps/s"
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write {name: array} as out_dir/<name>.npy in float32 within DUMP_LIMIT_BYTES (see --dump-outputs)."""
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    share = DUMP_LIMIT_BYTES // (4 * len(arrays))
+    for name, a in arrays.items():
+        a = np.ascontiguousarray(a, dtype=np.float32)
+        if a.size > share:
+            a = a.ravel()[np.unique(np.random.default_rng(0).integers(0, a.size, share))]
+        np.save(out / f"{name}.npy", a)
 
 
 def workload_config(envs_per_gpu, n_gpus, config=2, n_total=None):
@@ -431,6 +451,9 @@ def run_b200(args):
         obs_check = obs_dev.cpu().numpy()
         assert np.isfinite(obs_check).all(), "non-finite observation"
         assert env.running() == 0 and not env.flags().any()
+        if args.dump_outputs:   # the last timed step's results of the whole batch, in global env order
+            outputs = {nm: sharding.gather_observations(t, world).cpu().numpy()
+                       for nm, t in (("obs", obs_dev), ("reward", rew_dev), ("done", done_dev.float()))}
 
         # ---- end-to-end arm: host buffers through rlfc_env_step ----
         for _ in range(W):
@@ -493,6 +516,8 @@ def run_b200(args):
             line["nccl_ranks"] = dist.get_world_size()
         if world == 1 and not args.no_cpu_baseline:
             line["cpu_baseline"] = cpu_baseline(args.cpu_sample_env_steps)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -537,6 +562,8 @@ def run_wide(args):
         ms = sharding.max_over_ranks(e0.elapsed_time(e1), world, device="cuda")
         launches = env.launch_count - l0
         clk = clocks.stop() if rank == 0 else None
+        if args.dump_outputs and rank == 0:   # (the other ranks run identical replicas)
+            outputs = dict(zip(("ux", "uy", "p"), env.get_fields(0)))
         # ---- end-to-end: host action in, force + probes out, every step ----
         for _ in range(W):
             env.update2(act_host, want_probes=True)
@@ -588,6 +615,8 @@ def run_wide(args):
             line["config"]["workload"] += f" [scaled run: resolution {res}, grid {env.n - 2}x{env.m - 2}]"
         if world == 1 and not args.no_cpu_baseline and res == 128:
             line["cpu_baseline"] = cpu_baseline_wide(args.cpu_sample_wide_steps)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()
@@ -695,6 +724,8 @@ def run_slab(args):
         nv1 = nvlink_counters(nd)
         launches, barriers = env.launch_count - l0, env.slab_info()[1] - b0
         clk = clocks.stop()
+        if args.dump_outputs:
+            outputs = dict(zip(("ux", "uy", "p"), env.get_fields(0)))
         for _ in range(W):
             env.update2(act_host, want_probes=True)
         t0 = time.perf_counter()
@@ -740,6 +771,8 @@ def run_slab(args):
                          "model": "4 B x N_int x (28 + 16 (kP + kC)) = 240 B/cell at one MG iteration per solve (SURVEY 8d)"},
             "kernels": table, "mg_iters_per_solve": k_sum / 2,
         }
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line))
     if world > 1:
         dist.barrier()
@@ -763,7 +796,11 @@ def main():
                     help="configs 3 / 5: cells per diameter (default 128 = the 2048x1024 domain / 512 = the 8192x4096 domain)")
     ap.add_argument("--settle-steps", type=int, default=12, help="config 3: untimed solver steps after the impulsive start")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the timed path's outputs of its last timed step as DIR/<name>.npy (float32, at most 64 MB)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU path (--impl b200)")
     if args.resolution is None:
         args.resolution = 512 if args.config == 5 else 128
     if args.steps is None:

@@ -143,3 +143,20 @@ def test_bench_actions_are_deterministic_and_sharded():
     assert np.array_equal(a0, bench.make_actions(5, 8, 0)) and not np.array_equal(a0, a1)
     k = np.arange(5)
     assert np.array_equal(a0[:, 0, 0], (0.8 * np.sin(2 * np.pi * k / 25.0)).astype(np.float32))     # env 0: config-1 sequence
+
+
+def test_bench_dump_outputs_float32_within_budget(tmp_path):
+    """--dump-outputs: small arrays are written whole as float32, a field too large for the 64 MB budget is replaced by the
+    same sample of its elements in every run."""
+    import bench
+    done = np.array([0, 1, 0], np.int32)
+    big = np.arange(3 * 2000 * 2000, dtype=np.float32).reshape(3, 2000, 2000)          # 48 MB: over the share of one of two
+    for d in ("a", "b"):
+        bench.dump_outputs(tmp_path / d, {"done": done, "p": big})
+    got = {f.name: np.load(f) for f in sorted((tmp_path / "a").iterdir())}
+    assert sorted(got) == ["done.npy", "p.npy"] and all(a.dtype == np.float32 for a in got.values())
+    assert np.array_equal(got["done.npy"], done.astype(np.float32))
+    assert sum(f.stat().st_size for f in (tmp_path / "a").iterdir()) <= 64 << 20
+    p = got["p.npy"]                                      # element values = flat indices: distinct, in storage order
+    assert 1000 < p.size < big.size and np.all(np.diff(p) > 0) and np.all(p == np.floor(p)) and p[-1] < big.size
+    assert np.array_equal(p, np.load(tmp_path / "b" / "p.npy"))

@@ -1,11 +1,7 @@
 """The reference-run recipe (oracle/ref_java): the Processing pre-processor subset is checked on snippets (no JVM is needed
-for that), and -- where the reference tree is present -- on the real tabs: only literal suffixes, colours and conversion
-calls may change."""
+for that): only literal suffixes, colours and conversion calls may change."""
 import importlib.util
-import re
 from pathlib import Path
-
-import pytest
 
 ROOT = Path(__file__).resolve().parents[1]
 spec = importlib.util.spec_from_file_location("pde2java", ROOT / "oracle" / "ref_java" / "pde2java.py")
@@ -29,23 +25,3 @@ def test_strings_and_comments_are_left_alone():
     src = 'println("dt = 0.5, color #993333"); // scale by 0.5\n/* float(x) 1.0 */ char q = \'.\'; x = 1.0;'
     assert c(src) == 'println("dt = 0.5, color #993333"); // scale by 0.5\n/* float(x) 1.0 */ char q = \'.\'; x = 1.0f;'
 
-
-@pytest.mark.skipif(not Path("/root/reference/clientLilypad/BDIM.pde").exists(), reason="reference tree not present")
-def test_real_tabs_change_only_in_the_expected_ways():
-    tabs = ["Window", "OrthoNormal", "Body", "BodyUnion", "Field", "VectorField", "PoissonMatrix", "MG", "BDIM", "SaveScalar",
-            "AFCCylinder"]
-    number = re.compile(r"(?<![\w.])(\d+\.\d*|\.\d+|\d+[eE][+-]?\d+)(?:[eE][+-]?\d+)?f")
-    for t in tabs:
-        src = Path(f"/root/reference/clientLilypad/{t}.pde").read_text(errors="replace")
-        out = pde2java.convert(src)
-        a, b = src.split("\n"), out.split("\n")
-        assert len(a) == len(b)
-        for la, lb in zip(a, b):
-            if la == lb:
-                continue
-            # undo the permitted rewrites and require the original line
-            back = number.sub(lambda m: m.group(0)[:-1], lb)
-            back = back.replace("parseFloat(", "float(").replace("parseInt(", "int(")
-            back = re.sub(r"0xFF([0-9A-Fa-f]{6})\b", r"#\1", back)
-            la_norm = re.sub(r"\bcolor\b(?!\s*\()", "int", la)
-            assert back == la_norm, (t, la, lb)
