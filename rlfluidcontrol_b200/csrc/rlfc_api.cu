@@ -918,6 +918,9 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
   // than ~8 Mi cells does not give the marching kernel enough warps -- one 2048x1024 domain: 38 vs 31 us)
   if ((((g.n - 2) | (g.m - 2)) & 1) || (long long)B * (g.n - 2) * (g.m - 2) < (8ll << 20)) sp.resid_march = 0;
   if (const char* ev = std::getenv("RLFC_RESID")) if (std::strcmp(ev, "march") == 0 && !(((g.n - 2) | (g.m - 2)) & 1)) sp.resid_march = 1;
+  // slab mode keeps the tile kernel: the marching kernel bulk-copies its rows (cp.async.bulk), which here would read
+  // other devices' memory through the shared address range, a combination that has not been run on several devices
+  if (slab) sp.resid_march = 0;
   int n_groups = cfg->n_groups;
   if (const char* ev = std::getenv("RLFC_GROUPS")) n_groups = std::atoi(ev);
   // (measured, 256 default-grid envs, final round-2 kernels: 1 group 7 120, 2 groups 7 333-7 364, 3 groups 7 230, 4 groups 7 242

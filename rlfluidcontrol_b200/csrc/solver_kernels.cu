@@ -605,25 +605,42 @@ k_resid_down0(const __grid_constant__ SolverParams q, const float* __restrict__ 
 
 // ------------------------------------------------------------------------------------------------
 // The same fused first MG iteration as a MARCHING kernel (the default; k_resid_down0 above is kept as the cross-check,
-// RLFC_RESID=tile): a warp owns kRmCols columns (+2 halo lanes on either side, as k_advdif) and marches down kRmRows
-// rows.  Everything that is shared between neighbouring cells is loaded ONCE: p, ux, lx travel down the rows in
-// registers, the j-neighbours of p, uy, ly and d come from the adjacent lanes by shuffle -- 7 loads, 8 shuffles and
-// ~27 float operations per cell instead of the tile version's 15 + 5 loads and its shared-memory round trip
-// (225 -> ~75 thread instructions per fine cell).  Row i is finalised one iteration after its d is formed, when
-// d of row i+1 exists.  Arithmetic and its order are those of k_resid_down0 / the reference.
+// RLFC_RESID=tile): a compute warp owns kRmCols columns (+2 halo lanes on either side, as k_advdif) and marches down
+// the CTA's kRmRows rows.  Everything that is shared between neighbouring cells is read ONCE: p, ux, lx travel down the
+// rows in registers, the j-neighbours of p, uy, ly and d come from the adjacent lanes by shuffle -- 7 reads, 8 shuffles
+// and ~27 float operations per cell.  Row i is finalised one step after its d is formed, when d of row i+1 exists.
+// Arithmetic and its order are those of k_resid_down0 / the reference.
+//
+// Where the operands come from: the kernel streams at HBM speed only with enough bytes in flight, and register-target
+// loads cannot provide them (one row per lane in flight at 64 registers and 50 % occupancy: 2.4 TB/s; issuing them a
+// row or two ahead needed 88 registers and serialised on the warp's load scoreboards, 176 -> 241 us).  So the rows
+// come through a shared-memory ring: one lane of a loader warp bulk-copies (cp.async.bulk, UBLKCP) row q of all seven
+// operand arrays -- p, ux, uy and the L2-resident lx, ly, diag, inv -- into slot q % kRmDepth, completing on the
+// slot's `full` mbarrier; the compute warps read their lane's column out of the slot with plain shared loads and free
+// it through the slot's `empty` mbarrier (one arrival per compute warp) once no later step reads that row.  A CTA of
+// kRmWarps compute warps covers kRmWarps*kRmCols = 196 columns, the full width of the default grid (192 columns; one
+// 800-byte row per array), so all warps share every staged row and the halo columns of neighbouring warps cost no
+// extra copy; wider grids are cut into column windows of that width.  Step s (forming row ia-1+s) reads rows s..s+3 of
+// the ring (q = row - ia + 2; s-1 .. s+1 for finishing row ia-2+s) and releases row s-1, so the loader runs
+// kRmDepth - 5 rows ahead of the slowest warp.
 // ------------------------------------------------------------------------------------------------
 constexpr int kRmCols = 28;       // output columns per warp (even: 2x2 restriction pairs start at odd columns)
-#ifndef RLFC_RM_ROWS
-#define RLFC_RM_ROWS 32
-#endif
-#ifndef RLFC_RM_MINB
-#define RLFC_RM_MINB 8
-#endif
-constexpr int kRmRows = RLFC_RM_ROWS;   // rows per chunk (even)
+constexpr int kRmWarps = 7;       // compute warps per CTA (+1 loader warp)
+constexpr int kRmRows = 32;       // rows per CTA (even)
+constexpr int kRmDepth = 8;       // ring slots
+constexpr int kRmMinB = 4;        // CTAs per SM: 4 x 47 KB of ring, at most 64 registers
+constexpr int kRmArrays = 7;      // staged arrays: p, ux, uy, lx, ly, diag, inv
+constexpr int kRmSeg = 208;       // floats per staged row segment: kRmWarps*kRmCols + 4 halo columns, 16-byte aligned ends
+constexpr size_t kRmSmem = (size_t)kRmDepth * kRmArrays * kRmSeg * 4 + 2 * kRmDepth * 8;
 
-__global__ void __launch_bounds__(128, RLFC_RM_MINB)
+__global__ void __launch_bounds__(32 * (kRmWarps + 1), kRmMinB)
 k_resid_down0_march(const __grid_constant__ SolverParams q, const float* __restrict__ ux_all, const float* __restrict__ uy_all,
                     const float* __restrict__ pin_all, float* __restrict__ pout_all, float* __restrict__ rout_all, int which) {
+  using namespace rows_detail;
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  float* ring = reinterpret_cast<float*>(smem_raw);                  // [kRmDepth][kRmArrays][kRmSeg]
+  unsigned long long* full = reinterpret_cast<unsigned long long*>(ring + (size_t)kRmDepth * kRmArrays * kRmSeg);
+  unsigned long long* empty = full + kRmDepth;
   const DevLevel& L = q.lev[0];
   const DevLevel& C = q.lev[1];
   const int P = L.P, n = L.n, m = L.m, ni = n - 2, mj = m - 2;
@@ -632,39 +649,65 @@ k_resid_down0_march(const __grid_constant__ SolverParams q, const float* __restr
   if (slab_skip(blockIdx.y, gridDim.y, q.slab_rank, q.slab_n)) return;
   if (blockIdx.x == 0 && blockIdx.y == 0 && threadIdx.x == 0) { q.sc.active[e] = 1; q.sc.iters[2 * e + which] = 0; }
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int jw0 = 1 + blockIdx.x * kRmCols;                          // first output column of this warp (odd)
-  const int ia = 1 + (blockIdx.y * 4 + warp) * kRmRows;              // first row of this chunk (odd)
-  if (ia > ni) return;
+  const int jc0 = 1 + blockIdx.x * (kRmWarps * kRmCols);             // first output column of this CTA (odd)
+  const int c0 = max(jc0 - 2, 0) & ~3;                               // staged columns [c0, c1)
+  const int c1 = min(P, (jc0 - 2 + (kRmWarps - 1) * kRmCols + 32 + 3) & ~3);
+  const int ia = 1 + blockIdx.y * kRmRows;                           // first row of this chunk (odd)
   const int ib = min(ia + kRmRows - 1, ni);
+  const int nq = 2 + 2 * ((ib - ia + 2) / 2) + 3;                    // staged rows ia-2 .. : the prologue's three + one per form
   const size_t eo = (size_t)e * L.stride;
-  const float* __restrict__ ux = ux_all + eo;
-  const float* __restrict__ uy = uy_all + eo;
   const float* __restrict__ pin = pin_all + eo;
+  auto rowc = [&](int i) { return min(max(i, 0), n - 1); };
+  if (threadIdx.x == 0) {
+    for (int s = 0; s < kRmDepth; s++) { mbar_init(full + s, 1); mbar_init(empty + s, kRmWarps); }
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  }
+  __syncthreads();
+  if (warp == kRmWarps) {                                            // loader
+    if (lane == 0) {
+      const float* src[kRmArrays] = {pin, ux_all + eo, uy_all + eo, L.lx, L.ly, L.diag, L.inv};
+      const unsigned bytes = (unsigned)(c1 - c0) * 4u;
+      for (int qq = 0; qq < nq; qq++) {
+        const int s = qq % kRmDepth;
+        if (qq >= kRmDepth) mbar_wait(empty + s, (unsigned)(qq / kRmDepth - 1) & 1u);
+        const size_t off = (size_t)rowc(ia - 2 + qq) * P + c0;
+        mbar_expect_tx(full + s, kRmArrays * bytes);
+#pragma unroll
+        for (int a = 0; a < kRmArrays; a++) bulk_g2s(ring + ((size_t)s * kRmArrays + a) * kRmSeg, src[a] + off, bytes, full + s);
+      }
+    }
+    return;
+  }
   float* __restrict__ pout = pout_all + eo;
   float* __restrict__ rout = rout_all + eo;
-  const float* __restrict__ lx = L.lx;
-  const float* __restrict__ ly = L.ly;
-  const float* __restrict__ diag = L.diag;
-  const float* __restrict__ inv = L.inv;
+  const int jw0 = jc0 + warp * kRmCols;                              // first output column of this warp (odd)
   const int j = jw0 - 2 + lane;                                      // this lane's column (may be outside the array)
-  const int jl = min(max(j, 0), m - 1);                              // clamped for loads
+  const int cs = min(max(j, 0), m - 1) - c0;                         // its (clamped) column in the staged segments
   const bool out_lane = lane >= 2 && lane < 2 + kRmCols && j <= mj;
   const bool jfirst = j == 1, jlast = j == mj;
-  auto rowc = [&](int i) { return min(max(i, 0), n - 1); };
+  enum { aP, aUX, aUY, aLX, aLY, aDG, aIV };
+  auto slot = [&](int qq) { return ring + (size_t)(qq % kRmDepth) * kRmArrays * kRmSeg + cs; };
+  auto wait_row = [&](int qq) { mbar_wait(full + qq % kRmDepth, (unsigned)(qq / kRmDepth) & 1u); };
+  auto release_row = [&](int qq) {
+    __syncwarp();
+    if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(sm_addr(empty + qq % kRmDepth)) : "memory");
+  };
   // rolling rows: p of rows ir-1, ir, ir+1; ux and lx of rows ir, ir+1
   int ir = ia - 1;                                                   // the row whose r and d are formed next
-  float p_m = pin[IDX(rowc(ir - 1), jl)], p_c = pin[IDX(rowc(ir), jl)], p_n = pin[IDX(rowc(ir + 1), jl)];
-  float ux_c = ux[IDX(rowc(ir), jl)], lx_c = lx[IDX(rowc(ir), jl)];
+  int qr = 1;                                                        // its ring row
+  wait_row(0); wait_row(1); wait_row(2);
+  float p_m = slot(0)[aP * kRmSeg], p_c = slot(1)[aP * kRmSeg], p_n = slot(2)[aP * kRmSeg];
+  float ux_c = slot(1)[aUX * kRmSeg], lx_c = slot(1)[aLX * kRmSeg];
   // what finalising a row needs from the two rows formed before it
   float d_1 = 0.f, d_2 = 0.f, r_1 = 0.f, pq_1 = 0.f, pq_2 = 0.f, diag_1 = 0.f, lxw_1 = 0.f, ly_1 = 0.f, lyn_1 = 0.f;
   float acc = 0.f;
-  // forms r and d of row ir (garbage outside the interior, never used there) and advances the rolling rows.  (Issuing the
-  // seven loads one or two rows ahead of their use was measured: 176 -> 241 us -- 88 registers instead of 64, and deep
-  // register-target prefetches serialise on the warp's six load scoreboards.)
+  // forms r and d of row ir (garbage outside the interior, never used there) and advances the rolling rows
   auto form = [&](float& r_out, float& d_out, float& diag_o, float& lxw_o, float& ly_o, float& lyn_o) {
-    const int k = IDX(rowc(ir), jl), kn = IDX(rowc(ir + 1), jl);
-    const float ux_n = ux[kn], lx_n = lx[kn];
-    const float uy_c = uy[k], ly_c = ly[k], dg = diag[k], iv = inv[k];
+    wait_row(qr + 2);
+    const float* sc = slot(qr);
+    const float* sn = slot(qr + 1);
+    const float ux_n = sn[aUX * kRmSeg], lx_n = sn[aLX * kRmSeg];
+    const float uy_c = sc[aUY * kRmSeg], ly_c = sc[aLY * kRmSeg], dg = sc[aDG * kRmSeg], iv = sc[aIV * kRmSeg];
     const float p_s = __shfl_up_sync(0xffffffffu, p_c, 1), p_nn = __shfl_down_sync(0xffffffffu, p_c, 1);
     const float uy_n = __shfl_down_sync(0xffffffffu, uy_c, 1), ly_n = __shfl_down_sync(0xffffffffu, ly_c, 1);
     const float sdiv = ux_n - ux_c + uy_n - uy_c;                    // VectorField.pde:56-65
@@ -675,10 +718,11 @@ k_resid_down0_march(const __grid_constant__ SolverParams q, const float* __restr
     // advance: ir -> ir + 1
     ux_c = ux_n; lx_c = lx_n;
     p_m = p_c; p_c = p_n;
-    ir++;
-    p_n = pin[IDX(rowc(ir + 1), jl)];
+    ir++; qr++;
+    p_n = slot(qr + 1)[aP * kRmSeg];
   };
-  // finalises row i = ir - 2 (its d is d_1, the rows around it d_2 and d_0): smooth(0) increment, new p, restriction
+  // finalises row i = ir - 2 (its d is d_1, the rows around it d_2 and d_0): smooth(0) increment, new p, restriction;
+  // then row i - 1 is no longer read
   auto finish = [&](int i, float d_0, float lxe, float p_e, bool odd) {
     const float dc = d_1;
     const float dW = (i == 1) ? dc : d_2, dE = (i == ni) ? dc : d_0;             // d.setBC: ghost = adjacent interior value
@@ -695,10 +739,11 @@ k_resid_down0_march(const __grid_constant__ SolverParams q, const float* __restr
       // ghosts of x receive the clamped d (x.plusEq(d) runs over all cells, MG.pde:95); p's ghosts are live data
       const int di = (i == 1) ? -1 : (i == ni ? 1 : 0), dj = jfirst ? -1 : (jlast ? 1 : 0);
       if (di) pout[IDX(i + di, j)] = ((di < 0) ? pq_2 : p_e) + dc;
-      if (dj) pout[IDX(i, j + dj)] = pin[IDX(i, j + dj)] + dc;
-      if (di && dj) pout[IDX(i + di, j + dj)] = pin[IDX(i + di, j + dj)] + dc;
+      if (dj) pout[IDX(i, j + dj)] = slot(qr - 2)[aP * kRmSeg + dj] + dc;
+      if (di && dj) pout[IDX(i + di, j + dj)] = slot(qr - 2 + di)[aP * kRmSeg + dj] + dc;
       if (!odd && !(lane & 1)) C.r[(size_t)e * C.stride + (i >> 1) * C.P + ((j + 1) >> 1)] = acc;
     }
+    release_row(qr - 3);
   };
   // prologue: rows ia-1 and ia
   {
@@ -708,6 +753,7 @@ k_resid_down0_march(const __grid_constant__ SolverParams q, const float* __restr
     d_2 = d0; pq_2 = p_m;                                             // p_m is now p of row ia - 1
     form(r_1, d_1, diag_1, lxw_1, ly_1, lyn_1);                       // row ia
     pq_1 = p_m;                                                       // p of row ia
+    release_row(0);                                                   // row ia - 2
   }
   for (int i = ia; i <= ib; i += 2) {
     float r0, d0, g0, w0, y0, yn0;
@@ -846,72 +892,103 @@ k_mg_up0(const __grid_constant__ SolverParams q, float* __restrict__ r_all) {
 // xc[I][J]; their outward neighbours take the adjacent coarse cell's value, or -- at the domain edge, where
 // d.setBC copies the adjacent interior value (MG.pde:139-152) -- the cell's own.  x += d on the children and on the
 // ghost cells they border, r -= A d written to the smoother's skewed array.
-#ifndef RLFC_UP0_MINB
-#define RLFC_UP0_MINB 1
-#endif
-__global__ void __launch_bounds__(256, RLFC_UP0_MINB)
+// A CTA owns kUpRows fine rows of one environment over the full width (the row smoother's grids are at most 256 columns
+// wide).  Its rows of x and r and the coarse x rows around them are contiguous in memory: one thread bulk-copies them
+// into shared memory (three cp.async.bulk copies on one mbarrier), so a CTA's loads are in flight at once without
+// holding registers.  The new residual overwrites r in shared memory and leaves in a second phase in the skewed order:
+// the CTA's part of skewed entry tau (row tau - ln of lane ln, ln in [tau - i0 - kUpRows + 1, tau - i0]) is one
+// contiguous range, written by one warp with consecutive stores (the skewed index of a thread's own cells scatters
+// 4-byte stores over 24-byte lane blocks).
+constexpr int kUpRows = 16;       // fine rows per CTA (even)
+
+static size_t up0_smem(const SolverParams& q) {
+  return sizeof(float) * (2 * (size_t)kUpRows * q.P + (size_t)(kUpRows / 2 + 2) * q.lev[1].P) + 16;
+}
+
+__global__ void __launch_bounds__(256)
 k_mg_up0_blk(const __grid_constant__ SolverParams q, const float* __restrict__ r_all) {
-  const int e = blockIdx.z;
+  using namespace rows_detail;
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  const int e = blockIdx.y;
   if (!q.sc.active[e]) return;
   const DevLevel& L0 = q.lev[0];
   const DevLevel& L1 = q.lev[1];
-  const int P = L0.P, n = L0.n, m = L0.m, CPc = L1.P;
+  const int P = L0.P, n = L0.n, m = L0.m, ni = n - 2, mj = m - 2, CPc = L1.P;
   const int nci = L1.n - 2, ncj = L1.m - 2;
-  const int J = blockIdx.x * blockDim.x + threadIdx.x + 1;
-  const int I = blockIdx.y * blockDim.y + threadIdx.y + 1;
-  if (I > nci || J > ncj) return;
-  const float* __restrict__ xc = L1.x + (size_t)e * L1.stride;
+  const int i0 = 1 + blockIdx.x * kUpRows, rows = min(kUpRows, ni + 1 - i0);   // fine rows i0 .. i0+rows-1
+  const int I0 = (i0 + 1) / 2;                                                  // their first coarse row
+  float* s_x = reinterpret_cast<float*>(smem_raw);                              // [rows][P] from row i0
+  float* s_r = s_x + kUpRows * P;                                               // [rows][P] from row i0
+  float* s_xc = s_r + kUpRows * P;                                              // [rows/2 + 2][CPc] from coarse row I0-1
+  unsigned long long* bar = reinterpret_cast<unsigned long long*>(s_xc + (kUpRows / 2 + 2) * CPc);
   const size_t eo = (size_t)e * L0.stride;
   float* __restrict__ x = L0.x + eo;
-  const float* __restrict__ r = r_all + eo;
-  float* __restrict__ rsk = q.rsk + (size_t)e * q.rsk_stride;
-  const float dc = xc[I * CPc + J];
-  const float dWc = (I > 1) ? xc[(I - 1) * CPc + J] : dc, dEc = (I < nci) ? xc[(I + 1) * CPc + J] : dc;
-  const float dSc = (J > 1) ? xc[I * CPc + J - 1] : dc, dNc = (J < ncj) ? xc[I * CPc + J + 1] : dc;
-  const int i0 = 2 * I - 1, j0 = 2 * J - 1;
+  if (threadIdx.x == 0) {
+    mbar_init(bar, 1);
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    const unsigned fb = (unsigned)(rows * P) * 4u, cb = (unsigned)((rows / 2 + 2) * CPc) * 4u;
+    mbar_expect_tx(bar, 2 * fb + cb);
+    bulk_g2s(s_x, x + (size_t)i0 * P, fb, bar);
+    bulk_g2s(s_r, r_all + eo + (size_t)i0 * P, fb, bar);
+    bulk_g2s(s_xc, L1.x + (size_t)e * L1.stride + (size_t)(I0 - 1) * CPc, cb, bar);
+  }
+  __syncthreads();
+  mbar_wait(bar, 0);
   const int C = L0.rt.C, CP = rows_CP(C);
-  float xo[2][2], ro[2][2];
+  for (int t = threadIdx.x; t < (rows / 2) * ncj; t += blockDim.x) {
+    const int Il = t / ncj, J = t - Il * ncj + 1, I = I0 + Il;
+    const float* xc = s_xc + (Il + 1) * CPc;
+    const float dc = xc[J];
+    const float dWc = (I > 1) ? xc[J - CPc] : dc, dEc = (I < nci) ? xc[J + CPc] : dc;
+    const float dSc = (J > 1) ? xc[J - 1] : dc, dNc = (J < ncj) ? xc[J + 1] : dc;
+    const int a0 = 2 * Il, ig = i0 + a0, j0 = 2 * J - 1;
+    // the 2x2 block's face coefficients, each loaded once: lx on the three rows ig .. ig+2, ly on the three columns
+    // j0 .. j0+2; the diagonal is their plain sum (PoissonMatrix.pde:46-48; checked against the host table at create time)
+    float lxv[3][2], lyv[2][3];
 #pragma unroll
-  for (int a = 0; a < 2; a++)
+    for (int a = 0; a < 3; a++)
 #pragma unroll
-    for (int b = 0; b < 2; b++) { xo[a][b] = x[IDX(i0 + a, j0 + b)]; ro[a][b] = r[IDX(i0 + a, j0 + b)]; }
-  // the 2x2 block's face coefficients, each loaded once: lx on the three rows i0 .. i0+2, ly on the three columns j0 .. j0+2;
-  // the diagonal is their plain sum (PoissonMatrix.pde:46-48; checked against the host table at create time)
-  // (a single division per thread for the skewed index of both columns was measured: 62 registers instead of 48 and 195 us
-  // instead of 106 -- as with the template-parameter variant of round 1, fewer instructions but slower)
-  float lxv[3][2], lyv[2][3];
+      for (int b = 0; b < 2; b++) lxv[a][b] = L0.lx[IDX(ig + a, j0 + b)];
 #pragma unroll
-  for (int a = 0; a < 3; a++)
+    for (int a = 0; a < 2; a++)
 #pragma unroll
-    for (int b = 0; b < 2; b++) lxv[a][b] = L0.lx[IDX(i0 + a, j0 + b)];
-#pragma unroll
-  for (int a = 0; a < 2; a++)
-#pragma unroll
-    for (int b = 0; b < 3; b++) lyv[a][b] = L0.ly[IDX(i0 + a, j0 + b)];
-#pragma unroll
-  for (int a = 0; a < 2; a++)
-#pragma unroll
-    for (int b = 0; b < 2; b++) {
-      const int i = i0 + a, j = j0 + b, k = IDX(i, j);
-      const float dW = a ? dc : dWc, dE = a ? dEc : dc, dS = b ? dc : dSc, dN = b ? dNc : dc;
-      const float dg = -(lxv[a][b] + lxv[a + 1][b] + lyv[a][b] + lyv[a][b + 1]);
-      const float Ad = dc * dg + dW * lxv[a][b] + dE * lxv[a + 1][b] + dS * lyv[a][b] + dN * lyv[a][b + 1];
-      x[k] = xo[a][b] + dc;
-      const int ln = (j - 1) / C, c = (j - 1) - ln * C;
-      rsk[((size_t)(i + ln) * 32 + ln) * CP + c] = ro[a][b] - Ad;
-    }
-  // ghost cells bordering the block (only the blocks on the rim of the level)
-  if (I == 1 || I == nci || J == 1 || J == ncj) {
+      for (int b = 0; b < 3; b++) lyv[a][b] = L0.ly[IDX(ig + a, j0 + b)];
 #pragma unroll
     for (int a = 0; a < 2; a++)
 #pragma unroll
       for (int b = 0; b < 2; b++) {
-        const int i = i0 + a, j = j0 + b;
-        const int di = (i == 1) ? -1 : (i == n - 2 ? 1 : 0), dj = (j == 1) ? -1 : (j == m - 2 ? 1 : 0);
-        if (di) x[IDX(i + di, j)] += dc;
-        if (dj) x[IDX(i, j + dj)] += dc;
-        if (di && dj) x[IDX(i + di, j + dj)] += dc;
+        const int i = ig + a, j = j0 + b, ks = IDX(a0 + a, j);
+        const float dW = a ? dc : dWc, dE = a ? dEc : dc, dS = b ? dc : dSc, dN = b ? dNc : dc;
+        const float dg = -(lxv[a][b] + lxv[a + 1][b] + lyv[a][b] + lyv[a][b + 1]);
+        const float Ad = dc * dg + dW * lxv[a][b] + dE * lxv[a + 1][b] + dS * lyv[a][b] + dN * lyv[a][b + 1];
+        x[IDX(i, j)] = s_x[ks] + dc;
+        s_r[ks] = s_r[ks] - Ad;
       }
+    // ghost cells bordering the block (only the blocks on the rim of the level)
+    if (I == 1 || I == nci || J == 1 || J == ncj) {
+#pragma unroll
+      for (int a = 0; a < 2; a++)
+#pragma unroll
+        for (int b = 0; b < 2; b++) {
+          const int i = ig + a, j = j0 + b;
+          const int di = (i == 1) ? -1 : (i == n - 2 ? 1 : 0), dj = (j == 1) ? -1 : (j == m - 2 ? 1 : 0);
+          if (di) x[IDX(i + di, j)] += dc;
+          if (dj) x[IDX(i, j + dj)] += dc;
+          if (di && dj) x[IDX(i + di, j + dj)] += dc;
+        }
+    }
+  }
+  __syncthreads();
+  // skewed write-out: warp w takes the CTA's entries tau = i0 + t, t = w, w + 8, ...
+  float* __restrict__ rsk = q.rsk + (size_t)e * q.rsk_stride;
+  const int lane = threadIdx.x & 31, nw = blockDim.x >> 5;
+  for (int t = threadIdx.x >> 5; t < rows + 31; t += nw) {
+    const int lo = max(0, t - rows + 1) * CP, hi = (min(31, t) + 1) * CP;
+    float* __restrict__ ent = rsk + (size_t)(i0 + t) * 32 * CP;
+    for (int p = lo + lane; p < hi; p += 32) {
+      const int ln = p / CP, c = p - ln * CP, j = ln * C + c + 1;
+      if (c < C && j <= mj) ent[p] = s_r[IDX(t - ln, j)];
+    }
   }
 }
 
@@ -1468,8 +1545,8 @@ int launch_resid_down0(const SolverParams& q, const float* ux, const float* uy, 
   const DevLevel& L1 = q.lev[1];
   if (q.resid_march) {
     const int ni = q.n - 2, mj = q.m - 2;
-    dim3 grid((mj + kRmCols - 1) / kRmCols, ((ni + kRmRows - 1) / kRmRows + 3) / 4, q.B);
-    k_resid_down0_march<<<grid, 128, 0, st>>>(q, ux, uy, p_in, p_out, r_out, which);
+    dim3 grid((mj + kRmWarps * kRmCols - 1) / (kRmWarps * kRmCols), (ni + kRmRows - 1) / kRmRows, q.B);
+    k_resid_down0_march<<<grid, 32 * (kRmWarps + 1), kRmSmem, st>>>(q, ux, uy, p_in, p_out, r_out, which);
     return 1;
   }
   dim3 blk(kRdJ, kRdI);
@@ -1555,6 +1632,7 @@ int configure_kernels(const SolverParams& q) {
   }
   if (cudaFuncSetAttribute(k_xsum_chain_blocks<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kXsBlocksSmem) != cudaSuccess ||
       cudaFuncSetAttribute(k_xsum_chain_blocks<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kXsBlocksSmem) != cudaSuccess) return -1;
+  if (cudaFuncSetAttribute(k_resid_down0_march, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kRmSmem) != cudaSuccess) return -1;
   cudaError_t e3 = cudaFuncSetAttribute(k_mg_coarse_rows, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)coarse_rows_smem(q));
   if (q.chain_levels > 0 &&
       (cudaFuncSetAttribute(k_chain_sweeps, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(kChMaxWpb * sizeof(ChainRing))) != cudaSuccess ||
@@ -1638,7 +1716,7 @@ int launch_mg_coarse(const SolverParams& q, cudaStream_t st) {
 int launch_mg_up0(const SolverParams& q, float* r, cudaStream_t st) {
   dim3 blk(32, 8);
   if (q.lev[0].ch.on) return launch_chain_up(q, 0, r, st);
-  if (q.use_rows && !q.lev[0].wave) k_mg_up0_blk<<<grid2d(q.lev[1].m - 2, q.lev[1].n - 2, q.B, blk), blk, 0, st>>>(q, r);
+  if (q.use_rows && !q.lev[0].wave) k_mg_up0_blk<<<dim3((q.n - 2 + kUpRows - 1) / kUpRows, q.B), 256, up0_smem(q), st>>>(q, r);
   else k_mg_up0<false><<<grid2d(q.m, q.n, q.B, blk), blk, 0, st>>>(q, r);
   return 1;
 }
