@@ -14,7 +14,7 @@ PKG = Path(__file__).resolve().parent
 CSRC = PKG / "csrc"
 LIB = PKG / "librlfc.so"
 SOURCES = ["rlfc_api.cu", "solver_kernels.cu", "geometry.cpp", "vmm.cpp"]
-HEADERS = ["solver.h", "geometry.h", "vmm.h", "smooth_strip.cuh", "smooth_rows.cuh", "smooth_wave.cuh", "smooth_chain.cuh", "smooth_chain3.cuh", "smooth_tiny.cuh", "exact_sum.cuh",
+HEADERS = ["solver.h", "geometry.h", "vmm.h", "smooth_rows.cuh", "smooth_wave.cuh", "smooth_chain.cuh", "smooth_chain3.cuh", "smooth_tiny.cuh", "exact_sum.cuh",
            "exact_sum_kernels.cuh", "../../include/rlfc.h"]
 
 NVCC_FLAGS = [

@@ -213,12 +213,6 @@ k_xsum_tables(const __grid_constant__ SolverParams q) {
       }
     }
   }
-  // the chunk's records are complete: tell the serial pass, which may already be running (k_xsum_chain)
-  __syncthreads();
-  if (t == 0) {
-    __threadfence();
-    *(volatile unsigned*)(q.xs_rflag + (size_t)e * q.xs_nchunks + c) = q.xs_epoch[e] + 1u;
-  }
 }
 
 // Between the two table passes of a large domain: prefix sums of the batches' float increments = the refined prediction
@@ -266,7 +260,6 @@ __device__ __forceinline__ void xs_cp4(void* smem, const void* gmem) {
   asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"((unsigned)__cvta_generic_to_shared(smem)), "l"(gmem) : "memory");
 }
 
-template <bool WAIT>              // WAIT: k_xsum_tables may still be running (parallel graph branch): poll the chunk flags
 __global__ void __launch_bounds__(32)
 k_xsum_chain(const __grid_constant__ SolverParams q) {
   __shared__ __align__(16) uint32_t ring[2 * kXsGroup][kXsRecWords];
@@ -327,23 +320,7 @@ k_xsum_chain(const __grid_constant__ SolverParams q) {
 #pragma unroll 1
     for (int k = 0; k < 32; k++) redo(stage[k][lane]);
   };
-  // The records of chunk c are complete when xs_rflag[e][c] carries this pass's epoch.  k_xsum_tables may still be
-  // running (the two kernels are parallel branches of the step graph): wait chunk by chunk.  The wait is bounded --
-  // a flag that never comes is a bug, and a trap is better than a hung GPU.
   const int ngrp = (nb + kXsGroup - 1) / kXsGroup;
-  const unsigned ep = q.xs_epoch[e] + 1u;
-  const volatile unsigned* rf = q.xs_rflag + (size_t)e * q.xs_nchunks;
-  auto ready = [&](int grp) { return rf[grp] == ep; };
-  auto wait_chunk = [&](int grp) {
-    if (lane == 0) {
-      long long spins = 0;
-      while (!ready(grp)) {
-        if (++spins > (1ll << 26)) __trap();
-      }
-    }
-    __syncwarp();
-    __threadfence();
-  };
   float rawn[kXsRawPf];                                           // elements of the next batch's first serial segments
 #pragma unroll
   for (int i = 0; i < kXsRawPf; i++) rawn[i] = 0.f;
@@ -352,10 +329,9 @@ k_xsum_chain(const __grid_constant__ SolverParams q) {
     if (b % kXsGroup == 0) {                                      // chunk boundary
       const int grp = b / kXsGroup;
       __syncwarp();
-      if (!prefetched) { if (WAIT) wait_chunk(grp); fetch(grp); }
+      if (!prefetched) fetch(grp);
       prefetched = false;
-      if (grp + 1 < ngrp && (!WAIT || __shfl_sync(0xffffffffu, (int)ready(grp + 1), 0))) {   // next chunk there: in flight now
-        if (WAIT) __threadfence();
+      if (grp + 1 < ngrp) {                                       // next chunk's records: in flight now
         fetch(grp + 1);
         prefetched = true;
         asm volatile("cp.async.wait_group 1;" ::: "memory");

@@ -64,14 +64,14 @@ struct rlfc_env {
   // Environment groups: the batch is split into contiguous groups, each advanced by its own stream (and its own
   // CUDA graphs), so the latency-bound per-env kernels of one group overlap the bandwidth-bound kernels of another.
   struct Group {
-    int e0 = 0, B = 0, index = 0;
+    int e0 = 0, B = 0;
     SolverParams sp{};                       // view of the batch arrays restricted to [e0, e0 + B); lev[0].x = pressure buffer A
     SolverParams spB{};                      // same view with lev[0].x = pressure buffer B (p ping-pongs A -> B -> A per half step)
     float *uAx = nullptr, *uAy = nullptr, *uBx = nullptr, *uBy = nullptr, *uCx = nullptr, *uCy = nullptr;
     cudaStream_t st = nullptr;               // group 0 runs on the handle's stream
     cudaEvent_t done = nullptr;
     cudaGraphExec_t step_graph[2] = {nullptr, nullptr};   // [accumulate]
-    long long graph_launches[2] = {0, 0};    // kernel nodes of one replay outside / inside the MG loops
+    long long graph_launches = 0;            // kernel nodes of one replay outside the MG loops' WHILE bodies
   };
   std::vector<Group> groups;
   Group whole;                               // the entire batch on the handle's stream (eager / profiled path)
@@ -91,18 +91,10 @@ struct rlfc_env {
   long long slab_barriers = 0;
   cudaStream_t aux_stream = nullptr;         // used to capture the bodies of the conditional nodes
   cudaEvent_t fork_ev = nullptr;
-  cudaStream_t psum_stream = nullptr;        // side branch of the step graphs: Field.sum's serial pass (launch_psum_overlapped)
-  cudaEvent_t psum_fork = nullptr, psum_join = nullptr;
-  bool psum_overlap = false;                 // RLFC_PSUM_OVERLAP=1: serial pass as a parallel graph branch (measured slower)
   bool use_graph = true;
-  bool eager_groups = false;
-  bool fused = true;                         // RLFC_FUSED=0: unfused residual/down0 and project/shift kernels (A/B experiments)
-  int fixed_iters = 0;                       // experiment: > 0 = that many unconditional MG iterations per solve, no WHILE node
   // optional per-kernel CUDA-event timing (rlfc_env_set_profiling)
   bool profiling = false;
-  struct ProfRec { int id; cudaEvent_t e0, e1; int group; };
-  cudaEvent_t trace_base = nullptr;          // RLFC_TRACE=<csv path>: per-launch (group, kernel, start, end) timeline
-  std::string trace_path;
+  struct ProfRec { int id; cudaEvent_t e0, e1; };
   std::vector<ProfRec> prof_recs;
   std::vector<cudaEvent_t> event_pool;
   struct ProfAgg { std::string name; double ms = 0; long long count = 0; double floats_per_cell = 0; };
@@ -119,10 +111,10 @@ struct rlfc_env {
   }
   // run one kernel launch, optionally bracketed by events on the handle's stream
   template <typename F>
-  void run(const char* name, double floats_per_cell, F&& launch, cudaStream_t st = nullptr, int group = 0) {
+  void run(const char* name, double floats_per_cell, F&& launch, cudaStream_t st = nullptr) {
     if (!profiling) { launches += launch(); return; }
     if (!st) st = stream;
-    ProfRec r{prof_id(name, floats_per_cell), get_event(), get_event(), group};
+    ProfRec r{prof_id(name, floats_per_cell), get_event(), get_event()};
     cudaEventRecord(r.e0, st);
     launches += launch();
     cudaEventRecord(r.e1, st);
@@ -132,17 +124,6 @@ struct rlfc_env {
     if (prof_recs.empty()) return;
     cudaStreamSynchronize(stream);
     for (auto& G : groups) if (G.st) cudaStreamSynchronize(G.st);
-    if (!trace_path.empty() && trace_base) {
-      if (FILE* f = std::fopen(trace_path.c_str(), "a")) {
-        for (auto& r : prof_recs) {
-          float a = 0, b = 0;
-          cudaEventElapsedTime(&a, trace_base, r.e0);
-          cudaEventElapsedTime(&b, trace_base, r.e1);
-          std::fprintf(f, "%d,%s,%.4f,%.4f\n", r.group, prof[r.id].name.c_str(), a, b);
-        }
-        std::fclose(f);
-      }
-    }
     for (auto& r : prof_recs) {
       float ms = 0;
       cudaEventElapsedTime(&ms, r.e0, r.e1);
@@ -229,23 +210,20 @@ using Group = rlfc_env::Group;
 // (MG.pde:34) costs one 4-byte readback per iteration
 int project_eager(rlfc_env* E, Group& G, float* Ux, float* Uy, int which) {
   SolverParams& sp = G.sp;
-  SolverParams& sb = E->fused ? G.spB : G.sp;
+  SolverParams& sb = G.spB;
   cudaStream_t st = G.st;
-  const int gi = G.index;
   float* r = sp.lev[0].r;
   float* rs = sp.lev[0].d;
   float* pA = sp.lev[0].x;
   float* pB = sb.lev[0].x;
-  if (!E->fused) E->run("k_residual", 4, [&] { return launch_residual(sp, Ux, Uy, r, which, st); }, st, gi);
-  for (int it = 0; it < (E->fixed_iters > 0 ? E->fixed_iters : sp.mg_max_iters); it++) {
+  for (int it = 0; it < sp.mg_max_iters; it++) {
     CU(cudaMemsetAsync(sp.sc.any_active, 0, sizeof(int), st));
-    if (it == 0 && E->fused)
-      E->run("k_resid_down0", 5.25, [&] { return launch_resid_down0(sp, Ux, Uy, pA, pB, rs, which, st); }, st, gi);
+    if (it == 0)
+      E->run("k_resid_down0", 5.25, [&] { return launch_resid_down0(sp, Ux, Uy, pA, pB, rs, which, st); }, st);
     else {
-      // (the plain residual is fresh from k_residual in the first iteration of the unfused path; afterwards the row
-      // smoother has left it skewed)
-      if (it > 0) E->run("k_unskew_r", 2, [&] { return launch_unskew_r(sb, r, st); }, st, gi);
-      E->run("k_mg_down0", 4.25, [&] { return launch_mg_down0(sb, r, rs, st); }, st, gi);
+      // (the row smoother has left the residual skewed)
+      E->run("k_unskew_r", 2, [&] { return launch_unskew_r(sb, r, st); }, st);
+      E->run("k_mg_down0", 4.25, [&] { return launch_mg_down0(sb, r, rs, st); }, st);
     }
     if (sp.chain_levels > 0 && E->profiling) {   // per-kernel timing of the chained levels
       const int first = std::max(1, sp.chain_levels);
@@ -253,46 +231,40 @@ int project_eager(rlfc_env* E, Group& G, float* Ux, float* Uy, int which) {
                                      {"k_chain_down_L2", "k_chain_up_L2", "k_chain_sweeps_L2", "k_chain_incr_L2"},
                                      {"k_chain_down_L3", "k_chain_up_L3", "k_chain_sweeps_L3", "k_chain_incr_L3"},
                                      {"k_chain_down_L4+", "k_chain_up_L4+", "k_chain_sweeps_L4+", "k_chain_incr_L4+"}};
-      for (int l = 1; l < first; l++) E->run(nm[std::min(l, 4) - 1][0], 0, [&] { return launch_chain_down(sb, l, st); }, st, gi);
-      E->run("k_mg_coarse_cta", 0.5, [&] { return launch_coarse_cta(sb, st); }, st, gi);
+      for (int l = 1; l < first; l++) E->run(nm[std::min(l, 4) - 1][0], 0, [&] { return launch_chain_down(sb, l, st); }, st);
+      E->run("k_mg_coarse_cta", 0.5, [&] { return launch_coarse_cta(sb, st); }, st);
       for (int l = first - 1; l >= 1; l--) {
-        E->run(nm[std::min(l, 4) - 1][1], 0, [&] { return launch_chain_up(sb, l, nullptr, st); }, st, gi);
-        E->run(nm[std::min(l, 4) - 1][2], 0, [&] { return launch_chain_sweeps(sb, l, st); }, st, gi);
-        E->run(nm[std::min(l, 4) - 1][3], 0, [&] { return launch_chain_incr(sb, l, nullptr, 0, st); }, st, gi);
+        E->run(nm[std::min(l, 4) - 1][1], 0, [&] { return launch_chain_up(sb, l, nullptr, st); }, st);
+        E->run(nm[std::min(l, 4) - 1][2], 0, [&] { return launch_chain_sweeps(sb, l, st); }, st);
+        E->run(nm[std::min(l, 4) - 1][3], 0, [&] { return launch_chain_incr(sb, l, nullptr, 0, st); }, st);
       }
-      E->run("k_chain_up_L0", 4.25, [&] { return launch_chain_up(sb, 0, rs, st); }, st, gi);
-      E->run("k_chain_sweeps_L0", 3, [&] { return launch_chain_sweeps(sb, 0, st); }, st, gi);
-      E->run("k_chain_incr_L0", 4, [&] { return launch_chain_incr(sb, 0, r, which, st); }, st, gi);
+      E->run("k_chain_up_L0", 4.25, [&] { return launch_chain_up(sb, 0, rs, st); }, st);
+      E->run("k_chain_sweeps_L0", 3, [&] { return launch_chain_sweeps(sb, 0, st); }, st);
+      E->run("k_chain_incr_L0", 4, [&] { return launch_chain_incr(sb, 0, r, which, st); }, st);
     } else {
-    E->run("k_mg_coarse", 0.5, [&] { return launch_mg_coarse(sb, st); }, st, gi);
-    E->run("k_mg_up0", 4.25, [&] { return launch_mg_up0(sb, rs, st); }, st, gi);
-    E->run("k_smooth0", 4, [&] { return launch_smooth0(sb, rs, r, which, st); }, st, gi);
+    E->run("k_mg_coarse", 0.5, [&] { return launch_mg_coarse(sb, st); }, st);
+    E->run("k_mg_up0", 4.25, [&] { return launch_mg_up0(sb, rs, st); }, st);
+    E->run("k_smooth0", 4, [&] { return launch_smooth0(sb, rs, r, which, st); }, st);
     }
     E->mg_iter_launch_rounds++;
-    if (E->fixed_iters > 0) continue;
     CU(cudaMemcpyAsync(E->h_any, sp.sc.any_active, sizeof(int), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     if (!*E->h_any) break;
   }
   if (E->profiling && sb.xs_recs) {
-    E->run("k_xsum_tables", 1, [&] { return launch_psum_tables(sb, st); }, st, gi);
-    E->run("k_xsum_pass", 0, [&] { return launch_psum_pass(sb, st); }, st, gi);
+    E->run("k_xsum_tables", 1, [&] { return launch_psum_tables(sb, st); }, st);
+    E->run("k_xsum_pass", 0, [&] { return launch_psum_pass(sb, st); }, st);
   } else {
-    E->run("k_psum", 1, [&] { return launch_psum(sb, st); }, st, gi);
+    E->run("k_psum", 1, [&] { return launch_psum(sb, st); }, st);
   }
-  if (E->fused && which == 1 && sp.fast_bc) {
+  if (which == 1 && sp.fast_bc) {
     // corrector: Heun average fused into the projection and the boundary-condition kernels (BDIM.pde:95-96)
-    E->run("k_project_shift_heun", 8, [&] { return launch_project_shift_heun(sp, pB, pA, Ux, Uy, G.uBx, G.uBy, G.uAx, G.uAy, st); }, st, gi);
-    E->run("k_bc_heun", 0, [&] { return launch_bc_heun(sp, Ux, Uy, G.uBx, G.uBy, G.uAx, G.uAy, st); }, st, gi);
+    E->run("k_project_shift_heun", 8, [&] { return launch_project_shift_heun(sp, pB, pA, Ux, Uy, G.uBx, G.uBy, G.uAx, G.uAy, st); }, st);
+    E->run("k_bc_heun", 0, [&] { return launch_bc_heun(sp, Ux, Uy, G.uBx, G.uBy, G.uAx, G.uAy, st); }, st);
     return RLFC_OK;
   }
-  if (E->fused) {
-    E->run("k_project_shift", 6, [&] { return launch_project_shift(sp, pB, pA, Ux, Uy, st); }, st, gi);
-  } else {
-    E->run("k_project_u", 5, [&] { return launch_project_u(sp, Ux, Uy, st); }, st, gi);
-    E->run("k_shift_p", 2, [&] { return launch_shift_p(sp, st); }, st, gi);
-  }
-  E->run("k_bc", 0, [&] { return launch_bc(sp, Ux, Uy, st); }, st, gi);
+  E->run("k_project_shift", 6, [&] { return launch_project_shift(sp, pB, pA, Ux, Uy, st); }, st);
+  E->run("k_bc", 0, [&] { return launch_bc(sp, Ux, Uy, st); }, st);
   return RLFC_OK;
 }
 
@@ -300,19 +272,18 @@ int project_eager(rlfc_env* E, Group& G, float* Ux, float* Uy, int which) {
 int solver_step_eager(rlfc_env* E, Group& G, int accumulate) {
   SolverParams& sp = G.sp;
   cudaStream_t st = G.st;
-  const int gi = G.index;
   int rc;
   // predictor BDIM.update(): u0 = u (buffer A), F = AdvDif(u) -> B, updateUP
-  E->run("k_advdif", 5, [&] { return launch_advdif(sp, G.uAx, G.uAy, G.uAx, G.uAy, G.uBx, G.uBy, st); }, st, gi);
-  E->run("k_band_bc", 0, [&] { return launch_band_bc(sp, G.uBx, G.uBy, st); }, st, gi);
+  E->run("k_advdif", 5, [&] { return launch_advdif(sp, G.uAx, G.uAy, G.uAx, G.uAy, G.uBx, G.uBy, st); }, st);
+  E->run("k_band_bc", 0, [&] { return launch_band_bc(sp, G.uBx, G.uBy, st); }, st);
   if ((rc = project_eager(E, G, G.uBx, G.uBy, 0))) return rc;
   // corrector BDIM.update2(): us = u (B), F = AdvDif(u; + u0) -> C, updateUP, u = (u + us)/2 -> A
-  E->run("k_advdif", 5, [&] { return launch_advdif(sp, G.uBx, G.uBy, G.uAx, G.uAy, G.uCx, G.uCy, st); }, st, gi);
-  E->run("k_band_bc", 0, [&] { return launch_band_bc(sp, G.uCx, G.uCy, st); }, st, gi);
+  E->run("k_advdif", 5, [&] { return launch_advdif(sp, G.uBx, G.uBy, G.uAx, G.uAy, G.uCx, G.uCy, st); }, st);
+  E->run("k_band_bc", 0, [&] { return launch_band_bc(sp, G.uCx, G.uCy, st); }, st);
   if ((rc = project_eager(E, G, G.uCx, G.uCy, 1))) return rc;
-  if (!(E->fused && sp.fast_bc))
-    E->run("k_heun", 6, [&] { return launch_heun(sp, G.uCx, G.uCy, G.uBx, G.uBy, G.uAx, G.uAy, st); }, st, gi);
-  E->run("k_force", 0, [&] { return launch_force(sp, accumulate, st); }, st, gi);
+  if (!sp.fast_bc)
+    E->run("k_heun", 6, [&] { return launch_heun(sp, G.uCx, G.uCy, G.uBx, G.uBy, G.uAx, G.uAy, st); }, st);
+  E->run("k_force", 0, [&] { return launch_force(sp, accumulate, st); }, st);
   CU(cudaGetLastError());
   return RLFC_OK;
 }
@@ -320,7 +291,7 @@ int solver_step_eager(rlfc_env* E, Group& G, int accumulate) {
 // graph path: one CUDA graph per group = one solver step; each MGsolver loop is a WHILE conditional node whose
 // body is one iteration and whose condition is written on the device (k_loopcond), so no host round trip remains
 int capture_half_step(rlfc_env* E, Group& G, cudaStream_t st, const float* sx, const float* sy, const float* u0x,
-                      const float* u0y, float* dx, float* dy, int which, long long* n_outer, long long* n_body) {
+                      const float* u0y, float* dx, float* dy, int which, long long* n_outer) {
   SolverParams& sp = G.sp;
   SolverParams& sb = G.spB;
   float* r = sp.lev[0].r;
@@ -334,46 +305,36 @@ int capture_half_step(rlfc_env* E, Group& G, cudaStream_t st, const float* sx, c
   *n_outer += launch_mg_coarse(sb, st);
   *n_outer += launch_mg_up0(sb, rs, st);
   *n_outer += launch_smooth0(sb, rs, r, which, st);
-  if (E->fixed_iters <= 0) {
-    // ---- WHILE node: further iterations while any environment is still unconverged (rare) ----
-    cudaStreamCaptureStatus status;
-    cudaGraph_t graph;
-    const cudaGraphNode_t* deps;
-    size_t ndeps;
-    CU(cudaStreamGetCaptureInfo(st, &status, nullptr, &graph, &deps, &ndeps));
-    cudaGraphConditionalHandle handle;
-    CU(cudaGraphConditionalHandleCreate(&handle, graph, 0, cudaGraphCondAssignDefault));
-    // the condition is written by a kernel ahead of the node and again at the end of every body pass
-    *n_outer += launch_loopcond(sb, (unsigned long long)handle, st);
-    CU(cudaStreamGetCaptureInfo(st, &status, nullptr, &graph, &deps, &ndeps));
-    cudaGraphNodeParams np{};
-    np.type = cudaGraphNodeTypeConditional;
-    np.conditional.handle = handle;
-    np.conditional.type = cudaGraphCondTypeWhile;
-    np.conditional.size = 1;
-    cudaGraphNode_t cond;
-    CU(cudaGraphAddNode(&cond, graph, deps, ndeps, &np));
-    cudaGraph_t body = np.conditional.phGraph_out[0];
-    CU(cudaStreamBeginCaptureToGraph(E->aux_stream, body, nullptr, nullptr, 0, cudaStreamCaptureModeThreadLocal));
-    launch_unskew_r(sb, r, E->aux_stream);
-    launch_mg_down0(sb, r, rs, E->aux_stream);
-    launch_mg_coarse(sb, E->aux_stream);
-    launch_mg_up0(sb, rs, E->aux_stream);
-    launch_smooth0(sb, rs, r, which, E->aux_stream);
-    launch_loopcond(sb, (unsigned long long)handle, E->aux_stream);
-    CU(cudaStreamEndCapture(E->aux_stream, nullptr));
-    CU(cudaStreamUpdateCaptureDependencies(st, &cond, 1, cudaStreamSetCaptureDependencies));
-  } else {
-    for (int it = 1; it < E->fixed_iters; it++) {
-      *n_body += launch_unskew_r(sb, r, st);
-      *n_body += launch_mg_down0(sb, r, rs, st);
-      *n_body += launch_mg_coarse(sb, st);
-      *n_body += launch_mg_up0(sb, rs, st);
-      *n_body += launch_smooth0(sb, rs, r, which, st);
-    }
-  }
+  // ---- WHILE node: further iterations while any environment is still unconverged (rare) ----
+  cudaStreamCaptureStatus status;
+  cudaGraph_t graph;
+  const cudaGraphNode_t* deps;
+  size_t ndeps;
+  CU(cudaStreamGetCaptureInfo(st, &status, nullptr, &graph, &deps, &ndeps));
+  cudaGraphConditionalHandle handle;
+  CU(cudaGraphConditionalHandleCreate(&handle, graph, 0, cudaGraphCondAssignDefault));
+  // the condition is written by a kernel ahead of the node and again at the end of every body pass
+  *n_outer += launch_loopcond(sb, (unsigned long long)handle, st);
+  CU(cudaStreamGetCaptureInfo(st, &status, nullptr, &graph, &deps, &ndeps));
+  cudaGraphNodeParams np{};
+  np.type = cudaGraphNodeTypeConditional;
+  np.conditional.handle = handle;
+  np.conditional.type = cudaGraphCondTypeWhile;
+  np.conditional.size = 1;
+  cudaGraphNode_t cond;
+  CU(cudaGraphAddNode(&cond, graph, deps, ndeps, &np));
+  cudaGraph_t body = np.conditional.phGraph_out[0];
+  CU(cudaStreamBeginCaptureToGraph(E->aux_stream, body, nullptr, nullptr, 0, cudaStreamCaptureModeThreadLocal));
+  launch_unskew_r(sb, r, E->aux_stream);
+  launch_mg_down0(sb, r, rs, E->aux_stream);
+  launch_mg_coarse(sb, E->aux_stream);
+  launch_mg_up0(sb, rs, E->aux_stream);
+  launch_smooth0(sb, rs, r, which, E->aux_stream);
+  launch_loopcond(sb, (unsigned long long)handle, E->aux_stream);
+  CU(cudaStreamEndCapture(E->aux_stream, nullptr));
+  CU(cudaStreamUpdateCaptureDependencies(st, &cond, 1, cudaStreamSetCaptureDependencies));
   // ---- projection tail ----
-  *n_outer += E->psum_overlap ? launch_psum_overlapped(sb, st, E->psum_stream, E->psum_fork, E->psum_join) : launch_psum(sb, st);
+  *n_outer += launch_psum(sb, st);
   if (which == 1 && sp.fast_bc) {   // corrector: Heun average fused in (BDIM.pde:95-96); sx, sy = us, u0x, u0y = step-start buffer
     *n_outer += launch_project_shift_heun(sp, pB, pA, dx, dy, sx, sy, const_cast<float*>(u0x), const_cast<float*>(u0y), st);
     *n_outer += launch_bc_heun(sp, dx, dy, sx, sy, const_cast<float*>(u0x), const_cast<float*>(u0y), st);
@@ -386,10 +347,10 @@ int capture_half_step(rlfc_env* E, Group& G, cudaStream_t st, const float* sx, c
 
 int build_step_graph(rlfc_env* E, Group& G, int accumulate) {
   cudaStream_t st = G.st;
-  long long n_outer = 0, n_body = 0;
+  long long n_outer = 0;
   CU(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
-  int rc = capture_half_step(E, G, st, G.uAx, G.uAy, G.uAx, G.uAy, G.uBx, G.uBy, 0, &n_outer, &n_body);
-  if (!rc) rc = capture_half_step(E, G, st, G.uBx, G.uBy, G.uAx, G.uAy, G.uCx, G.uCy, 1, &n_outer, &n_body);
+  int rc = capture_half_step(E, G, st, G.uAx, G.uAy, G.uAx, G.uAy, G.uBx, G.uBy, 0, &n_outer);
+  if (!rc) rc = capture_half_step(E, G, st, G.uBx, G.uBy, G.uAx, G.uAy, G.uCx, G.uCy, 1, &n_outer);
   if (!rc) {
     if (!G.sp.fast_bc) n_outer += launch_heun(G.sp, G.uCx, G.uCy, G.uBx, G.uBy, G.uAx, G.uAy, st);
     n_outer += launch_force(G.sp, accumulate, st);
@@ -401,8 +362,7 @@ int build_step_graph(rlfc_env* E, Group& G, int accumulate) {
   ce = cudaGraphInstantiate(&G.step_graph[accumulate], graph, 0);
   cudaGraphDestroy(graph);
   if (ce != cudaSuccess) return fail(RLFC_ECUDA, std::string("cudaGraphInstantiate: ") + cudaGetErrorString(ce));
-  G.graph_launches[0] = n_outer;
-  G.graph_launches[1] = n_body;   // per MG iteration pair (predictor + corrector) with one iteration each
+  G.graph_launches = n_outer;
   return RLFC_OK;
 }
 
@@ -434,7 +394,7 @@ void slab_all(rlfc_env* E, const char* name, double fpc, F&& launch) {
   for (size_t d = 0; d < E->slab.size(); d++) {
     SlabDev& D = E->slab[d];
     cudaSetDevice(D.device);
-    if (d == 0) E->run(name, fpc, [&] { return launch(D); }, D.st, 0);
+    if (d == 0) E->run(name, fpc, [&] { return launch(D); }, D.st);
     else E->launches += launch(D);
   }
 }
@@ -442,7 +402,7 @@ template <typename F>
 void slab_first(rlfc_env* E, const char* name, double fpc, F&& launch) {
   SlabDev& D = E->slab[0];
   cudaSetDevice(D.device);
-  E->run(name, fpc, [&] { return launch(D); }, D.st, 0);
+  E->run(name, fpc, [&] { return launch(D); }, D.st);
 }
 void slab_barrier(rlfc_env* E) {
   slab_all(E, "k_slab_barrier", 0, [&](SlabDev& D) { return launch_slab_barrier(D.bar, D.st); });
@@ -543,26 +503,17 @@ int solver_steps(rlfc_env* E, int nsteps, int accumulate) {
       if ((rc = slab_step(E, accumulate))) return rc;
     return RLFC_OK;
   }
-  const bool graph = E->use_graph && !E->profiling;
-  if (!graph && !(E->fixed_iters > 0 && E->eager_groups)) {
+  if (!E->use_graph || E->profiling) {
     for (int s = 0; s < nsteps; s++)
       if ((rc = solver_step_eager(E, E->whole, accumulate))) return rc;
     return RLFC_OK;
   }
-  if (!graph) {   // experiment: eager launches on the group streams, fixed MG iteration count (no host sync)
-    if (E->profiling && !E->trace_base) { cudaEventCreate(&E->trace_base); cudaEventRecord(E->trace_base, E->stream); }
-    if ((rc = fork_groups(E))) return rc;
-    for (int s = 0; s < nsteps; s++)
-      for (auto& G : E->groups)
-        if ((rc = solver_step_eager(E, G, accumulate))) return rc;
-    return join_groups(E);
-  }
   if ((rc = fork_groups(E))) return rc;
   for (auto& G : E->groups) {
-    if (graph && !G.step_graph[accumulate] && (rc = build_step_graph(E, G, accumulate))) return rc;
+    if (!G.step_graph[accumulate] && (rc = build_step_graph(E, G, accumulate))) return rc;
     for (int s = 0; s < nsteps; s++) {
       CU(cudaGraphLaunch(G.step_graph[accumulate], G.st));
-      E->launches += G.graph_launches[0] + G.graph_launches[1];   // lower bound: one MG iteration per solve
+      E->launches += G.graph_launches;   // lower bound: one MG iteration per solve
     }
   }
   if ((rc = join_groups(E))) return rc;
@@ -634,9 +585,6 @@ void rlfc_env_destroy(rlfc_env* E) {
   }
   cudaSetDevice(E->device);
   if (E->aux_stream) cudaStreamDestroy(E->aux_stream);
-  if (E->psum_stream) cudaStreamDestroy(E->psum_stream);
-  if (E->psum_fork) cudaEventDestroy(E->psum_fork);
-  if (E->psum_join) cudaEventDestroy(E->psum_join);
   if (E->fork_ev) cudaEventDestroy(E->fork_ev);
   for (void* p : E->allocs) cudaFree(p);
   for (void* p : {(void*)E->h_actions, (void*)E->h_obs, (void*)E->h_reward, (void*)E->h_force, (void*)E->h_probes,
@@ -712,8 +660,6 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
   sp.action_scale = cfg->action_scale;
   sp.inv_cells = (float)((g.n - 2) * (g.m - 2));
   sp.mg_tol = g.mg_tol;
-  sp.use_rows = 1;
-  if (const char* ev = std::getenv("RLFC_SMOOTHER")) sp.use_rows = std::string(ev) != "strip";
   const bool force_wave = std::getenv("RLFC_SMOOTHER") && std::string(std::getenv("RLFC_SMOOTHER")) == "wave";
   // RLFC_SMOOTHER=chain: the chained strip smoother (smooth_chain.cuh) on every level but the coarsest (tests); by default it
   // takes the levels that are too wide for the row pipeline
@@ -722,12 +668,6 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
   int chain_min_cols = 33;            // RLFC_CHAIN_MIN_COLS: coarse levels at least this wide follow a chained level 0 (levels of
                                       // at most 32 columns are faster in the one-CTA kernel's single-warp smoother: 521 -> 528 steps/s)
   if (const char* ev = std::getenv("RLFC_CHAIN_MIN_COLS")) chain_min_cols = std::max(1, std::atoi(ev));
-  int chain_wpb = 1;
-  if (const char* ev = std::getenv("RLFC_CHAIN_WPB")) chain_wpb = std::min(3, std::max(1, std::atoi(ev)));
-  sp.chain_v = 3;                      // RLFC_CHAIN_V=1: the first generation of the sweep kernel (A/B, cross-check tests)
-  if (const char* ev = std::getenv("RLFC_CHAIN_V")) sp.chain_v = std::atoi(ev) == 1 ? 1 : 3;
-  if (slab) sp.chain_v = 3;
-  if (sp.chain_v == 3) chain_wpb = 1;  // (one compute warp + one loader warp per CTA)
   sp.nlevels = (int)g.levels.size();
   sp.resolution = cfg->resolution; sp.substeps = cfg->substeps; sp.mg_max_iters = cfg->mg_max_iters;
   sp.init_time = cfg->init_time; sp.episode_time = cfg->episode_time;
@@ -756,28 +696,6 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
     TRY(upload_static(E, H.ly, H.n, H.m, L.P, &L.ly));
     TRY(upload_static(E, H.inv, H.n, H.m, L.P, &L.inv));
     TRY(upload_static(E, H.diag, H.n, H.m, L.P, &L.diag));
-    {  // pre-skewed coefficient tables for the strip smoother (layout: solver.h SkewLevel)
-      const int ni = H.n - 2, mj = H.m - 2;
-      const int ns = (mj + 31) / 32, Tsk = 16 /*kSkewPad*/ + ni + 64 /*kSkewTail*/;
-      if (ns > 8 && !sp.use_rows) return bail(fail(RLFC_EGRID, "grids wider than 256 cells are not supported by the strip smoother"));
-      if (ns <= 8) {
-      std::vector<float4> A((size_t)ns * Tsk * 32, make_float4(0.f, 0.f, 0.f, 0.f));
-      std::vector<float2> nd((size_t)ns * Tsk * 32, make_float2(0.f, 0.f));
-      for (int k = 0; k < ns; k++)
-        for (int tp = 0; tp < Tsk; tp++)
-          for (int l = 0; l < 32; l++) {
-            const int tau = tp - 16, i = tau - l + 1, j = 32 * k + l + 1;
-            if (i < 1 || i > ni || j > mj) continue;
-            const size_t c = (size_t)i * H.m + j, o = ((size_t)k * Tsk + tp) * 32 + l;
-            A[o] = make_float4(H.lx[c], H.lx[c + H.m], H.ly[c], H.ly[c + 1]);
-            nd[o] = make_float2(-H.inv[c], H.diag[c]);
-          }
-      L.sk.nstrips = ns; L.sk.Tsk = Tsk;
-      TRY(upload_vec(E, A, &L.sk.A));
-      TRY(upload_vec(E, nd, &L.sk.nd));
-      if (l >= 1) sp.coarse_strips = std::max(sp.coarse_strips, ns);
-      }
-    }
     {  // pre-skewed coefficient table for the row-pipelined smoother (layout: solver.h RowTab)
       const int ni = H.n - 2, mj = H.m - 2;
       const int C = (mj + 31) / 32, K = (3 * C + 1 + 3) / 4, nl = (mj + C - 1) / C;
@@ -788,16 +706,13 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
       L.ch = ChainLevel{};
       // levels the row pipeline could take, but which are faster chained when one domain has the GPU to itself
       const bool prefer_chain = sp.chain_levels > 0 && l >= 1 && mj >= chain_min_cols;
-      if (sp.use_rows && !force_wave && l < sp.nlevels - 1 && (force_chain || L.wave || prefer_chain || (slab && l == 0)) && sp.chain_levels == l) {
+      if (!force_wave && l < sp.nlevels - 1 && (force_chain || L.wave || prefer_chain || (slab && l == 0)) && sp.chain_levels == l) {
         // chained strip smoother: static coefficient table in the strip-skewed layout (solver.h ChainLevel)
         ChainLevel& ch = L.ch;
         ch.on = 1; ch.NS = (mj + 31) / 32; ch.T = round_up(ni + 33, 32) + 32;   // (>= ni + 34; whole batches of up to 32 steps stay inside a strip)
         ch.s0 = 0; ch.ns_loc = ch.NS;
-        ch.wpb = std::min(chain_wpb, ch.NS); ch.nb = (ch.NS + ch.wpb - 1) / ch.wpb;
         ch.sk_stride = (size_t)ch.NS * ch.T * 32;
-        // (the sweeps form addresses up to kChPFS entries past a strip's end for copies of zero bytes: pad the arrays)
-        const size_t pad = (size_t)128 * 32;
-        std::vector<float4> ct(ch.sk_stride + pad, make_float4(0.f, 0.f, 0.f, 0.f));
+        std::vector<float4> ct(ch.sk_stride, make_float4(0.f, 0.f, 0.f, 0.f));
         for (int s = 0; s < ch.NS; s++)
           for (int t = 0; t < ch.T; t++)
             for (int ln = 0; ln < 32; ln++) {
@@ -813,8 +728,8 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
               ct[((size_t)s * ch.T + t) * 32 + ln] = v;
             }
         TRY(upload_vec(E, ct, &ch.ct));
-        TRY(E->dmalloc(&ch.rsk, ch.sk_stride * B + pad));
-        for (int gsw = 0; gsw < 5; gsw++) TRY(E->dmalloc(&ch.dsk[gsw], ch.sk_stride * B + pad));
+        TRY(E->dmalloc(&ch.rsk, ch.sk_stride * B));
+        for (int gsw = 0; gsw < 5; gsw++) TRY(E->dmalloc(&ch.dsk[gsw], ch.sk_stride * B));
         ch.TE = ch.T + 72;               // smooth_chain3.cuh: consumer steps 0 .. T-1 behind kC2EdgePad, producer indices up to T + 62
         ch.edge_arr = (size_t)B * ch.NS * ch.TE;
         TRY(E->dmalloc(&ch.edge, ch.edge_arr * 10 + 64));
@@ -931,10 +846,6 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
   n_groups = std::min(n_groups, B);
   if (slab) n_groups = 1;
   if (const char* ev = std::getenv("RLFC_NO_GRAPH")) E->use_graph = std::atoi(ev) == 0;
-  if (const char* ev = std::getenv("RLFC_FIXED_ITERS")) E->fixed_iters = std::atoi(ev);
-  if (const char* ev = std::getenv("RLFC_EAGER_GROUPS")) E->eager_groups = std::atoi(ev) != 0;
-  if (const char* ev = std::getenv("RLFC_TRACE")) E->trace_path = ev;
-  if (const char* ev = std::getenv("RLFC_FUSED")) E->fused = std::atoi(ev) != 0;
   TRY(E->dmalloc(&sp.sc.flow_t, B));
   TRY(E->dmalloc(&sp.sc.xi, 2 * B)); TRY(E->dmalloc(&sp.sc.t, B)); TRY(E->dmalloc(&sp.sc.force, 2 * B));
   TRY(E->dmalloc(&sp.sc.probes, (size_t)B * RLFC_NUM_PROBES));
@@ -971,7 +882,6 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
     if (summaries) {
       TRY(E->dmalloc(&sp.xs_ctot, (size_t)sp.xs_nchunks * B));
       TRY(E->dmalloc(&sp.xs_cflag, (size_t)sp.xs_nchunks * B));
-      TRY(E->dmalloc(&sp.xs_rflag, (size_t)sp.xs_nchunks * B));
       TRY(E->dmalloc(&sp.xs_epoch, (size_t)B));
       TRY(E->dmalloc(&sp.xs_recs, (size_t)sp.xs_nbatches * 192 * B));
       sp.xs_blk = nullptr;
@@ -1016,7 +926,7 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
   for (int g = 0; g < n_groups; g++) {
     rlfc_env::Group& G = E->groups[g];
     const int e0 = (int)((long long)B * g / n_groups), e1 = (int)((long long)B * (g + 1) / n_groups);
-    G.e0 = e0; G.B = e1 - e0; G.index = g;
+    G.e0 = e0; G.B = e1 - e0;
     G.sp = sp;
     SolverParams& v = G.sp;
     v.B = G.B;
@@ -1043,7 +953,7 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
     v.sc.psum += e0; v.sc.any_active += g;
     if (v.xs_recs) {
       v.xs_ctot += (size_t)e0 * v.xs_nchunks;
-      v.xs_cflag += (size_t)e0 * v.xs_nchunks; v.xs_rflag += (size_t)e0 * v.xs_nchunks; v.xs_epoch += e0;
+      v.xs_cflag += (size_t)e0 * v.xs_nchunks; v.xs_epoch += e0;
       v.xs_recs += (size_t)e0 * v.xs_nbatches * 192;
       if (v.xs_blk) {
         v.xs_blk += (size_t)e0 * ((v.xs_nbatches + 31) / 32) * 256;
@@ -1072,7 +982,7 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
     for (int gv = 0; gv <= n_groups; gv++)
       for (int l = 0; l < sp.chain_levels; l++) {
         const int Bv = gv < n_groups ? E->groups[gv].B : B;
-        init[(size_t)gv * kMaxLevels + l] = (unsigned long long)Bv * 4ull * (unsigned)sp.lev[l].ch.nb;
+        init[(size_t)gv * kMaxLevels + l] = (unsigned long long)Bv * 4ull * (unsigned)sp.lev[l].ch.ns_loc;
       }
     if (cudaMemcpyAsync(E->chain_tickets, init.data(), init.size() * sizeof(unsigned long long), cudaMemcpyHostToDevice, E->stream) != cudaSuccess ||
         cudaStreamSynchronize(E->stream) != cudaSuccess)
@@ -1112,7 +1022,6 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
         ChainLevel& ch = D.sp.lev[l].ch;
         ch.s0 = (int)((long long)ch.NS * d / nd);
         ch.ns_loc = (int)((long long)ch.NS * (d + 1) / nd) - ch.s0;
-        ch.wpb = 1; ch.nb = ch.ns_loc;
         ch.ticket = tickets + l;
         ch.tag_hi = 1u << 26;                                  // the same launch tags on every device
         init[l] = (unsigned long long)B * 4ull * (unsigned)std::max(ch.ns_loc, 1);
@@ -1126,11 +1035,7 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
     }
     cudaSetDevice(E->device);
   }
-  if (const char* ev = std::getenv("RLFC_PSUM_OVERLAP")) E->psum_overlap = std::atoi(ev) != 0;
   if (cudaStreamCreateWithFlags(&E->aux_stream, cudaStreamNonBlocking) != cudaSuccess ||
-      cudaStreamCreateWithFlags(&E->psum_stream, cudaStreamNonBlocking) != cudaSuccess ||
-      cudaEventCreateWithFlags(&E->psum_fork, cudaEventDisableTiming) != cudaSuccess ||
-      cudaEventCreateWithFlags(&E->psum_join, cudaEventDisableTiming) != cudaSuccess ||
       cudaEventCreateWithFlags(&E->fork_ev, cudaEventDisableTiming) != cudaSuccess)
     return bail(fail(RLFC_ECUDA, "stream/event creation failed"));
 

@@ -14,10 +14,8 @@
 //     lane 0's S is lane 31 of the previous strip's entry t+31 of the SAME sweep;
 //   * there is no barrier and no flag: every element a sweep writes is an 8-byte {value, launch tag} pair (one
 //     store), and a consumer that finds an older tag simply reloads until the tag of THIS launch appears (the LL
-//     protocol of NCCL).  Operands are prefetched kChPF steps ahead with cp.async.cg (L2, no stale L1 lines) into a
-//     per-warp shared-memory ring, so a producer that is far enough ahead is never waited for; strips settle about
-//     31 + kChPF + (L2 round trip) steps behind their left neighbour and sweeps about kChPF + (L2 round trip) steps
-//     behind the previous sweep;
+//     protocol of NCCL).  How the sweep kernel (smooth_chain3.cuh) fetches and validates its operands is described
+//     there;
 //   * CTAs take their role (environment, sweep, column block) from a ticket counter, so roles start in dependency
 //     order whatever the block scheduler does: a CTA only ever waits for CTAs that have already started;
 //   * out-of-domain cells have zero coefficients (host table), so they evaluate to +-0 by themselves; ghosts of d
@@ -27,51 +25,8 @@
 //     d = -(dW*lxW + dE*lxE + dS*lyS + dN*lyN - r) * inv      (the minus sign folded into ninv = -inv: exact)
 #pragma once
 
-#ifndef RLFC_CHPF
-#define RLFC_CHPF 12
-#endif
-#ifndef RLFC_CHPFS
-#define RLFC_CHPFS 48
-#endif
-constexpr int kChPF = RLFC_CHPF;     // steps of prefetch of the DYNAMIC operands (previous sweep, neighbour strips: L2 hits)
-constexpr int kChPFS = RLFC_CHPFS;   // steps of prefetch of the STATIC operands (coefficients, r: they stream from HBM --
-                                     // the arrays of one wide level fill the L2 -- and depend on no producer)
-constexpr int kChRing = 64;          // ring slots per warp (power of two > kChPFS)
-constexpr int kChMaxWpb = 3;         // strips (warps) per CTA at most
 constexpr unsigned kChSpinMax = 1u << 24;   // bounded reload spin: a tag that never comes is a bug, and a trap beats a hung GPU
 
-struct __align__(16) ChainRing {     // one warp's operand ring
-  float4 coef[kChRing][32];          // {lx[i+1][j], ly[i][j], ly[i][j+1], -inv[i][j]}
-  float r[kChRing][32];
-  uint2 e[kChRing][32];              // previous sweep, entry t+1
-  uint2 aux[kChRing][4];             // [0..1] next strip's entry t-31 lanes 0,1 (N of lane 31); [2..3] previous strip's
-                                     // entry t+31 lanes 30,31 of this sweep (S of lane 0)
-  float4 dummy[32];                  // landing area of the zero-byte copies of lanes without a share
-};
-
-// 16-byte async copy whose source size is 16 or 0 (0 = write zeros, nothing is read): no predicate, no branch
-__device__ __forceinline__ void ch_cp16z(unsigned smem, const void* gmem, unsigned src_bytes) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(smem), "l"(gmem), "r"(src_bytes) : "memory");
-}
-__device__ __forceinline__ void ch_cp16(unsigned smem, const void* gmem, bool pred) {
-  asm volatile("{ .reg .pred q; setp.ne.u32 q, %2, 0; @q cp.async.cg.shared.global [%0], [%1], 16; }" ::"r"(smem), "l"(gmem),
-               "r"((unsigned)pred) : "memory");
-}
-__device__ __forceinline__ uint2 ch_ld_volatile(const uint2* p) {
-  uint2 v;
-  asm volatile("ld.volatile.global.v2.u32 {%0,%1}, [%2];" : "=r"(v.x), "=r"(v.y) : "l"(p) : "memory");
-  return v;
-}
-__device__ __forceinline__ float4 ch_lds128(unsigned a) {
-  float4 v;
-  asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(a));
-  return v;
-}
-__device__ __forceinline__ uint2 ch_lds64(unsigned a) {
-  uint2 v;
-  asm volatile("ld.shared.v2.u32 {%0,%1}, [%2];" : "=r"(v.x), "=r"(v.y) : "r"(a));
-  return v;
-}
 __device__ __forceinline__ float ch_lds32(unsigned a) {
   float v;
   asm volatile("ld.shared.f32 %0, [%1];" : "=f"(v) : "r"(a));
@@ -89,222 +44,6 @@ constexpr int kC2EdgePad = 32;       // front padding of the edge arrays (smooth
 // the element a consumer needs at its step t sits at index t + kC2EdgePad
 __device__ __forceinline__ uint2* c2_edge(const ChainLevel& ch, int g, int which, int e, int s) {
   return ch.edge + (size_t)(2 * g + which) * ch.edge_arr + ((size_t)e * ch.NS + s) * ch.TE;
-}
-
-// ------------------------------------------------------------------------------------------------
-// the four sweeps of one level: grid = B * 4 * nb CTAs of 32*wpb threads
-// ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(32 * kChMaxWpb)
-k_chain_sweeps(const __grid_constant__ SolverParams q, int level) {
-  extern __shared__ __align__(16) unsigned char ch_smem[];
-  __shared__ unsigned long long s_ticket;
-  const DevLevel& Lv = q.lev[level];
-  const ChainLevel& ch = Lv.ch;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const unsigned long long G = (unsigned long long)q.B * 4ull * (unsigned)ch.nb;
-  if (threadIdx.x == 0) s_ticket = atomicAdd(ch.ticket, 1ull);
-  __syncthreads();
-  const unsigned long long ticket = s_ticket;
-  const unsigned tag = ch.tag_hi | (unsigned)((ticket / G) & 0x3ffffffull);      // same for every CTA of this launch
-  const unsigned role = (unsigned)(ticket % G);
-  const int e = (int)(role / (4u * ch.nb)), rem = (int)(role % (4u * ch.nb));
-  const int g = rem / ch.nb + 1, kb = rem % ch.nb;
-  const int s = kb * ch.wpb + warp;
-  if (!q.sc.active[e] || s >= ch.NS || warp >= ch.wpb) return;
-  const int ni = Lv.n - 2, T = ch.T, NS = ch.NS;
-  int Tend = ni + 32;                                         // entries 0 .. Tend: rows 0 .. ni+1 of every lane
-  const size_t eo = (size_t)e * ch.sk_stride;
-  const float4* ct = ch.ct + (size_t)s * T * 32;
-  const float* rsk = ch.rsk + eo + (size_t)s * T * 32;
-  const uint2* dprev = ch.dsk[g - 1] + eo;
-  uint2* dcur = ch.dsk[g] + eo;
-  const unsigned tag_prev = (g == 1) ? 0u : tag;              // sweep 0 (= r*inv) was written by the kernel before this one
-
-  // Copies of one step (16-byte chunks): every lane its coefficient vector; then lanes 0-7 r, 8-23 the previous sweep's
-  // entry q+1, 24 the next strip's entry q-31 (lanes 0,1), 25 the previous strip's entry q+31 of this sweep (lanes 30,31).
-  // A copy is issued for steps q2lo <= q <= q2lo + q2span.
-  const unsigned ring_base = (unsigned)__cvta_generic_to_shared(ch_smem + (size_t)warp * sizeof(ChainRing));
-  const char* g2 = reinterpret_cast<const char*>(rsk);
-  unsigned s2 = ring_base + (unsigned)offsetof(ChainRing, dummy) + 16u * lane, sh2 = 0, stride2 = 0, q2span = 0;
-  int q2lo = 1 << 30;
-  if (lane < 8) {
-    g2 = reinterpret_cast<const char*>(rsk + 4 * lane);
-    s2 = ring_base + (unsigned)offsetof(ChainRing, r) + 16u * lane; sh2 = 7; stride2 = 128; q2lo = 0; q2span = Tend;
-  } else if (lane < 24) {
-    g2 = reinterpret_cast<const char*>(dprev + ((size_t)s * T + 1) * 32 + 2 * (lane - 8));
-    s2 = ring_base + (unsigned)offsetof(ChainRing, e) + 16u * (lane - 8); sh2 = 8; stride2 = 256; q2lo = 0; q2span = Tend;
-  } else if (lane == 24 && s + 1 < NS) {
-    g2 = reinterpret_cast<const char*>(dprev + ((size_t)(s + 1) * T + 1) * 32) - 32 * 256;   // entry q-31 at step q
-    s2 = ring_base + (unsigned)offsetof(ChainRing, aux); sh2 = 5; stride2 = 256; q2lo = 32; q2span = ni - 1;
-  } else if (lane == 25 && s > 0) {
-    g2 = reinterpret_cast<const char*>(dcur + ((size_t)(s - 1) * T + 31) * 32 + 30);         // entry q+31 at step q
-    s2 = ring_base + (unsigned)offsetof(ChainRing, aux) + 16u; sh2 = 5; stride2 = 256; q2lo = 1; q2span = ni - 1;
-  }
-  const char* g1 = reinterpret_cast<const char*>(ct + lane);
-  const unsigned s1 = ring_base + (unsigned)offsetof(ChainRing, coef) + 16u * lane;
-  // zero the aux slots (entries that are never copied must read as finite values)
-  {
-    uint2* aux0 = reinterpret_cast<uint2*>(ch_smem + (size_t)warp * sizeof(ChainRing) + offsetof(ChainRing, aux));
-    for (int k = lane; k < kChRing * 4; k += 32) aux0[k] = make_uint2(0u, 0u);
-  }
-  __syncwarp();
-  float W = 0.f, cxW = 0.f;
-  uint2* out = dcur + (size_t)s * T * 32 + lane;
-  const uint2* e_src = dprev + ((size_t)s * T + 1) * 32 + lane;                 // entry t+1, this lane (reload path)
-  const bool aux_lane = (lane == 0 && s > 0) || (lane == 31 && s + 1 < NS);
-  const uint2* aux_src = e_src;
-  if (aux_lane) aux_src = (lane == 0) ? dcur + ((size_t)(s - 1) * T + 31) * 32 + 31 : dprev + ((size_t)(s + 1) * T + 1) * 32 - 32 * 32;
-  const unsigned aux_tag = (lane == 0) ? tag : tag_prev;
-  const int aux_lo = aux_lane ? (lane == 0 ? 1 : 32) : (1 << 30);               // steps at which the aux operand is a cell
-  const unsigned aux_span = ni - 1;
-  // shared addresses of this lane's operands in slot 0
-  const unsigned a_coef = s1;
-  const unsigned a_r = ring_base + (unsigned)offsetof(ChainRing, r) + 4u * lane;
-  const unsigned a_e = ring_base + (unsigned)offsetof(ChainRing, e) + 8u * lane;
-  const unsigned a_aux = ring_base + (unsigned)offsetof(ChainRing, aux) + (lane == 0 ? 24u : 0u);
-#ifdef RLFC_CHAIN_STATS        // one launch's pipeline shape: start/end time, reload events and spins per (sweep, strip)
-  unsigned long long st_t0, st_t1;
-  unsigned st_miss = 0, st_spins = 0;
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(st_t0));
-#endif
-  unsigned l0 = lane == 0, l31 = lane == 31;
-  unsigned a_coef_ = a_coef, a_r_ = a_r, a_e_ = a_e, a_aux_ = a_aux, s1_ = s1, tagp = tag_prev, tagc = tag, taga = aux_tag;
-  int aux_lo_ = aux_lo;
-  unsigned aux_span_ = aux_span;
-  // pin the loop invariants in registers (otherwise they are rematerialised from the kernel parameters / special registers
-  // in every step)
-  asm volatile("" : "+r"(Tend), "+r"(l0), "+r"(l31), "+r"(a_coef_), "+r"(a_r_), "+r"(a_e_), "+r"(a_aux_), "+r"(s1_), "+r"(s2),
-               "+r"(sh2), "+r"(stride2), "+r"(q2lo), "+r"(q2span), "+r"(tagp), "+r"(tagc), "+r"(taga), "+r"(aux_lo_),
-               "+r"(aux_span_));
-  // One cp.async group per step, two copy instructions, no branches: every lane its coefficient vector of step
-  // i + kChPFS, and its share of the other operands -- of step i + kChPFS for the lanes that copy r, of step i + kChPF
-  // for the lanes that copy the previous sweep / the neighbour strips (lanes without a share copy 0 bytes into a dummy).
-  int qq = 0;                                                 // next step whose dynamic operands are fetched
-  unsigned qslot = 0;
-  const unsigned lead2 = (lane < 8) ? (unsigned)(kChPFS - kChPF) : 0u;
-  unsigned mask2 = (q2lo == (1 << 30)) ? 0u : (unsigned)(kChRing - 1);    // lanes without a share always use their one dummy slot
-  asm volatile("" : "+r"(mask2));
-  int q2lo_ = q2lo - (int)lead2;                              // in terms of qq
-  asm volatile("" : "+r"(q2lo_));
-  auto issue = [&]() {
-    const unsigned sslot = (qslot + (kChPFS - kChPF)) & (kChRing - 1);
-    ch_cp16z(s1_ + (sslot << 9), g1, (qq + (kChPFS - kChPF) <= Tend) ? 16u : 0u);
-    ch_cp16z(s2 + (((qslot + lead2) & mask2) << sh2), g2, ((unsigned)(qq - q2lo_) <= q2span) ? 16u : 0u);
-    asm volatile("cp.async.commit_group;" ::: "memory");
-    g1 += 512; g2 += stride2;
-    qq++; qslot = (qslot + 1) & (kChRing - 1);
-  };
-  // When a step finds an operand with an older tag, its producer is less than the prefetch distance ahead, and then every
-  // copy in flight is stale as well.  Wait until the operands of the FURTHEST step in flight are visible (a strip's
-  // entries become visible in order; nothing depends on that: every operand's tag is checked when it is used), copy the
-  // dynamic operands of all steps in flight again and wait for them: one round trip instead of one per step.  This is
-  // also how a strip starts: its first step finds nothing and waits here until the producers are far enough ahead.
-  const char* g2base = g2;                                    // (re-issue path, lanes >= 8: source of step q = g2base + q*stride2)
-  auto refill = [&](int t) {
-    const int tt = min(t + kChPF + 1, Tend);                  // steps t .. tt are in flight
-    const int te = min(tt, Tend - 1);                         // last step whose E operand is checked
-    const int ta = min(tt, aux_lo_ + (int)aux_span_);         // last step in flight that needs the aux operand
-    const bool chk_e = te >= t, chk_a = ta >= t && ta >= aux_lo_;
-    unsigned spins = 0;
-    while (true) {
-      bool ok = true;
-      if (chk_e) ok = ch_ld_volatile(e_src + (size_t)te * 32).y == tagp;
-      if (chk_a) ok = ok && ch_ld_volatile(aux_src + (size_t)ta * 32).y == taga;
-      if (__all_sync(0xffffffffu, ok)) break;
-      if (++spins > kChSpinMax) __trap();
-#ifdef RLFC_CHAIN_STATS
-      st_spins++;
-#endif
-    }
-    asm volatile("cp.async.wait_group 0;" ::: "memory");     // (the stale copies must not land after their replacements)
-    if (lane >= 8)
-      for (int qv = t; qv <= tt; qv++)
-        ch_cp16(s2 + (((unsigned)qv & (kChRing - 1)) << sh2), g2base + (size_t)qv * stride2, (unsigned)(qv - q2lo) <= q2span);
-    asm volatile("cp.async.commit_group;" ::: "memory");
-    asm volatile("cp.async.wait_group 0;" ::: "memory");
-    __syncwarp();
-  };
-  for (int k = 0; k < kChPFS - kChPF; k++) {                  // static operands of steps 0 .. kChPFS - kChPF - 1
-    ch_cp16(s1_ + ((unsigned)k << 9), g1, k <= Tend);
-    if (lane < 8) { ch_cp16(s2 + ((unsigned)k << sh2), g2, k <= Tend); g2 += stride2; }
-    g1 += 512;
-  }
-  for (int k = 0; k <= kChPF; k++) issue();                   // dynamic operands of steps 0 .. kChPF (static: up to kChPFS)
-  asm volatile("cp.async.wait_group %0;" ::"n"(kChPF) : "memory");
-  __syncwarp();
-  // operands of the current step live in registers, loaded one step ahead (the shared-memory latency hides behind the
-  // previous step's arithmetic)
-  float4 c = ch_lds128(a_coef_);
-  float rv = ch_lds32(a_r_);
-  uint2 ev = ch_lds64(a_e_);
-  uint2 ax = ch_lds64(a_aux_);
-  unsigned tslot = 1;
-  // the tag test and the N operand of a step are prepared at the end of the step before it (vote and shuffle latencies
-  // overlap the start of the next step)
-  auto stale = [&](int t, const uint2& ev_, const uint2& ax_, bool& need_aux) {
-    need_aux = (unsigned)(t - aux_lo_) <= aux_span_;
-#ifdef RLFC_CH_NOCHECK
-    return false;
-#else
-    return (t < Tend && ev_.y != tagp) || (need_aux && ax_.y != taga);
-#endif
-  };
-  bool need_aux;
-  bool any_bad = __any_sync(0xffffffffu, stale(0, ev, ax, need_aux));
-  float N = __shfl_down_sync(0xffffffffu, __uint_as_float(ev.x), 1);
-#pragma unroll 2
-  for (int t = 0; t <= Tend; t++) {
-    float S = __shfl_up_sync(0xffffffffu, W, 1);              // the loop-carried chain starts first
-    const float WcxW = W * cxW;
-#ifndef RLFC_CH_NOISSUE
-    issue();                                                  // copies of step t + kChPF + 1
-#endif
-    if (any_bad) {
-#ifdef RLFC_CHAIN_STATS
-      st_miss++;
-#endif
-      unsigned spins = 0;
-      do {
-        refill(t);
-        const unsigned sl = (unsigned)t & (kChRing - 1);
-        ev = ch_lds64(a_e_ + (sl << 8));
-        ax = ch_lds64(a_aux_ + (sl << 5));
-        if (++spins > 1024u) __trap();
-      } while (__any_sync(0xffffffffu, stale(t, ev, ax, need_aux)));
-      N = __shfl_down_sync(0xffffffffu, __uint_as_float(ev.x), 1);
-    }
-    const float E = __uint_as_float(ev.x);
-    const float axv = need_aux ? __uint_as_float(ax.x) : 0.f;
-    const float4 cc = c;
-    const float rc = rv;
-    // next step's operands (independent of the arithmetic below)
-#ifndef RLFC_CH_NOWAIT
-    asm volatile("cp.async.wait_group %0;" ::"n"(kChPF) : "memory");
-#endif
-    __syncwarp();
-    c = ch_lds128(a_coef_ + (tslot << 9));
-    rv = ch_lds32(a_r_ + (tslot << 7));
-    ev = ch_lds64(a_e_ + (tslot << 8));
-    ax = ch_lds64(a_aux_ + (tslot << 5));
-    tslot = (tslot + 1) & (kChRing - 1);
-    if (l31) N = axv;
-    if (l0) S = axv;
-    const float res = (WcxW + E * cc.x + S * cc.y + N * cc.z - rc) * cc.w;      // MG.pde:85-86
-#ifndef RLFC_CH_NOSTORE
-    *out = make_uint2(__float_as_uint(res), tagc);
-#endif
-    out += 32;
-    W = res;
-    cxW = cc.x;
-    any_bad = __any_sync(0xffffffffu, stale(t + 1, ev, ax, need_aux));
-    N = __shfl_down_sync(0xffffffffu, __uint_as_float(ev.x), 1);
-  }
-  asm volatile("cp.async.wait_group 0;" ::: "memory");
-#ifdef RLFC_CHAIN_STATS
-  asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(st_t1));
-  if (lane == 0 && (ticket / G) == RLFC_CHAIN_STATS)
-    printf("chain L%d g%d s%d start %llu end %llu miss %u spins %u steps %d\n", level, g, s, st_t0, st_t1, st_miss, st_spins, Tend + 1);
-#endif
 }
 
 // ------------------------------------------------------------------------------------------------

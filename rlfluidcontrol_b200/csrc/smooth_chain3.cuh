@@ -1,12 +1,12 @@
 // smooth_chain3.cuh -- sweep kernel of the chained strip smoother (smooth_chain.cuh explains the mapping and the
-// {value, launch tag} protocol), third generation: WARP-SPECIALISED.  Same arithmetic, arrays, tags and ticket roles.
+// {value, launch tag} protocol), third generation: WARP-SPECIALISED.
 // Included by solver_kernels.cu after smooth_chain.cuh, inside namespace rlfc::{anonymous}.
 //
 // Measured on B200 (tools/ubench/shfl_lat.cu, profiles/r02_chain_sweeps.md): the loop-carried chain of one step
-// (SHFL.UP of the previous result, select, 6 dependent FP ops without FMA) is 51.5 cycles; the first kernel spent 156
-// cycles per step (cp.async bookkeeping, tag votes and operand addressing in the same warp), a batched single-warp
-// variant 166 (two mbarrier waits at ~90 cycles and five bulk-copy issues per 8 steps).  So everything that is not the
-// chain moves to a second warp:
+// (SHFL.UP of the previous result, select, 6 dependent FP ops without FMA) is 51.5 cycles; the first generation of the
+// kernel (since removed) spent 156 cycles per step (cp.async bookkeeping, tag votes and operand addressing in the same
+// warp), a batched single-warp variant 166 (two mbarrier waits at ~90 cycles and five bulk-copy issues per 8 steps).
+// So everything that is not the chain moves to a second warp:
 //   * CTA = one COMPUTE warp + one LOADER warp + one EDGE-FORWARDER warp per (sweep, strip);
 //   * the loader streams the strip's operands in batches of kC3B steps with bulk copies (coefficients, r, previous
 //     sweep's entries: contiguous along t in the strip-skewed layout), VALIDATES the tags of the previous sweep's entries

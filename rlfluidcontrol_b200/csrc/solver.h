@@ -17,14 +17,6 @@ namespace rlfc {
 
 constexpr int kMaxLevels = 16;
 
-// Pre-skewed static coefficient tables of one level for the strip smoother (smooth_strip.cuh):
-// entry [(k*Tsk + tau + kSkewPad)*32 + lane] belongs to cell (i = tau - lane + 1, j = 32k + lane + 1).
-struct SkewLevel {
-  const float4* A;          // (lx[i][j], lx[i+1][j], ly[i][j], ly[i][j+1])
-  const float2* nd;         // (-inv[i][j], diag[i][j])
-  int nstrips, Tsk;
-};
-
 // Pre-skewed static coefficient table of one level for the row-pipelined smoother (smooth_rows.cuh):
 // entry tau (stored at index tau + kTabFront) holds, for lane l, the coefficients of row tau - l of the
 // lane's C columns j0 = C*l+1 .. C*l+C as the float stream [ly[row][j0+c] (C+1) | -inv[row][j0+c] (C) |
@@ -44,7 +36,6 @@ struct RowTab {
 struct ChainLevel {
   int on;                   // 1 = this level is smoothed by the chained strip smoother
   int NS, T;                // strips, entries per strip
-  int wpb, nb;              // strips (warps) per CTA, CTAs per sweep
   size_t sk_stride;         // elements per environment of a skewed array = NS*T*32
   const float4* ct;         // static coefficients {lx[i+1][j], ly[i][j], ly[i][j+1], -inv[i][j]}   [NS][T][32]
   float* rsk;               // [B] residual entering smooth(4)                                     (4 B / element)
@@ -60,7 +51,6 @@ struct ChainLevel {
 };
 
 struct DevLevel {
-  SkewLevel sk;
   RowTab rt;
   int n, m, P;              // dims incl. ghosts, pitch
   size_t stride;            // per-env stride (floats) of r/x/d at this level
@@ -120,8 +110,6 @@ struct SolverParams {
   float inv_cells;          // (float)((n-2)*(m-2))
   float mg_tol;
   int   nlevels;
-  int   coarse_strips;      // max strip count over levels >= 1 (warps of k_mg_coarse)
-  int   chain_v;            // sweep kernel generation: 1 = smooth_chain.cuh, 3 (default) = smooth_chain3.cuh
   int   chain_levels;       // levels 0 .. chain_levels-1 run as grid-wide kernels with the chained strip smoother; the
                             // one-CTA-per-env coarse kernel starts at level max(chain_levels, 1)
   double *rr_chain;         // [B][rr_chain_n] per-CTA partial sums of r.r of the level-0 chain increment
@@ -130,7 +118,6 @@ struct SolverParams {
   int   tiny;               // 1 = levels of at most 32 columns are smoothed by one warp in registers (smooth_tiny.cuh; RLFC_TINY=0: row pipeline)
   int   resid_march;        // 1 = k_resid_down0_march (default), 0 = the shared-memory tile version (RLFC_RESID=tile)
   int   fast_bc;            // 1 = two-phase setBC kernels (no band face on the lines setBC reads; grid fits one CTA)
-  int   use_rows;           // 1 = row-pipelined smoother (smooth_rows.cuh), 0 = strip smoother (smooth_strip.cuh)
   int   resolution, substeps, mg_max_iters;
   float init_time, episode_time;
   DevLevel lev[kMaxLevels];
@@ -148,7 +135,6 @@ struct SolverParams {
   // Field.sum as segment summaries (exact_sum.cuh); xs_recs == nullptr selects the plain serial chain (k_psum)
   double *xs_ctot;          // [B][xs_nchunks] chunk totals, valid when xs_cflag == xs_epoch + 1
   unsigned *xs_cflag;       // [B][xs_nchunks]
-  unsigned *xs_rflag;       // [B][xs_nchunks] == xs_epoch + 1 once the chunk's batch records are written
   unsigned *xs_epoch;       // [B] passes completed
   unsigned *xs_recs;        // [B][xs_nbatches][192] batch records (32 summaries condensed)
   unsigned *xs_blk;         // [B][ceil(xs_nbatches/32)][8][32] blocks of 32 records condensed (large domains; else nullptr)
@@ -183,7 +169,6 @@ int chain_incr_blocks(int ni, int NS);
 int launch_advdif(const SolverParams& P, const float* srcx, const float* srcy, const float* u0x, const float* u0y,
                   float* dstx, float* dsty, cudaStream_t st);
 int launch_band_bc(const SolverParams& P, float* ux, float* uy, cudaStream_t st);
-int launch_residual(const SolverParams& P, const float* ux, const float* uy, float* r, int which, cudaStream_t st);
 // first MG iteration fused: residual + level-0 smooth(0)/increment/restriction; p_in -> p_out (different buffers)
 int launch_resid_down0(const SolverParams& P, const float* ux, const float* uy, const float* p_in, float* p_out, float* r_out,
                        int which, cudaStream_t st);
@@ -214,11 +199,6 @@ int launch_loopcond(const SolverParams& P, unsigned long long cond_handle, cudaS
 int launch_psum(const SolverParams& P, cudaStream_t st);
 int launch_psum_tables(const SolverParams& P, cudaStream_t st);   // (the two kernels of launch_psum, segment-summary mode)
 int launch_psum_pass(const SolverParams& P, cudaStream_t st);
-// same, with the serial pass on `side` (forked from / joined to `st` through the two events) so that it runs WHILE the
-// table kernel produces the records it consumes chunk by chunk; for stream capture (parallel branches of the graph)
-int launch_psum_overlapped(const SolverParams& P, cudaStream_t st, cudaStream_t side, cudaEvent_t fork, cudaEvent_t join);
-int launch_project_u(const SolverParams& P, float* ux, float* uy, cudaStream_t st);
-int launch_shift_p(const SolverParams& P, cudaStream_t st);
 int launch_bc(const SolverParams& P, float* ux, float* uy, cudaStream_t st);
 int launch_heun(const SolverParams& P, const float* ucx, const float* ucy, const float* ubx, const float* uby,
                 float* uax, float* uay, cudaStream_t st);

@@ -8,30 +8,23 @@
 // Kernel inventory (one launch handles the whole batch; blockIdx.z / blockIdx.x = environment):
 //   k_advdif      VectorField.AdvDif (QUICK, median-limited)            VectorField.pde:170-222
 //   k_band_bc     BDIM blend + mu1 term on the body band, then u.setBC   BDIM.pde:109-122, Field.pde:209-234
-//   k_residual    r = div(u) - A p                                      VectorField.pde:56-65, PoissonMatrix.pde:53-68
 //   k_mg_down0    level-0 smooth(0) + increment + residual restriction  MG.pde:68-70,79-97,124-137
-//   k_mg_coarse   levels >= 1 of the V-cycle in one CTA per env          MG.pde:68-97,124-152
+//   k_mg_coarse_rows levels >= 1 of the V-cycle in one CTA per env       MG.pde:68-97,124-152
 //   k_mg_up0      level-0 prolongation + increment                       MG.pde:75-76,139-152
-//   k_smooth0     level-0 smooth(4) + increment + r.r + loop test (strip sweep) MG.pde:30-38,79-97, Field.pde:302-310
+//   k_smooth0_rows level-0 smooth(4) + increment + r.r + loop test       MG.pde:30-38,79-97, Field.pde:302-310
 //   k_psum        serial float interior sum of p                        Field.pde:311-318
-//   k_project_u   gradient of the mean-shifted p, velocity correction   VectorField.pde:136-139
-//   k_shift_p     p += -sum(p)/N on all cells                            VectorField.pde:136
+//   k_project_shift p += -sum(p)/N, velocity correction by grad p        VectorField.pde:136-139
 //   k_bc          u.setBC after the projection                          VectorField.pde:140
 //   k_heun        u = (u + us) * 0.5                                     BDIM.pde:95-96
 //   k_force       pressForce + probes + time + draw() accumulation       Body.pde:296-303, SaveScalar.pde:61-72, clientCFD.pde:39-47
 #include "solver.h"
-#include "smooth_strip.cuh"
 #include "smooth_rows.cuh"
 #include "smooth_wave.cuh"
 #include "exact_sum.cuh"
 
-#ifndef RLFC_DOWN_UNROLL
-#define RLFC_DOWN_UNROLL 2      // coarse down pass: blocks in flight per thread
-#endif
 #ifndef RLFC_UP_ROWS
 #define RLFC_UP_ROWS 4          // coarse up pass: rows in flight per warp
 #endif
-constexpr int kDownUnroll = RLFC_DOWN_UNROLL;
 
 namespace rlfc {
 namespace {
@@ -433,30 +426,11 @@ k_bc2(const __grid_constant__ SolverParams q, float* ux_all, float* uy_all, cons
 }
 
 // ------------------------------------------------------------------------------------------------
-// residual r = div(u) - A p   (VectorField.pde:56-65, PoissonMatrix.pde:53-68); also opens the solve
+// A p of the residual r = div(u) - A p   (VectorField.pde:56-65, PoissonMatrix.pde:53-68)
 // ------------------------------------------------------------------------------------------------
 __device__ __forceinline__ float apply_A(const float* x, const float* __restrict__ lx, const float* __restrict__ ly,
                                          const float* __restrict__ diag, int P, int k) {
   return x[k] * diag[k] + x[k - P] * lx[k] + x[k + P] * lx[k + P] + x[k - 1] * ly[k] + x[k + 1] * ly[k + 1];
-}
-
-__global__ void __launch_bounds__(256)
-k_residual(const __grid_constant__ SolverParams q, const float* __restrict__ ux_all, const float* __restrict__ uy_all,
-           float* __restrict__ r_all, int which) {
-  const int P = q.P;
-  const int j = blockIdx.x * blockDim.x + threadIdx.x;
-  const int i = blockIdx.y * blockDim.y + threadIdx.y;
-  const int e = blockIdx.z;
-  if (q.sc.frozen[e]) return;                          // (active[e] is 0 after every completed solve: the MG kernels skip it too)
-  if (i == 0 && j == 0) { q.sc.active[e] = 1; q.sc.iters[2 * e + which] = 0; }
-  if (i < 1 || j < 1 || i > q.n - 2 || j > q.m - 2) return;
-  const size_t eo = (size_t)e * q.stride;
-  const float* ux = ux_all + eo;
-  const float* uy = uy_all + eo;
-  const float* p = q.lev[0].x + eo;
-  const int k = IDX(i, j);
-  float s = ux[k + P] - ux[k] + uy[k + 1] - uy[k];
-  r_all[eo + k] = s - apply_A(p, q.lev[0].lx, q.lev[0].ly, q.lev[0].diag, P, k);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -812,50 +786,9 @@ __device__ __forceinline__ void coarse_up_pass(const DevLevel& L, const DevLevel
   }
 }
 
-__global__ void __launch_bounds__(256, 2)
-k_mg_coarse(const __grid_constant__ SolverParams q) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  StripShared* sh = reinterpret_cast<StripShared*>(smem_raw);
-  StripMail* mail = reinterpret_cast<StripMail*>(smem_raw + sizeof(StripShared) * q.coarse_strips);
-  const int e = blockIdx.x;
-  if (!q.sc.active[e]) return;
-  const int last = q.nlevels - 1;
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
-  // ---- down: smooth(0) + restrict; warps own coarse rows, lanes own coarse columns ----
-  for (int l = 1; l < last; l++) {
-    const DevLevel& L = q.lev[l];
-    const DevLevel& C = q.lev[l + 1];
-    const int nci = C.n - 2, ncj = C.m - 2;
-    const size_t eo = (size_t)e * L.stride;
-    for (int J = 1 + lane; J <= ncj; J += 32)
-#pragma unroll kDownUnroll
-      for (int I = 1 + warp; I <= nci; I += nw)
-        down_block<false>(L, C, L.r + eo, L.d + eo, L.x + eo, C.r + (size_t)e * C.stride, I, J);
-    __syncthreads();
-  }
-  // ---- coarsest level: smooth(its) only (MG.pde:72-73), x = 0 + d ----
-  {
-    const DevLevel& L = q.lev[last];
-    strip_smooth<1>(L, L.r + (size_t)e * L.stride, L.x + (size_t)e * L.stride, sh, mail);
-  }
-  // ---- up: prolongate + increment, then smooth(its): x += GS(r)  (MG.pde:73-76) ----
-  for (int l = last - 1; l >= 1; l--) {
-    const DevLevel& L = q.lev[l];
-    const DevLevel& C = q.lev[l + 1];
-    const size_t eo = (size_t)e * L.stride;
-    float* r = L.d + eo;            // smoothed residual left by the down pass
-    float* x = L.x + eo;
-    coarse_up_pass(L, C, r, x, C.x + (size_t)e * C.stride);
-    __syncthreads();
-    strip_smooth<2>(L, r, x, sh, mail);
-  }
-}
-
 // ------------------------------------------------------------------------------------------------
 // level 0, up: d = prolongate(x1) (+setBC), x += d, r -= A d   (MG.pde:75-76)
 // ------------------------------------------------------------------------------------------------
-// SKEWED: the updated residual goes to the row smoother's skewed array (solver.h rsk) instead of back in place
-template <bool SKEWED>
 __global__ void __launch_bounds__(256)
 k_mg_up0(const __grid_constant__ SolverParams q, float* __restrict__ r_all) {
   const int e = blockIdx.z;
@@ -878,13 +811,7 @@ k_mg_up0(const __grid_constant__ SolverParams q, float* __restrict__ r_all) {
   if (i >= 1 && j >= 1 && i <= n - 2 && j <= m - 2) {
     float Ad = dc * L0.diag[k] + dval(i - 1, j) * L0.lx[k] + dval(i + 1, j) * L0.lx[k + P] + dval(i, j - 1) * L0.ly[k] +
                dval(i, j + 1) * L0.ly[k + 1];
-    if (SKEWED) {
-      const int C = L0.rt.C, CP = rows_CP(C);
-      const int ln = (j - 1) / C, c = (j - 1) - ln * C;
-      q.rsk[(size_t)e * q.rsk_stride + ((size_t)(i + ln) * 32 + ln) * CP + c] = r_all[eo + k] - Ad;
-    } else {
-      r_all[eo + k] -= Ad;
-    }
+    r_all[eo + k] -= Ad;
   }
 }
 
@@ -1006,45 +933,6 @@ k_unskew_r(const __grid_constant__ SolverParams q, float* __restrict__ r_all) {
   const int C = L0.rt.C, CP = rows_CP(C);
   const int ln = (j - 1) / C, c = (j - 1) - ln * C;
   r_all[(size_t)e * L0.stride + IDX(i, j)] = q.rsk[(size_t)e * q.rsk_stride + ((size_t)(i + ln) * 32 + ln) * CP + c];
-}
-
-// level 0 smooth(4) complete (MG.pde:79-97) + the MGsolver loop test (MG.pde:32-35), one CTA per env with one
-// warp per 32-column strip (smooth_strip.cuh, XMODE 3): d = r*inv, four lexicographic Gauss-Seidel sweeps,
-// d.setBC, x += d (p, ghosts included), r -= A d, r.r accumulated in double, then iter++ and the
-// `r.r < tol` / `iter == itmx` decision for this environment.
-__global__ void __launch_bounds__(256)
-k_smooth0(const __grid_constant__ SolverParams q, const float* r_in_all, float* r_out_all, int which) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  const DevLevel& L = q.lev[0];
-  const int ns = L.sk.nstrips, n = L.n, m = L.m, P = L.P, ni = n - 2, mj = m - 2;
-  StripShared* sh = reinterpret_cast<StripShared*>(smem_raw);
-  StripMail* mail = reinterpret_cast<StripMail*>(smem_raw + sizeof(StripShared) * ns);
-  float* gbuf = reinterpret_cast<float*>(smem_raw + sizeof(StripShared) * ns + sizeof(StripMail) * (ns + 2));
-  __shared__ double wsum[32];
-  const int e = blockIdx.x;
-  if (!q.sc.active[e]) return;
-  float* p = L.x + (size_t)e * L.stride;
-  double rr = strip_smooth<3>(L, r_in_all + (size_t)e * L.stride, p, sh, mail, gbuf, r_out_all + (size_t)e * L.stride);
-  // ghost cells of x: x.plusEq(d) runs over all cells and d.setBC copied the adjacent interior value (MG.pde:90,95)
-  const float *gtop = gbuf, *gbot = gbuf + mj, *gleft = gbuf + 2 * mj, *gright = gbuf + 2 * mj + ni;
-  for (int c = threadIdx.x; c < mj; c += blockDim.x) { p[IDX(0, c + 1)] += gtop[c]; p[IDX(n - 1, c + 1)] += gbot[c]; }
-  for (int c = threadIdx.x; c < ni; c += blockDim.x) { p[IDX(c + 1, 0)] += gleft[c]; p[IDX(c + 1, m - 1)] += gright[c]; }
-  if (threadIdx.x == 0) {
-    p[IDX(0, 0)] += gtop[0]; p[IDX(0, m - 1)] += gtop[mj - 1];
-    p[IDX(n - 1, 0)] += gbot[0]; p[IDX(n - 1, m - 1)] += gbot[mj - 1];
-  }
-  // r.r: fixed-order reduction (lanes by shuffle tree, then warps in order)
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) rr += __shfl_down_sync(0xffffffffu, rr, o);
-  if ((threadIdx.x & 31) == 0) wsum[threadIdx.x >> 5] = rr;
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    double s = 0;
-    for (int w = 0; w < (int)(blockDim.x >> 5); w++) s += wsum[w];
-    const int it = ++q.sc.iters[2 * e + which];
-    if ((float)s < q.mg_tol || it >= q.mg_max_iters) q.sc.active[e] = 0;
-    else atomicExch(q.sc.any_active, 1);
-  }
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1237,43 +1125,8 @@ k_psum(const __grid_constant__ SolverParams q) {
 // projection tail (VectorField.pde:136-139): p += -sum/N on all cells; dp = grad p with its setBC
 // (dp.x[1][*] = dp.y[*][1] = 0); u += c * (dp * -1) on the interior.  u.setBC follows in k_bc.
 // ------------------------------------------------------------------------------------------------
-// p must not be shifted in place while neighbouring blocks still read the unshifted values, so the
-// velocity correction (k_project_u) and the shift itself (k_shift_p) are separate passes
-__global__ void __launch_bounds__(256)
-k_project_u(const __grid_constant__ SolverParams q, float* __restrict__ ux_all, float* __restrict__ uy_all) {
-  const int P = q.P, n = q.n, m = q.m;
-  const int j = blockIdx.x * blockDim.x + threadIdx.x;
-  const int i = blockIdx.y * blockDim.y + threadIdx.y;
-  const int e = blockIdx.z;
-  if (i < 1 || j < 1 || i > n - 2 || j > m - 2 || q.sc.frozen[e]) return;
-  const size_t eo = (size_t)e * q.stride;
-  const float* p = q.lev[0].x + eo;
-  const float shift = -1 * q.sc.psum[e] / q.inv_cells;
-  const int k = IDX(i, j);
-  const float pc = p[k] + shift;
-  if (i >= 2) {
-    float dpx = pc - (p[k - P] + shift);
-    ux_all[eo + k] += q.c_x[k] * (dpx * -1);
-  }
-  if (j >= 2) {
-    float dpy = pc - (p[k - 1] + shift);
-    uy_all[eo + k] += q.c_y[k] * (dpy * -1);
-  }
-}
-__global__ void __launch_bounds__(256)
-k_shift_p(const __grid_constant__ SolverParams q) {
-  const int P = q.P;
-  const int j = blockIdx.x * blockDim.x + threadIdx.x;
-  const int i = blockIdx.y * blockDim.y + threadIdx.y;
-  const int e = blockIdx.z;
-  if (i >= q.n || j >= q.m || q.sc.frozen[e]) return;
-  float* p = q.lev[0].x + (size_t)e * q.stride;
-  const float shift = -1 * q.sc.psum[e] / q.inv_cells;
-  p[IDX(i, j)] += shift;
-}
-
-// projection tail fused (VectorField.pde:136-139): p_out = p_in + shift on all cells (p ping-pongs B -> A, so no
-// thread reads a value another thread has already shifted), u += c * (grad(p_in + shift) * -1) on the interior.
+// One kernel: p_out = p_in + shift on all cells (p ping-pongs B -> A, so no thread reads a value another thread has
+// already shifted), u += c * (grad(p_in + shift) * -1) on the interior.
 // One thread handles four consecutive columns (aligned float4 accesses; the pitch is a multiple of 8 floats).
 // HEUN (corrector, BDIM.pde:95-96): away from the lines u.setBC touches the projected velocity goes straight into
 // the Heun average  u = (u + us) * 0.5  written to the step-start buffer; inside that zone (heun_zone) the projected
@@ -1534,12 +1387,6 @@ int launch_bc(const SolverParams& q, float* ux, float* uy, cudaStream_t st) {
   return 1;
 }
 
-int launch_residual(const SolverParams& q, const float* ux, const float* uy, float* r, int which, cudaStream_t st) {
-  dim3 blk(32, 8);
-  k_residual<<<grid2d(q.m, q.n, q.B, blk), blk, 0, st>>>(q, ux, uy, r, which);
-  return 1;
-}
-
 int launch_resid_down0(const SolverParams& q, const float* ux, const float* uy, const float* p_in, float* p_out, float* r_out,
                        int which, cudaStream_t st) {
   const DevLevel& L1 = q.lev[1];
@@ -1593,12 +1440,6 @@ int launch_mg_down0(const SolverParams& q, const float* r_in, float* r_out, cuda
   return 1;
 }
 
-static size_t strip_smem(int nstrips) { return sizeof(StripShared) * nstrips + sizeof(StripMail) * (nstrips + 2); }
-
-static size_t smooth0_smem(const SolverParams& q) {
-  return strip_smem(q.lev[0].sk.nstrips) + sizeof(float) * (2 * (q.n - 2) + 2 * (q.m - 2));
-}
-
 // opt-in shared-memory sizes; called once per handle, outside any stream capture
 static size_t coarse_rows_smem(const SolverParams& q) {
   size_t s = 0;
@@ -1619,11 +1460,6 @@ static cudaError_t set_smooth0_rows_attr(const SolverParams& q) {
 }
 
 int configure_kernels(const SolverParams& q) {
-  cudaError_t e1 = cudaSuccess, e2 = cudaSuccess;
-  if (!q.use_rows) {
-    e1 = cudaFuncSetAttribute(k_mg_coarse, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)strip_smem(q.coarse_strips));
-    e2 = cudaFuncSetAttribute(k_smooth0, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smooth0_smem(q));
-  }
   if (q.fast_bc) {
     if (cudaFuncSetAttribute(k_bc2<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bc2_smem(q)) != cudaSuccess ||
         cudaFuncSetAttribute(k_bc2<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bc2_smem(q)) != cudaSuccess ||
@@ -1635,8 +1471,7 @@ int configure_kernels(const SolverParams& q) {
   if (cudaFuncSetAttribute(k_resid_down0_march, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kRmSmem) != cudaSuccess) return -1;
   cudaError_t e3 = cudaFuncSetAttribute(k_mg_coarse_rows, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)coarse_rows_smem(q));
   if (q.chain_levels > 0 &&
-      (cudaFuncSetAttribute(k_chain_sweeps, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(kChMaxWpb * sizeof(ChainRing))) != cudaSuccess ||
-       cudaFuncSetAttribute(k_chain_sweeps3<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Chain3Smem)) != cudaSuccess ||
+      (cudaFuncSetAttribute(k_chain_sweeps3<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Chain3Smem)) != cudaSuccess ||
        cudaFuncSetAttribute(k_chain_sweeps3<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Chain3Smem)) != cudaSuccess))
     return -1;
   cudaError_t e4 = cudaSuccess;
@@ -1650,14 +1485,13 @@ int configure_kernels(const SolverParams& q) {
     case 7: e4 = set_smooth0_rows_attr<7>(q); break;
     default: e4 = set_smooth0_rows_attr<8>(q); break;
   }
-  return (e1 == cudaSuccess && e2 == cudaSuccess && e3 == cudaSuccess && e4 == cudaSuccess) ? 0 : -1;
+  return (e3 == cudaSuccess && e4 == cudaSuccess) ? 0 : -1;
 }
 
 // chained strip smoother (smooth_chain.cuh): the pieces of one level, individually launchable (profiling) ...
 int launch_chain_sweeps(const SolverParams& q, int l, cudaStream_t st) {
   const ChainLevel& ch = q.lev[l].ch;
-  if (q.chain_v == 1) k_chain_sweeps<<<q.B * 4 * ch.nb, 32 * ch.wpb, ch.wpb * sizeof(ChainRing), st>>>(q, l);
-  else if (ch.ns_loc > 0) {
+  if (ch.ns_loc > 0) {
     // (slab mode: strips on other devices hand their edge operands over through peer memory: system-scope accesses)
     if (q.slab_n > 1) k_chain_sweeps3<true><<<q.B * 4 * ch.ns_loc, 96, sizeof(Chain3Smem), st>>>(q, l);
     else k_chain_sweeps3<false><<<q.B * 4 * ch.ns_loc, 96, sizeof(Chain3Smem), st>>>(q, l);
@@ -1695,34 +1529,29 @@ int chain_incr_blocks(int ni, int NS) {
 
 // ... and as the composites the step graph captures
 int launch_mg_coarse(const SolverParams& q, cudaStream_t st) {
-  if (q.use_rows) {
-    // wide levels run as grid-wide kernels around the one-CTA-per-environment kernel of the small levels
-    int nl = 0;
-    const int first = max(1, q.chain_levels);
-    for (int l = 1; l < first; l++) nl += launch_chain_down(q, l, st);
-    nl += launch_coarse_cta(q, st);
-    for (int l = first - 1; l >= 1; l--) {
-      nl += launch_chain_up(q, l, nullptr, st);
-      nl += launch_chain_sweeps(q, l, st);
-      nl += launch_chain_incr(q, l, nullptr, 0, st);
-    }
-    return nl;
+  // wide levels run as grid-wide kernels around the one-CTA-per-environment kernel of the small levels
+  int nl = 0;
+  const int first = max(1, q.chain_levels);
+  for (int l = 1; l < first; l++) nl += launch_chain_down(q, l, st);
+  nl += launch_coarse_cta(q, st);
+  for (int l = first - 1; l >= 1; l--) {
+    nl += launch_chain_up(q, l, nullptr, st);
+    nl += launch_chain_sweeps(q, l, st);
+    nl += launch_chain_incr(q, l, nullptr, 0, st);
   }
-  const size_t smem = strip_smem(q.coarse_strips);
-  k_mg_coarse<<<q.B, max(256, 32 * q.coarse_strips), smem, st>>>(q);
-  return 1;
+  return nl;
 }
 
 int launch_mg_up0(const SolverParams& q, float* r, cudaStream_t st) {
   dim3 blk(32, 8);
   if (q.lev[0].ch.on) return launch_chain_up(q, 0, r, st);
-  if (q.use_rows && !q.lev[0].wave) k_mg_up0_blk<<<dim3((q.n - 2 + kUpRows - 1) / kUpRows, q.B), 256, up0_smem(q), st>>>(q, r);
-  else k_mg_up0<false><<<grid2d(q.m, q.n, q.B, blk), blk, 0, st>>>(q, r);
+  if (!q.lev[0].wave) k_mg_up0_blk<<<dim3((q.n - 2 + kUpRows - 1) / kUpRows, q.B), 256, up0_smem(q), st>>>(q, r);
+  else k_mg_up0<<<grid2d(q.m, q.n, q.B, blk), blk, 0, st>>>(q, r);
   return 1;
 }
 
 int launch_unskew_r(const SolverParams& q, float* r, cudaStream_t st) {
-  if (!q.use_rows || q.lev[0].wave || q.lev[0].ch.on) return 0;   // (the chain increment writes the plain residual itself)
+  if (q.lev[0].wave || q.lev[0].ch.on) return 0;   // (the chain increment writes the plain residual itself)
   dim3 blk(32, 8);
   k_unskew_r<<<grid2d(q.m, q.n, q.B, blk), blk, 0, st>>>(q, r);
   return 1;
@@ -1730,27 +1559,21 @@ int launch_unskew_r(const SolverParams& q, float* r, cudaStream_t st) {
 
 int launch_smooth0(const SolverParams& q, const float* r_in, float* r_out, int which, cudaStream_t st) {
   if (q.lev[0].ch.on) return launch_chain_sweeps(q, 0, st) + launch_chain_incr(q, 0, r_out, which, st);
-  if (q.use_rows && q.lev[0].wave) {
+  if (q.lev[0].wave) {
     k_smooth0_wave<<<q.B, 1024, 0, st>>>(q, r_in, r_out, which);
     return 1;
   }
-  if (q.use_rows) {
-    const size_t sm = smooth0_rows_smem(q);
-    switch (q.lev[0].rt.C) {
-      case 1: k_smooth0_rows<1><<<q.B, kRows0Threads, sm, st>>>(q, which); break;
-      case 2: k_smooth0_rows<2><<<q.B, kRows0Threads, sm, st>>>(q, which); break;
-      case 3: k_smooth0_rows<3><<<q.B, kRows0Threads, sm, st>>>(q, which); break;
-      case 4: k_smooth0_rows<4><<<q.B, kRows0Threads, sm, st>>>(q, which); break;
-      case 5: k_smooth0_rows<5><<<q.B, kRows0Threads, sm, st>>>(q, which); break;
-      case 6: k_smooth0_rows<6><<<q.B, kRows0Threads, sm, st>>>(q, which); break;
-      case 7: k_smooth0_rows<7><<<q.B, kRows0Threads, sm, st>>>(q, which); break;
-      default: k_smooth0_rows<8><<<q.B, kRows0Threads, sm, st>>>(q, which); break;
-    }
-    return 1;
+  const size_t sm = smooth0_rows_smem(q);
+  switch (q.lev[0].rt.C) {
+    case 1: k_smooth0_rows<1><<<q.B, kRows0Threads, sm, st>>>(q, which); break;
+    case 2: k_smooth0_rows<2><<<q.B, kRows0Threads, sm, st>>>(q, which); break;
+    case 3: k_smooth0_rows<3><<<q.B, kRows0Threads, sm, st>>>(q, which); break;
+    case 4: k_smooth0_rows<4><<<q.B, kRows0Threads, sm, st>>>(q, which); break;
+    case 5: k_smooth0_rows<5><<<q.B, kRows0Threads, sm, st>>>(q, which); break;
+    case 6: k_smooth0_rows<6><<<q.B, kRows0Threads, sm, st>>>(q, which); break;
+    case 7: k_smooth0_rows<7><<<q.B, kRows0Threads, sm, st>>>(q, which); break;
+    default: k_smooth0_rows<8><<<q.B, kRows0Threads, sm, st>>>(q, which); break;
   }
-  const int ns = q.lev[0].sk.nstrips;
-  const size_t smem = smooth0_smem(q);
-  k_smooth0<<<q.B, 32 * ns, smem, st>>>(q, r_in, r_out, which);
   return 1;
 }
 
@@ -1778,7 +1601,7 @@ int launch_psum_pass(const SolverParams& q, cudaStream_t st) {
     else k_xsum_chain_blocks<false><<<q.B, 32, kXsBlocksSmem, st>>>(q);
     return 2;
   }
-  k_xsum_chain<false><<<q.B, 32, 0, st>>>(q);
+  k_xsum_chain<<<q.B, 32, 0, st>>>(q);
   return 1;
 }
 int launch_psum(const SolverParams& q, cudaStream_t st) {
@@ -1787,30 +1610,6 @@ int launch_psum(const SolverParams& q, cudaStream_t st) {
     return 1;
   }
   return launch_psum_tables(q, st) + launch_psum_pass(q, st);
-}
-
-int launch_psum_overlapped(const SolverParams& q, cudaStream_t st, cudaStream_t side, cudaEvent_t fork, cudaEvent_t join) {
-  if (!q.xs_recs) return launch_psum(q, st);
-  cudaEventRecord(fork, st);
-  cudaStreamWaitEvent(side, fork, 0);
-  const dim3 grid(q.B, q.xs_nchunks);
-  k_xsum_tables<0><<<grid, kXsThreads, 0, st>>>(q);
-  k_xsum_chain<true><<<q.B, 32, 0, side>>>(q);       // waits for each chunk's record flag (bounded), see the kernel
-  cudaEventRecord(join, side);
-  cudaStreamWaitEvent(st, join, 0);
-  return 2;
-}
-
-int launch_project_u(const SolverParams& q, float* ux, float* uy, cudaStream_t st) {
-  dim3 blk(32, 8);
-  k_project_u<<<grid2d(q.m, q.n, q.B, blk), blk, 0, st>>>(q, ux, uy);
-  return 1;
-}
-
-int launch_shift_p(const SolverParams& q, cudaStream_t st) {
-  dim3 blk(32, 8);
-  k_shift_p<<<grid2d(q.m, q.n, q.B, blk), blk, 0, st>>>(q);
-  return 1;
 }
 
 int launch_heun(const SolverParams& q, const float* ucx, const float* ucy, const float* ubx, const float* uby,

@@ -175,17 +175,15 @@ def test_other_grids(rlfc, oracle, resolution, xl, yl):
             assert_same(a, b, nm)
 
 
-@pytest.mark.parametrize("envvar,value", [("RLFC_SMOOTHER", "strip"), ("RLFC_SMOOTHER", "wave"), ("RLFC_SMOOTHER", "chain"),
-                                          ("RLFC_NO_GRAPH", "1"), ("RLFC_FUSED", "0"),
+@pytest.mark.parametrize("envvar,value", [("RLFC_SMOOTHER", "wave"), ("RLFC_SMOOTHER", "chain"),
+                                          ("RLFC_NO_GRAPH", "1"),
                                           ("RLFC_GROUPS", "3"), ("RLFC_GROUPS", "4"), ("RLFC_FAST_BC", "0"), ("RLFC_PSUM", "serial"),
                                           ("RLFC_RESID", "tile"), ("RLFC_RESID", "march"), ("RLFC_TINY", "0")])
 def test_alternative_execution_paths(rlfc, oracle, init_state, monkeypatch, envvar, value):
-    """The strip smoother, the wavefront fallback smoother, eager launches, odd env-group splits, the literal setBC kernels and the plain
+    """The wavefront fallback smoother, the chained smoother, eager launches, odd env-group splits, the literal setBC kernels and the plain
     serial Field.sum chain are different
     schedules of the same arithmetic: all must reproduce the oracle bit for bit."""
     monkeypatch.setenv(envvar, value)
-    if envvar == "RLFC_FUSED":                     # the unfused kernels only exist on the eager path
-        monkeypatch.setenv("RLFC_NO_GRAPH", "1")
     ref = make_oracle(oracle, init_state)
     ref.set_xi(-0.6, 0.9)
     B = 7
@@ -200,15 +198,13 @@ def test_alternative_execution_paths(rlfc, oracle, init_state, monkeypatch, envv
             assert_same(a, b, nm)
 
 
-@pytest.mark.parametrize("resolution,dims,chain_v", [(64, (1026, 514), 3), (128, (2050, 1026), 3), (64, (1026, 514), 1),
-                                                     (256, (4098, 2050), 3)])
-def test_wide_grid(rlfc, oracle, monkeypatch, resolution, dims, chain_v):
+@pytest.mark.parametrize("resolution,dims", [(64, (1026, 514)), (128, (2050, 1026)), (256, (4098, 2050))])
+def test_wide_grid(rlfc, oracle, resolution, dims):
     """Single-domain-style grids wider than the row pipeline's 256 columns: BASELINE config 3 (2048x1024, SURVEY 8d:
     resolution 128, t_step = 0.18/128 so dt stays 0.18 grid units) and its half-scale version.  The wide levels fall
     back to the wavefront smoother, setBC to the literal kernels.  Impulsive start, a non-zero action, every float
-    equal to the oracle's.  chain_v: the two generations of the chained sweep kernel (smooth_chain.cuh, smooth_chain3.cuh).
-    The 4096x2048 case (8 Mi cells) also runs the three-pass Field.sum of very large domains; its oracle needs ~20 s."""
-    monkeypatch.setenv("RLFC_CHAIN_V", str(chain_v))
+    equal to the oracle's.  The 4096x2048 case (8 Mi cells) also runs the three-pass Field.sum of very large domains;
+    its oracle needs ~20 s."""
     kw = dict(resolution=resolution, x_lengths=16, y_lengths=8)
     t_step = np.float32(0.18) / np.float32(resolution)
     ref = oracle.OracleEnv(literal=False, resolution=resolution, xLengths=16, yLengths=8, tStep=float(t_step))

@@ -15,12 +15,10 @@ run() {  # name tool env... -- args
 }
 run memcheck_default memcheck --
 run memcheck_chain memcheck RLFC_SMOOTHER=chain --
-run memcheck_strip memcheck RLFC_SMOOTHER=strip --
 run memcheck_wave memcheck RLFC_SMOOTHER=wave -- --small
 run initcheck_default initcheck --
 run initcheck_chain initcheck RLFC_SMOOTHER=chain --
 run racecheck_default racecheck -- --small
-run racecheck_strip racecheck RLFC_SMOOTHER=strip -- --small
 run racecheck_wave racecheck RLFC_SMOOTHER=wave -- --small
 run racecheck_chain racecheck RLFC_SMOOTHER=chain -- --small
 run synccheck_default synccheck -- --small

@@ -1,9 +1,5 @@
 mkdir -p gpurun_out
-for fi in 0 1; do for g in 1 2 4 8 16; do
-  v=$(RLFC_FIXED_ITERS=$fi RLFC_GROUPS=$g timeout 120 python bench.py --no-cpu-baseline --steps 4 --warmup 3 --profile-steps 0 2>/dev/null | python -c "import sys,json; d=json.loads(sys.stdin.read().strip().splitlines()[-1]); print(round(d['value'],1), round(d['e2e']['value'],1))")
-  echo "fixed_iters=$fi groups=$g -> $v"
-done; done
-for g in 4 8; do
-  v=$(RLFC_PSUM=serial RLFC_FIXED_ITERS=1 RLFC_GROUPS=$g timeout 120 python bench.py --no-cpu-baseline --steps 4 --warmup 3 --profile-steps 0 2>/dev/null | python -c "import sys,json; d=json.loads(sys.stdin.read().strip().splitlines()[-1]); print(round(d['value'],1), round(d['e2e']['value'],1))")
-  echo "serial psum fixed_iters=1 groups=$g -> $v"
+for g in 1 2 4 8 16; do
+  v=$(RLFC_GROUPS=$g timeout 120 python bench.py --no-cpu-baseline --steps 4 --warmup 3 --profile-steps 0 2>/dev/null | python -c "import sys,json; d=json.loads(sys.stdin.read().strip().splitlines()[-1]); print(round(d['value'],1), round(d['e2e']['value'],1))")
+  echo "groups=$g -> $v"
 done
