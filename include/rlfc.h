@@ -75,6 +75,12 @@ typedef struct {
                            NVLink): rows / strips are distributed, halo operands are ordinary peer loads, the
                            lexicographic Gauss-Seidel sweeps cross devices strip to strip, results are bit-identical
                            to the single-device run (BASELINE config 5; DESIGN.md 5)                         */
+  int   adaptive_dt;    /* 0 (default) = every solver step is AFCCylinder.update2 with the fixed dt = t_step*resolution.
+                           1 = every solver step of every entry point is AFCCylinder.update() (AFCCylinder.pde:63-84):
+                           each environment taking part in the step first sets dt[e] = min(CFL(u[e], nu), 1)
+                           (BDIM.checkCFL) and then runs the update2 statements with it.  The Poisson hierarchy
+                           (c = del*dt and every coarse level) is rebuilt per environment on the device before each step.
+                           Not available in slab mode or with the chained / wavefront smoothers (RLFC_EINVAL).       */
 } rlfc_config;
 
 void rlfc_default_config(rlfc_config *cfg);
@@ -83,7 +89,7 @@ int  rlfc_env_create(const rlfc_config *cfg, rlfc_env **out);
 void rlfc_env_destroy(rlfc_env *env);
 
 /* Reload the initial state into the listed environments (NULL = all): u, p from the init
-   checkpoint (or uniform flow), t = 0, xi = 0.  The draw()-loop accumulators (callLearn, Cd, Cl)
+   checkpoint (or uniform flow), t = 0, xi = 0, dt = t_step*resolution.  The draw()-loop accumulators (callLearn, Cd, Cl)
    are sketch globals in the reference and survive setUpNewSim (clientCFD.pde:11-13); pass
    reset_accumulators != 0 to also restore them to (16, 0, 0). */
 int  rlfc_env_reset(rlfc_env *env, const int *env_ids, int n, int reset_accumulators);
@@ -147,15 +153,26 @@ int  rlfc_env_field_sum(rlfc_env *env, float *sums);
    All zero with RLFC_PSUM=serial. */
 int  rlfc_env_field_sum_stats(rlfc_env *env, int *stats);
 
-/* Text checkpoint of one environment in the BDIM.write format (readable by BDIM.resume). */
+/* Text checkpoint of one environment in the BDIM.write format (readable by BDIM.resume).  Line 1 holds the dt: the
+   handle's fixed dt, or in adaptive mode the environment's own.  Loading requires the handle's dt in fixed mode and
+   accepts any positive dt in adaptive mode, where it becomes the environment's current dt. */
 int  rlfc_env_save_bdim(rlfc_env *env, int e, const char *path);
 int  rlfc_env_load_bdim(rlfc_env *env, int e, const char *path);
 
 /* BDIM.checkCFL (BDIM.pde:217-219, VectorField.CFL VectorField.pde:225-235) of every environment's current velocity:
    dt[n_envs] = min(1 / (max_interior(|ux| + |uy|) + 3 nu), 1), the time step the reference's adaptive variant
-   AFCCylinder.update() (AFCCylinder.pde:63-84) would take next.  The environment step itself runs the fixed dt of
-   AFCCylinder.update2 (what clientCFD.pde calls); stepping with a per-environment dt is not implemented (DESIGN.md 6). */
+   AFCCylinder.update() (AFCCylinder.pde:63-84) would take next.  A handle created with adaptive_dt = 1 takes exactly
+   that dt in its next solver step; with adaptive_dt = 0 the steps run the fixed dt of AFCCylinder.update2 (what
+   clientCFD.pde calls). */
 int  rlfc_env_check_cfl(rlfc_env *env, float *dt);
+/* dt[n_envs]: the time step (grid units) of each environment's last solver step.  Fixed mode: t_step*resolution for every
+   environment.  Adaptive mode: the CFL step the environment took last; t_step*resolution after create / reset, the
+   checkpoint's dt after rlfc_env_load_bdim.  Synchronises the handle's stream. */
+int  rlfc_env_get_dt(rlfc_env *env, float *dt);
+/* Environment e's Poisson coefficients as its last solver step used them, reference layout at the given MG level:
+   "lower.x", "lower.y", "inv", "diag" (any level), "c.x", "c.y" (level 0 only).  Fixed mode: the same fields as
+   rlfc_env_get_static.  Adaptive mode: the per-environment hierarchy built on the device from c = del*dt[e]. */
+int  rlfc_env_get_coeffs(rlfc_env *env, int e, const char *name, int level, float *out, int *n, int *m);
 
 /* Introspection. */
 int  rlfc_env_dims(const rlfc_env *env, int *n_with_ghosts, int *m_with_ghosts, int *n_envs);

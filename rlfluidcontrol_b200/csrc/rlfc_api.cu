@@ -273,6 +273,12 @@ int solver_step_eager(rlfc_env* E, Group& G, int accumulate) {
   SolverParams& sp = G.sp;
   cudaStream_t st = G.st;
   int rc;
+  if (sp.adaptive) {
+    // AFCCylinder.update (AFCCylinder.pde:63-84): dt = flow.checkCFL(), then the Poisson hierarchy of c = del*dt
+    E->run("k_check_cfl", 2, [&] { return launch_step_cfl(sp, G.uAx, G.uAy, st); }, st);
+    E->run("k_poisson_rebuild0", 0, [&] { return launch_poisson_rebuild0(sp, st); }, st);
+    E->run("k_poisson_rebuild_coarse", 0, [&] { return launch_poisson_rebuild_coarse(sp, st); }, st);
+  }
   // predictor BDIM.update(): u0 = u (buffer A), F = AdvDif(u) -> B, updateUP
   E->run("k_advdif", 5, [&] { return launch_advdif(sp, G.uAx, G.uAy, G.uAx, G.uAy, G.uBx, G.uBy, st); }, st);
   E->run("k_band_bc", 0, [&] { return launch_band_bc(sp, G.uBx, G.uBy, st); }, st);
@@ -349,6 +355,11 @@ int build_step_graph(rlfc_env* E, Group& G, int accumulate) {
   cudaStream_t st = G.st;
   long long n_outer = 0;
   CU(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
+  if (G.sp.adaptive) {   // dt = flow.checkCFL() and the hierarchy of c = del*dt, on the device (dt never goes to the host)
+    n_outer += launch_step_cfl(G.sp, G.uAx, G.uAy, st);
+    n_outer += launch_poisson_rebuild0(G.sp, st);
+    n_outer += launch_poisson_rebuild_coarse(G.sp, st);
+  }
   int rc = capture_half_step(E, G, st, G.uAx, G.uAy, G.uAx, G.uAy, G.uBx, G.uBy, 0, &n_outer);
   if (!rc) rc = capture_half_step(E, G, st, G.uBx, G.uBy, G.uAx, G.uAy, G.uCx, G.uCy, 1, &n_outer);
   if (!rc) {
@@ -602,6 +613,8 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
   if ((long long)cfg->resolution * cfg->x_lengths * cfg->resolution * cfg->y_lengths >= (1ll << 31))
     return fail(RLFC_EINVAL, "grid too large (the kernels index cells with 32 bits)");
   if (cfg->substeps < 1 || cfg->mg_max_iters < 1) return fail(RLFC_EINVAL, "substeps and mg_max_iters must be >= 1");
+  if (cfg->adaptive_dt != 0 && cfg->adaptive_dt != 1) return fail(RLFC_EINVAL, "adaptive_dt must be 0 or 1");
+  if (cfg->adaptive_dt && cfg->n_devices > 1) return fail(RLFC_EINVAL, "adaptive_dt is not available in slab mode (n_devices > 1)");
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
     return fail(RLFC_ENODEV, "no CUDA device available (rlfc has no CPU fallback)");
@@ -665,6 +678,8 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
   // takes the levels that are too wide for the row pipeline
   const bool force_chain = std::getenv("RLFC_SMOOTHER") && std::string(std::getenv("RLFC_SMOOTHER")) == "chain";
   const bool slab = E->cfg.n_devices > 1;   // slab mode: level 0 always runs the chained smoother (its sweeps span devices)
+  const bool adaptive = cfg->adaptive_dt == 1;
+  sp.adaptive = adaptive ? 1 : 0;
   int chain_min_cols = 33;            // RLFC_CHAIN_MIN_COLS: coarse levels at least this wide follow a chained level 0 (levels of
                                       // at most 32 columns are faster in the one-CTA kernel's single-warp smoother: 521 -> 528 steps/s)
   if (const char* ev = std::getenv("RLFC_CHAIN_MIN_COLS")) chain_min_cols = std::max(1, std::atoi(ev));
@@ -676,8 +691,10 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
 
 #define TRY(x) do { rc = (x); if (rc) return bail(rc); } while (0)
   // static level-0 fields
-  TRY(upload_static(E, g.c_x, g.n, g.m, sp.P, &sp.c_x));
-  TRY(upload_static(E, g.c_y, g.n, g.m, sp.P, &sp.c_y));
+  if (!adaptive) {
+    TRY(upload_static(E, g.c_x, g.n, g.m, sp.P, &sp.c_x));
+    TRY(upload_static(E, g.c_y, g.n, g.m, sp.P, &sp.c_y));
+  }
   TRY(upload_static(E, g.w1_x, g.n, g.m, sp.P, &sp.w1_x));
   TRY(upload_static(E, g.w2_x, g.n, g.m, sp.P, &sp.w2_x));
   TRY(upload_static(E, g.ry1_x, g.n, g.m, sp.P, &sp.ry1_x));
@@ -692,10 +709,17 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
     DevLevel& L = sp.lev[l];
     L.n = H.n; L.m = H.m; L.P = round_up(H.m, 8);
     L.stride = (size_t)round_up(L.n * L.P, 32);
-    TRY(upload_static(E, H.lx, H.n, H.m, L.P, &L.lx));
-    TRY(upload_static(E, H.ly, H.n, H.m, L.P, &L.ly));
-    TRY(upload_static(E, H.inv, H.n, H.m, L.P, &L.inv));
-    TRY(upload_static(E, H.diag, H.n, H.m, L.P, &L.diag));
+    if (adaptive) {
+      // one copy per environment at the level's stride, rebuilt on the device from each environment's dt
+      float* a[4] = {nullptr, nullptr, nullptr, nullptr};
+      for (int k = 0; k < 4; k++) TRY(E->dmalloc(&a[k], L.stride * B));
+      L.lx = a[0]; L.ly = a[1]; L.inv = a[2]; L.diag = a[3];
+    } else {
+      TRY(upload_static(E, H.lx, H.n, H.m, L.P, &L.lx));
+      TRY(upload_static(E, H.ly, H.n, H.m, L.P, &L.ly));
+      TRY(upload_static(E, H.inv, H.n, H.m, L.P, &L.inv));
+      TRY(upload_static(E, H.diag, H.n, H.m, L.P, &L.diag));
+    }
     {  // pre-skewed coefficient table for the row-pipelined smoother (layout: solver.h RowTab)
       const int ni = H.n - 2, mj = H.m - 2;
       const int C = (mj + 31) / 32, K = (3 * C + 1 + 3) / 4, nl = (mj + C - 1) / C;
@@ -737,7 +761,13 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
         sp.chain_levels = l + 1;
       }
       L.rt.C = C; L.rt.K = K; L.rt.entries = 0; L.rt.copies = 1; L.rt.T = nullptr;
-      if (!L.wave && !L.ch.on) {
+      if (adaptive && !L.wave && !L.ch.on) {
+        // one table per environment (k_poisson_rebuild*); a view of the batch sets `copies` to its B, so the smoother's
+        // CTA e (= environment e of the view) reads table e
+        float4* T = nullptr;
+        TRY(E->dmalloc(&T, (size_t)entries * K * 32 * B));
+        L.rt.entries = entries; L.rt.copies = B; L.rt.T = T;
+      } else if (!L.wave && !L.ch.on) {
       std::vector<float4> T((size_t)entries * K * 32, make_float4(0.f, 0.f, 0.f, 0.f));
       std::vector<float> f(4 * K);
       for (int e = 0; e < entries; e++)
@@ -779,6 +809,19 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
     L.r2 = nullptr;
     L.w = nullptr;
     if (l == 0 && L.wave) TRY(E->dmalloc(&L.w, L.stride * B));
+  }
+  if (adaptive) {
+    // the per-environment hierarchy exists for the row-pipeline and single-warp smoothers only
+    if (sp.chain_levels > 0)
+      return bail(fail(RLFC_EINVAL, "adaptive_dt is not available with the chained strip smoother (a level too wide for the "
+                                    "row pipeline, or RLFC_SMOOTHER=chain)"));
+    for (int l = 0; l < sp.nlevels; l++)
+      if (sp.lev[l].wave)
+        return bail(fail(RLFC_EINVAL, "adaptive_dt is not available with the wavefront smoother (RLFC_SMOOTHER=wave, or a "
+                                      "coarsest level wider than the row pipeline)"));
+    TRY(upload_static(E, g.del_x, g.n, g.m, sp.P, &sp.del_x));
+    TRY(upload_static(E, g.del_y, g.n, g.m, sp.P, &sp.del_y));
+    sp.c_x = sp.lev[0].lx; sp.c_y = sp.lev[0].ly;   // c = del*(1*dt) is level 0's lower (geometry.cpp)
   }
   // body band: faces where the BDIM blend is not the identity (del != 1, del1 != 0, or a control
   // cylinder's velocity kernel is non-zero)
@@ -854,6 +897,7 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
   TRY(E->dmalloc(&sp.sc.frozen, B)); TRY(E->dmalloc(&sp.sc.non_finite, B)); TRY(E->dmalloc(&sp.sc.n_running, 1));
   sp.sc.rr_part = nullptr;
   TRY(E->dmalloc(&sp.sc.psum, B));
+  TRY(E->dmalloc(&sp.sc.dt, B));
   {
     // Field.sum: segment summaries (exact_sum.cuh) or the plain dependent-add chain (k_psum).  The chain costs
     // 6 cycles per cell of pure latency whatever the batch size and next to no issue slots; the summaries cost
@@ -934,7 +978,12 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
       const size_t o = (size_t)e0 * v.lev[l].stride;
       v.lev[l].r += o; v.lev[l].x += o; v.lev[l].d += o;
       if (v.lev[l].w) v.lev[l].w += o;
+      if (v.adaptive) {
+        v.lev[l].lx += o; v.lev[l].ly += o; v.lev[l].inv += o; v.lev[l].diag += o;
+        if (v.lev[l].rt.T) { v.lev[l].rt.T += (size_t)e0 * v.lev[l].rt.entries * v.lev[l].rt.K * 32; v.lev[l].rt.copies = G.B; }
+      }
     }
+    if (v.adaptive) { v.c_x = v.lev[0].lx; v.c_y = v.lev[0].ly; v.sc.dt += e0; }
     for (int l = 0; l < v.chain_levels; l++) {
       ChainLevel& ch = v.lev[l].ch;
       ch.rsk += (size_t)e0 * ch.sk_stride;
@@ -1041,6 +1090,11 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
 
   if ((rc = load_initial_state(E))) return bail(rc);
   if ((rc = rlfc_env_reset(E, nullptr, B, 1))) return bail(rc);
+  if (adaptive) {   // the hierarchy of the initial dt, so that rlfc_env_get_coeffs is defined before the first step
+    E->launches += launch_poisson_rebuild0(E->whole.sp, E->stream);
+    E->launches += launch_poisson_rebuild_coarse(E->whole.sp, E->stream);
+    if (cudaGetLastError() != cudaSuccess) return bail(fail(RLFC_ECUDA, "initial Poisson hierarchy build failed"));
+  }
   if (cudaStreamSynchronize(E->stream) != cudaSuccess) return bail(fail(RLFC_ECUDA, "initialisation failed"));
   *out = E;
   return RLFC_OK;
@@ -1067,6 +1121,7 @@ int rlfc_env_reset(rlfc_env* E, const int* env_ids, int n, int reset_accumulator
     CU(cudaMemsetAsync(sp.sc.force + 2 * e, 0, 2 * sizeof(float), E->stream));
     CU(cudaMemsetAsync(sp.sc.frozen + e, 0, sizeof(int), E->stream));
     CU(cudaMemsetAsync(sp.sc.non_finite + e, 0, sizeof(int), E->stream));
+    CU(cudaMemcpyAsync(sp.sc.dt + e, &E->geo.dt, sizeof(float), cudaMemcpyHostToDevice, E->stream));   // t_step*resolution
     if (reset_accumulators) {
       CU(cudaMemcpyAsync(sp.sc.callLearn + e, &one16, sizeof(int), cudaMemcpyHostToDevice, E->stream));
       CU(cudaMemsetAsync(sp.sc.Cd + e, 0, sizeof(float), E->stream));
@@ -1107,7 +1162,11 @@ int rlfc_env_step(rlfc_env* E, const float* actions, float* obs, float* reward, 
   // Every environment advances to ITS next observation (clientCFD.pde:39-50).  Environments at a callLearn boundary need
   // exactly `substeps` solver steps -- one round; an environment fresh from a reset first runs uncontrolled until
   // t > init_time and then through its first accumulation window, over several rounds, while the others stay frozen.
-  const int max_rounds = 3 + (int)((sp.init_time > 0 ? sp.init_time : 0) / sp.dt_over_res) / sp.substeps;
+  // (adaptive mode: the bound follows the smallest dt any environment has taken in the rounds so far)
+  const float init_time = sp.init_time > 0 ? sp.init_time : 0;
+  int max_rounds = 3 + (int)(init_time / sp.dt_over_res) / sp.substeps;
+  float dt_min = sp.dt;
+  std::vector<float> h_dt(sp.adaptive ? B : 0);
   for (int round = 0;; round++) {
     int rc = step_round(E, E->d_actions, E->d_obs, E->d_reward, E->d_done);
     if (rc) return rc;
@@ -1115,8 +1174,13 @@ int rlfc_env_step(rlfc_env* E, const float* actions, float* obs, float* reward, 
     CU(cudaMemcpyAsync(E->h_obs, E->d_obs, 2 * B * sizeof(float), cudaMemcpyDeviceToHost, E->stream));
     if (reward) CU(cudaMemcpyAsync(E->h_reward, E->d_reward, B * sizeof(float), cudaMemcpyDeviceToHost, E->stream));
     if (done) CU(cudaMemcpyAsync(E->h_done, E->d_done, B * sizeof(int), cudaMemcpyDeviceToHost, E->stream));
+    if (sp.adaptive) CU(cudaMemcpyAsync(h_dt.data(), sp.sc.dt, B * sizeof(float), cudaMemcpyDeviceToHost, E->stream));
     CU(cudaStreamSynchronize(E->stream));
     if (*E->h_any == 0) break;
+    if (sp.adaptive) {
+      for (float d : h_dt) if (d > 0 && d < dt_min) dt_min = d;
+      max_rounds = 3 + (int)(init_time / (dt_min / sp.resolution)) / sp.substeps;
+    }
     if (round >= max_rounds) return fail(RLFC_ENOTCONV, "an environment did not reach its next observation");
   }
   std::memcpy(obs, E->h_obs, 2 * B * sizeof(float));
@@ -1195,11 +1259,12 @@ int rlfc_env_save_bdim(rlfc_env* E, int e, const char* path) {
   int rc = rlfc_env_get_fields(E, e, ux.data(), uy.data(), p.data());
   if (rc) return rc;
   // BDIM.t counts grid-unit time: set by resume, += dt per solver step (AFCCylinder.t advances by dt/resolution instead)
-  float flow_t = 0;
+  float flow_t = 0, dt = E->sp.dt;
   CU(cudaMemcpyAsync(&flow_t, E->sp.sc.flow_t + e, sizeof(float), cudaMemcpyDeviceToHost, E->stream));
+  if (E->sp.adaptive) CU(cudaMemcpyAsync(&dt, E->sp.sc.dt + e, sizeof(float), cudaMemcpyDeviceToHost, E->stream));
   CU(cudaStreamSynchronize(E->stream));
   std::string err;
-  rc = write_bdim_text(path, E->sp.n, E->sp.m, flow_t, E->sp.dt, ux.data(), uy.data(), p.data(), err);
+  rc = write_bdim_text(path, E->sp.n, E->sp.m, flow_t, dt, ux.data(), uy.data(), p.data(), err);
   return rc ? fail(rc, err) : RLFC_OK;
 }
 
@@ -1210,9 +1275,13 @@ int rlfc_env_load_bdim(rlfc_env* E, int e, const char* path) {
   std::string err;
   int rc = read_checkpoint(path, E->sp.n, E->sp.m, t, dt, ux, uy, p, err);
   if (rc) return fail(rc, err);
-  if (dt != E->sp.dt && !(std::fabs(dt - E->sp.dt) <= 1e-6f * E->sp.dt))
+  if (E->sp.adaptive) {
+    // adaptive mode: any positive dt; it becomes the environment's current dt
+    if (!(dt > 0) || !std::isfinite(dt)) return fail(RLFC_EIO, "checkpoint dt " + std::to_string(dt) + " is not a positive number");
+  } else if (dt != E->sp.dt && !(std::fabs(dt - E->sp.dt) <= 1e-6f * E->sp.dt))
     return fail(RLFC_EIO, "checkpoint dt " + std::to_string(dt) + " does not match the handle's " + std::to_string(E->sp.dt));
   CU(cudaSetDevice(E->device));
+  if (E->sp.adaptive) CU(cudaMemcpyAsync(E->sp.sc.dt + e, &dt, sizeof(float), cudaMemcpyHostToDevice, E->stream));
   CU(cudaMemcpyAsync(E->sp.sc.flow_t + e, &t, sizeof(float), cudaMemcpyHostToDevice, E->stream));   // BDIM.resume: t = stuff[0]
   CU(cudaStreamSynchronize(E->stream));
   return rlfc_env_set_fields(E, e, ux.data(), uy.data(), p.data());
@@ -1260,6 +1329,18 @@ int rlfc_env_check_cfl(rlfc_env* E, float* dt) {
   CU(cudaMemcpyAsync(E->h_reward, E->d_reward, E->sp.B * sizeof(float), cudaMemcpyDeviceToHost, E->stream));
   CU(cudaStreamSynchronize(E->stream));
   std::memcpy(dt, E->h_reward, E->sp.B * sizeof(float));
+  return RLFC_OK;
+}
+
+int rlfc_env_get_dt(rlfc_env* E, float* dt) {
+  if (!E || !dt) return fail(RLFC_EINVAL, "null argument");
+  if (!E->sp.adaptive) {
+    for (int e = 0; e < E->sp.B; e++) dt[e] = E->sp.dt;
+    return RLFC_OK;
+  }
+  CU(cudaSetDevice(E->device));
+  CU(cudaMemcpyAsync(dt, E->sp.sc.dt, E->sp.B * sizeof(float), cudaMemcpyDeviceToHost, E->stream));
+  CU(cudaStreamSynchronize(E->stream));
   return RLFC_OK;
 }
 
@@ -1322,6 +1403,27 @@ static int static_lookup(const Geometry& g, const char* name, int level, float* 
 int rlfc_env_get_static(rlfc_env* E, const char* name, int level, float* out, int* n, int* m) {
   if (!E || !name) return fail(RLFC_EINVAL, "null argument");
   return static_lookup(E->geo, name, level, out, n, m);
+}
+
+int rlfc_env_get_coeffs(rlfc_env* E, int e, const char* name, int level, float* out, int* n, int* m) {
+  if (!E || !name) return fail(RLFC_EINVAL, "null argument");
+  if (e < 0 || e >= E->sp.B) return fail(RLFC_EINVAL, "env index out of range");
+  if (level < 0 || level >= E->sp.nlevels) return fail(RLFC_EINVAL, "level out of range");
+  const std::string nm(name);
+  const bool c0 = level == 0 && (nm == "c.x" || nm == "c.y");
+  if (!c0 && nm != "lower.x" && nm != "lower.y" && nm != "inv" && nm != "diag")
+    return fail(RLFC_EINVAL, "unknown Poisson coefficient field " + nm);
+  if (!E->sp.adaptive) return static_lookup(E->geo, name, level, out, n, m);
+  const DevLevel& L = E->sp.lev[level];
+  if (n) *n = L.n;
+  if (m) *m = L.m;
+  if (!out) return RLFC_OK;
+  const float* src = (nm == "lower.x" || nm == "c.x") ? L.lx : (nm == "lower.y" || nm == "c.y") ? L.ly : nm == "inv" ? L.inv : L.diag;
+  CU(cudaSetDevice(E->device));
+  CU(cudaMemcpy2DAsync(out, L.m * sizeof(float), src + (size_t)e * L.stride, L.P * sizeof(float), L.m * sizeof(float), L.n,
+                       cudaMemcpyDeviceToHost, E->stream));
+  CU(cudaStreamSynchronize(E->stream));
+  return RLFC_OK;
 }
 
 int rlfc_geometry_static(const rlfc_config* cfg, const char* name, int level, float* out, int* n, int* m, int* nlevels) {

@@ -59,7 +59,7 @@ k_chain_down(const __grid_constant__ SolverParams q, int level) {
   const int I = blockIdx.y * blockDim.y + threadIdx.y + 1;
   if (I > C.n - 2 || J > C.m - 2) return;
   const size_t eo = (size_t)e * L.stride;
-  down_block<false>(L, C, L.r + eo, L.d + eo, L.x + eo, C.r + (size_t)e * C.stride, I, J);
+  down_block<false>(L, C, L.r + eo, L.d + eo, L.x + eo, C.r + (size_t)e * C.stride, I, J, 0);
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -23,15 +23,15 @@ __host__ __device__ inline bool tiny_level(int ni, int mj) { return mj <= 32 && 
 // XMODE 1: x = 0 + d (coarsest level), 2: x = x + d.  Called by ALL threads of the CTA (any block size >= 32).
 template <int XMODE>
 __device__ __forceinline__ void tiny_smooth(const DevLevel& L, const float* __restrict__ r, float* __restrict__ x,
-                                            unsigned char* smem_raw) {
+                                            unsigned char* smem_raw, size_t co) {
   const int ni = L.n - 2, mj = L.m - 2, P = L.P;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   float4* s_a = reinterpret_cast<float4*>(smem_raw);                       // [ni+2][32] {lxW, lxE, lyS, lyN}
   float2* s_b = reinterpret_cast<float2*>(s_a + (size_t)(ni + 2) * 32);    // [ni+2][32] {-inv, r}
   float* s_x = reinterpret_cast<float*>(s_b + (size_t)(ni + 2) * 32);      // [ni+2][32] x
-  const float* __restrict__ lx = L.lx;
-  const float* __restrict__ ly = L.ly;
-  const float* __restrict__ inv = L.inv;
+  const float* __restrict__ lx = L.lx + co;                                // co: this environment's coefficients (adaptive mode)
+  const float* __restrict__ ly = L.ly + co;
+  const float* __restrict__ inv = L.inv + co;
   // ---- stage: rows 0 .. ni+1, lanes 0 .. 31 (zeros outside the interior) ----
   for (int t = threadIdx.x; t < (ni + 2) * 32; t += blockDim.x) {
     const int i = t >> 5, l = t & 31, j = l + 1;

@@ -88,6 +88,7 @@ struct EnvScalars {
   double *rr_part;  // [B][rr_blocks] partial sums of r.r
   float *psum;      // [B]    serial interior sum of p
   int   *any_active;// [1]
+  float *dt;        // [B]    adaptive mode: dt of the env's current / last solver step (k_check_cfl<true> writes it)
 };
 
 // Slab mode (BASELINE config 5): one domain advanced by several devices that share every array through one virtual
@@ -145,6 +146,12 @@ struct SolverParams {
   int xs_flags;             // cross-check switches: bit 0 = redo batches as plain additions (RLFC_XS_REDO=serial)
   int *xs_stats;            // [B][8] counters of the last serial pass (rlfc_env_field_sum_stats)
   EnvScalars sc;
+  // (appended last, so the fields above keep their offsets in the kernels' parameter space)
+  int   adaptive;           // 1 = per-environment dt (sc.dt) and Poisson hierarchy: every level's lx, ly, inv, diag hold one
+                            // copy per environment at the level's `stride` (like r, x, d), c_x / c_y are level 0's lx / ly,
+                            // and each row-pipeline level's RowTab holds one table per environment (rt.copies = the view's B,
+                            // so the row smoother's `blockIdx.x % copies` pick selects environment blockIdx.x's table)
+  const float *del_x, *del_y;   // adaptive mode: level-0 BDIM del (reference layout incl. ghosts, pitched), c = del*(1*dt)
 };
 
 #ifdef __CUDACC__
@@ -206,6 +213,12 @@ int launch_heun(const SolverParams& P, const float* ucx, const float* ucy, const
 int launch_force(const SolverParams& P, int accumulate, cudaStream_t st);
 // BDIM.checkCFL of every environment's current velocity: d_dt[B] = min(1/(max(|ux|+|uy|) + 3 nu), 1)
 int launch_check_cfl(const SolverParams& P, const float* ux, const float* uy, float* d_dt, cudaStream_t st);
+// adaptive mode, start of a solver step: sc.dt[e] = BDIM.checkCFL of u for every environment not frozen (frozen ones keep theirs)
+int launch_step_cfl(const SolverParams& P, const float* ux, const float* uy, cudaStream_t st);
+// adaptive mode: every level's lx, ly, inv, diag and row tables of the environments not frozen, from c = del*(1*dt[e])
+// (geometry.cpp finish_level / coarsen restated); level 0 grid-wide, then the coarse levels one CTA per environment
+int launch_poisson_rebuild0(const SolverParams& P, cudaStream_t st);
+int launch_poisson_rebuild_coarse(const SolverParams& P, cudaStream_t st);
 // mode 0 (single solver steps): xi = actions (NULL keeps xi), every env runs.  mode 1 (RL step): an env takes its
 // action only where the reference would have asked for one (t > init_time and at a callLearn boundary); envs whose
 // episode is over (t >= episode_time) are frozen for the call

@@ -81,12 +81,15 @@ __device__ __forceinline__ float face_value(float uf, float bLL, float bL, float
 #ifndef RLFC_ADV_MINB
 #define RLFC_ADV_MINB 9      // 56 registers, 9 CTAs per SM: 202 -> 193 us (8: 198, 10 and 12 spill: 201, 217)
 #endif
-template <bool PREDICTOR>
+// ADT (adaptive mode): the environment's own dt, dts[blockIdx.z], replaces the handle's fixed `dt`
+template <bool PREDICTOR, bool ADT>
 __global__ void __launch_bounds__(128, RLFC_ADV_MINB)
 k_advdif(const float* __restrict__ srcx, const float* __restrict__ srcy, const float* __restrict__ u0x,
          const float* __restrict__ u0y, float* __restrict__ dstx, float* __restrict__ dsty, int n, int m, int P,
-         size_t stride, float dt, float nu, const int* __restrict__ frozen, int slab_rank, int slab_n, int chunk_rows) {
+         size_t stride, float dt_fixed, float nu, const int* __restrict__ frozen, int slab_rank, int slab_n, int chunk_rows,
+         const float* __restrict__ dts) {
   if (frozen[blockIdx.z] || slab_skip(blockIdx.y, gridDim.y, slab_rank, slab_n)) return;
+  const float dt = ADT ? dts[blockIdx.z] : dt_fixed;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int ni = n - 2, mj = m - 2;
   const int jw0 = 1 + blockIdx.x * kAdvCols;                         // first output column of this warp
@@ -221,24 +224,25 @@ __device__ void cta_setBC(float* a, int n, int m, int P, int btype, float bval, 
 }
 
 // body velocity from the static basis (BodyUnion.velocity BodyUnion.pde:84-92, Body.velocity Body.pde:234-240)
-__device__ __forceinline__ float ub_x(const SolverParams& q, int k, float dphi1, float dphi2) {
-  float u1 = (0.f - q.ry1_x[k] * dphi1) / q.dt;
-  float u2 = (0.f - q.ry2_x[k] * dphi2) / q.dt;
+__device__ __forceinline__ float ub_x(const SolverParams& q, int k, float dphi1, float dphi2, float dt) {
+  float u1 = (0.f - q.ry1_x[k] * dphi1) / dt;
+  float u2 = (0.f - q.ry2_x[k] * dphi2) / dt;
   float v = 0.f + u1 * q.w1_x[k];
   return v + u2 * q.w2_x[k];
 }
-__device__ __forceinline__ float ub_y(const SolverParams& q, int k, float dphi1, float dphi2) {
-  float u1 = (0.f + q.rx1_y[k] * dphi1) / q.dt;
-  float u2 = (0.f + q.rx2_y[k] * dphi2) / q.dt;
+__device__ __forceinline__ float ub_y(const SolverParams& q, int k, float dphi1, float dphi2, float dt) {
+  float u1 = (0.f + q.rx1_y[k] * dphi1) / dt;
+  float u2 = (0.f + q.rx2_y[k] * dphi2) / dt;
   float v = 0.f + u1 * q.w1_y[k];
   return v + u2 * q.w2_y[k];
 }
 
 // BDIM.updateUP blend of one band face (BDIM.pde:109-122): u = del*R - ub*(del + (-1)) + del1 * normalGrad(R - ub)
 template <bool XCOMP>
-__device__ __forceinline__ float band_face(const SolverParams& q, const float* u, const BandFace& f, float dphi1, float dphi2) {
+__device__ __forceinline__ float band_face(const SolverParams& q, const float* u, const BandFace& f, float dphi1, float dphi2,
+                                           float dt) {
   const int P = q.P, k = IDX(f.i, f.j);
-  auto ub = [&](int kk) { return XCOMP ? ub_x(q, kk, dphi1, dphi2) : ub_y(q, kk, dphi1, dphi2); };
+  auto ub = [&](int kk) { return XCOMP ? ub_x(q, kk, dphi1, dphi2, dt) : ub_y(q, kk, dphi1, dphi2, dt); };
   const float R = u[k], ubc = ub(k);
   const float v = f.del * R - ubc * (f.del + (-1.f));
   const float duE = u[k + P] - ub(k + P), duW = u[k - P] - ub(k - P);
@@ -247,7 +251,12 @@ __device__ __forceinline__ float band_face(const SolverParams& q, const float* u
   return v + f.del1 * g;
 }
 
+// dt of environment e's solver step: the handle's fixed dt, or (ADT, adaptive mode) the environment's own
+template <bool ADT>
+__device__ __forceinline__ float env_dt(const SolverParams& q, int e) { return ADT ? q.sc.dt[e] : q.dt; }
+
 // the blend for a whole (large) band, grid-wide: values go to band_tmp, k_band_bc<true> writes them back
+template <bool ADT>
 __global__ void __launch_bounds__(256)
 k_band_blend(const __grid_constant__ SolverParams q, const float* ux_all, const float* uy_all) {
   const int e = blockIdx.y, b = blockIdx.x * blockDim.x + threadIdx.x;
@@ -256,13 +265,14 @@ k_band_blend(const __grid_constant__ SolverParams q, const float* ux_all, const 
   const float* uy = uy_all + (size_t)e * q.stride;
   float* tmp = q.band_tmp + (size_t)e * (q.nband_x + q.nband_y);
   const float xi1_m = q.action_scale * q.sc.xi[2 * e], xi2_m = q.action_scale * q.sc.xi[2 * e + 1];   // AFCCylinder.pde:48-49
-  const float dphi1 = (2 * xi1_m * q.dt) / q.dRD, dphi2 = (2 * xi2_m * q.dt) / q.dRD;
-  tmp[b] = (b < q.nband_x) ? band_face<true>(q, ux, q.band_x[b], dphi1, dphi2)
-                           : band_face<false>(q, uy, q.band_y[b - q.nband_x], dphi1, dphi2);
+  const float dt = env_dt<ADT>(q, e);
+  const float dphi1 = (2 * xi1_m * dt) / q.dRD, dphi2 = (2 * xi2_m * dt) / q.dRD;
+  tmp[b] = (b < q.nband_x) ? band_face<true>(q, ux, q.band_x[b], dphi1, dphi2, dt)
+                           : band_face<false>(q, uy, q.band_y[b - q.nband_x], dphi1, dphi2, dt);
 }
 
 // BDIM.updateUP blend on the body band (everywhere else it is the identity), then u.setBC()
-template <bool PREBLENDED>
+template <bool PREBLENDED, bool ADT>
 __global__ void __launch_bounds__(1024)
 k_band_bc(const __grid_constant__ SolverParams q, float* ux_all, float* uy_all) {
   extern __shared__ float scol[];
@@ -274,9 +284,10 @@ k_band_bc(const __grid_constant__ SolverParams q, float* ux_all, float* uy_all) 
   if (!PREBLENDED) {
     // AFCCylinder.pde:48-49
     const float xi1_m = q.action_scale * q.sc.xi[2 * e], xi2_m = q.action_scale * q.sc.xi[2 * e + 1];
-    const float dphi1 = (2 * xi1_m * q.dt) / q.dRD, dphi2 = (2 * xi2_m * q.dt) / q.dRD;
-    for (int b = threadIdx.x; b < q.nband_x; b += blockDim.x) tmp[b] = band_face<true>(q, ux, q.band_x[b], dphi1, dphi2);
-    for (int b = threadIdx.x; b < q.nband_y; b += blockDim.x) tmp[q.nband_x + b] = band_face<false>(q, uy, q.band_y[b], dphi1, dphi2);
+    const float dt = env_dt<ADT>(q, e);
+    const float dphi1 = (2 * xi1_m * dt) / q.dRD, dphi2 = (2 * xi2_m * dt) / q.dRD;
+    for (int b = threadIdx.x; b < q.nband_x; b += blockDim.x) tmp[b] = band_face<true>(q, ux, q.band_x[b], dphi1, dphi2, dt);
+    for (int b = threadIdx.x; b < q.nband_y; b += blockDim.x) tmp[q.nband_x + b] = band_face<false>(q, uy, q.band_y[b], dphi1, dphi2, dt);
     __syncthreads();
   }
   for (int b = threadIdx.x; b < q.nband_x; b += blockDim.x) ux[IDX(q.band_x[b].i, q.band_x[b].j)] = tmp[b];
@@ -340,7 +351,7 @@ __device__ __forceinline__ void bc_store(const BcLines& s, float* a, int tid, in
   }
 }
 
-template <bool BAND, bool HEUN>
+template <bool BAND, bool HEUN, bool ADT>
 __global__ void __launch_bounds__(1024)
 k_bc2(const __grid_constant__ SolverParams q, float* ux_all, float* uy_all, const float* usx_all, const float* usy_all,
       float* uox_all, float* uoy_all) {
@@ -364,24 +375,25 @@ k_bc2(const __grid_constant__ SolverParams q, float* ux_all, float* uy_all, cons
   if (BAND) {
     // BDIM.updateUP blend on the body band (BDIM.pde:109-122), identical arithmetic to k_band_bc
     const float xi1_m = q.action_scale * q.sc.xi[2 * e], xi2_m = q.action_scale * q.sc.xi[2 * e + 1];
-    const float dphi1 = (2 * xi1_m * q.dt) / q.dRD, dphi2 = (2 * xi2_m * q.dt) / q.dRD;
+    const float dt = env_dt<ADT>(q, e);
+    const float dphi1 = (2 * xi1_m * dt) / q.dRD, dphi2 = (2 * xi2_m * dt) / q.dRD;
     for (int b = tid; b < q.nband_x; b += blockDim.x) {
       const BandFace f = q.band_x[b];
       const int k = IDX(f.i, f.j);
-      float R = ux[k], ub = ub_x(q, k, dphi1, dphi2);
+      float R = ux[k], ub = ub_x(q, k, dphi1, dphi2, dt);
       float v = f.del * R - ub * (f.del + (-1.f));
-      float duE = ux[k + P] - ub_x(q, k + P, dphi1, dphi2), duW = ux[k - P] - ub_x(q, k - P, dphi1, dphi2);
-      float duN = ux[k + 1] - ub_x(q, k + 1, dphi1, dphi2), duS = ux[k - 1] - ub_x(q, k - 1, dphi1, dphi2);
+      float duE = ux[k + P] - ub_x(q, k + P, dphi1, dphi2, dt), duW = ux[k - P] - ub_x(q, k - P, dphi1, dphi2, dt);
+      float duN = ux[k + 1] - ub_x(q, k + 1, dphi1, dphi2, dt), duS = ux[k - 1] - ub_x(q, k - 1, dphi1, dphi2, dt);
       float g = 0.5f * (f.wnx * (duE - duW) + f.wny * (duN - duS));       // VectorField.pde:50
       tmp[b] = v + f.del1 * g;
     }
     for (int b = tid; b < q.nband_y; b += blockDim.x) {
       const BandFace f = q.band_y[b];
       const int k = IDX(f.i, f.j);
-      float R = uy[k], ub = ub_y(q, k, dphi1, dphi2);
+      float R = uy[k], ub = ub_y(q, k, dphi1, dphi2, dt);
       float v = f.del * R - ub * (f.del + (-1.f));
-      float duE = uy[k + P] - ub_y(q, k + P, dphi1, dphi2), duW = uy[k - P] - ub_y(q, k - P, dphi1, dphi2);
-      float duN = uy[k + 1] - ub_y(q, k + 1, dphi1, dphi2), duS = uy[k - 1] - ub_y(q, k - 1, dphi1, dphi2);
+      float duE = uy[k + P] - ub_y(q, k + P, dphi1, dphi2, dt), duW = uy[k - P] - ub_y(q, k - P, dphi1, dphi2, dt);
+      float duN = uy[k + 1] - ub_y(q, k + 1, dphi1, dphi2, dt), duS = uy[k - 1] - ub_y(q, k - 1, dphi1, dphi2, dt);
       float g = 0.5f * (f.wnx * (duE - duW) + f.wny * (duN - duS));       // VectorField.pde:51
       tmp[q.nband_x + b] = v + f.del1 * g;
     }
@@ -438,11 +450,15 @@ __device__ __forceinline__ float apply_A(const float* x, const float* __restrict
 //   smooth(0): d = r*inv, d.setBC (ghost = clamped interior), x += d, r -= A d;  then restrict r.
 // `rin` is read with its 4x4 neighbourhood, so the new residual goes to a different buffer `rout`.
 // ------------------------------------------------------------------------------------------------
+// `co`: offset of this environment's coefficients (adaptive mode: e * L.stride; 0 for the shared static tables)
 template <bool LEVEL0>
 __device__ __forceinline__ void down_block(const DevLevel& L, const DevLevel& C, const float* __restrict__ rin,
                                            float* __restrict__ rout, float* __restrict__ x, float* __restrict__ rc,
-                                           int I, int J) {
+                                           int I, int J, size_t co) {
   const int P = L.P, n = L.n, m = L.m;
+  const float* __restrict__ Linv = L.inv + co;
+  const float* __restrict__ Llx = L.lx + co;
+  const float* __restrict__ Lly = L.ly + co;
   const int i0 = (I - 1) * 2 + 1, j0 = (J - 1) * 2 + 1;
   float d[4][4], rv[2][2];
 #pragma unroll
@@ -452,7 +468,7 @@ __device__ __forceinline__ void down_block(const DevLevel& L, const DevLevel& C,
       if ((a == 0 || a == 3) && (b == 0 || b == 3)) { d[a][b] = 0.f; continue; }
       int ci = min(max(i0 - 1 + a, 1), n - 2), cj = min(max(j0 - 1 + b, 1), m - 2);
       const float rr = rin[IDX(ci, cj)];
-      d[a][b] = rr * L.inv[IDX(ci, cj)];
+      d[a][b] = rr * Linv[IDX(ci, cj)];
       if (a >= 1 && a <= 2 && b >= 1 && b <= 2) rv[a - 1][b - 1] = rr;       // (the block's own cells are never clamped)
     }
   // the block's face coefficients, each loaded once: lx on rows i0 .. i0+2, ly on columns j0 .. j0+2; the diagonal is
@@ -461,11 +477,11 @@ __device__ __forceinline__ void down_block(const DevLevel& L, const DevLevel& C,
 #pragma unroll
   for (int a = 0; a < 3; a++)
 #pragma unroll
-    for (int b = 0; b < 2; b++) lxv[a][b] = L.lx[IDX(i0 + a, j0 + b)];
+    for (int b = 0; b < 2; b++) lxv[a][b] = Llx[IDX(i0 + a, j0 + b)];
 #pragma unroll
   for (int a = 0; a < 2; a++)
 #pragma unroll
-    for (int b = 0; b < 3; b++) lyv[a][b] = L.ly[IDX(i0 + a, j0 + b)];
+    for (int b = 0; b < 3; b++) lyv[a][b] = Lly[IDX(i0 + a, j0 + b)];
   float rn[2][2];
 #pragma unroll
   for (int a = 0; a < 2; a++)
@@ -493,6 +509,7 @@ __device__ __forceinline__ void down_block(const DevLevel& L, const DevLevel& C,
   rc[I * C.P + J] = rn[0][0] + rn[0][1] + rn[1][0] + rn[1][1];
 }
 
+template <bool ADT>
 __global__ void __launch_bounds__(256)
 k_mg_down0(const __grid_constant__ SolverParams q, const float* __restrict__ rin_all, float* __restrict__ rout_all) {
   const int e = blockIdx.z;
@@ -503,7 +520,7 @@ k_mg_down0(const __grid_constant__ SolverParams q, const float* __restrict__ rin
   const int I = blockIdx.y * blockDim.y + threadIdx.y + 1;
   if (I > L1.n - 2 || J > L1.m - 2) return;
   const size_t eo = (size_t)e * L0.stride;
-  down_block<true>(L0, L1, rin_all + eo, rout_all + eo, L0.x + eo, L1.r + (size_t)e * L1.stride, I, J);
+  down_block<true>(L0, L1, rin_all + eo, rout_all + eo, L0.x + eo, L1.r + (size_t)e * L1.stride, I, J, ADT ? eo : 0);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -518,6 +535,7 @@ k_mg_down0(const __grid_constant__ SolverParams q, const float* __restrict__ rin
 constexpr int kRdI = 8, kRdJ = 32;                       // coarse cells per CTA (one per thread)
 constexpr int kRdTI = 2 * kRdI + 2, kRdTJ = 2 * kRdJ + 2;
 
+template <bool ADT>
 __global__ void __launch_bounds__(kRdI * kRdJ)
 k_resid_down0(const __grid_constant__ SolverParams q, const float* __restrict__ ux_all, const float* __restrict__ uy_all,
               const float* __restrict__ pin_all, float* __restrict__ pout_all, float* __restrict__ rout_all, int which) {
@@ -535,6 +553,7 @@ k_resid_down0(const __grid_constant__ SolverParams q, const float* __restrict__ 
   const float* __restrict__ ux = ux_all + eo;
   const float* __restrict__ uy = uy_all + eo;
   const float* __restrict__ pin = pin_all + eo;
+  const size_t co = ADT ? eo : 0;                                       // this environment's coefficients
   const int I0 = blockIdx.y * kRdI + 1, J0 = blockIdx.x * kRdJ + 1;     // first coarse cell of the tile
   const int i0 = (I0 - 1) * 2 + 1, j0 = (J0 - 1) * 2 + 1;              // first fine cell
   // ---- phase 1: r and d = r*inv on the tile + halo, at clamped coordinates ----
@@ -543,9 +562,9 @@ k_resid_down0(const __grid_constant__ SolverParams q, const float* __restrict__ 
     const int i = min(max(i0 - 1 + a, 1), n - 2), j = min(max(j0 - 1 + b, 1), m - 2);
     const int k = IDX(i, j);
     const float sdiv = ux[k + P] - ux[k] + uy[k + 1] - uy[k];
-    const float rv = sdiv - apply_A(pin, L.lx, L.ly, L.diag, P, k);
+    const float rv = sdiv - apply_A(pin, L.lx + co, L.ly + co, L.diag + co, P, k);
     s_r[a][b] = rv;
-    s_d[a][b] = rv * L.inv[k];
+    s_d[a][b] = rv * L.inv[co + k];
   }
   __syncthreads();
   // ---- phase 2: smooth(0) increment and restriction for this thread's coarse cell ----
@@ -562,8 +581,8 @@ k_resid_down0(const __grid_constant__ SolverParams q, const float* __restrict__ 
     for (int b = 0; b < 2; b++) {
       const int i = fi + a, j = fj + b, k = IDX(i, j);
       const float dc = s_d[ta + a][tb + b];
-      const float Ad = dc * L.diag[k] + s_d[ta + a - 1][tb + b] * L.lx[k] + s_d[ta + a + 1][tb + b] * L.lx[k + P] +
-                       s_d[ta + a][tb + b - 1] * L.ly[k] + s_d[ta + a][tb + b + 1] * L.ly[k + 1];
+      const float Ad = dc * L.diag[co + k] + s_d[ta + a - 1][tb + b] * L.lx[co + k] + s_d[ta + a + 1][tb + b] * L.lx[co + k + P] +
+                       s_d[ta + a][tb + b - 1] * L.ly[co + k] + s_d[ta + a][tb + b + 1] * L.ly[co + k + 1];
       rn[a][b] = s_r[ta + a][tb + b] - Ad;
       rout[k] = rn[a][b];
       pout[k] = pin[k] + dc;
@@ -607,6 +626,7 @@ constexpr int kRmArrays = 7;      // staged arrays: p, ux, uy, lx, ly, diag, inv
 constexpr int kRmSeg = 208;       // floats per staged row segment: kRmWarps*kRmCols + 4 halo columns, 16-byte aligned ends
 constexpr size_t kRmSmem = (size_t)kRmDepth * kRmArrays * kRmSeg * 4 + 2 * kRmDepth * 8;
 
+template <bool ADT>
 __global__ void __launch_bounds__(32 * (kRmWarps + 1), kRmMinB)
 k_resid_down0_march(const __grid_constant__ SolverParams q, const float* __restrict__ ux_all, const float* __restrict__ uy_all,
                     const float* __restrict__ pin_all, float* __restrict__ pout_all, float* __restrict__ rout_all, int which) {
@@ -639,7 +659,8 @@ k_resid_down0_march(const __grid_constant__ SolverParams q, const float* __restr
   __syncthreads();
   if (warp == kRmWarps) {                                            // loader
     if (lane == 0) {
-      const float* src[kRmArrays] = {pin, ux_all + eo, uy_all + eo, L.lx, L.ly, L.diag, L.inv};
+      const size_t co = ADT ? eo : 0;                              // this environment's coefficients
+      const float* src[kRmArrays] = {pin, ux_all + eo, uy_all + eo, L.lx + co, L.ly + co, L.diag + co, L.inv + co};
       const unsigned bytes = (unsigned)(c1 - c0) * 4u;
       for (int qq = 0; qq < nq; qq++) {
         const int s = qq % kRmDepth;
@@ -753,11 +774,11 @@ k_resid_down0_march(const __grid_constant__ SolverParams q, const float* __restr
 // MG.pde:139-152), x += d, r -= A d (MG.pde:75-76,94-97).  Warps own rows, lanes own columns; four rows are in
 // flight per warp so the L2 round trips overlap.
 __device__ __forceinline__ void coarse_up_pass(const DevLevel& L, const DevLevel& C, float* __restrict__ r,
-                                               float* __restrict__ x, const float* __restrict__ xc) {
+                                               float* __restrict__ x, const float* __restrict__ xc, size_t co) {
   const int n = L.n, m = L.m, P = L.P, ni = n - 2, mj = m - 2, CP = C.P;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
-  const float* __restrict__ lx = L.lx;
-  const float* __restrict__ ly = L.ly;
+  const float* __restrict__ lx = L.lx + co;
+  const float* __restrict__ ly = L.ly + co;
   constexpr int U = RLFC_UP_ROWS;
   for (int j = 1 + lane; j <= mj; j += 32) {
     const int cj = (j - 1) / 2 + 1, cjm = (max(j - 1, 1) - 1) / 2 + 1, cjp = (min(j + 1, mj) - 1) / 2 + 1;
@@ -832,6 +853,7 @@ static size_t up0_smem(const SolverParams& q) {
   return sizeof(float) * (2 * (size_t)kUpRows * q.P + (size_t)(kUpRows / 2 + 2) * q.lev[1].P) + 16;
 }
 
+template <bool ADT>
 __global__ void __launch_bounds__(256)
 k_mg_up0_blk(const __grid_constant__ SolverParams q, const float* __restrict__ r_all) {
   using namespace rows_detail;
@@ -850,6 +872,8 @@ k_mg_up0_blk(const __grid_constant__ SolverParams q, const float* __restrict__ r
   unsigned long long* bar = reinterpret_cast<unsigned long long*>(s_xc + (kUpRows / 2 + 2) * CPc);
   const size_t eo = (size_t)e * L0.stride;
   float* __restrict__ x = L0.x + eo;
+  const float* __restrict__ L0lx = L0.lx + (ADT ? eo : 0);           // this environment's coefficients
+  const float* __restrict__ L0ly = L0.ly + (ADT ? eo : 0);
   if (threadIdx.x == 0) {
     mbar_init(bar, 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
@@ -875,11 +899,11 @@ k_mg_up0_blk(const __grid_constant__ SolverParams q, const float* __restrict__ r
 #pragma unroll
     for (int a = 0; a < 3; a++)
 #pragma unroll
-      for (int b = 0; b < 2; b++) lxv[a][b] = L0.lx[IDX(ig + a, j0 + b)];
+      for (int b = 0; b < 2; b++) lxv[a][b] = L0lx[IDX(ig + a, j0 + b)];
 #pragma unroll
     for (int a = 0; a < 2; a++)
 #pragma unroll
-      for (int b = 0; b < 3; b++) lyv[a][b] = L0.ly[IDX(ig + a, j0 + b)];
+      for (int b = 0; b < 3; b++) lyv[a][b] = L0ly[IDX(ig + a, j0 + b)];
 #pragma unroll
     for (int a = 0; a < 2; a++)
 #pragma unroll
@@ -950,6 +974,8 @@ __device__ __forceinline__ void rows_dispatch(const DevLevel& L, float* r, float
   }
 }
 
+// ADT (adaptive mode): every level's coefficients are the environment's own (the row tables pick env e's by blockIdx.x)
+template <bool ADT>
 __global__ void __launch_bounds__(kRowsThreads, 2)
 k_mg_coarse_rows(const __grid_constant__ SolverParams q, int first) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -974,7 +1000,7 @@ k_mg_coarse_rows(const __grid_constant__ SolverParams q, int first) {
     for (int J = 1 + lane; J <= ncj; J += 32)
 #pragma unroll 2
       for (int I = 1 + warp; I <= nci; I += nw)
-        down_block<false>(L, C, L.r + eo, L.d + eo, L.x + eo, C.r + (size_t)e * C.stride, I, J);
+        down_block<false>(L, C, L.r + eo, L.d + eo, L.x + eo, C.r + (size_t)e * C.stride, I, J, ADT ? eo : 0);
     __syncthreads();
     TICK("down", l);
   }
@@ -982,7 +1008,7 @@ k_mg_coarse_rows(const __grid_constant__ SolverParams q, int first) {
     const DevLevel& L = q.lev[last];
     const size_t eo = (size_t)e * L.stride;
     if (L.wave) wave_smooth<1>(L, L.r + eo, L.x + eo, L.d + eo, nullptr, 4);     // L.d is unused on the coarsest level
-    else if (q.tiny && tiny_level(L.n - 2, L.m - 2)) tiny_smooth<1>(L, L.r + eo, L.x + eo, smem_raw);
+    else if (q.tiny && tiny_level(L.n - 2, L.m - 2)) tiny_smooth<1>(L, L.r + eo, L.x + eo, smem_raw, ADT ? eo : 0);
     else rows_dispatch<1>(L, L.r + eo, L.x + eo, smem_raw);
     TICK("smooth", last);
   }
@@ -992,11 +1018,11 @@ k_mg_coarse_rows(const __grid_constant__ SolverParams q, int first) {
     const size_t eo = (size_t)e * L.stride;
     float* r = L.d + eo;
     float* x = L.x + eo;
-    coarse_up_pass(L, C, r, x, C.x + (size_t)e * C.stride);
+    coarse_up_pass(L, C, r, x, C.x + (size_t)e * C.stride, ADT ? eo : 0);
     __syncthreads();
     TICK("up", l);
     if (L.wave) wave_smooth<2>(L, r, x, L.r + eo, nullptr, 4);   // the level's restricted residual is dead after the down pass
-    else if (q.tiny && tiny_level(L.n - 2, L.m - 2)) tiny_smooth<2>(L, r, x, smem_raw);
+    else if (q.tiny && tiny_level(L.n - 2, L.m - 2)) tiny_smooth<2>(L, r, x, smem_raw, ADT ? eo : 0);
     else rows_dispatch<2>(L, r, x, smem_raw);
     TICK("smooth", l);
   }
@@ -1135,7 +1161,7 @@ __device__ __forceinline__ bool heun_zone(int i, int j4, int n, int m) {        
   return i < 2 || i > n - 3 || j4 < 4 || j4 >= 4 * ((m - 2) / 4);
 }
 
-template <bool HEUN>
+template <bool HEUN, bool ADT>
 __global__ void __launch_bounds__(256)
 k_project_shift(const __grid_constant__ SolverParams q, const float* __restrict__ pin_all, float* __restrict__ pout_all,
                 float* __restrict__ ux_all, float* __restrict__ uy_all, const float* __restrict__ usx_all,
@@ -1157,8 +1183,9 @@ k_project_shift(const __grid_constant__ SolverParams q, const float* __restrict_
   float4 uyv = *reinterpret_cast<const float4*>(uy_all + eo + k);
   float uxa[4] = {uxv.x, uxv.y, uxv.z, uxv.w}, uya[4] = {uyv.x, uyv.y, uyv.z, uyv.w};
   if (i >= 1 && i <= n - 2 && j4 <= m - 2) {
-    const float4 cxv = *reinterpret_cast<const float4*>(q.c_x + k);
-    const float4 cyv = *reinterpret_cast<const float4*>(q.c_y + k);
+    const size_t co = ADT ? eo : 0;                               // this environment's c (adaptive mode)
+    const float4 cxv = *reinterpret_cast<const float4*>(q.c_x + co + k);
+    const float4 cyv = *reinterpret_cast<const float4*>(q.c_y + co + k);
     const float cxa[4] = {cxv.x, cxv.y, cxv.z, cxv.w}, cya[4] = {cyv.x, cyv.y, cyv.z, cyv.w};
     float pw[4] = {0.f, 0.f, 0.f, 0.f};
     if (i >= 2) {
@@ -1214,6 +1241,7 @@ __device__ __forceinline__ float sample_linear(const float* a, int P, int i, int
   return s * (t * a[IDX(i + 1, j + 1)] + (1 - t) * a[IDX(i + 1, j)]) + (1 - s) * (t * a[IDX(i, j + 1)] + (1 - t) * a[IDX(i, j)]);
 }
 
+template <bool ADT>
 __global__ void __launch_bounds__(64)
 k_force(const __grid_constant__ SolverParams q, int accumulate) {
   const int e = blockIdx.x, tid = threadIdx.x, P = q.P;
@@ -1237,9 +1265,9 @@ k_force(const __grid_constant__ SolverParams q, int accumulate) {
     const float fx = pvx * -1, fy = pvy * -1;                                     // AFCCylinder.pde:58
     q.sc.force[2 * e] = fx;
     q.sc.force[2 * e + 1] = fy;
-    const float t = q.sc.t[e] + q.dt_over_res;                                    // AFCCylinder.pde:56
+    const float t = q.sc.t[e] + (ADT ? q.sc.dt[e] / q.resolution : q.dt_over_res);   // AFCCylinder.pde:56
     q.sc.t[e] = t;
-    q.sc.flow_t[e] += q.dt;                                                       // BDIM.update2: t += dt (BDIM.pde:106)
+    q.sc.flow_t[e] += env_dt<ADT>(q, e);                                          // BDIM.update2: t += dt (BDIM.pde:106)
     if (!isfinite(fx) || !isfinite(fy)) q.sc.non_finite[e] = 1;                   // diverged environment (sticky flag)
     if (accumulate && t >= q.episode_time) q.sc.frozen[e] = 1;                    // clientCFD.pde:36: no frame past Time
     if (accumulate && t > q.init_time) {                                          // clientCFD.pde:39-47
@@ -1268,11 +1296,14 @@ k_force(const __grid_constant__ SolverParams q, int accumulate) {
 // b = max(|ux|+|uy|) over the interior, started from cell [0][0].  A maximum does not depend on the order it is taken in,
 // so the reduction is parallel and still exact.  One CTA per environment (a diagnostic / adaptive-dt read-out, not on
 // the fixed-dt step path).
+// STEP (adaptive mode, start of a solver step): frozen environments are skipped and keep their dt.
+template <bool STEP>
 __global__ void __launch_bounds__(1024)
 k_check_cfl(const __grid_constant__ SolverParams q, const float* __restrict__ ux_all, const float* __restrict__ uy_all,
             float* __restrict__ dt_out) {
   __shared__ float wmax[32];
   const int e = blockIdx.x, P = q.P, ni = q.n - 2, mj = q.m - 2;
+  if (STEP && q.sc.frozen[e]) return;
   const float* ux = ux_all + (size_t)e * q.stride;
   const float* uy = uy_all + (size_t)e * q.stride;
   float b = fabsf(ux[0]) + fabsf(uy[0]);
@@ -1349,6 +1380,159 @@ __global__ void k_loopcond(cudaGraphConditionalHandle h, int* any_active) {
   }
 }
 
+// ------------------------------------------------------------------------------------------------
+// Adaptive dt (AFCCylinder.update, AFCCylinder.pde:63-84): the Poisson hierarchy of every environment not frozen, rebuilt
+// from its dt before the step.  The host formulas of geometry.cpp restated operation for operation (built with
+// --fmad=false like everything else), so the tables are bit-identical to what the host would build for that dt:
+//   level 0:  lx = del.x * (1*dt), ly = del.y * (1*dt) on all cells (BDIM.pde:59-61,81), then finish_level;
+//   finish_level (PoissonMatrix.pde:38-51): interior diag = -sumd, inv = -1/sumd where sumd > 1e-5, else 1; ghosts 0 / 1;
+//   coarsen (MG.pde:108-122): interior (a + b) * 0.5 of the fine pair, lx.setBC(btype 1, 0), ly.setBC(btype 2, 0);
+//   and each row-pipeline level's pre-skewed table (solver.h RowTab) from those arrays.
+// ------------------------------------------------------------------------------------------------
+// one float4 of a row table: entry `ent`, vector kv, lane ln (layout solver.h RowTab, host build in rlfc_api.cu)
+__device__ __forceinline__ float4 rowtab_vec(const RowTab& rt, int ent, int kv, int ln, int ni, int mj, int Pl,
+                                             const float* lx, const float* ly, const float* inv) {
+  const int C = rt.C, row = (ent - kTabFront) - ln, j0 = C * ln + 1;
+  float f[4];
+#pragma unroll
+  for (int u = 0; u < 4; u++) {
+    const int idx = 4 * kv + u;
+    float v = 0.f;
+    if (idx <= C) {                                   // ly of columns j0 .. j0 + C
+      const int j = j0 + idx;
+      if (row >= 1 && row <= ni && j <= mj + 1) v = ly[row * Pl + j];
+    } else if (idx <= 2 * C) {                        // -inv of columns j0 .. j0 + C - 1
+      const int j = j0 + idx - (C + 1);
+      if (row >= 1 && row <= ni && j <= mj) v = -inv[row * Pl + j];
+    } else if (idx <= 3 * C) {                        // lx of columns j0 .. j0 + C - 1
+      const int j = j0 + idx - (2 * C + 1);
+      if (row >= 1 && row <= ni + 1 && j <= mj) v = lx[row * Pl + j];
+    }
+    f[u] = v;
+  }
+  return make_float4(f[0], f[1], f[2], f[3]);
+}
+
+// level 0: lx, ly, diag, inv of every cell and the level's row table (if any), grid-wide; blockIdx.y = environment
+__global__ void __launch_bounds__(256)
+k_poisson_rebuild0(const __grid_constant__ SolverParams q) {
+  const int e = blockIdx.y;
+  if (q.sc.frozen[e]) return;
+  const DevLevel& L = q.lev[0];
+  const int n = L.n, m = L.m, P = L.P, ni = n - 2, mj = m - 2;
+  const float dt = q.sc.dt[e];
+  const size_t co = (size_t)e * L.stride;
+  float* lx = const_cast<float*>(L.lx) + co;
+  float* ly = const_cast<float*>(L.ly) + co;
+  float* diag = const_cast<float*>(L.diag) + co;
+  float* inv = const_cast<float*>(L.inv) + co;
+  const int cells = n * m;
+  const int tab = L.rt.entries ? L.rt.entries * L.rt.K * 32 : 0;
+  const float cdt = 1.f * dt;
+  for (int t = blockIdx.x * blockDim.x + threadIdx.x; t < cells + tab; t += gridDim.x * blockDim.x) {
+    if (t < cells) {
+      const int i = t / m, j = t - i * m, k = IDX(i, j);
+      lx[k] = q.del_x[k] * cdt;
+      ly[k] = q.del_y[k] * cdt;
+      float dg = 0.f, iv = 1.f;
+      if (i >= 1 && i <= ni && j >= 1 && j <= mj) {
+        const float sumd = q.del_x[k] * cdt + q.del_x[k + P] * cdt + q.del_y[k] * cdt + q.del_y[k + 1] * cdt;
+        dg = -sumd;
+        if (sumd > 1e-5f) iv = -1.f / sumd;
+      }
+      diag[k] = dg;
+      inv[k] = iv;
+    } else {
+      // the row table reads lx, ly, inv of other cells: recomputed here from del (the same operations, the same values)
+      const int u = t - cells, ln = u & 31, kv = (u >> 5) % L.rt.K, ent = (u >> 5) / L.rt.K;
+      const int C = L.rt.C, row = (ent - kTabFront) - ln, j0 = C * ln + 1;
+      float f[4];
+#pragma unroll
+      for (int w = 0; w < 4; w++) {
+        const int idx = 4 * kv + w;
+        float v = 0.f;
+        if (idx <= C) {
+          const int j = j0 + idx;
+          if (row >= 1 && row <= ni && j <= mj + 1) v = q.del_y[IDX(row, j)] * cdt;
+        } else if (idx <= 2 * C) {
+          const int j = j0 + idx - (C + 1);
+          if (row >= 1 && row <= ni && j <= mj) {
+            const int k = IDX(row, j);
+            const float sumd = q.del_x[k] * cdt + q.del_x[k + P] * cdt + q.del_y[k] * cdt + q.del_y[k + 1] * cdt;
+            v = -((sumd > 1e-5f) ? -1.f / sumd : 1.f);
+          }
+        } else if (idx <= 3 * C) {
+          const int j = j0 + idx - (2 * C + 1);
+          if (row >= 1 && row <= ni + 1 && j <= mj) v = q.del_x[IDX(row, j)] * cdt;
+        }
+        f[w] = v;
+      }
+      reinterpret_cast<float4*>(const_cast<float4*>(L.rt.T))[(size_t)e * tab + u] = make_float4(f[0], f[1], f[2], f[3]);
+    }
+  }
+}
+
+// levels 1 .. nlevels-1, one CTA per environment, level by level from the one above
+__global__ void __launch_bounds__(1024)
+k_poisson_rebuild_coarse(const __grid_constant__ SolverParams q) {
+  const int e = blockIdx.x, tid = threadIdx.x, nt = blockDim.x;
+  if (q.sc.frozen[e]) return;
+  for (int l = 1; l < q.nlevels; l++) {
+    const DevLevel& F = q.lev[l - 1];
+    const DevLevel& L = q.lev[l];
+    const int n = L.n, m = L.m, P = L.P, FP = F.P, ni = n - 2, mj = m - 2;
+    const size_t cf = (size_t)e * F.stride, co = (size_t)e * L.stride;
+    const float* flx = F.lx + cf;
+    const float* fly = F.ly + cf;
+    float* lx = const_cast<float*>(L.lx) + co;
+    float* ly = const_cast<float*>(L.ly) + co;
+    float* diag = const_cast<float*>(L.diag) + co;
+    float* inv = const_cast<float*>(L.inv) + co;
+    for (int t = tid; t < ni * mj; t += nt) {                  // interior: (a + b) * 0.5 of the fine pair
+      const int i = 1 + t / mj, j = 1 + t % mj;
+      const int kf = ((i - 1) * 2 + 1) * FP + (j - 1) * 2 + 1;
+      lx[IDX(i, j)] = (flx[kf] + flx[kf + 1]) * 0.5f;
+      ly[IDX(i, j)] = (fly[kf] + fly[kf + FP]) * 0.5f;
+    }
+    __syncthreads();
+    for (int j = tid; j < m; j += nt) {                        // Field.setBC, row statements (each column independent)
+      lx[IDX(0, j)] = lx[IDX(1, j)];
+      lx[IDX(n - 1, j)] = lx[IDX(n - 2, j)];
+      lx[IDX(1, j)] = 0.f; lx[IDX(n - 1, j)] = 0.f;           // btype 1, bval 0
+      ly[IDX(0, j)] = ly[IDX(1, j)];
+      ly[IDX(n - 1, j)] = ly[IDX(n - 2, j)];
+    }
+    __syncthreads();
+    for (int i = tid; i < n; i += nt) {                        // column statements (each row independent)
+      lx[IDX(i, 0)] = lx[IDX(i, 1)];
+      lx[IDX(i, m - 1)] = lx[IDX(i, m - 2)];
+      ly[IDX(i, 0)] = ly[IDX(i, 1)];
+      ly[IDX(i, m - 1)] = ly[IDX(i, m - 2)];
+      ly[IDX(i, 1)] = 0.f; ly[IDX(i, m - 1)] = 0.f;           // btype 2, bval 0
+    }
+    __syncthreads();
+    for (int t = tid; t < n * m; t += nt) {                    // finish_level
+      const int i = t / m, j = t - (t / m) * m, k = IDX(i, j);
+      float dg = 0.f, iv = 1.f;
+      if (i >= 1 && i <= ni && j >= 1 && j <= mj) {
+        const float sumd = lx[k] + lx[k + P] + ly[k] + ly[k + 1];
+        dg = -sumd;
+        if (sumd > 1e-5f) iv = -1.f / sumd;
+      }
+      diag[k] = dg;
+      inv[k] = iv;
+    }
+    __syncthreads();
+    if (L.rt.entries) {                                        // this level's row table
+      const int tab = L.rt.entries * L.rt.K * 32;
+      float4* T = const_cast<float4*>(L.rt.T) + (size_t)e * tab;
+      for (int u = tid; u < tab; u += nt)
+        T[u] = rowtab_vec(L.rt, (u >> 5) / L.rt.K, (u >> 5) % L.rt.K, u & 31, ni, mj, P, lx, ly, inv);
+    }
+    __syncthreads();
+  }
+}
+
 inline dim3 grid2d(int m, int n, int B, dim3 blk) { return dim3((m + blk.x - 1) / blk.x, (n + blk.y - 1) / blk.y, B); }
 
 }  // namespace
@@ -1362,27 +1546,35 @@ int launch_advdif(const SolverParams& q, const float* srcx, const float* srcy, c
   // rows a warp marches: 48 amortise the 4-row window best; a small batch (one wide domain) needs more warps instead
   const int rows = (long long)q.B * ni * mj < (8ll << 20) ? 16 : kAdvRows;
   dim3 grid((mj + kAdvCols - 1) / kAdvCols, ((ni + rows - 1) / rows + 3) / 4, q.B);
-  if (srcx == u0x && srcy == u0y)
-    k_advdif<true><<<grid, 128, 0, st>>>(srcx, srcy, u0x, u0y, dstx, dsty, q.n, q.m, q.P, q.stride, q.dt, q.nu, q.sc.frozen, q.slab_rank, q.slab_n, rows);
+  const bool pred = srcx == u0x && srcy == u0y;
+  if (q.adaptive) {
+    if (pred) k_advdif<true, true><<<grid, 128, 0, st>>>(srcx, srcy, u0x, u0y, dstx, dsty, q.n, q.m, q.P, q.stride, q.dt, q.nu, q.sc.frozen, q.slab_rank, q.slab_n, rows, q.sc.dt);
+    else k_advdif<false, true><<<grid, 128, 0, st>>>(srcx, srcy, u0x, u0y, dstx, dsty, q.n, q.m, q.P, q.stride, q.dt, q.nu, q.sc.frozen, q.slab_rank, q.slab_n, rows, q.sc.dt);
+  } else if (pred)
+    k_advdif<true, false><<<grid, 128, 0, st>>>(srcx, srcy, u0x, u0y, dstx, dsty, q.n, q.m, q.P, q.stride, q.dt, q.nu, q.sc.frozen, q.slab_rank, q.slab_n, rows, nullptr);
   else
-    k_advdif<false><<<grid, 128, 0, st>>>(srcx, srcy, u0x, u0y, dstx, dsty, q.n, q.m, q.P, q.stride, q.dt, q.nu, q.sc.frozen, q.slab_rank, q.slab_n, rows);
+    k_advdif<false, false><<<grid, 128, 0, st>>>(srcx, srcy, u0x, u0y, dstx, dsty, q.n, q.m, q.P, q.stride, q.dt, q.nu, q.sc.frozen, q.slab_rank, q.slab_n, rows, nullptr);
   return 1;
 }
 
 static size_t bc2_smem(const SolverParams& q) { return sizeof(float) * (2 * (3 * q.m + 2 * q.n) + q.nband_x + q.nband_y); }
 
-int launch_band_bc(const SolverParams& q, float* ux, float* uy, cudaStream_t st) {
-  if (q.fast_bc) k_bc2<true, false><<<q.B, 1024, bc2_smem(q), st>>>(q, ux, uy, nullptr, nullptr, nullptr, nullptr);
+template <bool ADT>
+static int launch_band_bc_t(const SolverParams& q, float* ux, float* uy, cudaStream_t st) {
+  if (q.fast_bc) k_bc2<true, false, ADT><<<q.B, 1024, bc2_smem(q), st>>>(q, ux, uy, nullptr, nullptr, nullptr, nullptr);
   else if (q.nband_x + q.nband_y > 4096) {             // a large band (single wide domain): blend grid-wide first
-    k_band_blend<<<dim3((q.nband_x + q.nband_y + 255) / 256, q.B), 256, 0, st>>>(q, ux, uy);
-    k_band_bc<true><<<q.B, 1024, sizeof(float) * q.m, st>>>(q, ux, uy);
+    k_band_blend<ADT><<<dim3((q.nband_x + q.nband_y + 255) / 256, q.B), 256, 0, st>>>(q, ux, uy);
+    k_band_bc<true, ADT><<<q.B, 1024, sizeof(float) * q.m, st>>>(q, ux, uy);
     return 2;
-  } else k_band_bc<false><<<q.B, 1024, sizeof(float) * q.m, st>>>(q, ux, uy);
+  } else k_band_bc<false, ADT><<<q.B, 1024, sizeof(float) * q.m, st>>>(q, ux, uy);
   return 1;
+}
+int launch_band_bc(const SolverParams& q, float* ux, float* uy, cudaStream_t st) {
+  return q.adaptive ? launch_band_bc_t<true>(q, ux, uy, st) : launch_band_bc_t<false>(q, ux, uy, st);
 }
 
 int launch_bc(const SolverParams& q, float* ux, float* uy, cudaStream_t st) {
-  if (q.fast_bc) k_bc2<false, false><<<q.B, 1024, bc2_smem(q), st>>>(q, ux, uy, nullptr, nullptr, nullptr, nullptr);
+  if (q.fast_bc) k_bc2<false, false, false><<<q.B, 1024, bc2_smem(q), st>>>(q, ux, uy, nullptr, nullptr, nullptr, nullptr);
   else k_bc<<<q.B, 512, sizeof(float) * q.m, st>>>(q, ux, uy);
   return 1;
 }
@@ -1393,19 +1585,22 @@ int launch_resid_down0(const SolverParams& q, const float* ux, const float* uy, 
   if (q.resid_march) {
     const int ni = q.n - 2, mj = q.m - 2;
     dim3 grid((mj + kRmWarps * kRmCols - 1) / (kRmWarps * kRmCols), (ni + kRmRows - 1) / kRmRows, q.B);
-    k_resid_down0_march<<<grid, 32 * (kRmWarps + 1), kRmSmem, st>>>(q, ux, uy, p_in, p_out, r_out, which);
+    if (q.adaptive) k_resid_down0_march<true><<<grid, 32 * (kRmWarps + 1), kRmSmem, st>>>(q, ux, uy, p_in, p_out, r_out, which);
+    else k_resid_down0_march<false><<<grid, 32 * (kRmWarps + 1), kRmSmem, st>>>(q, ux, uy, p_in, p_out, r_out, which);
     return 1;
   }
   dim3 blk(kRdJ, kRdI);
   dim3 grid((L1.m - 2 + kRdJ - 1) / kRdJ, (L1.n - 2 + kRdI - 1) / kRdI, q.B);
-  k_resid_down0<<<grid, blk, 0, st>>>(q, ux, uy, p_in, p_out, r_out, which);
+  if (q.adaptive) k_resid_down0<true><<<grid, blk, 0, st>>>(q, ux, uy, p_in, p_out, r_out, which);
+  else k_resid_down0<false><<<grid, blk, 0, st>>>(q, ux, uy, p_in, p_out, r_out, which);
   return 1;
 }
 
 int launch_project_shift(const SolverParams& q, const float* p_in, float* p_out, float* ux, float* uy, cudaStream_t st) {
   const int items = q.n * (q.P >> 2);
   dim3 grid((items + 255) / 256, q.B);
-  k_project_shift<false><<<grid, 256, 0, st>>>(q, p_in, p_out, ux, uy, nullptr, nullptr, nullptr, nullptr);
+  if (q.adaptive) k_project_shift<false, true><<<grid, 256, 0, st>>>(q, p_in, p_out, ux, uy, nullptr, nullptr, nullptr, nullptr);
+  else k_project_shift<false, false><<<grid, 256, 0, st>>>(q, p_in, p_out, ux, uy, nullptr, nullptr, nullptr, nullptr);
   return 1;
 }
 
@@ -1413,13 +1608,14 @@ int launch_project_shift_heun(const SolverParams& q, const float* p_in, float* p
                               const float* usy, float* uox, float* uoy, cudaStream_t st) {
   const int items = q.n * (q.P >> 2);
   dim3 grid((items + 255) / 256, q.B);
-  k_project_shift<true><<<grid, 256, 0, st>>>(q, p_in, p_out, ux, uy, usx, usy, uox, uoy);
+  if (q.adaptive) k_project_shift<true, true><<<grid, 256, 0, st>>>(q, p_in, p_out, ux, uy, usx, usy, uox, uoy);
+  else k_project_shift<true, false><<<grid, 256, 0, st>>>(q, p_in, p_out, ux, uy, usx, usy, uox, uoy);
   return 1;
 }
 
 int launch_bc_heun(const SolverParams& q, float* ux, float* uy, const float* usx, const float* usy, float* uox, float* uoy,
                    cudaStream_t st) {
-  k_bc2<false, true><<<q.B, 1024, bc2_smem(q), st>>>(q, ux, uy, usx, usy, uox, uoy);
+  k_bc2<false, true, false><<<q.B, 1024, bc2_smem(q), st>>>(q, ux, uy, usx, usy, uox, uoy);
   return 1;
 }
 
@@ -1436,7 +1632,8 @@ int launch_loopcond(const SolverParams& q, unsigned long long handle, cudaStream
 int launch_mg_down0(const SolverParams& q, const float* r_in, float* r_out, cudaStream_t st) {
   dim3 blk(32, 8);
   const DevLevel& L1 = q.lev[1];
-  k_mg_down0<<<grid2d(L1.m - 2, L1.n - 2, q.B, blk), blk, 0, st>>>(q, r_in, r_out);
+  if (q.adaptive) k_mg_down0<true><<<grid2d(L1.m - 2, L1.n - 2, q.B, blk), blk, 0, st>>>(q, r_in, r_out);
+  else k_mg_down0<false><<<grid2d(L1.m - 2, L1.n - 2, q.B, blk), blk, 0, st>>>(q, r_in, r_out);
   return 1;
 }
 
@@ -1461,15 +1658,23 @@ static cudaError_t set_smooth0_rows_attr(const SolverParams& q) {
 
 int configure_kernels(const SolverParams& q) {
   if (q.fast_bc) {
-    if (cudaFuncSetAttribute(k_bc2<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bc2_smem(q)) != cudaSuccess ||
-        cudaFuncSetAttribute(k_bc2<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bc2_smem(q)) != cudaSuccess ||
-        cudaFuncSetAttribute(k_bc2<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bc2_smem(q)) != cudaSuccess)
+    if (cudaFuncSetAttribute(k_bc2<true, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bc2_smem(q)) != cudaSuccess ||
+        cudaFuncSetAttribute(k_bc2<false, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bc2_smem(q)) != cudaSuccess ||
+        cudaFuncSetAttribute(k_bc2<false, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bc2_smem(q)) != cudaSuccess)
+      return -1;
+    if (q.adaptive &&
+        cudaFuncSetAttribute(k_bc2<true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bc2_smem(q)) != cudaSuccess)
       return -1;
   }
   if (cudaFuncSetAttribute(k_xsum_chain_blocks<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kXsBlocksSmem) != cudaSuccess ||
       cudaFuncSetAttribute(k_xsum_chain_blocks<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kXsBlocksSmem) != cudaSuccess) return -1;
-  if (cudaFuncSetAttribute(k_resid_down0_march, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kRmSmem) != cudaSuccess) return -1;
-  cudaError_t e3 = cudaFuncSetAttribute(k_mg_coarse_rows, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)coarse_rows_smem(q));
+  if (cudaFuncSetAttribute(k_resid_down0_march<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kRmSmem) != cudaSuccess) return -1;
+  cudaError_t e3 = cudaFuncSetAttribute(k_mg_coarse_rows<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)coarse_rows_smem(q));
+  if (q.adaptive) {
+    if (cudaFuncSetAttribute(k_resid_down0_march<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kRmSmem) != cudaSuccess) return -1;
+    if (e3 == cudaSuccess)
+      e3 = cudaFuncSetAttribute(k_mg_coarse_rows<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)coarse_rows_smem(q));
+  }
   if (q.chain_levels > 0 &&
       (cudaFuncSetAttribute(k_chain_sweeps3<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Chain3Smem)) != cudaSuccess ||
        cudaFuncSetAttribute(k_chain_sweeps3<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Chain3Smem)) != cudaSuccess))
@@ -1518,7 +1723,8 @@ int launch_chain_up(const SolverParams& q, int l, const float* r, cudaStream_t s
   return 1;
 }
 int launch_coarse_cta(const SolverParams& q, cudaStream_t st) {
-  k_mg_coarse_rows<<<q.B, kRowsThreads, coarse_rows_smem(q), st>>>(q, max(1, q.chain_levels));
+  if (q.adaptive) k_mg_coarse_rows<true><<<q.B, kRowsThreads, coarse_rows_smem(q), st>>>(q, max(1, q.chain_levels));
+  else k_mg_coarse_rows<false><<<q.B, kRowsThreads, coarse_rows_smem(q), st>>>(q, max(1, q.chain_levels));
   return 1;
 }
 
@@ -1545,7 +1751,10 @@ int launch_mg_coarse(const SolverParams& q, cudaStream_t st) {
 int launch_mg_up0(const SolverParams& q, float* r, cudaStream_t st) {
   dim3 blk(32, 8);
   if (q.lev[0].ch.on) return launch_chain_up(q, 0, r, st);
-  if (!q.lev[0].wave) k_mg_up0_blk<<<dim3((q.n - 2 + kUpRows - 1) / kUpRows, q.B), 256, up0_smem(q), st>>>(q, r);
+  if (!q.lev[0].wave) {
+    if (q.adaptive) k_mg_up0_blk<true><<<dim3((q.n - 2 + kUpRows - 1) / kUpRows, q.B), 256, up0_smem(q), st>>>(q, r);
+    else k_mg_up0_blk<false><<<dim3((q.n - 2 + kUpRows - 1) / kUpRows, q.B), 256, up0_smem(q), st>>>(q, r);
+  }
   else k_mg_up0<<<grid2d(q.m, q.n, q.B, blk), blk, 0, st>>>(q, r);
   return 1;
 }
@@ -1620,12 +1829,31 @@ int launch_heun(const SolverParams& q, const float* ucx, const float* ucy, const
 }
 
 int launch_force(const SolverParams& q, int accumulate, cudaStream_t st) {
-  k_force<<<q.B, 64, 0, st>>>(q, accumulate);
+  if (q.adaptive) k_force<true><<<q.B, 64, 0, st>>>(q, accumulate);
+  else k_force<false><<<q.B, 64, 0, st>>>(q, accumulate);
   return 1;
 }
 
 int launch_check_cfl(const SolverParams& q, const float* ux, const float* uy, float* d_dt, cudaStream_t st) {
-  k_check_cfl<<<q.B, 1024, 0, st>>>(q, ux, uy, d_dt);
+  k_check_cfl<false><<<q.B, 1024, 0, st>>>(q, ux, uy, d_dt);
+  return 1;
+}
+
+int launch_step_cfl(const SolverParams& q, const float* ux, const float* uy, cudaStream_t st) {
+  k_check_cfl<true><<<q.B, 1024, 0, st>>>(q, ux, uy, q.sc.dt);
+  return 1;
+}
+
+int launch_poisson_rebuild0(const SolverParams& q, cudaStream_t st) {
+  const DevLevel& L = q.lev[0];
+  const long long items = (long long)L.n * L.m + (long long)L.rt.entries * L.rt.K * 32;
+  const long long blocks = (items + 255) / 256;
+  k_poisson_rebuild0<<<dim3((unsigned)(blocks < 1024 ? blocks : 1024), q.B), 256, 0, st>>>(q);
+  return 1;
+}
+
+int launch_poisson_rebuild_coarse(const SolverParams& q, cudaStream_t st) {
+  k_poisson_rebuild_coarse<<<q.B, 1024, 0, st>>>(q);
   return 1;
 }
 

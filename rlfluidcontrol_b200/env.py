@@ -29,7 +29,7 @@ class Config(C.Structure):
         ("action_scale", C.c_float), ("substeps", C.c_int), ("init_time", C.c_float),
         ("episode_time", C.c_float), ("n_envs", C.c_int), ("device", C.c_int), ("exact", C.c_int),
         ("mg_max_iters", C.c_int), ("init_bdim_path", C.c_char_p), ("stream", C.c_void_p),
-        ("n_groups", C.c_int), ("n_devices", C.c_int),
+        ("n_groups", C.c_int), ("n_devices", C.c_int), ("adaptive_dt", C.c_int),
     ]
 
 
@@ -74,6 +74,8 @@ def load_library():
     L.rlfc_env_get_time.argtypes = [vp, fp]
     L.rlfc_env_get_mg_iters.argtypes = [vp, ip]
     L.rlfc_env_check_cfl.argtypes = [vp, fp]
+    L.rlfc_env_get_dt.argtypes = [vp, fp]
+    L.rlfc_env_get_coeffs.argtypes = [vp, C.c_int, C.c_char_p, C.c_int, fp, ip, ip]
     L.rlfc_env_running.argtypes = [vp, ip]
     L.rlfc_env_get_flags.argtypes = [vp, ip]
     L.rlfc_env_field_sum.argtypes = [vp, fp]
@@ -180,7 +182,11 @@ class AFCCylinderBatch:
         self._check(rc, "rlfc_env_step_device")
 
     def update2(self, actions=None, want_probes=False):
-        """One solver step (AFCCylinder.update2).  Returns force (n_envs, 2) [, probes (n_envs, 32)]."""
+        """One solver step.  Returns force (n_envs, 2) [, probes (n_envs, 32)].
+
+        The step is the one the handle was created for: AFCCylinder.update2 with the fixed dt = t_step*resolution
+        (adaptive_dt=0, the default), or AFCCylinder.update (adaptive_dt=1): every environment first takes
+        dt = min(CFL, 1) of its own velocity (`check_cfl`) and then the update2 statements with it (see `dt`)."""
         a = None if actions is None else np.ascontiguousarray(actions, dtype=np.float32).reshape(self.n_envs, 2)
         force = np.empty((self.n_envs, 2), np.float32)
         probes = np.empty((self.n_envs, NUM_PROBES), np.float32) if want_probes else None
@@ -219,6 +225,22 @@ class AFCCylinderBatch:
         dt = np.empty(self.n_envs, np.float32)
         self._check(self._L.rlfc_env_check_cfl(self._h, _fp(dt)), "rlfc_env_check_cfl")
         return dt
+
+    def dt(self):
+        """dt (grid units) of each environment's last solver step: t_step*resolution in fixed mode, the environment's
+        own CFL step in adaptive mode (t_step*resolution after create / reset, the checkpoint's after load_bdim)."""
+        dt = np.empty(self.n_envs, np.float32)
+        self._check(self._L.rlfc_env_get_dt(self._h, _fp(dt)), "rlfc_env_get_dt")
+        return dt
+
+    def get_coeffs(self, e, name, level=0):
+        """Environment e's Poisson coefficients as its last step used them ("lower.x", "lower.y", "inv", "diag" at any
+        level, "c.x", "c.y" at level 0), reference layout.  Fixed mode: the same as `get_static`."""
+        n, m = C.c_int(), C.c_int()
+        self._check(self._L.rlfc_env_get_coeffs(self._h, e, name.encode(), level, None, C.byref(n), C.byref(m)), "rlfc_env_get_coeffs")
+        out = np.empty((n.value, m.value), np.float32)
+        self._check(self._L.rlfc_env_get_coeffs(self._h, e, name.encode(), level, _fp(out), None, None), "rlfc_env_get_coeffs")
+        return out
 
     def running(self):
         """Environments that had not emitted their observation when the last RL-step round ended."""
