@@ -47,6 +47,14 @@ extern "C" {
 
 typedef struct rlfc_env rlfc_env;   /* opaque; owns all device + pinned-host memory */
 
+/* The per-environment arguments of the AFCCylinder constructor (AFCCylinder.pde:11-42).  resolution, x_lengths and
+   y_lengths fix the grid and stay handle-wide.  Valid sets: re >= 1, 0 < dR <= 1, gR >= 0, theta finite, t_step finite
+   and > 0, convex bodies (Body.pde:90-96), and no body-band face on rows 0, 1, n-2, n-1 or columns 0, 1, m-2, m-1. */
+typedef struct {
+  int   re;
+  float dR, gR, theta, t_step;
+} rlfc_env_params;
+
 typedef struct {
   /* defaults (rlfc_default_config) reproduce clientCFD.pde:5-14,94-96 and AFCCylinder.pde:4-7 */
   int   resolution;     /* 24   cells per main-cylinder diameter                     */
@@ -81,6 +89,13 @@ typedef struct {
                            (BDIM.checkCFL) and then runs the update2 statements with it.  The Poisson hierarchy
                            (c = del*dt and every coarse level) is rebuilt per environment on the device before each step.
                            Not available in slab mode or with the chained / wavefront smoothers (RLFC_EINVAL).       */
+  const rlfc_env_params *env_params;
+                        /* NULL (default) = every environment uses re, dR, gR, theta, t_step above.  Else n_envs entries:
+                           PER-ENVIRONMENT MODE, environment e is new AFCCylinder(resolution, env_params[e]..., x_lengths,
+                           y_lengths) with its own Reynolds number, control cylinders, fixed dt = t_step*resolution and
+                           Poisson hierarchy.  Combines with adaptive_dt 0 and 1; has the same restrictions as adaptive_dt
+                           (RLFC_EINVAL in slab mode and with the chained / wavefront smoothers).  The entries are copied
+                           and validated before any device call; an invalid one fails with RLFC_EINVAL.                */
 } rlfc_config;
 
 void rlfc_default_config(rlfc_config *cfg);
@@ -93,6 +108,16 @@ void rlfc_env_destroy(rlfc_env *env);
    are sketch globals in the reference and survive setUpNewSim (clientCFD.pde:11-13); pass
    reset_accumulators != 0 to also restore them to (16, 0, 0). */
 int  rlfc_env_reset(rlfc_env *env, const int *env_ids, int n, int reset_accumulators);
+
+/* setUpNewSim with new constructor arguments (clientCFD.pde:93-102), per-environment handles only (else RLFC_EINVAL):
+   environment env_ids[k] takes params[k], its geometry and Poisson hierarchy, and then exactly what rlfc_env_reset does.
+   Every set is validated and every geometry built before anything on the device changes: if one set is invalid
+   (RLFC_EINVAL) no environment changes.  The environments not listed are untouched. */
+int  rlfc_env_reset_params(rlfc_env *env, const int *env_ids, int n, const rlfc_env_params *params,
+                           int reset_accumulators);
+/* params[n_envs]: each environment's constructor arguments (the scalar config's for every environment of a handle
+   created without env_params). */
+int  rlfc_env_get_params(rlfc_env *env, rlfc_env_params *params);
 
 /* One RL step for every environment, with the cadence of clientCFD.draw() (clientCFD.pde:35-55).  All pointers are
    HOST memory.
@@ -154,24 +179,25 @@ int  rlfc_env_field_sum(rlfc_env *env, float *sums);
 int  rlfc_env_field_sum_stats(rlfc_env *env, int *stats);
 
 /* Text checkpoint of one environment in the BDIM.write format (readable by BDIM.resume).  Line 1 holds the dt: the
-   handle's fixed dt, or in adaptive mode the environment's own.  Loading requires the handle's dt in fixed mode and
-   accepts any positive dt in adaptive mode, where it becomes the environment's current dt. */
+   handle's fixed dt, or in adaptive or per-environment mode the environment's own.  Loading requires the environment's
+   fixed dt in fixed mode and accepts any positive dt in adaptive mode, where it becomes the environment's current dt. */
 int  rlfc_env_save_bdim(rlfc_env *env, int e, const char *path);
 int  rlfc_env_load_bdim(rlfc_env *env, int e, const char *path);
 
 /* BDIM.checkCFL (BDIM.pde:217-219, VectorField.CFL VectorField.pde:225-235) of every environment's current velocity:
-   dt[n_envs] = min(1 / (max_interior(|ux| + |uy|) + 3 nu), 1), the time step the reference's adaptive variant
+   dt[n_envs] = min(1 / (max_interior(|ux| + |uy|) + 3 nu[e]), 1), the time step the reference's adaptive variant
    AFCCylinder.update() (AFCCylinder.pde:63-84) would take next.  A handle created with adaptive_dt = 1 takes exactly
    that dt in its next solver step; with adaptive_dt = 0 the steps run the fixed dt of AFCCylinder.update2 (what
    clientCFD.pde calls). */
 int  rlfc_env_check_cfl(rlfc_env *env, float *dt);
-/* dt[n_envs]: the time step (grid units) of each environment's last solver step.  Fixed mode: t_step*resolution for every
-   environment.  Adaptive mode: the CFL step the environment took last; t_step*resolution after create / reset, the
-   checkpoint's dt after rlfc_env_load_bdim.  Synchronises the handle's stream. */
+/* dt[n_envs]: the time step (grid units) of each environment's last solver step.  Fixed mode: t_step*resolution (the
+   environment's own t_step in per-environment mode).  Adaptive mode: the CFL step the environment took last;
+   t_step*resolution after create / reset, the checkpoint's dt after rlfc_env_load_bdim.  Synchronises the handle's stream. */
 int  rlfc_env_get_dt(rlfc_env *env, float *dt);
 /* Environment e's Poisson coefficients as its last solver step used them, reference layout at the given MG level:
-   "lower.x", "lower.y", "inv", "diag" (any level), "c.x", "c.y" (level 0 only).  Fixed mode: the same fields as
-   rlfc_env_get_static.  Adaptive mode: the per-environment hierarchy built on the device from c = del*dt[e]. */
+   "lower.x", "lower.y", "inv", "diag" (any level), "c.x", "c.y", "del.x", "del.y" (level 0 only).  Fixed mode without
+   env_params: the same fields as rlfc_env_get_static.  Adaptive or per-environment mode: the environment's own hierarchy,
+   built on the device from c = del[e]*dt[e]. */
 int  rlfc_env_get_coeffs(rlfc_env *env, int e, const char *name, int level, float *out, int *n, int *m);
 
 /* Introspection. */

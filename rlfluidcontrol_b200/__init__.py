@@ -5,6 +5,6 @@ this package is the thin Python mirror of the reference's environment interface
 (clientLilypad/AFCCylinder.pde + clientCFD.pde) on top of it.  There is no CPU fallback: creating an
 environment without the CUDA library / a CUDA device raises.
 """
-from .env import AFCCylinderBatch, RlfcError, Config, load_library, library_path, default_init_state  # noqa: F401
+from .env import AFCCylinderBatch, RlfcError, Config, EnvParams, load_library, library_path, default_init_state  # noqa: F401
 
 __version__ = "0.1.0"

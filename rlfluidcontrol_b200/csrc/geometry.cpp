@@ -207,7 +207,7 @@ Sample resolve_sample(int n, int m, float x0, float y0) {
 
 }  // namespace
 
-int build_geometry(const rlfc_config& cfg, Geometry& g, std::string& err) {
+int build_geometry(const rlfc_config& cfg, Geometry& g, std::string& err, bool hierarchy) {
   if (cfg.resolution < 2 || cfg.x_lengths < 1 || cfg.y_lengths < 1 || cfg.re <= 0) {
     err = "resolution/x_lengths/y_lengths/re must be positive";
     return RLFC_EINVAL;
@@ -279,6 +279,7 @@ int build_geometry(const rlfc_config& cfg, Geometry& g, std::string& err) {
   // multigrid hierarchy (MG.pde:68-77,99-122): the finest level always restricts; a coarse level
   // recurses only while divisible
   g.levels.clear();
+  if (hierarchy) {
   {
     HostLevel L0;
     L0.n = n; L0.m = m; L0.lx = g.c_x; L0.ly = g.c_y;
@@ -298,6 +299,7 @@ int build_geometry(const rlfc_config& cfg, Geometry& g, std::string& err) {
       break;
     }
     g.levels.push_back(coarsen(F));
+  }
   }
 
   // MG.tol MG.pde:49-50: inner product of a field of 1e-4f with itself (float products, double sum)

@@ -49,8 +49,10 @@ struct Geometry {
   float mg_tol = 0;                 // MG.tol at level 0 (MG.pde:49-50)
 };
 
-// Builds the geometry for a configuration.  Returns 0 or an RLFC_E* code (err gets a message).
-int build_geometry(const rlfc_config& cfg, Geometry& g, std::string& err);
+// Builds the geometry for a configuration.  Returns 0 or an RLFC_E* code (err gets a message).  hierarchy = false leaves
+// `levels` empty (and skips the grid checks that come with it): the per-environment geometries, whose hierarchy the device
+// builds.
+int build_geometry(const rlfc_config& cfg, Geometry& g, std::string& err, bool hierarchy = true);
 
 // Checkpoint IO (BDIM.write / BDIM.resume text format BDIM.pde:226-251, and the .bdimb binary form).
 int read_checkpoint(const std::string& path, int n, int m, float& t, float& dt,

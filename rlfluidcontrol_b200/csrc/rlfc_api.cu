@@ -10,6 +10,7 @@
 #include <cmath>
 #include <cstring>
 #include <string>
+#include <thread>
 #include <vector>
 
 #include "../../include/rlfc.h"
@@ -43,6 +44,13 @@ struct rlfc_env {
   std::string init_path;
   Geometry geo;
   SolverParams sp{};
+  // per-environment constructor arguments (rlfc_config.env_params): env_mode = the handle was created with them
+  bool env_mode = false;
+  std::vector<rlfc_env_params> params;     // [B]
+  std::vector<float> dt0;                  // [B] t_step*resolution: sc.dt after a reset, the fixed dt without adaptive_dt
+  std::vector<float> h_nu, h_dRD;          // [B] host copies of sp.env_nu, sp.env_dRD
+  std::vector<int> h_nbx, h_nby;           // [B] host copies of sp.env_nband_x / y
+  int* d_skip = nullptr;                   // [B] mask of launch_poisson_rebuild* outside a step (1 = keep)
   int device = 0;
   cudaStream_t stream = nullptr;
   bool own_stream = false;
@@ -199,6 +207,140 @@ int broadcast_field(rlfc_env* E, float* batch, const float* one, const int* ids,
   return RLFC_OK;
 }
 
+// ---- per-environment geometry (rlfc_config.env_params) ----
+
+rlfc_env_params params_of(const rlfc_config& c) { return rlfc_env_params{c.re, c.dR, c.gR, c.theta, c.t_step}; }
+
+bool same_params(const rlfc_env_params& a, const rlfc_env_params& b) {
+  return a.re == b.re && !std::memcmp(&a.dR, &b.dR, 4) && !std::memcmp(&a.gR, &b.gR, 4) && !std::memcmp(&a.theta, &b.theta, 4) &&
+         !std::memcmp(&a.t_step, &b.t_step, 4);
+}
+
+// body band: faces where the BDIM blend is not the identity (del != 1, del1 != 0, or a control cylinder's velocity kernel
+// is non-zero)
+void band_lists(const Geometry& g, std::vector<BandFace>& bx, std::vector<BandFace>& by) {
+  bx.clear(); by.clear();
+  for (int i = 1; i < g.n - 1; i++)
+    for (int j = 1; j < g.m - 1; j++) {
+      size_t k = (size_t)i * g.m + j;
+      if (g.del_x[k] != 1.f || g.del1_x[k] != 0.f || g.w1_x[k] != 0.f || g.w2_x[k] != 0.f)
+        bx.push_back({i, j, g.del_x[k], g.del1_x[k], g.wnx_x[k], g.wny_x[k]});
+      if (g.del_y[k] != 1.f || g.del1_y[k] != 0.f || g.w1_y[k] != 0.f || g.w2_y[k] != 0.f)
+        by.push_back({i, j, g.del_y[k], g.del1_y[k], g.wnx_y[k], g.wny_y[k]});
+    }
+}
+
+// Band faces per component that one geometry slot holds.  Every band face lies within 3 cells of a body's surface (mu0 /
+// mu1 have half-width eps = 2, the union weights behind w1 / w2 vanish from distance 3 on), so inside one of the three
+// bodies' bounding boxes grown by 4 cells; the largest body has diameter D (dR <= 1), and a square of side D + 8 holds at
+// most (D + 9)^2 faces of one component.  With this capacity a new parameter set never needs more room.
+int band_capacity(const rlfc_config& c) {
+  const long long side = c.resolution + 9, cap = 3 * side * side;
+  const long long faces = (long long)c.x_lengths * c.resolution * c.y_lengths * c.resolution;
+  return (int)std::min(cap, faces);
+}
+
+struct EnvGeometry {
+  Geometry g;
+  std::vector<BandFace> bx, by;
+};
+
+// Validates the parameter sets p[0 .. n-1] for the grid of `cfg` and builds their geometries (without the hierarchy, which
+// the device builds): equal sets once, on a few threads.  set_of[k] = the entry of `out` that p[k] uses.  Touches no device.
+int build_env_geometries(const rlfc_config& cfg, const rlfc_env_params* p, int n, std::vector<EnvGeometry>& out,
+                         std::vector<int>& set_of, std::string& err) {
+  std::vector<int> uniq;                   // index into p of the first occurrence of each distinct set
+  set_of.assign(n, 0);
+  for (int k = 0; k < n; k++) {
+    const rlfc_env_params& q = p[k];
+    const std::string at = "env_params[" + std::to_string(k) + "]: ";
+    if (q.re < 1) { err = at + "re must be >= 1"; return RLFC_EINVAL; }
+    if (!(q.dR > 0 && q.dR <= 1)) { err = at + "dR must be in (0, 1]"; return RLFC_EINVAL; }
+    if (!(q.gR >= 0) || !std::isfinite(q.gR)) { err = at + "gR must be finite and >= 0"; return RLFC_EINVAL; }
+    if (!std::isfinite(q.theta)) { err = at + "theta must be finite"; return RLFC_EINVAL; }
+    if (!std::isfinite(q.t_step) || !(q.t_step > 0)) { err = at + "t_step must be finite and > 0"; return RLFC_EINVAL; }
+    size_t u = 0;
+    while (u < uniq.size() && !same_params(p[uniq[u]], q)) u++;
+    if (u == uniq.size()) uniq.push_back(k);
+    set_of[k] = (int)u;
+  }
+  out.clear();
+  out.resize(uniq.size());
+  std::vector<int> rc(uniq.size(), RLFC_OK);
+  std::vector<std::string> msg(uniq.size());
+  const int cap = band_capacity(cfg);
+  auto build = [&](size_t u) {
+    rlfc_config c = cfg;
+    const rlfc_env_params& q = p[uniq[u]];
+    c.re = q.re; c.dR = q.dR; c.gR = q.gR; c.theta = q.theta; c.t_step = q.t_step; c.env_params = nullptr;
+    EnvGeometry& G = out[u];
+    if ((rc[u] = build_geometry(c, G.g, msg[u], false))) return;
+    band_lists(G.g, G.bx, G.by);
+    // the two-phase setBC kernel (k_bc2) reads rows 1, n-2 and columns 1, m-2 before it blends the band
+    for (const auto* v : {&G.bx, &G.by})
+      for (const BandFace& f : *v)
+        if (f.i <= 1 || f.i >= G.g.n - 2 || f.j <= 1 || f.j >= G.g.m - 2) {
+          rc[u] = RLFC_EINVAL;
+          msg[u] = "the body band reaches the lines next to the domain boundary (face " + std::to_string(f.i) + ", " +
+                   std::to_string(f.j) + ")";
+          return;
+        }
+    if ((int)G.bx.size() > cap || (int)G.by.size() > cap) {
+      rc[u] = RLFC_EINVAL;
+      msg[u] = "body band larger than the slot capacity of " + std::to_string(cap) + " faces";
+    }
+  };
+  const int nth = (int)std::min<size_t>(uniq.size(), std::max(1u, std::min(8u, std::thread::hardware_concurrency())));
+  std::vector<std::thread> th;
+  for (int t = 1; t < nth; t++)
+    th.emplace_back([&, t] { for (size_t u = t; u < uniq.size(); u += nth) build(u); });
+  for (size_t u = 0; u < uniq.size(); u += std::max(nth, 1)) build(u);
+  for (auto& x : th) x.join();
+  for (size_t u = 0; u < uniq.size(); u++)
+    if (rc[u]) {
+      err = "env_params[" + std::to_string(uniq[u]) + "]: " + msg[u];
+      return RLFC_EINVAL;
+    }
+  return RLFC_OK;
+}
+
+// environment e's parameters: its geometry into slot e (del, the body-velocity basis, the band lists) and the host copies of
+// its scalars; the caller uploads the per-environment arrays and rebuilds the hierarchy
+int upload_env_geometry(rlfc_env* E, int e, const rlfc_env_params& p, const EnvGeometry& G) {
+  SolverParams& sp = E->sp;
+  const Geometry& g = G.g;
+  const std::vector<float>* src[10] = {&g.del_x, &g.del_y, &g.w1_x, &g.w2_x, &g.ry1_x, &g.ry2_x, &g.w1_y, &g.w2_y, &g.rx1_y, &g.rx2_y};
+  const float* dst[10] = {sp.del_x, sp.del_y, sp.w1_x, sp.w2_x, sp.ry1_x, sp.ry2_x, sp.w1_y, sp.w2_y, sp.rx1_y, sp.rx2_y};
+  for (int f = 0; f < 10; f++)
+    CU(cudaMemcpy2DAsync(const_cast<float*>(dst[f]) + (size_t)e * sp.stride, sp.P * sizeof(float), src[f]->data(),
+                         g.m * sizeof(float), g.m * sizeof(float), g.n, cudaMemcpyHostToDevice, E->stream));
+  if (!G.bx.empty())
+    CU(cudaMemcpyAsync(const_cast<BandFace*>(sp.band_x) + (size_t)e * sp.nband_x, G.bx.data(), G.bx.size() * sizeof(BandFace),
+                       cudaMemcpyHostToDevice, E->stream));
+  if (!G.by.empty())
+    CU(cudaMemcpyAsync(const_cast<BandFace*>(sp.band_y) + (size_t)e * sp.nband_y, G.by.data(), G.by.size() * sizeof(BandFace),
+                       cudaMemcpyHostToDevice, E->stream));
+  E->params[e] = p;
+  E->dt0[e] = g.dt;
+  E->h_nu[e] = g.nu;
+  E->h_dRD[e] = g.dR * g.D;
+  E->h_nbx[e] = (int)G.bx.size();
+  E->h_nby[e] = (int)G.by.size();
+  return RLFC_OK;
+}
+
+// the host copies of the per-environment scalars -> sp.env_*
+int upload_env_scalars(rlfc_env* E) {
+  SolverParams& sp = E->sp;
+  const size_t B = E->params.size();
+  CU(cudaMemcpyAsync(const_cast<float*>(sp.env_nu), E->h_nu.data(), B * sizeof(float), cudaMemcpyHostToDevice, E->stream));
+  CU(cudaMemcpyAsync(const_cast<float*>(sp.env_dRD), E->h_dRD.data(), B * sizeof(float), cudaMemcpyHostToDevice, E->stream));
+  CU(cudaMemcpyAsync(const_cast<int*>(sp.env_nband_x), E->h_nbx.data(), B * sizeof(int), cudaMemcpyHostToDevice, E->stream));
+  CU(cudaMemcpyAsync(const_cast<int*>(sp.env_nband_y), E->h_nby.data(), B * sizeof(int), cudaMemcpyHostToDevice, E->stream));
+  CU(cudaStreamSynchronize(E->stream));
+  return RLFC_OK;
+}
+
 // ---- one MG-projected half step on velocity buffer U (BDIM.updateUP tail + VectorField.project) ----
 // The floats-per-interior-cell figures are each kernel's ALGORITHMIC traffic per env (SURVEY 8d
 // convention: per-env arrays only, one read per input and one write per output).
@@ -276,8 +418,8 @@ int solver_step_eager(rlfc_env* E, Group& G, int accumulate) {
   if (sp.adaptive) {
     // AFCCylinder.update (AFCCylinder.pde:63-84): dt = flow.checkCFL(), then the Poisson hierarchy of c = del*dt
     E->run("k_check_cfl", 2, [&] { return launch_step_cfl(sp, G.uAx, G.uAy, st); }, st);
-    E->run("k_poisson_rebuild0", 0, [&] { return launch_poisson_rebuild0(sp, st); }, st);
-    E->run("k_poisson_rebuild_coarse", 0, [&] { return launch_poisson_rebuild_coarse(sp, st); }, st);
+    E->run("k_poisson_rebuild0", 0, [&] { return launch_poisson_rebuild0(sp, sp.sc.frozen, st); }, st);
+    E->run("k_poisson_rebuild_coarse", 0, [&] { return launch_poisson_rebuild_coarse(sp, sp.sc.frozen, st); }, st);
   }
   // predictor BDIM.update(): u0 = u (buffer A), F = AdvDif(u) -> B, updateUP
   E->run("k_advdif", 5, [&] { return launch_advdif(sp, G.uAx, G.uAy, G.uAx, G.uAy, G.uBx, G.uBy, st); }, st);
@@ -357,8 +499,8 @@ int build_step_graph(rlfc_env* E, Group& G, int accumulate) {
   CU(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
   if (G.sp.adaptive) {   // dt = flow.checkCFL() and the hierarchy of c = del*dt, on the device (dt never goes to the host)
     n_outer += launch_step_cfl(G.sp, G.uAx, G.uAy, st);
-    n_outer += launch_poisson_rebuild0(G.sp, st);
-    n_outer += launch_poisson_rebuild_coarse(G.sp, st);
+    n_outer += launch_poisson_rebuild0(G.sp, G.sp.sc.frozen, st);
+    n_outer += launch_poisson_rebuild_coarse(G.sp, G.sp.sc.frozen, st);
   }
   int rc = capture_half_step(E, G, st, G.uAx, G.uAy, G.uAx, G.uAy, G.uBx, G.uBy, 0, &n_outer);
   if (!rc) rc = capture_half_step(E, G, st, G.uBx, G.uBy, G.uAx, G.uAy, G.uCx, G.uCy, 1, &n_outer);
@@ -615,6 +757,14 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
   if (cfg->substeps < 1 || cfg->mg_max_iters < 1) return fail(RLFC_EINVAL, "substeps and mg_max_iters must be >= 1");
   if (cfg->adaptive_dt != 0 && cfg->adaptive_dt != 1) return fail(RLFC_EINVAL, "adaptive_dt must be 0 or 1");
   if (cfg->adaptive_dt && cfg->n_devices > 1) return fail(RLFC_EINVAL, "adaptive_dt is not available in slab mode (n_devices > 1)");
+  // per-environment parameters: every set validated and its geometry built before any device call
+  std::vector<EnvGeometry> env_geo;
+  std::vector<int> env_set;
+  if (cfg->env_params) {
+    if (cfg->n_devices > 1) return fail(RLFC_EINVAL, "env_params is not available in slab mode (n_devices > 1)");
+    std::string err;
+    if (build_env_geometries(*cfg, cfg->env_params, cfg->n_envs, env_geo, env_set, err)) return fail(RLFC_EINVAL, err);
+  }
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
     return fail(RLFC_ENODEV, "no CUDA device available (rlfc has no CPU fallback)");
@@ -622,6 +772,8 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
   E->cfg = *cfg;
   if (cfg->init_bdim_path) E->init_path = cfg->init_bdim_path;
   E->cfg.init_bdim_path = nullptr;
+  E->env_mode = cfg->env_params != nullptr;
+  E->cfg.env_params = nullptr;              // (copied into E->params below)
   int rc = RLFC_OK;
   auto bail = [&](int code) { rlfc_env_destroy(E); return code; };
 
@@ -679,7 +831,10 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
   const bool force_chain = std::getenv("RLFC_SMOOTHER") && std::string(std::getenv("RLFC_SMOOTHER")) == "chain";
   const bool slab = E->cfg.n_devices > 1;   // slab mode: level 0 always runs the chained smoother (its sweeps span devices)
   const bool adaptive = cfg->adaptive_dt == 1;
+  const bool env_mode = E->env_mode;
+  const bool per_env = adaptive || env_mode;   // per-environment dt, hierarchy and geometry slots
   sp.adaptive = adaptive ? 1 : 0;
+  sp.per_env = per_env ? 1 : 0;
   int chain_min_cols = 33;            // RLFC_CHAIN_MIN_COLS: coarse levels at least this wide follow a chained level 0 (levels of
                                       // at most 32 columns are faster in the one-CTA kernel's single-warp smoother: 521 -> 528 steps/s)
   if (const char* ev = std::getenv("RLFC_CHAIN_MIN_COLS")) chain_min_cols = std::max(1, std::atoi(ev));
@@ -691,10 +846,19 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
 
 #define TRY(x) do { rc = (x); if (rc) return bail(rc); } while (0)
   // static level-0 fields
-  if (!adaptive) {
+  if (!per_env) {
     TRY(upload_static(E, g.c_x, g.n, g.m, sp.P, &sp.c_x));
     TRY(upload_static(E, g.c_y, g.n, g.m, sp.P, &sp.c_y));
   }
+  if (env_mode) {
+    // one geometry slot per environment: del and the body-velocity basis at e * stride (filled by upload_env_geometry)
+    const float** slot[10] = {&sp.del_x, &sp.del_y, &sp.w1_x, &sp.w2_x, &sp.ry1_x, &sp.ry2_x, &sp.w1_y, &sp.w2_y, &sp.rx1_y, &sp.rx2_y};
+    for (const float** f : slot) {
+      float* d = nullptr;
+      TRY(E->dmalloc(&d, sp.stride * B));
+      *f = d;
+    }
+  } else {
   TRY(upload_static(E, g.w1_x, g.n, g.m, sp.P, &sp.w1_x));
   TRY(upload_static(E, g.w2_x, g.n, g.m, sp.P, &sp.w2_x));
   TRY(upload_static(E, g.ry1_x, g.n, g.m, sp.P, &sp.ry1_x));
@@ -703,13 +867,14 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
   TRY(upload_static(E, g.w2_y, g.n, g.m, sp.P, &sp.w2_y));
   TRY(upload_static(E, g.rx1_y, g.n, g.m, sp.P, &sp.rx1_y));
   TRY(upload_static(E, g.rx2_y, g.n, g.m, sp.P, &sp.rx2_y));
+  }
   // multigrid hierarchy
   for (int l = 0; l < sp.nlevels; l++) {
     const HostLevel& H = g.levels[l];
     DevLevel& L = sp.lev[l];
     L.n = H.n; L.m = H.m; L.P = round_up(H.m, 8);
     L.stride = (size_t)round_up(L.n * L.P, 32);
-    if (adaptive) {
+    if (per_env) {
       // one copy per environment at the level's stride, rebuilt on the device from each environment's dt
       float* a[4] = {nullptr, nullptr, nullptr, nullptr};
       for (int k = 0; k < 4; k++) TRY(E->dmalloc(&a[k], L.stride * B));
@@ -761,7 +926,7 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
         sp.chain_levels = l + 1;
       }
       L.rt.C = C; L.rt.K = K; L.rt.entries = 0; L.rt.copies = 1; L.rt.T = nullptr;
-      if (adaptive && !L.wave && !L.ch.on) {
+      if (per_env && !L.wave && !L.ch.on) {
         // one table per environment (k_poisson_rebuild*); a view of the batch sets `copies` to its B, so the smoother's
         // CTA e (= environment e of the view) reads table e
         float4* T = nullptr;
@@ -810,45 +975,78 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
     L.w = nullptr;
     if (l == 0 && L.wave) TRY(E->dmalloc(&L.w, L.stride * B));
   }
-  if (adaptive) {
+  if (per_env) {
     // the per-environment hierarchy exists for the row-pipeline and single-warp smoothers only
+    const std::string what = adaptive ? "adaptive_dt" : "env_params";
     if (sp.chain_levels > 0)
-      return bail(fail(RLFC_EINVAL, "adaptive_dt is not available with the chained strip smoother (a level too wide for the "
-                                    "row pipeline, or RLFC_SMOOTHER=chain)"));
+      return bail(fail(RLFC_EINVAL, what + " is not available with the chained strip smoother (a level too wide for the "
+                                           "row pipeline, or RLFC_SMOOTHER=chain)"));
     for (int l = 0; l < sp.nlevels; l++)
       if (sp.lev[l].wave)
-        return bail(fail(RLFC_EINVAL, "adaptive_dt is not available with the wavefront smoother (RLFC_SMOOTHER=wave, or a "
-                                      "coarsest level wider than the row pipeline)"));
-    TRY(upload_static(E, g.del_x, g.n, g.m, sp.P, &sp.del_x));
-    TRY(upload_static(E, g.del_y, g.n, g.m, sp.P, &sp.del_y));
+        return bail(fail(RLFC_EINVAL, what + " is not available with the wavefront smoother (RLFC_SMOOTHER=wave, or a "
+                                             "coarsest level wider than the row pipeline)"));
+    if (!env_mode) {   // one geometry slot, shared by every environment
+      TRY(upload_static(E, g.del_x, g.n, g.m, sp.P, &sp.del_x));
+      TRY(upload_static(E, g.del_y, g.n, g.m, sp.P, &sp.del_y));
+    }
     sp.c_x = sp.lev[0].lx; sp.c_y = sp.lev[0].ly;   // c = del*(1*dt) is level 0's lower (geometry.cpp)
   }
-  // body band: faces where the BDIM blend is not the identity (del != 1, del1 != 0, or a control
-  // cylinder's velocity kernel is non-zero)
   {
     std::vector<BandFace> bx, by;
-    for (int i = 1; i < g.n - 1; i++)
-      for (int j = 1; j < g.m - 1; j++) {
-        size_t k = (size_t)i * g.m + j;
-        if (g.del_x[k] != 1.f || g.del1_x[k] != 0.f || g.w1_x[k] != 0.f || g.w2_x[k] != 0.f)
-          bx.push_back({i, j, g.del_x[k], g.del1_x[k], g.wnx_x[k], g.wny_x[k]});
-        if (g.del_y[k] != 1.f || g.del1_y[k] != 0.f || g.w1_y[k] != 0.f || g.w2_y[k] != 0.f)
-          by.push_back({i, j, g.del_y[k], g.del1_y[k], g.wnx_y[k], g.wny_y[k]});
-      }
+    band_lists(g, bx, by);
     sp.nband_x = (int)bx.size(); sp.nband_y = (int)by.size();
+    if (env_mode) sp.nband_x = sp.nband_y = band_capacity(E->cfg);   // every slot's lists at this capacity
     // the two-phase setBC kernel fetches rows 1, n-2 and columns 1, m-2 before the band is blended: no band face may
     // sit on them, and the shared-memory image of the lines (+ the blended band) must fit one CTA.  The kernel strides over
     // longer lines too, but ONE CTA blending the band of a 2048x1024 domain is slower than the grid-wide k_band_blend + the
     // literal kernels (measured: 122 vs 52 us), so large grids keep those.
     sp.fast_bc = (g.n <= 1024 && g.m <= 1024 &&
                   sizeof(float) * (2 * (3 * (size_t)g.m + 2 * (size_t)g.n) + bx.size() + by.size()) <= 200 * 1024) ? 1 : 0;
-    for (const auto* v : {&bx, &by})
-      for (const BandFace& f : *v)
-        if (f.i <= 1 || f.i >= g.n - 2 || f.j <= 1 || f.j >= g.m - 2) sp.fast_bc = 0;
+    // (per-environment sets are validated to keep the band off those lines; the scalar config's band is not used then)
+    if (!env_mode)
+      for (const auto* v : {&bx, &by})
+        for (const BandFace& f : *v)
+          if (f.i <= 1 || f.i >= g.n - 2 || f.j <= 1 || f.j >= g.m - 2) sp.fast_bc = 0;
+    if (env_mode)
+      sp.fast_bc = (g.n <= 1024 && g.m <= 1024 &&
+                    sizeof(float) * (2 * (3 * (size_t)g.m + 2 * (size_t)g.n) + (size_t)sp.nband_x + sp.nband_y) <= 200 * 1024) ? 1 : 0;
     if (const char* ev = std::getenv("RLFC_FAST_BC")) sp.fast_bc = sp.fast_bc && std::atoi(ev) != 0;
-    TRY(upload_vec(E, bx, &sp.band_x));
-    TRY(upload_vec(E, by, &sp.band_y));
-    TRY(E->dmalloc(&sp.band_tmp, (size_t)B * (bx.size() + by.size())));
+    if (env_mode) {
+      BandFace* d = nullptr;
+      TRY(E->dmalloc(&d, (size_t)sp.nband_x * B)); sp.band_x = d;
+      TRY(E->dmalloc(&d, (size_t)sp.nband_y * B)); sp.band_y = d;
+    } else {
+      TRY(upload_vec(E, bx, &sp.band_x));
+      TRY(upload_vec(E, by, &sp.band_y));
+    }
+    TRY(E->dmalloc(&sp.band_tmp, (size_t)B * (sp.nband_x + sp.nband_y)));
+  }
+  // per-environment parameters: the scalar config's for every environment unless env_params gives them
+  E->params.assign(B, params_of(E->cfg));
+  E->dt0.assign(B, g.dt);
+  E->h_nu.assign(B, g.nu); E->h_dRD.assign(B, g.dR * g.D);
+  E->h_nbx.assign(B, sp.nband_x); E->h_nby.assign(B, sp.nband_y);
+  if (per_env) {
+    std::vector<int> slot(B, 0);
+    if (env_mode) {
+      for (int e = 0; e < B; e++) {
+        slot[e] = e;
+        TRY(upload_env_geometry(E, e, cfg->env_params[e], env_geo[env_set[e]]));
+      }
+      if (cudaStreamSynchronize(E->stream) != cudaSuccess) return bail(fail(RLFC_ECUDA, "geometry upload failed"));
+      env_geo.clear();
+    }
+    int* d = nullptr;
+    TRY(E->dmalloc(&d, B)); sp.env_slot = d;
+    TRY(E->dmalloc(&d, B)); sp.env_nband_x = d;
+    TRY(E->dmalloc(&d, B)); sp.env_nband_y = d;
+    TRY(E->dmalloc(&E->d_skip, B));
+    float* f = nullptr;
+    TRY(E->dmalloc(&f, B)); sp.env_nu = f;
+    TRY(E->dmalloc(&f, B)); sp.env_dRD = f;
+    if (cudaMemcpyAsync(d = const_cast<int*>(sp.env_slot), slot.data(), B * sizeof(int), cudaMemcpyHostToDevice, E->stream) != cudaSuccess)
+      return bail(fail(RLFC_ECUDA, "slot table upload failed"));
+    TRY(upload_env_scalars(E));
   }
   {
     std::vector<ForcePt> fp;
@@ -978,12 +1176,15 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
       const size_t o = (size_t)e0 * v.lev[l].stride;
       v.lev[l].r += o; v.lev[l].x += o; v.lev[l].d += o;
       if (v.lev[l].w) v.lev[l].w += o;
-      if (v.adaptive) {
+      if (v.per_env) {
         v.lev[l].lx += o; v.lev[l].ly += o; v.lev[l].inv += o; v.lev[l].diag += o;
         if (v.lev[l].rt.T) { v.lev[l].rt.T += (size_t)e0 * v.lev[l].rt.entries * v.lev[l].rt.K * 32; v.lev[l].rt.copies = G.B; }
       }
     }
-    if (v.adaptive) { v.c_x = v.lev[0].lx; v.c_y = v.lev[0].ly; v.sc.dt += e0; }
+    if (v.per_env) {
+      v.c_x = v.lev[0].lx; v.c_y = v.lev[0].ly; v.sc.dt += e0;
+      v.env_slot += e0; v.env_nu += e0; v.env_dRD += e0; v.env_nband_x += e0; v.env_nband_y += e0;
+    }
     for (int l = 0; l < v.chain_levels; l++) {
       ChainLevel& ch = v.lev[l].ch;
       ch.rsk += (size_t)e0 * ch.sk_stride;
@@ -1090,9 +1291,9 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
 
   if ((rc = load_initial_state(E))) return bail(rc);
   if ((rc = rlfc_env_reset(E, nullptr, B, 1))) return bail(rc);
-  if (adaptive) {   // the hierarchy of the initial dt, so that rlfc_env_get_coeffs is defined before the first step
-    E->launches += launch_poisson_rebuild0(E->whole.sp, E->stream);
-    E->launches += launch_poisson_rebuild_coarse(E->whole.sp, E->stream);
+  if (per_env) {   // the hierarchy of the initial dt (d_skip: all zero)
+    E->launches += launch_poisson_rebuild0(E->whole.sp, E->d_skip, E->stream);
+    E->launches += launch_poisson_rebuild_coarse(E->whole.sp, E->d_skip, E->stream);
     if (cudaGetLastError() != cudaSuccess) return bail(fail(RLFC_ECUDA, "initial Poisson hierarchy build failed"));
   }
   if (cudaStreamSynchronize(E->stream) != cudaSuccess) return bail(fail(RLFC_ECUDA, "initialisation failed"));
@@ -1121,7 +1322,7 @@ int rlfc_env_reset(rlfc_env* E, const int* env_ids, int n, int reset_accumulator
     CU(cudaMemsetAsync(sp.sc.force + 2 * e, 0, 2 * sizeof(float), E->stream));
     CU(cudaMemsetAsync(sp.sc.frozen + e, 0, sizeof(int), E->stream));
     CU(cudaMemsetAsync(sp.sc.non_finite + e, 0, sizeof(int), E->stream));
-    CU(cudaMemcpyAsync(sp.sc.dt + e, &E->geo.dt, sizeof(float), cudaMemcpyHostToDevice, E->stream));   // t_step*resolution
+    CU(cudaMemcpyAsync(sp.sc.dt + e, &E->dt0[e], sizeof(float), cudaMemcpyHostToDevice, E->stream));   // t_step*resolution
     if (reset_accumulators) {
       CU(cudaMemcpyAsync(sp.sc.callLearn + e, &one16, sizeof(int), cudaMemcpyHostToDevice, E->stream));
       CU(cudaMemsetAsync(sp.sc.Cd + e, 0, sizeof(float), E->stream));
@@ -1130,6 +1331,47 @@ int rlfc_env_reset(rlfc_env* E, const int* env_ids, int n, int reset_accumulator
     }
   }
   CU(cudaStreamSynchronize(E->stream));
+  return RLFC_OK;
+}
+
+int rlfc_env_reset_params(rlfc_env* E, const int* env_ids, int n, const rlfc_env_params* params, int reset_accumulators) {
+  if (!E) return fail(RLFC_EINVAL, "null handle");
+  if (!E->env_mode) return fail(RLFC_EINVAL, "rlfc_env_reset_params needs a handle created with env_params");
+  const int B = E->sp.B;
+  if (n < 0 || n > B) return fail(RLFC_EINVAL, "bad env count");
+  if (n > 0 && (!env_ids || !params)) return fail(RLFC_EINVAL, "null argument");
+  std::vector<char> listed(B, 0);
+  for (int k = 0; k < n; k++) {
+    if (env_ids[k] < 0 || env_ids[k] >= B) return fail(RLFC_EINVAL, "env id out of range");
+    if (listed[env_ids[k]]++) return fail(RLFC_EINVAL, "env id " + std::to_string(env_ids[k]) + " listed twice");
+  }
+  // all or nothing: every set validated and every geometry built before the device changes
+  std::vector<EnvGeometry> geo;
+  std::vector<int> set;
+  {
+    std::string err;
+    if (build_env_geometries(E->cfg, params, n, geo, set, err)) return fail(RLFC_EINVAL, err);
+  }
+  CU(cudaSetDevice(E->device));
+  int rc;
+  for (int k = 0; k < n; k++)
+    if ((rc = upload_env_geometry(E, env_ids[k], params[k], geo[set[k]]))) return rc;
+  if ((rc = upload_env_scalars(E))) return rc;
+  if ((rc = rlfc_env_reset(E, env_ids, n, reset_accumulators))) return rc;   // (sc.dt = the new t_step*resolution)
+  // the new hierarchies, of the listed environments only
+  std::vector<int> skip(B);
+  for (int e = 0; e < B; e++) skip[e] = listed[e] ? 0 : 1;
+  CU(cudaMemcpyAsync(E->d_skip, skip.data(), B * sizeof(int), cudaMemcpyHostToDevice, E->stream));
+  E->launches += launch_poisson_rebuild0(E->whole.sp, E->d_skip, E->stream);
+  E->launches += launch_poisson_rebuild_coarse(E->whole.sp, E->d_skip, E->stream);
+  CU(cudaGetLastError());
+  CU(cudaStreamSynchronize(E->stream));
+  return RLFC_OK;
+}
+
+int rlfc_env_get_params(rlfc_env* E, rlfc_env_params* params) {
+  if (!E || !params) return fail(RLFC_EINVAL, "null argument");
+  std::copy(E->params.begin(), E->params.end(), params);
   return RLFC_OK;
 }
 
@@ -1163,9 +1405,12 @@ int rlfc_env_step(rlfc_env* E, const float* actions, float* obs, float* reward, 
   // exactly `substeps` solver steps -- one round; an environment fresh from a reset first runs uncontrolled until
   // t > init_time and then through its first accumulation window, over several rounds, while the others stay frozen.
   // (adaptive mode: the bound follows the smallest dt any environment has taken in the rounds so far)
+  // (per-environment mode: the smallest t_step*resolution to start with)
   const float init_time = sp.init_time > 0 ? sp.init_time : 0;
-  int max_rounds = 3 + (int)(init_time / sp.dt_over_res) / sp.substeps;
   float dt_min = sp.dt;
+  if (sp.per_env) dt_min = *std::min_element(E->dt0.begin(), E->dt0.end());
+  int max_rounds = sp.per_env ? 3 + (int)(init_time / (dt_min / sp.resolution)) / sp.substeps
+                              : 3 + (int)(init_time / sp.dt_over_res) / sp.substeps;
   std::vector<float> h_dt(sp.adaptive ? B : 0);
   for (int round = 0;; round++) {
     int rc = step_round(E, E->d_actions, E->d_obs, E->d_reward, E->d_done);
@@ -1261,7 +1506,7 @@ int rlfc_env_save_bdim(rlfc_env* E, int e, const char* path) {
   // BDIM.t counts grid-unit time: set by resume, += dt per solver step (AFCCylinder.t advances by dt/resolution instead)
   float flow_t = 0, dt = E->sp.dt;
   CU(cudaMemcpyAsync(&flow_t, E->sp.sc.flow_t + e, sizeof(float), cudaMemcpyDeviceToHost, E->stream));
-  if (E->sp.adaptive) CU(cudaMemcpyAsync(&dt, E->sp.sc.dt + e, sizeof(float), cudaMemcpyDeviceToHost, E->stream));
+  if (E->sp.per_env) CU(cudaMemcpyAsync(&dt, E->sp.sc.dt + e, sizeof(float), cudaMemcpyDeviceToHost, E->stream));
   CU(cudaStreamSynchronize(E->stream));
   std::string err;
   rc = write_bdim_text(path, E->sp.n, E->sp.m, flow_t, dt, ux.data(), uy.data(), p.data(), err);
@@ -1278,8 +1523,11 @@ int rlfc_env_load_bdim(rlfc_env* E, int e, const char* path) {
   if (E->sp.adaptive) {
     // adaptive mode: any positive dt; it becomes the environment's current dt
     if (!(dt > 0) || !std::isfinite(dt)) return fail(RLFC_EIO, "checkpoint dt " + std::to_string(dt) + " is not a positive number");
-  } else if (dt != E->sp.dt && !(std::fabs(dt - E->sp.dt) <= 1e-6f * E->sp.dt))
-    return fail(RLFC_EIO, "checkpoint dt " + std::to_string(dt) + " does not match the handle's " + std::to_string(E->sp.dt));
+  } else {
+    const float fixed = E->dt0[e];   // the environment's t_step*resolution (the handle's without env_params)
+    if (dt != fixed && !(std::fabs(dt - fixed) <= 1e-6f * fixed))
+      return fail(RLFC_EIO, "checkpoint dt " + std::to_string(dt) + " does not match the environment's " + std::to_string(fixed));
+  }
   CU(cudaSetDevice(E->device));
   if (E->sp.adaptive) CU(cudaMemcpyAsync(E->sp.sc.dt + e, &dt, sizeof(float), cudaMemcpyHostToDevice, E->stream));
   CU(cudaMemcpyAsync(E->sp.sc.flow_t + e, &t, sizeof(float), cudaMemcpyHostToDevice, E->stream));   // BDIM.resume: t = stuff[0]
@@ -1334,7 +1582,7 @@ int rlfc_env_check_cfl(rlfc_env* E, float* dt) {
 
 int rlfc_env_get_dt(rlfc_env* E, float* dt) {
   if (!E || !dt) return fail(RLFC_EINVAL, "null argument");
-  if (!E->sp.adaptive) {
+  if (!E->sp.per_env) {
     for (int e = 0; e < E->sp.B; e++) dt[e] = E->sp.dt;
     return RLFC_OK;
   }
@@ -1410,17 +1658,22 @@ int rlfc_env_get_coeffs(rlfc_env* E, int e, const char* name, int level, float* 
   if (e < 0 || e >= E->sp.B) return fail(RLFC_EINVAL, "env index out of range");
   if (level < 0 || level >= E->sp.nlevels) return fail(RLFC_EINVAL, "level out of range");
   const std::string nm(name);
-  const bool c0 = level == 0 && (nm == "c.x" || nm == "c.y");
+  const bool c0 = level == 0 && (nm == "c.x" || nm == "c.y" || nm == "del.x" || nm == "del.y");
   if (!c0 && nm != "lower.x" && nm != "lower.y" && nm != "inv" && nm != "diag")
     return fail(RLFC_EINVAL, "unknown Poisson coefficient field " + nm);
-  if (!E->sp.adaptive) return static_lookup(E->geo, name, level, out, n, m);
+  if (!E->sp.per_env) return static_lookup(E->geo, name, level, out, n, m);
   const DevLevel& L = E->sp.lev[level];
   if (n) *n = L.n;
   if (m) *m = L.m;
   if (!out) return RLFC_OK;
   const float* src = (nm == "lower.x" || nm == "c.x") ? L.lx : (nm == "lower.y" || nm == "c.y") ? L.ly : nm == "inv" ? L.inv : L.diag;
+  size_t off = (size_t)e * L.stride;
+  if (nm == "del.x" || nm == "del.y") {   // the environment's geometry slot
+    src = nm == "del.x" ? E->sp.del_x : E->sp.del_y;
+    off = E->env_mode ? (size_t)e * E->sp.stride : 0;
+  }
   CU(cudaSetDevice(E->device));
-  CU(cudaMemcpy2DAsync(out, L.m * sizeof(float), src + (size_t)e * L.stride, L.P * sizeof(float), L.m * sizeof(float), L.n,
+  CU(cudaMemcpy2DAsync(out, L.m * sizeof(float), src + off, L.P * sizeof(float), L.m * sizeof(float), L.n,
                        cudaMemcpyDeviceToHost, E->stream));
   CU(cudaStreamSynchronize(E->stream));
   return RLFC_OK;

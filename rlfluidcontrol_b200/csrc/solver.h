@@ -147,11 +147,23 @@ struct SolverParams {
   int *xs_stats;            // [B][8] counters of the last serial pass (rlfc_env_field_sum_stats)
   EnvScalars sc;
   // (appended last, so the fields above keep their offsets in the kernels' parameter space)
-  int   adaptive;           // 1 = per-environment dt (sc.dt) and Poisson hierarchy: every level's lx, ly, inv, diag hold one
-                            // copy per environment at the level's `stride` (like r, x, d), c_x / c_y are level 0's lx / ly,
-                            // and each row-pipeline level's RowTab holds one table per environment (rt.copies = the view's B,
-                            // so the row smoother's `blockIdx.x % copies` pick selects environment blockIdx.x's table)
-  const float *del_x, *del_y;   // adaptive mode: level-0 BDIM del (reference layout incl. ghosts, pitched), c = del*(1*dt)
+  int   adaptive;           // 1 = every solver step opens with k_check_cfl<true> and the hierarchy rebuild (adaptive dt)
+                            // per_env (below) = per-environment dt (sc.dt) and Poisson hierarchy: every level's lx, ly, inv,
+                            // diag hold one copy per environment at the level's `stride` (like r, x, d), c_x / c_y are level
+                            // 0's lx / ly, and each row-pipeline level's RowTab holds one table per environment (rt.copies = the
+                            // view's B, so the row smoother's `blockIdx.x % copies` pick selects environment blockIdx.x's table)
+  const float *del_x, *del_y;   // per_env: level-0 BDIM del of every geometry slot (pitched, slot s at s * stride), c = del*(1*dt)
+  // per_env = 1 (adaptive mode, or per-environment parameters, rlfc_config.env_params): the kernels run their
+  // per-environment instances (ADT), which read sc.dt[e], the per-environment hierarchy above and the arrays below.  An
+  // environment's geometry lives in its SLOT: del_x/del_y and the body-velocity basis w1_x .. rx2_y at env_slot[e] *
+  // stride, its band lists at band_x + env_slot[e] * nband_x and band_y + env_slot[e] * nband_y (nband_x / nband_y are
+  // then the per-slot capacities; band_tmp keeps its [B][nband_x + nband_y] layout).  `adaptive` alone says whether a
+  // step opens with the CFL and rebuild kernels.
+  int   per_env;
+  const int   *env_slot;    // [B] geometry slot of each environment (adaptive mode without env_params: all 0)
+  const float *env_nu;      // [B] D/Re
+  const float *env_dRD;     // [B] dR*D
+  const int   *env_nband_x, *env_nband_y;   // [B] band faces of each environment (<= nband_x / nband_y)
 };
 
 #ifdef __CUDACC__
@@ -217,8 +229,9 @@ int launch_check_cfl(const SolverParams& P, const float* ux, const float* uy, fl
 int launch_step_cfl(const SolverParams& P, const float* ux, const float* uy, cudaStream_t st);
 // adaptive mode: every level's lx, ly, inv, diag and row tables of the environments not frozen, from c = del*(1*dt[e])
 // (geometry.cpp finish_level / coarsen restated); level 0 grid-wide, then the coarse levels one CTA per environment
-int launch_poisson_rebuild0(const SolverParams& P, cudaStream_t st);
-int launch_poisson_rebuild_coarse(const SolverParams& P, cudaStream_t st);
+// `skip` [B] (the view's environments): 1 = leave this environment's hierarchy as it is (the step passes sc.frozen)
+int launch_poisson_rebuild0(const SolverParams& P, const int* skip, cudaStream_t st);
+int launch_poisson_rebuild_coarse(const SolverParams& P, const int* skip, cudaStream_t st);
 // mode 0 (single solver steps): xi = actions (NULL keeps xi), every env runs.  mode 1 (RL step): an env takes its
 // action only where the reference would have asked for one (t > init_time and at a callLearn boundary); envs whose
 // episode is over (t >= episode_time) are frozen for the call

@@ -81,15 +81,17 @@ __device__ __forceinline__ float face_value(float uf, float bLL, float bL, float
 #ifndef RLFC_ADV_MINB
 #define RLFC_ADV_MINB 9      // 56 registers, 9 CTAs per SM: 202 -> 193 us (8: 198, 10 and 12 spill: 201, 217)
 #endif
-// ADT (adaptive mode): the environment's own dt, dts[blockIdx.z], replaces the handle's fixed `dt`
+// ADT (per-environment mode): the environment's own dt and nu, dts[blockIdx.z] and nus[blockIdx.z], replace the handle's
+// `dt_fixed` and `nu_fixed`
 template <bool PREDICTOR, bool ADT>
 __global__ void __launch_bounds__(128, RLFC_ADV_MINB)
 k_advdif(const float* __restrict__ srcx, const float* __restrict__ srcy, const float* __restrict__ u0x,
          const float* __restrict__ u0y, float* __restrict__ dstx, float* __restrict__ dsty, int n, int m, int P,
-         size_t stride, float dt_fixed, float nu, const int* __restrict__ frozen, int slab_rank, int slab_n, int chunk_rows,
-         const float* __restrict__ dts) {
+         size_t stride, float dt_fixed, float nu_fixed, const int* __restrict__ frozen, int slab_rank, int slab_n, int chunk_rows,
+         const float* __restrict__ dts, const float* __restrict__ nus) {
   if (frozen[blockIdx.z] || slab_skip(blockIdx.y, gridDim.y, slab_rank, slab_n)) return;
   const float dt = ADT ? dts[blockIdx.z] : dt_fixed;
+  const float nu = ADT ? nus[blockIdx.z] : nu_fixed;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int ni = n - 2, mj = m - 2;
   const int jw0 = 1 + blockIdx.x * kAdvCols;                         // first output column of this warp
@@ -223,26 +225,51 @@ __device__ void cta_setBC(float* a, int n, int m, int P, int btype, float bval, 
   __syncthreads();
 }
 
-// body velocity from the static basis (BodyUnion.velocity BodyUnion.pde:84-92, Body.velocity Body.pde:234-240)
-__device__ __forceinline__ float ub_x(const SolverParams& q, int k, float dphi1, float dphi2, float dt) {
-  float u1 = (0.f - q.ry1_x[k] * dphi1) / dt;
-  float u2 = (0.f - q.ry2_x[k] * dphi2) / dt;
-  float v = 0.f + u1 * q.w1_x[k];
-  return v + u2 * q.w2_x[k];
+// body velocity from the static basis (BodyUnion.velocity BodyUnion.pde:84-92, Body.velocity Body.pde:234-240); `so` (ADT):
+// offset of the environment's geometry slot
+template <bool ADT>
+__device__ __forceinline__ float ub_x(const SolverParams& q, int k, size_t so, float dphi1, float dphi2, float dt) {
+  const float *ry1 = q.ry1_x + (ADT ? so : 0), *ry2 = q.ry2_x + (ADT ? so : 0);
+  const float *w1 = q.w1_x + (ADT ? so : 0), *w2 = q.w2_x + (ADT ? so : 0);
+  float u1 = (0.f - ry1[k] * dphi1) / dt;
+  float u2 = (0.f - ry2[k] * dphi2) / dt;
+  float v = 0.f + u1 * w1[k];
+  return v + u2 * w2[k];
 }
-__device__ __forceinline__ float ub_y(const SolverParams& q, int k, float dphi1, float dphi2, float dt) {
-  float u1 = (0.f + q.rx1_y[k] * dphi1) / dt;
-  float u2 = (0.f + q.rx2_y[k] * dphi2) / dt;
-  float v = 0.f + u1 * q.w1_y[k];
-  return v + u2 * q.w2_y[k];
+template <bool ADT>
+__device__ __forceinline__ float ub_y(const SolverParams& q, int k, size_t so, float dphi1, float dphi2, float dt) {
+  const float *rx1 = q.rx1_y + (ADT ? so : 0), *rx2 = q.rx2_y + (ADT ? so : 0);
+  const float *w1 = q.w1_y + (ADT ? so : 0), *w2 = q.w2_y + (ADT ? so : 0);
+  float u1 = (0.f + rx1[k] * dphi1) / dt;
+  float u2 = (0.f + rx2[k] * dphi2) / dt;
+  float v = 0.f + u1 * w1[k];
+  return v + u2 * w2[k];
 }
 
+// environment e's band (ADT: its slot's lists and its own counts and dR*D; else the handle's)
+template <bool ADT>
+struct EnvBand {
+  const BandFace *bx, *by;
+  int nbx, nby;
+  size_t so;
+  float dRD;
+  __device__ __forceinline__ EnvBand(const SolverParams& q, int e) {
+    const int s = ADT ? q.env_slot[e] : 0;
+    bx = q.band_x + (ADT ? (size_t)s * q.nband_x : 0);
+    by = q.band_y + (ADT ? (size_t)s * q.nband_y : 0);
+    nbx = ADT ? q.env_nband_x[e] : q.nband_x;
+    nby = ADT ? q.env_nband_y[e] : q.nband_y;
+    so = ADT ? (size_t)s * q.stride : 0;
+    dRD = ADT ? q.env_dRD[e] : q.dRD;
+  }
+};
+
 // BDIM.updateUP blend of one band face (BDIM.pde:109-122): u = del*R - ub*(del + (-1)) + del1 * normalGrad(R - ub)
-template <bool XCOMP>
-__device__ __forceinline__ float band_face(const SolverParams& q, const float* u, const BandFace& f, float dphi1, float dphi2,
-                                           float dt) {
+template <bool XCOMP, bool ADT>
+__device__ __forceinline__ float band_face(const SolverParams& q, const float* u, const BandFace& f, size_t so, float dphi1,
+                                           float dphi2, float dt) {
   const int P = q.P, k = IDX(f.i, f.j);
-  auto ub = [&](int kk) { return XCOMP ? ub_x(q, kk, dphi1, dphi2, dt) : ub_y(q, kk, dphi1, dphi2, dt); };
+  auto ub = [&](int kk) { return XCOMP ? ub_x<ADT>(q, kk, so, dphi1, dphi2, dt) : ub_y<ADT>(q, kk, so, dphi1, dphi2, dt); };
   const float R = u[k], ubc = ub(k);
   const float v = f.del * R - ubc * (f.del + (-1.f));
   const float duE = u[k + P] - ub(k + P), duW = u[k - P] - ub(k - P);
@@ -261,14 +288,16 @@ __global__ void __launch_bounds__(256)
 k_band_blend(const __grid_constant__ SolverParams q, const float* ux_all, const float* uy_all) {
   const int e = blockIdx.y, b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= q.nband_x + q.nband_y || q.sc.frozen[e] || slab_skip(blockIdx.x, gridDim.x, q.slab_rank, q.slab_n)) return;
+  const EnvBand<ADT> eb(q, e);
+  if (ADT && (b < q.nband_x ? b >= eb.nbx : b - q.nband_x >= eb.nby)) return;   // past this environment's band
   const float* ux = ux_all + (size_t)e * q.stride;
   const float* uy = uy_all + (size_t)e * q.stride;
   float* tmp = q.band_tmp + (size_t)e * (q.nband_x + q.nband_y);
   const float xi1_m = q.action_scale * q.sc.xi[2 * e], xi2_m = q.action_scale * q.sc.xi[2 * e + 1];   // AFCCylinder.pde:48-49
   const float dt = env_dt<ADT>(q, e);
-  const float dphi1 = (2 * xi1_m * dt) / q.dRD, dphi2 = (2 * xi2_m * dt) / q.dRD;
-  tmp[b] = (b < q.nband_x) ? band_face<true>(q, ux, q.band_x[b], dphi1, dphi2, dt)
-                           : band_face<false>(q, uy, q.band_y[b - q.nband_x], dphi1, dphi2, dt);
+  const float dphi1 = (2 * xi1_m * dt) / eb.dRD, dphi2 = (2 * xi2_m * dt) / eb.dRD;
+  tmp[b] = (b < q.nband_x) ? band_face<true, ADT>(q, ux, eb.bx[b], eb.so, dphi1, dphi2, dt)
+                           : band_face<false, ADT>(q, uy, eb.by[b - q.nband_x], eb.so, dphi1, dphi2, dt);
 }
 
 // BDIM.updateUP blend on the body band (everywhere else it is the identity), then u.setBC()
@@ -281,17 +310,18 @@ k_band_bc(const __grid_constant__ SolverParams q, float* ux_all, float* uy_all) 
   float* ux = ux_all + (size_t)e * q.stride;
   float* uy = uy_all + (size_t)e * q.stride;
   float* tmp = q.band_tmp + (size_t)e * (q.nband_x + q.nband_y);
+  const EnvBand<ADT> eb(q, e);
   if (!PREBLENDED) {
     // AFCCylinder.pde:48-49
     const float xi1_m = q.action_scale * q.sc.xi[2 * e], xi2_m = q.action_scale * q.sc.xi[2 * e + 1];
     const float dt = env_dt<ADT>(q, e);
-    const float dphi1 = (2 * xi1_m * dt) / q.dRD, dphi2 = (2 * xi2_m * dt) / q.dRD;
-    for (int b = threadIdx.x; b < q.nband_x; b += blockDim.x) tmp[b] = band_face<true>(q, ux, q.band_x[b], dphi1, dphi2, dt);
-    for (int b = threadIdx.x; b < q.nband_y; b += blockDim.x) tmp[q.nband_x + b] = band_face<false>(q, uy, q.band_y[b], dphi1, dphi2, dt);
+    const float dphi1 = (2 * xi1_m * dt) / eb.dRD, dphi2 = (2 * xi2_m * dt) / eb.dRD;
+    for (int b = threadIdx.x; b < eb.nbx; b += blockDim.x) tmp[b] = band_face<true, ADT>(q, ux, eb.bx[b], eb.so, dphi1, dphi2, dt);
+    for (int b = threadIdx.x; b < eb.nby; b += blockDim.x) tmp[q.nband_x + b] = band_face<false, ADT>(q, uy, eb.by[b], eb.so, dphi1, dphi2, dt);
     __syncthreads();
   }
-  for (int b = threadIdx.x; b < q.nband_x; b += blockDim.x) ux[IDX(q.band_x[b].i, q.band_x[b].j)] = tmp[b];
-  for (int b = threadIdx.x; b < q.nband_y; b += blockDim.x) uy[IDX(q.band_y[b].i, q.band_y[b].j)] = tmp[q.nband_x + b];
+  for (int b = threadIdx.x; b < eb.nbx; b += blockDim.x) ux[IDX(eb.bx[b].i, eb.bx[b].j)] = tmp[b];
+  for (int b = threadIdx.x; b < eb.nby; b += blockDim.x) uy[IDX(eb.by[b].i, eb.by[b].j)] = tmp[q.nband_x + b];
   __syncthreads();
   cta_setBC(ux, q.n, q.m, P, 1, 1.f, true, scol);     // u.x: btype 1, bval 1, gradientExit (BDIM.pde:52)
   cta_setBC(uy, q.n, q.m, P, 2, 0.f, false, scol);
@@ -372,28 +402,56 @@ k_bc2(const __grid_constant__ SolverParams q, float* ux_all, float* uy_all, cons
   // u.x: btype 1, bval 1, gradientExit (BDIM.pde:52); u.y: btype 2, bval 0
   bc_stage(sx, ux, tid, blockDim.x, n, m, P, 1, 1.f, true);
   bc_stage(sy, uy, tid, blockDim.x, n, m, P, 2, 0.f, false);
-  if (BAND) {
-    // BDIM.updateUP blend on the body band (BDIM.pde:109-122), identical arithmetic to k_band_bc
+  if constexpr (BAND && ADT) {
+    // BDIM.updateUP blend on the body band (BDIM.pde:109-122), identical arithmetic to k_band_bc; the environment's own
+    // band, basis slot and dR*D
+    const EnvBand<ADT> eb(q, e);
+    const float xi1_m = q.action_scale * q.sc.xi[2 * e], xi2_m = q.action_scale * q.sc.xi[2 * e + 1];
+    const float dt = env_dt<ADT>(q, e);
+    const float dphi1 = (2 * xi1_m * dt) / eb.dRD, dphi2 = (2 * xi2_m * dt) / eb.dRD;
+    const size_t so = eb.so;
+    for (int b = tid; b < eb.nbx; b += blockDim.x) {
+      const BandFace f = eb.bx[b];
+      const int k = IDX(f.i, f.j);
+      float R = ux[k], ub = ub_x<ADT>(q, k, so, dphi1, dphi2, dt);
+      float v = f.del * R - ub * (f.del + (-1.f));
+      float duE = ux[k + P] - ub_x<ADT>(q, k + P, so, dphi1, dphi2, dt), duW = ux[k - P] - ub_x<ADT>(q, k - P, so, dphi1, dphi2, dt);
+      float duN = ux[k + 1] - ub_x<ADT>(q, k + 1, so, dphi1, dphi2, dt), duS = ux[k - 1] - ub_x<ADT>(q, k - 1, so, dphi1, dphi2, dt);
+      float g = 0.5f * (f.wnx * (duE - duW) + f.wny * (duN - duS));       // VectorField.pde:50
+      tmp[b] = v + f.del1 * g;
+    }
+    for (int b = tid; b < eb.nby; b += blockDim.x) {
+      const BandFace f = eb.by[b];
+      const int k = IDX(f.i, f.j);
+      float R = uy[k], ub = ub_y<ADT>(q, k, so, dphi1, dphi2, dt);
+      float v = f.del * R - ub * (f.del + (-1.f));
+      float duE = uy[k + P] - ub_y<ADT>(q, k + P, so, dphi1, dphi2, dt), duW = uy[k - P] - ub_y<ADT>(q, k - P, so, dphi1, dphi2, dt);
+      float duN = uy[k + 1] - ub_y<ADT>(q, k + 1, so, dphi1, dphi2, dt), duS = uy[k - 1] - ub_y<ADT>(q, k - 1, so, dphi1, dphi2, dt);
+      float g = 0.5f * (f.wnx * (duE - duW) + f.wny * (duN - duS));       // VectorField.pde:51
+      tmp[q.nband_x + b] = v + f.del1 * g;
+    }
+  }
+  if constexpr (BAND && !ADT) {   // (the handle-wide band: kept apart so that this instance compiles as before)
     const float xi1_m = q.action_scale * q.sc.xi[2 * e], xi2_m = q.action_scale * q.sc.xi[2 * e + 1];
     const float dt = env_dt<ADT>(q, e);
     const float dphi1 = (2 * xi1_m * dt) / q.dRD, dphi2 = (2 * xi2_m * dt) / q.dRD;
     for (int b = tid; b < q.nband_x; b += blockDim.x) {
       const BandFace f = q.band_x[b];
       const int k = IDX(f.i, f.j);
-      float R = ux[k], ub = ub_x(q, k, dphi1, dphi2, dt);
+      float R = ux[k], ub = ub_x<false>(q, k, 0, dphi1, dphi2, dt);
       float v = f.del * R - ub * (f.del + (-1.f));
-      float duE = ux[k + P] - ub_x(q, k + P, dphi1, dphi2, dt), duW = ux[k - P] - ub_x(q, k - P, dphi1, dphi2, dt);
-      float duN = ux[k + 1] - ub_x(q, k + 1, dphi1, dphi2, dt), duS = ux[k - 1] - ub_x(q, k - 1, dphi1, dphi2, dt);
+      float duE = ux[k + P] - ub_x<false>(q, k + P, 0, dphi1, dphi2, dt), duW = ux[k - P] - ub_x<false>(q, k - P, 0, dphi1, dphi2, dt);
+      float duN = ux[k + 1] - ub_x<false>(q, k + 1, 0, dphi1, dphi2, dt), duS = ux[k - 1] - ub_x<false>(q, k - 1, 0, dphi1, dphi2, dt);
       float g = 0.5f * (f.wnx * (duE - duW) + f.wny * (duN - duS));       // VectorField.pde:50
       tmp[b] = v + f.del1 * g;
     }
     for (int b = tid; b < q.nband_y; b += blockDim.x) {
       const BandFace f = q.band_y[b];
       const int k = IDX(f.i, f.j);
-      float R = uy[k], ub = ub_y(q, k, dphi1, dphi2, dt);
+      float R = uy[k], ub = ub_y<false>(q, k, 0, dphi1, dphi2, dt);
       float v = f.del * R - ub * (f.del + (-1.f));
-      float duE = uy[k + P] - ub_y(q, k + P, dphi1, dphi2, dt), duW = uy[k - P] - ub_y(q, k - P, dphi1, dphi2, dt);
-      float duN = uy[k + 1] - ub_y(q, k + 1, dphi1, dphi2, dt), duS = uy[k - 1] - ub_y(q, k - 1, dphi1, dphi2, dt);
+      float duE = uy[k + P] - ub_y<false>(q, k + P, 0, dphi1, dphi2, dt), duW = uy[k - P] - ub_y<false>(q, k - P, 0, dphi1, dphi2, dt);
+      float duN = uy[k + 1] - ub_y<false>(q, k + 1, 0, dphi1, dphi2, dt), duS = uy[k - 1] - ub_y<false>(q, k - 1, 0, dphi1, dphi2, dt);
       float g = 0.5f * (f.wnx * (duE - duW) + f.wny * (duN - duS));       // VectorField.pde:51
       tmp[q.nband_x + b] = v + f.del1 * g;
     }
@@ -404,7 +462,11 @@ k_bc2(const __grid_constant__ SolverParams q, float* ux_all, float* uy_all, cons
     s_mean = s / (float)(m - 2);
   }
   // ---- phase 2: every store ----
-  if (BAND) {
+  if constexpr (BAND && ADT) {
+    const EnvBand<ADT> eb(q, e);
+    for (int b = tid; b < eb.nbx; b += blockDim.x) ux[IDX(eb.bx[b].i, eb.bx[b].j)] = tmp[b];
+    for (int b = tid; b < eb.nby; b += blockDim.x) uy[IDX(eb.by[b].i, eb.by[b].j)] = tmp[q.nband_x + b];
+  } else if constexpr (BAND) {
     for (int b = tid; b < q.nband_x; b += blockDim.x) ux[IDX(q.band_x[b].i, q.band_x[b].j)] = tmp[b];
     for (int b = tid; b < q.nband_y; b += blockDim.x) uy[IDX(q.band_y[b].i, q.band_y[b].j)] = tmp[q.nband_x + b];
   }
@@ -1296,8 +1358,9 @@ k_force(const __grid_constant__ SolverParams q, int accumulate) {
 // b = max(|ux|+|uy|) over the interior, started from cell [0][0].  A maximum does not depend on the order it is taken in,
 // so the reduction is parallel and still exact.  One CTA per environment (a diagnostic / adaptive-dt read-out, not on
 // the fixed-dt step path).
-// STEP (adaptive mode, start of a solver step): frozen environments are skipped and keep their dt.
-template <bool STEP>
+// STEP (adaptive mode, start of a solver step): frozen environments are skipped and keep their dt.  ADT: the environment's
+// own nu.
+template <bool STEP, bool ADT>
 __global__ void __launch_bounds__(1024)
 k_check_cfl(const __grid_constant__ SolverParams q, const float* __restrict__ ux_all, const float* __restrict__ uy_all,
             float* __restrict__ dt_out) {
@@ -1318,7 +1381,7 @@ k_check_cfl(const __grid_constant__ SolverParams q, const float* __restrict__ ux
   __syncthreads();
   if (threadIdx.x == 0) {
     for (int w = 1; w < (int)(blockDim.x >> 5); w++) if (wmax[w] > b) b = wmax[w];
-    const float cfl = 1.f / (b + 3.f * q.nu);
+    const float cfl = 1.f / (b + 3.f * (ADT ? q.env_nu[e] : q.nu));
     dt_out[e] = cfl < 1.f ? cfl : 1.f;                                      // PApplet.min(u.CFL(nu), 1)
   }
 }
@@ -1415,10 +1478,12 @@ __device__ __forceinline__ float4 rowtab_vec(const RowTab& rt, int ent, int kv, 
 
 // level 0: lx, ly, diag, inv of every cell and the level's row table (if any), grid-wide; blockIdx.y = environment
 __global__ void __launch_bounds__(256)
-k_poisson_rebuild0(const __grid_constant__ SolverParams q) {
+k_poisson_rebuild0(const __grid_constant__ SolverParams q, const int* __restrict__ skip) {
   const int e = blockIdx.y;
-  if (q.sc.frozen[e]) return;
+  if (skip[e]) return;
   const DevLevel& L = q.lev[0];
+  const float* __restrict__ del_x = q.del_x + (size_t)q.env_slot[e] * q.stride;   // this environment's geometry slot
+  const float* __restrict__ del_y = q.del_y + (size_t)q.env_slot[e] * q.stride;
   const int n = L.n, m = L.m, P = L.P, ni = n - 2, mj = m - 2;
   const float dt = q.sc.dt[e];
   const size_t co = (size_t)e * L.stride;
@@ -1432,11 +1497,11 @@ k_poisson_rebuild0(const __grid_constant__ SolverParams q) {
   for (int t = blockIdx.x * blockDim.x + threadIdx.x; t < cells + tab; t += gridDim.x * blockDim.x) {
     if (t < cells) {
       const int i = t / m, j = t - i * m, k = IDX(i, j);
-      lx[k] = q.del_x[k] * cdt;
-      ly[k] = q.del_y[k] * cdt;
+      lx[k] = del_x[k] * cdt;
+      ly[k] = del_y[k] * cdt;
       float dg = 0.f, iv = 1.f;
       if (i >= 1 && i <= ni && j >= 1 && j <= mj) {
-        const float sumd = q.del_x[k] * cdt + q.del_x[k + P] * cdt + q.del_y[k] * cdt + q.del_y[k + 1] * cdt;
+        const float sumd = del_x[k] * cdt + del_x[k + P] * cdt + del_y[k] * cdt + del_y[k + 1] * cdt;
         dg = -sumd;
         if (sumd > 1e-5f) iv = -1.f / sumd;
       }
@@ -1453,17 +1518,17 @@ k_poisson_rebuild0(const __grid_constant__ SolverParams q) {
         float v = 0.f;
         if (idx <= C) {
           const int j = j0 + idx;
-          if (row >= 1 && row <= ni && j <= mj + 1) v = q.del_y[IDX(row, j)] * cdt;
+          if (row >= 1 && row <= ni && j <= mj + 1) v = del_y[IDX(row, j)] * cdt;
         } else if (idx <= 2 * C) {
           const int j = j0 + idx - (C + 1);
           if (row >= 1 && row <= ni && j <= mj) {
             const int k = IDX(row, j);
-            const float sumd = q.del_x[k] * cdt + q.del_x[k + P] * cdt + q.del_y[k] * cdt + q.del_y[k + 1] * cdt;
+            const float sumd = del_x[k] * cdt + del_x[k + P] * cdt + del_y[k] * cdt + del_y[k + 1] * cdt;
             v = -((sumd > 1e-5f) ? -1.f / sumd : 1.f);
           }
         } else if (idx <= 3 * C) {
           const int j = j0 + idx - (2 * C + 1);
-          if (row >= 1 && row <= ni + 1 && j <= mj) v = q.del_x[IDX(row, j)] * cdt;
+          if (row >= 1 && row <= ni + 1 && j <= mj) v = del_x[IDX(row, j)] * cdt;
         }
         f[w] = v;
       }
@@ -1474,9 +1539,9 @@ k_poisson_rebuild0(const __grid_constant__ SolverParams q) {
 
 // levels 1 .. nlevels-1, one CTA per environment, level by level from the one above
 __global__ void __launch_bounds__(1024)
-k_poisson_rebuild_coarse(const __grid_constant__ SolverParams q) {
+k_poisson_rebuild_coarse(const __grid_constant__ SolverParams q, const int* __restrict__ skip) {
   const int e = blockIdx.x, tid = threadIdx.x, nt = blockDim.x;
-  if (q.sc.frozen[e]) return;
+  if (skip[e]) return;
   for (int l = 1; l < q.nlevels; l++) {
     const DevLevel& F = q.lev[l - 1];
     const DevLevel& L = q.lev[l];
@@ -1547,13 +1612,13 @@ int launch_advdif(const SolverParams& q, const float* srcx, const float* srcy, c
   const int rows = (long long)q.B * ni * mj < (8ll << 20) ? 16 : kAdvRows;
   dim3 grid((mj + kAdvCols - 1) / kAdvCols, ((ni + rows - 1) / rows + 3) / 4, q.B);
   const bool pred = srcx == u0x && srcy == u0y;
-  if (q.adaptive) {
-    if (pred) k_advdif<true, true><<<grid, 128, 0, st>>>(srcx, srcy, u0x, u0y, dstx, dsty, q.n, q.m, q.P, q.stride, q.dt, q.nu, q.sc.frozen, q.slab_rank, q.slab_n, rows, q.sc.dt);
-    else k_advdif<false, true><<<grid, 128, 0, st>>>(srcx, srcy, u0x, u0y, dstx, dsty, q.n, q.m, q.P, q.stride, q.dt, q.nu, q.sc.frozen, q.slab_rank, q.slab_n, rows, q.sc.dt);
+  if (q.per_env) {
+    if (pred) k_advdif<true, true><<<grid, 128, 0, st>>>(srcx, srcy, u0x, u0y, dstx, dsty, q.n, q.m, q.P, q.stride, q.dt, q.nu, q.sc.frozen, q.slab_rank, q.slab_n, rows, q.sc.dt, q.env_nu);
+    else k_advdif<false, true><<<grid, 128, 0, st>>>(srcx, srcy, u0x, u0y, dstx, dsty, q.n, q.m, q.P, q.stride, q.dt, q.nu, q.sc.frozen, q.slab_rank, q.slab_n, rows, q.sc.dt, q.env_nu);
   } else if (pred)
-    k_advdif<true, false><<<grid, 128, 0, st>>>(srcx, srcy, u0x, u0y, dstx, dsty, q.n, q.m, q.P, q.stride, q.dt, q.nu, q.sc.frozen, q.slab_rank, q.slab_n, rows, nullptr);
+    k_advdif<true, false><<<grid, 128, 0, st>>>(srcx, srcy, u0x, u0y, dstx, dsty, q.n, q.m, q.P, q.stride, q.dt, q.nu, q.sc.frozen, q.slab_rank, q.slab_n, rows, nullptr, nullptr);
   else
-    k_advdif<false, false><<<grid, 128, 0, st>>>(srcx, srcy, u0x, u0y, dstx, dsty, q.n, q.m, q.P, q.stride, q.dt, q.nu, q.sc.frozen, q.slab_rank, q.slab_n, rows, nullptr);
+    k_advdif<false, false><<<grid, 128, 0, st>>>(srcx, srcy, u0x, u0y, dstx, dsty, q.n, q.m, q.P, q.stride, q.dt, q.nu, q.sc.frozen, q.slab_rank, q.slab_n, rows, nullptr, nullptr);
   return 1;
 }
 
@@ -1570,7 +1635,7 @@ static int launch_band_bc_t(const SolverParams& q, float* ux, float* uy, cudaStr
   return 1;
 }
 int launch_band_bc(const SolverParams& q, float* ux, float* uy, cudaStream_t st) {
-  return q.adaptive ? launch_band_bc_t<true>(q, ux, uy, st) : launch_band_bc_t<false>(q, ux, uy, st);
+  return q.per_env ? launch_band_bc_t<true>(q, ux, uy, st) : launch_band_bc_t<false>(q, ux, uy, st);
 }
 
 int launch_bc(const SolverParams& q, float* ux, float* uy, cudaStream_t st) {
@@ -1585,13 +1650,13 @@ int launch_resid_down0(const SolverParams& q, const float* ux, const float* uy, 
   if (q.resid_march) {
     const int ni = q.n - 2, mj = q.m - 2;
     dim3 grid((mj + kRmWarps * kRmCols - 1) / (kRmWarps * kRmCols), (ni + kRmRows - 1) / kRmRows, q.B);
-    if (q.adaptive) k_resid_down0_march<true><<<grid, 32 * (kRmWarps + 1), kRmSmem, st>>>(q, ux, uy, p_in, p_out, r_out, which);
+    if (q.per_env) k_resid_down0_march<true><<<grid, 32 * (kRmWarps + 1), kRmSmem, st>>>(q, ux, uy, p_in, p_out, r_out, which);
     else k_resid_down0_march<false><<<grid, 32 * (kRmWarps + 1), kRmSmem, st>>>(q, ux, uy, p_in, p_out, r_out, which);
     return 1;
   }
   dim3 blk(kRdJ, kRdI);
   dim3 grid((L1.m - 2 + kRdJ - 1) / kRdJ, (L1.n - 2 + kRdI - 1) / kRdI, q.B);
-  if (q.adaptive) k_resid_down0<true><<<grid, blk, 0, st>>>(q, ux, uy, p_in, p_out, r_out, which);
+  if (q.per_env) k_resid_down0<true><<<grid, blk, 0, st>>>(q, ux, uy, p_in, p_out, r_out, which);
   else k_resid_down0<false><<<grid, blk, 0, st>>>(q, ux, uy, p_in, p_out, r_out, which);
   return 1;
 }
@@ -1599,7 +1664,7 @@ int launch_resid_down0(const SolverParams& q, const float* ux, const float* uy, 
 int launch_project_shift(const SolverParams& q, const float* p_in, float* p_out, float* ux, float* uy, cudaStream_t st) {
   const int items = q.n * (q.P >> 2);
   dim3 grid((items + 255) / 256, q.B);
-  if (q.adaptive) k_project_shift<false, true><<<grid, 256, 0, st>>>(q, p_in, p_out, ux, uy, nullptr, nullptr, nullptr, nullptr);
+  if (q.per_env) k_project_shift<false, true><<<grid, 256, 0, st>>>(q, p_in, p_out, ux, uy, nullptr, nullptr, nullptr, nullptr);
   else k_project_shift<false, false><<<grid, 256, 0, st>>>(q, p_in, p_out, ux, uy, nullptr, nullptr, nullptr, nullptr);
   return 1;
 }
@@ -1608,7 +1673,7 @@ int launch_project_shift_heun(const SolverParams& q, const float* p_in, float* p
                               const float* usy, float* uox, float* uoy, cudaStream_t st) {
   const int items = q.n * (q.P >> 2);
   dim3 grid((items + 255) / 256, q.B);
-  if (q.adaptive) k_project_shift<true, true><<<grid, 256, 0, st>>>(q, p_in, p_out, ux, uy, usx, usy, uox, uoy);
+  if (q.per_env) k_project_shift<true, true><<<grid, 256, 0, st>>>(q, p_in, p_out, ux, uy, usx, usy, uox, uoy);
   else k_project_shift<true, false><<<grid, 256, 0, st>>>(q, p_in, p_out, ux, uy, usx, usy, uox, uoy);
   return 1;
 }
@@ -1632,7 +1697,7 @@ int launch_loopcond(const SolverParams& q, unsigned long long handle, cudaStream
 int launch_mg_down0(const SolverParams& q, const float* r_in, float* r_out, cudaStream_t st) {
   dim3 blk(32, 8);
   const DevLevel& L1 = q.lev[1];
-  if (q.adaptive) k_mg_down0<true><<<grid2d(L1.m - 2, L1.n - 2, q.B, blk), blk, 0, st>>>(q, r_in, r_out);
+  if (q.per_env) k_mg_down0<true><<<grid2d(L1.m - 2, L1.n - 2, q.B, blk), blk, 0, st>>>(q, r_in, r_out);
   else k_mg_down0<false><<<grid2d(L1.m - 2, L1.n - 2, q.B, blk), blk, 0, st>>>(q, r_in, r_out);
   return 1;
 }
@@ -1662,7 +1727,7 @@ int configure_kernels(const SolverParams& q) {
         cudaFuncSetAttribute(k_bc2<false, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bc2_smem(q)) != cudaSuccess ||
         cudaFuncSetAttribute(k_bc2<false, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bc2_smem(q)) != cudaSuccess)
       return -1;
-    if (q.adaptive &&
+    if (q.per_env &&
         cudaFuncSetAttribute(k_bc2<true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bc2_smem(q)) != cudaSuccess)
       return -1;
   }
@@ -1670,7 +1735,7 @@ int configure_kernels(const SolverParams& q) {
       cudaFuncSetAttribute(k_xsum_chain_blocks<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kXsBlocksSmem) != cudaSuccess) return -1;
   if (cudaFuncSetAttribute(k_resid_down0_march<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kRmSmem) != cudaSuccess) return -1;
   cudaError_t e3 = cudaFuncSetAttribute(k_mg_coarse_rows<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)coarse_rows_smem(q));
-  if (q.adaptive) {
+  if (q.per_env) {
     if (cudaFuncSetAttribute(k_resid_down0_march<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kRmSmem) != cudaSuccess) return -1;
     if (e3 == cudaSuccess)
       e3 = cudaFuncSetAttribute(k_mg_coarse_rows<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)coarse_rows_smem(q));
@@ -1723,7 +1788,7 @@ int launch_chain_up(const SolverParams& q, int l, const float* r, cudaStream_t s
   return 1;
 }
 int launch_coarse_cta(const SolverParams& q, cudaStream_t st) {
-  if (q.adaptive) k_mg_coarse_rows<true><<<q.B, kRowsThreads, coarse_rows_smem(q), st>>>(q, max(1, q.chain_levels));
+  if (q.per_env) k_mg_coarse_rows<true><<<q.B, kRowsThreads, coarse_rows_smem(q), st>>>(q, max(1, q.chain_levels));
   else k_mg_coarse_rows<false><<<q.B, kRowsThreads, coarse_rows_smem(q), st>>>(q, max(1, q.chain_levels));
   return 1;
 }
@@ -1752,7 +1817,7 @@ int launch_mg_up0(const SolverParams& q, float* r, cudaStream_t st) {
   dim3 blk(32, 8);
   if (q.lev[0].ch.on) return launch_chain_up(q, 0, r, st);
   if (!q.lev[0].wave) {
-    if (q.adaptive) k_mg_up0_blk<true><<<dim3((q.n - 2 + kUpRows - 1) / kUpRows, q.B), 256, up0_smem(q), st>>>(q, r);
+    if (q.per_env) k_mg_up0_blk<true><<<dim3((q.n - 2 + kUpRows - 1) / kUpRows, q.B), 256, up0_smem(q), st>>>(q, r);
     else k_mg_up0_blk<false><<<dim3((q.n - 2 + kUpRows - 1) / kUpRows, q.B), 256, up0_smem(q), st>>>(q, r);
   }
   else k_mg_up0<<<grid2d(q.m, q.n, q.B, blk), blk, 0, st>>>(q, r);
@@ -1829,31 +1894,32 @@ int launch_heun(const SolverParams& q, const float* ucx, const float* ucy, const
 }
 
 int launch_force(const SolverParams& q, int accumulate, cudaStream_t st) {
-  if (q.adaptive) k_force<true><<<q.B, 64, 0, st>>>(q, accumulate);
+  if (q.per_env) k_force<true><<<q.B, 64, 0, st>>>(q, accumulate);
   else k_force<false><<<q.B, 64, 0, st>>>(q, accumulate);
   return 1;
 }
 
 int launch_check_cfl(const SolverParams& q, const float* ux, const float* uy, float* d_dt, cudaStream_t st) {
-  k_check_cfl<false><<<q.B, 1024, 0, st>>>(q, ux, uy, d_dt);
+  if (q.per_env) k_check_cfl<false, true><<<q.B, 1024, 0, st>>>(q, ux, uy, d_dt);
+  else k_check_cfl<false, false><<<q.B, 1024, 0, st>>>(q, ux, uy, d_dt);
   return 1;
 }
 
 int launch_step_cfl(const SolverParams& q, const float* ux, const float* uy, cudaStream_t st) {
-  k_check_cfl<true><<<q.B, 1024, 0, st>>>(q, ux, uy, q.sc.dt);
+  k_check_cfl<true, true><<<q.B, 1024, 0, st>>>(q, ux, uy, q.sc.dt);
   return 1;
 }
 
-int launch_poisson_rebuild0(const SolverParams& q, cudaStream_t st) {
+int launch_poisson_rebuild0(const SolverParams& q, const int* skip, cudaStream_t st) {
   const DevLevel& L = q.lev[0];
   const long long items = (long long)L.n * L.m + (long long)L.rt.entries * L.rt.K * 32;
   const long long blocks = (items + 255) / 256;
-  k_poisson_rebuild0<<<dim3((unsigned)(blocks < 1024 ? blocks : 1024), q.B), 256, 0, st>>>(q);
+  k_poisson_rebuild0<<<dim3((unsigned)(blocks < 1024 ? blocks : 1024), q.B), 256, 0, st>>>(q, skip);
   return 1;
 }
 
-int launch_poisson_rebuild_coarse(const SolverParams& q, cudaStream_t st) {
-  k_poisson_rebuild_coarse<<<q.B, 1024, 0, st>>>(q);
+int launch_poisson_rebuild_coarse(const SolverParams& q, const int* skip, cudaStream_t st) {
+  k_poisson_rebuild_coarse<<<q.B, 1024, 0, st>>>(q, skip);
   return 1;
 }
 

@@ -13,7 +13,10 @@ rlfluidcontrol_b200/peer/agent_server.py; the unchanged single-environment proto
     the peer (`finish_envs`), it restarts from the init state with xi = 0 and -- like the sketch globals callLearn/Cd/Cl
     (clientCFD.pde:11-13) -- keeps its force accumulators unless `reset_accumulators` is set.  Its first observation after
     the reset comes out of the uncontrolled start (rlfc.h: rlfc_env_step), during which the others wait;
-  * after every `train_every` finished environment-episodes: train(train_steps), save(train_steps) (clientCFD.pde:72-81).
+  * after every `train_every` finished environment-episodes: train(train_steps), save(train_steps) (clientCFD.pde:72-81);
+  * `sample_params` (a handle created with env_params): setUpNewSim builds a new AFCCylinder (clientCFD.pde:93-102), so a
+    finished environment may start its next episode with new constructor arguments: sample_params(rng, env_ids) returns
+    one parameter set per finished environment (dicts or a structured array, see AFCCylinderBatch.reset).
 """
 from __future__ import annotations
 
@@ -25,7 +28,7 @@ import numpy as np
 
 class BatchedEpisodeDriver:
     def __init__(self, env, url="http://localhost:8000", train_steps=1000, train_every=None, reset_accumulators=False,
-                 proxy=None, quiet=True):
+                 proxy=None, quiet=True, sample_params=None, seed=None):
         self.env = env
         self.B = env.n_envs
         self.peer = proxy if proxy is not None else xmlrpc.client.ServerProxy(url, allow_none=True)
@@ -33,6 +36,8 @@ class BatchedEpisodeDriver:
         self.train_every = train_every if train_every is not None else self.B
         self.reset_accumulators = reset_accumulators
         self.quiet = quiet
+        self.sample_params = sample_params
+        self.rng = np.random.default_rng(seed)
         self.finished_episodes = 0
         self.rl_steps = 0
         self.episode_returns = []
@@ -97,7 +102,8 @@ class BatchedEpisodeDriver:
             if self.finished_episodes // self.train_every > before:      # clientCFD.pde:72-81
                 self._rpc("train", self.train_steps, True)
                 self._rpc("save", self.train_steps, True)
-            self.env.reset(fin, reset_accumulators=self.reset_accumulators)
+            params = None if self.sample_params is None else self.sample_params(self.rng, fin)
+            self.env.reset(fin, reset_accumulators=self.reset_accumulators, params=params)
             # the reset environments produce their first observation during the next env.step (uncontrolled start,
             # actions ignored); what they hold now is the previous episode's last observation: not sent to the agent
             self._has_obs[fin] = False

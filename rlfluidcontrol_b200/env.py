@@ -22,6 +22,14 @@ class RlfcError(RuntimeError):
     pass
 
 
+class EnvParams(C.Structure):
+    """rlfc_env_params: the per-environment arguments of the AFCCylinder constructor."""
+    _fields_ = [("re", C.c_int), ("dR", C.c_float), ("gR", C.c_float), ("theta", C.c_float), ("t_step", C.c_float)]
+
+
+ENV_PARAM_KEYS = tuple(name for name, _ in EnvParams._fields_)
+
+
 class Config(C.Structure):
     _fields_ = [
         ("resolution", C.c_int), ("x_lengths", C.c_int), ("y_lengths", C.c_int), ("re", C.c_int),
@@ -30,6 +38,7 @@ class Config(C.Structure):
         ("episode_time", C.c_float), ("n_envs", C.c_int), ("device", C.c_int), ("exact", C.c_int),
         ("mg_max_iters", C.c_int), ("init_bdim_path", C.c_char_p), ("stream", C.c_void_p),
         ("n_groups", C.c_int), ("n_devices", C.c_int), ("adaptive_dt", C.c_int),
+        ("env_params", C.POINTER(EnvParams)),
     ]
 
 
@@ -62,6 +71,8 @@ def load_library():
     L.rlfc_env_destroy.argtypes = [vp]
     L.rlfc_env_destroy.restype = None
     L.rlfc_env_reset.argtypes = [vp, ip, C.c_int, C.c_int]
+    L.rlfc_env_reset_params.argtypes = [vp, ip, C.c_int, C.POINTER(EnvParams), C.c_int]
+    L.rlfc_env_get_params.argtypes = [vp, C.POINTER(EnvParams)]
     L.rlfc_env_step.argtypes = [vp, fp, fp, fp, ip]
     L.rlfc_env_step_device.argtypes = [vp, vp, vp, vp, vp]
     L.rlfc_env_substep.argtypes = [vp, fp, fp, fp]
@@ -103,10 +114,28 @@ def _fp(a):
     return a.ctypes.data_as(C.POINTER(C.c_float)) if a is not None else None
 
 
+def _env_params_array(params, cfg):
+    """A sequence of dicts (or a structured array with some of the fields re, dR, gR, theta, t_step) -> EnvParams[n]; a
+    missing key takes the scalar config's value."""
+    if isinstance(params, np.ndarray) and params.dtype.names:
+        params = [{k: params[k][i] for k in params.dtype.names} for i in range(len(params))]
+    params = list(params)
+    arr = (EnvParams * len(params))()
+    for i, p in enumerate(params):
+        unknown = set(p) - set(ENV_PARAM_KEYS)
+        if unknown:
+            raise TypeError(f"unknown environment parameter(s) {sorted(unknown)}")
+        for k in ENV_PARAM_KEYS:
+            setattr(arr[i], k, int(p[k]) if k == "re" and k in p else p.get(k, getattr(cfg, k)))
+    return arr
+
+
 class AFCCylinderBatch:
     """A batch of AFCCylinder environments on one GPU."""
 
-    def __init__(self, n_envs=1, init_state="default", device=-1, stream=None, **overrides):
+    def __init__(self, n_envs=1, init_state="default", device=-1, stream=None, env_params=None, **overrides):
+        """env_params: None (every environment uses the scalar config's re, dR, gR, theta, t_step), or n_envs entries, dicts
+        or a structured array, each environment's own constructor arguments (missing keys: the scalar config's)."""
         self._L = load_library()
         cfg = Config()
         self._L.rlfc_default_config(C.byref(cfg))
@@ -122,6 +151,11 @@ class AFCCylinderBatch:
             if not hasattr(cfg, k):
                 raise TypeError(f"unknown config field {k}")
             setattr(cfg, k, v)
+        if env_params is not None:
+            self._env_params = _env_params_array(env_params, cfg)
+            if len(self._env_params) != cfg.n_envs:
+                raise ValueError(f"env_params has {len(self._env_params)} entries for {cfg.n_envs} environments")
+            cfg.env_params = C.cast(self._env_params, C.POINTER(EnvParams))
         self.cfg = cfg
         h = C.c_void_p()
         rc = self._L.rlfc_env_create(C.byref(cfg), C.byref(h))
@@ -155,13 +189,36 @@ class AFCCylinderBatch:
             raise RlfcError(f"{what} failed ({rc}): {self._L.rlfc_last_error().decode()}")
 
     # -- reference-facing interface ---------------------------------------------------------
-    def reset(self, env_ids=None, reset_accumulators=False):
+    def reset(self, env_ids=None, reset_accumulators=False, params=None):
+        """setUpNewSim for the listed environments (None = all).  params (per-environment handles only): one entry per
+        listed environment, dicts or a structured array; the environment takes these constructor arguments (missing keys:
+        the scalar config's) with its geometry and Poisson hierarchy.  An invalid entry changes no environment."""
+        if params is not None:
+            ids = np.arange(self.n_envs, dtype=np.int32) if env_ids is None else np.ascontiguousarray(env_ids, dtype=np.int32)
+            arr = _env_params_array(params, self.cfg)
+            if len(arr) != len(ids):
+                raise ValueError(f"{len(arr)} parameter sets for {len(ids)} environments")
+            rc = self._L.rlfc_env_reset_params(self._h, ids.ctypes.data_as(C.POINTER(C.c_int)), len(ids), arr,
+                                               int(reset_accumulators))
+            self._check(rc, "rlfc_env_reset_params")
+            return
         if env_ids is None:
             rc = self._L.rlfc_env_reset(self._h, None, self.n_envs, int(reset_accumulators))
         else:
             ids = np.ascontiguousarray(env_ids, dtype=np.int32)
             rc = self._L.rlfc_env_reset(self._h, ids.ctypes.data_as(C.POINTER(C.c_int)), len(ids), int(reset_accumulators))
         self._check(rc, "rlfc_env_reset")
+
+    def params(self):
+        """Each environment's constructor arguments: a structured array with the fields re, dR, gR, theta, t_step."""
+        arr = (EnvParams * self.n_envs)()
+        self._check(self._L.rlfc_env_get_params(self._h, arr), "rlfc_env_get_params")
+        out = np.zeros(self.n_envs, dtype=[("re", np.int32), ("dR", np.float32), ("gR", np.float32), ("theta", np.float32),
+                                           ("t_step", np.float32)])
+        for i in range(self.n_envs):
+            for k in ENV_PARAM_KEYS:
+                out[k][i] = getattr(arr[i], k)
+        return out
 
     def step(self, actions, want_reward=True, want_done=True):
         """One RL step: actions (n_envs, 2) in [-1, 1] -> obs (n_envs, 2) = (Cl, Cd), reward, done."""
@@ -235,7 +292,8 @@ class AFCCylinderBatch:
 
     def get_coeffs(self, e, name, level=0):
         """Environment e's Poisson coefficients as its last step used them ("lower.x", "lower.y", "inv", "diag" at any
-        level, "c.x", "c.y" at level 0), reference layout.  Fixed mode: the same as `get_static`."""
+        level, "c.x", "c.y", "del.x", "del.y" at level 0), reference layout.  Fixed mode without env_params: the same as
+        `get_static`."""
         n, m = C.c_int(), C.c_int()
         self._check(self._L.rlfc_env_get_coeffs(self._h, e, name.encode(), level, None, C.byref(n), C.byref(m)), "rlfc_env_get_coeffs")
         out = np.empty((n.value, m.value), np.float32)
