@@ -96,6 +96,9 @@ typedef struct {
                            Poisson hierarchy.  Combines with adaptive_dt 0 and 1; has the same restrictions as adaptive_dt
                            (RLFC_EINVAL in slab mode and with the chained / wavefront smoothers).  The entries are copied
                            and validated before any device call; an invalid one fails with RLFC_EINVAL.                */
+  int   n_snapshots;    /* 0 (default) = no snapshot slots: nothing is allocated or launched for them.  > 0 = that many
+                           device slots, each holding one environment's complete state (rlfc_env_snapshot below; about
+                           0.93 MB per slot at the default grid).  RLFC_EINVAL if < 0, or > 0 in slab mode.             */
 } rlfc_config;
 
 void rlfc_default_config(rlfc_config *cfg);
@@ -152,8 +155,32 @@ int  rlfc_env_step_device(rlfc_env *env, const float *d_actions, float *d_obs, f
 int  rlfc_env_running(rlfc_env *env, int *n_running);
 
 /* Per-environment health flags, flags[n_envs]: bit 0 = a non-finite force was produced since the last reset (the
-   environment has diverged; SURVEY section 5 failure detection).  Synchronises the handle's stream. */
+   environment has diverged; SURVEY section 5 failure detection).  Bit 1 = the last restore aimed at the environment was
+   skipped because its slot was never written or holds a state of another parameter set (rlfc_env_restore_device; a restore
+   that applies clears it).  Synchronises the handle's stream. */
 int  rlfc_env_get_flags(rlfc_env *env, int *flags);
+
+/* Snapshots of complete environment states in the handle's rlfc_config.n_snapshots device slots (ALE cloneState /
+   restoreState for the batch).  A state is everything the next solver or RL step reads and the read-outs return: u, p
+   (the MG initial guess), xi, t, BDIM.t, dt, force, probes, callLearn, Cd, Cl, the last observation, the frozen and
+   non-finite flags, the MG iteration counts and the parameter set.  After rlfc_env_snapshot(e -> s) and
+   rlfc_env_restore(s -> e'), e' continues bit-identically to what e did from the snapshot, through every entry point.
+   A state moves only between environments with bitwise equal (re, dR, gR, theta, t_step); in adaptive mode a restore
+   rebuilds the destination's Poisson hierarchy from the restored dt.
+     rlfc_env_snapshot: environment env_ids[k] -> slot slots[k];  rlfc_env_restore: slot slots[k] -> environment env_ids[k].
+     keep_accumulators != 0: the destination keeps its own callLearn, Cd, Cl and obs (sketch globals that survive
+       setUpNewSim); 0 takes the snapshot's.  With S0 taken right after rlfc_env_reset(all, reset_accumulators = 1),
+       rlfc_env_restore(e, S0, k) is rlfc_env_reset({e}, reset_accumulators = !k) for every step that follows.
+   HOST arrays, synchronous on return, all or nothing: RLFC_EINVAL (and nothing changes) for a handle without slots, an id
+   or slot out of range, a destination listed twice, a restore from a slot never written or of another parameter set. */
+int  rlfc_env_snapshot(rlfc_env *env, const int *env_ids, const int *slots, int n);
+int  rlfc_env_restore(rlfc_env *env, const int *env_ids, const int *slots, int n, int keep_accumulators);
+/* Same with DEVICE int arrays of length n, asynchronous on the handle's stream (the host never sees the ids).  Defined for
+   every input: a pair with an entry out of range is skipped (a negative entry is the way to skip one, e.g.
+   slots = where(done, S0, -1)); of pairs with the same destination the last in-range pair wins; a restore from a slot never
+   written or of another parameter set is skipped and sets flags bit 1 of the destination. */
+int  rlfc_env_snapshot_device(rlfc_env *env, const int *d_env_ids, const int *d_slots, int n);
+int  rlfc_env_restore_device(rlfc_env *env, const int *d_env_ids, const int *d_slots, int n, int keep_accumulators);
 
 /* One solver step (AFCCylinder.update2) without the draw() accumulation.  HOST pointers.
      actions [n_envs][2] (NULL = keep current xi); force [n_envs][2] raw (fx, fy) = -pressForce;

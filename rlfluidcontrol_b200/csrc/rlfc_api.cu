@@ -51,6 +51,8 @@ struct rlfc_env {
   std::vector<float> h_nu, h_dRD;          // [B] host copies of sp.env_nu, sp.env_dRD
   std::vector<int> h_nbx, h_nby;           // [B] host copies of sp.env_nband_x / y
   int* d_skip = nullptr;                   // [B] mask of launch_poisson_rebuild* outside a step (1 = keep)
+  SnapSlots snap{};                        // rlfc_config.n_snapshots slots (snap.S = 0: none)
+  int *snap_env = nullptr, *snap_slot = nullptr;   // [max(B, S)] the pairs of a host snapshot / restore call
   int device = 0;
   cudaStream_t stream = nullptr;
   bool own_stream = false;
@@ -337,6 +339,92 @@ int upload_env_scalars(rlfc_env* E) {
   CU(cudaMemcpyAsync(const_cast<float*>(sp.env_dRD), E->h_dRD.data(), B * sizeof(float), cudaMemcpyHostToDevice, E->stream));
   CU(cudaMemcpyAsync(const_cast<int*>(sp.env_nband_x), E->h_nbx.data(), B * sizeof(int), cudaMemcpyHostToDevice, E->stream));
   CU(cudaMemcpyAsync(const_cast<int*>(sp.env_nband_y), E->h_nby.data(), B * sizeof(int), cudaMemcpyHostToDevice, E->stream));
+  CU(cudaStreamSynchronize(E->stream));
+  return RLFC_OK;
+}
+
+// ---- snapshot slots (rlfc_config.n_snapshots) ----
+
+// the bits of a parameter tuple as a slot header stores them (words 1 .. 5)
+void param_bits(const rlfc_env_params& p, unsigned out[5]) {
+  std::memcpy(&out[0], &p.re, 4); std::memcpy(&out[1], &p.dR, 4); std::memcpy(&out[2], &p.gR, 4);
+  std::memcpy(&out[3], &p.theta, 4); std::memcpy(&out[4], &p.t_step, 4);
+}
+
+// E->params -> snap.env_par (what a restore compares a slot's header with)
+int upload_snapshot_params(rlfc_env* E) {
+  if (!E->snap.S) return RLFC_OK;
+  const int B = (int)E->params.size();
+  std::vector<unsigned> bits((size_t)5 * B);
+  for (int e = 0; e < B; e++) {
+    unsigned b[5];
+    param_bits(E->params[e], b);
+    for (int w = 0; w < 5; w++) bits[(size_t)w * B + e] = b[w];
+  }
+  CU(cudaMemcpyAsync(E->snap.env_par, bits.data(), bits.size() * sizeof(unsigned), cudaMemcpyHostToDevice, E->stream));
+  CU(cudaStreamSynchronize(E->stream));
+  return RLFC_OK;
+}
+
+// the one copy path of both variants: n pairs in device memory, enqueued on the handle's stream; an adaptive-dt restore
+// then rebuilds the Poisson hierarchy of the environments it restored from their restored dt
+int snapshot_enqueue(rlfc_env* E, const int* d_env, const int* d_slot, int n, int restore, int keep) {
+  if (n <= 0) return RLFC_OK;
+  SolverParams& sp = E->whole.sp;
+  const bool rebuild = restore && sp.adaptive;
+  if (rebuild) CU(cudaMemsetAsync(E->d_skip, 1, sp.B * sizeof(int), E->stream));   // nonzero = keep; the copy clears
+  E->run("k_snapshot_copy", 0, [&] {
+    return launch_snapshot_copy(sp, E->snap, E->uAx, E->uAy, d_env, d_slot, n, restore, keep, rebuild ? E->d_skip : nullptr, E->stream);
+  });
+  if (rebuild) {
+    E->run("k_poisson_rebuild0", 0, [&] { return launch_poisson_rebuild0(sp, E->d_skip, E->stream); });
+    E->run("k_poisson_rebuild_coarse", 0, [&] { return launch_poisson_rebuild_coarse(sp, E->d_skip, E->stream); });
+  }
+  CU(cudaGetLastError());
+  return RLFC_OK;
+}
+
+int snapshot_check_handle(rlfc_env* E, int n, bool have_ptrs) {
+  if (!E) return fail(RLFC_EINVAL, "null handle");
+  if (!E->snap.S) return fail(RLFC_EINVAL, "the handle has no snapshot slots (rlfc_config.n_snapshots = 0)");
+  if (n < 0) return fail(RLFC_EINVAL, "bad pair count");
+  if (n > 0 && !have_ptrs) return fail(RLFC_EINVAL, "null argument");
+  return RLFC_OK;
+}
+
+// the host variants: validated all or nothing, then the device path, synchronous on return
+int snapshot_host(rlfc_env* E, const int* env_ids, const int* slots, int n, int restore, int keep) {
+  int rc = snapshot_check_handle(E, n, env_ids && slots);
+  if (rc) return rc;
+  const int B = E->sp.B, S = E->snap.S;
+  std::vector<char> seen(restore ? B : S, 0);
+  for (int k = 0; k < n; k++) {
+    if (env_ids[k] < 0 || env_ids[k] >= B) return fail(RLFC_EINVAL, "env id " + std::to_string(env_ids[k]) + " out of range");
+    if (slots[k] < 0 || slots[k] >= S) return fail(RLFC_EINVAL, "slot " + std::to_string(slots[k]) + " out of range");
+    const int dst = restore ? env_ids[k] : slots[k];
+    if (seen[dst]++) return fail(RLFC_EINVAL, std::string(restore ? "env id " : "slot ") + std::to_string(dst) + " listed twice");
+  }
+  CU(cudaSetDevice(E->device));
+  if (restore && n > 0) {
+    // device snapshots write slots the host never sees: read the headers back
+    std::vector<unsigned> hdr((size_t)kSnapHdr * S);
+    CU(cudaMemcpyAsync(hdr.data(), E->snap.hdr, hdr.size() * sizeof(unsigned), cudaMemcpyDeviceToHost, E->stream));
+    CU(cudaStreamSynchronize(E->stream));
+    for (int k = 0; k < n; k++) {
+      const int e = env_ids[k], s = slots[k];
+      if (!hdr[s]) return fail(RLFC_EINVAL, "slot " + std::to_string(s) + " has never been written");
+      unsigned b[5];
+      param_bits(E->params[e], b);
+      for (int w = 0; w < 5; w++)
+        if (hdr[(size_t)(1 + w) * S + s] != b[w])
+          return fail(RLFC_EINVAL, "slot " + std::to_string(s) + " holds a state of another parameter set than env " + std::to_string(e));
+    }
+  }
+  if (n > 0) {
+    CU(cudaMemcpyAsync(E->snap_env, env_ids, n * sizeof(int), cudaMemcpyHostToDevice, E->stream));
+    CU(cudaMemcpyAsync(E->snap_slot, slots, n * sizeof(int), cudaMemcpyHostToDevice, E->stream));
+  }
+  if ((rc = snapshot_enqueue(E, E->snap_env, E->snap_slot, n, restore, keep))) return rc;
   CU(cudaStreamSynchronize(E->stream));
   return RLFC_OK;
 }
@@ -757,6 +845,9 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
   if (cfg->substeps < 1 || cfg->mg_max_iters < 1) return fail(RLFC_EINVAL, "substeps and mg_max_iters must be >= 1");
   if (cfg->adaptive_dt != 0 && cfg->adaptive_dt != 1) return fail(RLFC_EINVAL, "adaptive_dt must be 0 or 1");
   if (cfg->adaptive_dt && cfg->n_devices > 1) return fail(RLFC_EINVAL, "adaptive_dt is not available in slab mode (n_devices > 1)");
+  if (cfg->n_snapshots < 0) return fail(RLFC_EINVAL, "n_snapshots must be >= 0");
+  if (cfg->n_snapshots > 0 && cfg->n_devices > 1)
+    return fail(RLFC_EINVAL, "n_snapshots is not available in slab mode (n_devices > 1)");
   // per-environment parameters: every set validated and its geometry built before any device call
   std::vector<EnvGeometry> env_geo;
   std::vector<int> env_set;
@@ -1096,6 +1187,16 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
   sp.sc.rr_part = nullptr;
   TRY(E->dmalloc(&sp.sc.psum, B));
   TRY(E->dmalloc(&sp.sc.dt, B));
+  if (cfg->n_snapshots > 0) {
+    // snapshot slots (solver.h SnapSlots); the zeroed headers mark every slot unwritten
+    SnapSlots& s = E->snap;
+    s.S = cfg->n_snapshots;
+    TRY(E->dmalloc(&s.ux, sp.stride * s.S)); TRY(E->dmalloc(&s.uy, sp.stride * s.S)); TRY(E->dmalloc(&s.p, sp.stride * s.S));
+    TRY(E->dmalloc(&s.rec, (size_t)kSnapWords * s.S)); TRY(E->dmalloc(&s.hdr, (size_t)kSnapHdr * s.S));
+    TRY(E->dmalloc(&s.env_par, (size_t)5 * B)); TRY(E->dmalloc(&s.refused, B));
+    TRY(E->dmalloc(&E->snap_env, std::max(B, s.S))); TRY(E->dmalloc(&E->snap_slot, std::max(B, s.S)));
+    TRY(upload_snapshot_params(E));
+  }
   {
     // Field.sum: segment summaries (exact_sum.cuh) or the plain dependent-add chain (k_psum).  The chain costs
     // 6 cycles per cell of pure latency whatever the batch size and next to no issue slots; the summaries cost
@@ -1357,6 +1458,7 @@ int rlfc_env_reset_params(rlfc_env* E, const int* env_ids, int n, const rlfc_env
   for (int k = 0; k < n; k++)
     if ((rc = upload_env_geometry(E, env_ids[k], params[k], geo[set[k]]))) return rc;
   if ((rc = upload_env_scalars(E))) return rc;
+  if ((rc = upload_snapshot_params(E))) return rc;
   if ((rc = rlfc_env_reset(E, env_ids, n, reset_accumulators))) return rc;   // (sc.dt = the new t_step*resolution)
   // the new hierarchies, of the listed environments only
   std::vector<int> skip(B);
@@ -1563,10 +1665,34 @@ int rlfc_env_running(rlfc_env* E, int* n_running) {
 int rlfc_env_get_flags(rlfc_env* E, int* flags) {
   if (!E || !flags) return fail(RLFC_EINVAL, "null argument");
   CU(cudaSetDevice(E->device));
+  std::vector<int> refused(E->snap.S ? E->sp.B : 0);
   CU(cudaMemcpyAsync(E->h_done, E->sp.sc.non_finite, E->sp.B * sizeof(int), cudaMemcpyDeviceToHost, E->stream));
+  if (E->snap.S) CU(cudaMemcpyAsync(refused.data(), E->snap.refused, E->sp.B * sizeof(int), cudaMemcpyDeviceToHost, E->stream));
   CU(cudaStreamSynchronize(E->stream));
-  for (int e = 0; e < E->sp.B; e++) flags[e] = E->h_done[e] ? 1 : 0;
+  for (int e = 0; e < E->sp.B; e++) flags[e] = (E->h_done[e] ? 1 : 0) | (E->snap.S && refused[e] ? 2 : 0);
   return RLFC_OK;
+}
+
+int rlfc_env_snapshot(rlfc_env* E, const int* env_ids, const int* slots, int n) {
+  return snapshot_host(E, env_ids, slots, n, 0, 0);
+}
+
+int rlfc_env_restore(rlfc_env* E, const int* env_ids, const int* slots, int n, int keep_accumulators) {
+  return snapshot_host(E, env_ids, slots, n, 1, keep_accumulators != 0);
+}
+
+int rlfc_env_snapshot_device(rlfc_env* E, const int* d_env_ids, const int* d_slots, int n) {
+  int rc = snapshot_check_handle(E, n, d_env_ids && d_slots);
+  if (rc) return rc;
+  CU(cudaSetDevice(E->device));
+  return snapshot_enqueue(E, d_env_ids, d_slots, n, 0, 0);
+}
+
+int rlfc_env_restore_device(rlfc_env* E, const int* d_env_ids, const int* d_slots, int n, int keep_accumulators) {
+  int rc = snapshot_check_handle(E, n, d_env_ids && d_slots);
+  if (rc) return rc;
+  CU(cudaSetDevice(E->device));
+  return snapshot_enqueue(E, d_env_ids, d_slots, n, 1, keep_accumulators != 0);
 }
 
 int rlfc_env_check_cfl(rlfc_env* E, float* dt) {

@@ -166,6 +166,21 @@ struct SolverParams {
   const int   *env_nband_x, *env_nband_y;   // [B] band faces of each environment (<= nband_x / nband_y)
 };
 
+// Snapshot slots (rlfc_config.n_snapshots; snapshot.cuh).  Slot s holds one environment's state: u.x, u.y (step-start
+// buffer A) and p (lev[0].x) at s * stride in the level-0 pitched layout, the scalar record rec[w * S + s] (word w of
+// snap_word in snapshot.cuh) and the header hdr[w * S + s]: w = 0 written (0 = never), w = 1 .. 5 the bits of the
+// (re, dR, gR, theta, t_step) tuple of the environment it was taken from.
+constexpr int kSnapWords = 48;
+constexpr int kSnapHdr = 6;
+struct SnapSlots {
+  int S;                    // slots (0 = none allocated)
+  float *ux, *uy, *p;       // [S] fields at s * stride
+  unsigned *rec;            // [kSnapWords][S]
+  unsigned *hdr;            // [kSnapHdr][S]
+  unsigned *env_par;        // [5][B] each environment's parameter tuple (bits), what a restore compares the header with
+  int *refused;             // [B] 1 = the last restore into the environment was skipped (rlfc_env_get_flags bit 1)
+};
+
 #ifdef __CUDACC__
 // true = block `blk` of `nblk` (a kernel's row-block or strip index) belongs to another device
 __device__ __forceinline__ bool slab_skip(unsigned blk, unsigned nblk, int rank, int n) {
@@ -238,5 +253,13 @@ int launch_poisson_rebuild_coarse(const SolverParams& P, const int* skip, cudaSt
 int launch_set_actions(const SolverParams& P, const float* d_actions, int mode, cudaStream_t st);
 int launch_emit_obs(const SolverParams& P, const float* d_actions, float* d_obs, float* d_reward, int* d_done,
                     cudaStream_t st);
+// Snapshot copy of n (environment, slot) pairs, device arrays d_env[n], d_slot[n]: restore = 0 copies environment
+// d_env[k]'s state (u.x = ux, u.y = uy, p = P.lev[0].x, P.sc) to slot d_slot[k], restore = 1 slot d_slot[k] to
+// environment d_env[k].  A pair with an entry out of range is skipped; of pairs with the same destination the last wins;
+// a restore from an unwritten slot or a slot of another parameter tuple is skipped and sets refused[e] (else clears it).
+// keep_accumulators = 1: a restore leaves callLearn, Cd, Cl and obs as they are.  skip != nullptr: a restore writes
+// skip[e] = 0 for every environment it restored (the mask of a following launch_poisson_rebuild*).
+int launch_snapshot_copy(const SolverParams& P, const SnapSlots& s, float* ux, float* uy, const int* d_env, const int* d_slot,
+                         int n, int restore, int keep_accumulators, int* skip, cudaStream_t st);
 
 }  // namespace rlfc

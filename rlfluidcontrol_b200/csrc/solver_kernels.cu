@@ -1935,3 +1935,5 @@ int launch_emit_obs(const SolverParams& q, const float* d_actions, float* d_obs,
 }
 
 }  // namespace rlfc
+
+#include "snapshot.cuh"

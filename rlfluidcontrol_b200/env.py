@@ -38,7 +38,7 @@ class Config(C.Structure):
         ("episode_time", C.c_float), ("n_envs", C.c_int), ("device", C.c_int), ("exact", C.c_int),
         ("mg_max_iters", C.c_int), ("init_bdim_path", C.c_char_p), ("stream", C.c_void_p),
         ("n_groups", C.c_int), ("n_devices", C.c_int), ("adaptive_dt", C.c_int),
-        ("env_params", C.POINTER(EnvParams)),
+        ("env_params", C.POINTER(EnvParams)), ("n_snapshots", C.c_int),
     ]
 
 
@@ -89,6 +89,10 @@ def load_library():
     L.rlfc_env_get_coeffs.argtypes = [vp, C.c_int, C.c_char_p, C.c_int, fp, ip, ip]
     L.rlfc_env_running.argtypes = [vp, ip]
     L.rlfc_env_get_flags.argtypes = [vp, ip]
+    L.rlfc_env_snapshot.argtypes = [vp, ip, ip, C.c_int]
+    L.rlfc_env_restore.argtypes = [vp, ip, ip, C.c_int, C.c_int]
+    L.rlfc_env_snapshot_device.argtypes = [vp, vp, vp, C.c_int]
+    L.rlfc_env_restore_device.argtypes = [vp, vp, vp, C.c_int, C.c_int]
     L.rlfc_env_field_sum.argtypes = [vp, fp]
     L.rlfc_env_field_sum_stats.argtypes = [vp, ip]
     L.rlfc_env_get_static.argtypes = [vp, C.c_char_p, C.c_int, fp, ip, ip]
@@ -112,6 +116,10 @@ def load_library():
 
 def _fp(a):
     return a.ctypes.data_as(C.POINTER(C.c_float)) if a is not None else None
+
+
+def _ip(a):
+    return a.ctypes.data_as(C.POINTER(C.c_int))
 
 
 def _env_params_array(params, cfg):
@@ -238,6 +246,40 @@ class AFCCylinderBatch:
                                           C.c_void_p(d_done) if d_done else None)
         self._check(rc, "rlfc_env_step_device")
 
+    def snapshot(self, env_ids, slots):
+        """Environment env_ids[k]'s complete state -> snapshot slot slots[k] (AFCCylinderBatch(n, n_snapshots=K) has K
+        slots).  All or nothing: an id or slot out of range or a slot listed twice raises and changes nothing."""
+        ids, sl = self._pairs(env_ids, slots)
+        self._check(self._L.rlfc_env_snapshot(self._h, _ip(ids), _ip(sl), len(ids)), "rlfc_env_snapshot")
+
+    def restore(self, env_ids, slots, keep_accumulators=False):
+        """Slot slots[k] -> environment env_ids[k], which then continues bit-identically to the environment the slot was
+        taken from.  keep_accumulators: the destination keeps its own callLearn, Cd, Cl and obs.  All or nothing: also
+        raises for a slot never written or taken from an environment with another parameter set."""
+        ids, sl = self._pairs(env_ids, slots)
+        self._check(self._L.rlfc_env_restore(self._h, _ip(ids), _ip(sl), len(ids), int(keep_accumulators)), "rlfc_env_restore")
+
+    def snapshot_device(self, d_env_ids, d_slots, n):
+        """snapshot() with device int32 arrays of length n (data_ptr() ints), asynchronous on the handle's stream.  Pairs
+        with an entry out of range (e.g. -1) are skipped; of pairs with the same slot the last wins."""
+        self._check(self._L.rlfc_env_snapshot_device(self._h, C.c_void_p(d_env_ids), C.c_void_p(d_slots), int(n)),
+                    "rlfc_env_snapshot_device")
+
+    def restore_device(self, d_env_ids, d_slots, n, keep_accumulators=False):
+        """restore() with device int32 arrays, asynchronous: restore_device(arange(B), where(done, S0, -1), B) resets the
+        finished environments without the host.  Pairs out of range are skipped, the last pair per environment wins, and a
+        restore from an unwritten slot or one of another parameter set is skipped and sets flags() bit 1."""
+        self._check(self._L.rlfc_env_restore_device(self._h, C.c_void_p(d_env_ids), C.c_void_p(d_slots), int(n),
+                                                    int(keep_accumulators)), "rlfc_env_restore_device")
+
+    @staticmethod
+    def _pairs(env_ids, slots):
+        ids = np.ascontiguousarray(env_ids, dtype=np.int32).reshape(-1)
+        sl = np.ascontiguousarray(slots, dtype=np.int32).reshape(-1)
+        if len(ids) != len(sl):
+            raise ValueError(f"{len(ids)} environment ids for {len(sl)} slots")
+        return ids, sl
+
     def update2(self, actions=None, want_probes=False):
         """One solver step.  Returns force (n_envs, 2) [, probes (n_envs, 32)].
 
@@ -307,7 +349,8 @@ class AFCCylinderBatch:
         return n.value
 
     def flags(self):
-        """Per-environment health flags (bit 0: a non-finite force was produced since the last reset)."""
+        """Per-environment health flags (bit 0: a non-finite force was produced since the last reset; bit 1: the last
+        restore aimed at the environment was skipped, its slot unwritten or of another parameter set)."""
         f = np.empty(self.n_envs, np.int32)
         self._check(self._L.rlfc_env_get_flags(self._h, f.ctypes.data_as(C.POINTER(C.c_int))), "rlfc_env_get_flags")
         return f

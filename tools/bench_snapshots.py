@@ -1,0 +1,121 @@
+"""Snapshot slots (rlfc_config.n_snapshots) on one GPU: 256 default-grid environments from init.bdim and 256 slots.
+
+  * restore_device and snapshot_device of all 256 environments (slot e <-> environment e): time from CUDA events over
+    --calls calls, and the effective bandwidth (bytes read + bytes written, of the three fields and the scalar record, per
+    second).  Alternated in the same run with cudaMemcpyAsync device-to-device of the same number of bytes (one block,
+    larger than the L2, so it comes from HBM like the copies).
+  * rlfc_env_reset of all 256 environments against rlfc_env_restore of all 256 from the slot S0 taken right after a
+    reset (host clock around each call; both synchronise before they return).
+
+The cases run --rounds times, alternated, to show the spread.  Records the card's name and power limit in the same run.
+Prints one JSON object; --out also writes it.  Needs a GPU.
+    python tools/bench_snapshots.py --out profiles/snapshots_b200.json
+"""
+from __future__ import annotations
+
+import argparse
+import ctypes as C
+import json
+import sys
+import time
+from pathlib import Path
+
+import numpy as np
+
+ROOT = Path(__file__).resolve().parents[1]
+sys.path.insert(0, str(ROOT))
+sys.path.insert(0, str(ROOT / "tools"))
+
+from bench_adaptive import card_info  # noqa: E402
+
+SNAP_WORDS = 48   # solver.h kSnapWords: the scalar record, 32-bit words
+
+
+def main():
+    ap = argparse.ArgumentParser(description=__doc__, formatter_class=argparse.RawDescriptionHelpFormatter)
+    ap.add_argument("--envs", type=int, default=256)
+    ap.add_argument("--calls", type=int, default=20)
+    ap.add_argument("--rounds", type=int, default=3)
+    ap.add_argument("--out", default=None)
+    args = ap.parse_args()
+    import torch
+    if not torch.cuda.is_available():
+        raise SystemExit("no CUDA device: this benchmark measures the GPU path only")
+    import rlfluidcontrol_b200 as R
+    R.load_library()
+    cudart = C.CDLL("libcudart.so.12")       # the runtime librlfc.so is linked against
+    cudart.cudaMemcpyAsync.argtypes = [C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]
+    B, K = args.envs, args.calls
+    stream = torch.cuda.Stream()
+    env = R.AFCCylinderBatch(B, n_snapshots=B, stream=stream.cuda_stream)
+    P = (env.m + 7) // 8 * 8
+    field_bytes = env.n * P * 4
+    moved = B * (3 * field_bytes + SNAP_WORDS * 4)          # bytes read = bytes written per call
+    src = torch.empty(moved, dtype=torch.uint8, device="cuda")
+    dst = torch.empty_like(src)
+    src.fill_(1)
+    ids = torch.arange(B, dtype=torch.int32, device="cuda")
+    env.reset(None, reset_accumulators=True)
+    torch.cuda.synchronize()
+
+    def memcpy():
+        rc = cudart.cudaMemcpyAsync(C.c_void_p(dst.data_ptr()), C.c_void_p(src.data_ptr()), moved, 3, C.c_void_p(stream.cuda_stream))
+        assert rc == 0, rc
+
+    cases = {
+        "snapshot_device": lambda: env.snapshot_device(ids.data_ptr(), ids.data_ptr(), B),
+        "restore_device": lambda: env.restore_device(ids.data_ptr(), ids.data_ptr(), B),
+        "memcpy_d2d": memcpy,
+    }
+
+    def timed(fn):
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record(stream)
+        for _ in range(K):
+            fn()
+        e1.record(stream)
+        e1.synchronize()
+        return e0.elapsed_time(e1) / K
+
+    for fn in cases.values():                 # warm-up (the first snapshot also writes every slot)
+        fn(); fn()
+    torch.cuda.synchronize()
+    res = {k: [] for k in cases}
+    for _ in range(args.rounds):
+        for name, fn in cases.items():
+            ms = timed(fn)
+            res[name].append({"ms_per_call": ms, "gb_per_s": 2 * moved / (ms * 1e-3) / 1e9})
+    assert not env.flags().any()
+
+    # host reset of every environment against a restore of every environment from S0
+    env.reset(None, reset_accumulators=True)
+    env.snapshot([0], [0])
+    all_ids, zeros = np.arange(B, dtype=np.int32), np.zeros(B, np.int32)
+    host = {"rlfc_env_reset": [], "rlfc_env_restore": []}
+    for _ in range(args.rounds * 3):
+        t0 = time.perf_counter()
+        env.reset(all_ids, reset_accumulators=True)
+        host["rlfc_env_reset"].append((time.perf_counter() - t0) * 1e3)
+        t0 = time.perf_counter()
+        env.restore(all_ids, zeros)
+        host["rlfc_env_restore"].append((time.perf_counter() - t0) * 1e3)
+    env.close()
+
+    summary = {k: {"median_ms": float(np.median([x["ms_per_call"] for x in v])),
+                   "median_gb_per_s": float(np.median([x["gb_per_s"] for x in v]))} for k, v in res.items()}
+    for k in ("snapshot_device", "restore_device"):
+        summary[k]["over_memcpy"] = summary[k]["median_gb_per_s"] / summary["memcpy_d2d"]["median_gb_per_s"]
+    for k, v in host.items():
+        summary[k] = {"median_ms": float(np.median(v))}
+    out = {"workload": f"{B} default-grid envs ({env.n}x{env.m} incl. ghosts, pitch {P}) from init.bdim, {B} slots; "
+                       f"{K} calls per timing, {args.rounds} alternated rounds; {moved} bytes read and as many written per "
+                       f"call of all {B} pairs",
+           "card": card_info(), "device": res, "host_ms": host, "summary": summary}
+    s = json.dumps(out, indent=1)
+    print(s)
+    if args.out:
+        Path(args.out).write_text(s + "\n")
+
+
+if __name__ == "__main__":
+    main()
