@@ -55,6 +55,19 @@ typedef struct {
   float dR, gR, theta, t_step;
 } rlfc_env_params;
 
+/* A flow sensor: the value of one field at one point, sampled on the device after every solver step (rlfc_env_get_sensors).
+   (x, y) are grid coordinates as Body and SaveScalar use them: one unit is one cell, the main cylinder's centre is at
+   (x_lengths*resolution/4, y_lengths*resolution/2).  The value is the reference's Field.linear(x, y) (Field.pde:175-190) of
+   that field with the field's own btype: the point is clamped to [0.5, n-1.5] x [0.5, m-1.5], then shifted by +0.5 in x
+   for u.x and in y for u.y, and interpolated bilinearly.  A p sensor at a SaveScalar point equals that probe bit for bit. */
+#define RLFC_SENSOR_P   0   /* pressure p (btype 0)                                                  */
+#define RLFC_SENSOR_UX  1   /* velocity u.x (btype 1)                                                */
+#define RLFC_SENSOR_UY  2   /* velocity u.y (btype 2)                                                */
+typedef struct {
+  int   field;          /* RLFC_SENSOR_P, _UX or _UY                                                */
+  float x, y;
+} rlfc_sensor;
+
 typedef struct {
   /* defaults (rlfc_default_config) reproduce clientCFD.pde:5-14,94-96 and AFCCylinder.pde:4-7 */
   int   resolution;     /* 24   cells per main-cylinder diameter                     */
@@ -99,6 +112,12 @@ typedef struct {
   int   n_snapshots;    /* 0 (default) = no snapshot slots: nothing is allocated or launched for them.  > 0 = that many
                            device slots, each holding one environment's complete state (rlfc_env_snapshot below; about
                            0.93 MB per slot at the default grid).  RLFC_EINVAL if < 0, or > 0 in slab mode.             */
+  int   n_sensors;      /* 0 (default) = no sensors: nothing is allocated or launched for them.  > 0 = the number of entries
+                           of `sensors`, sampled in every environment (rlfc_env_get_sensors below).  The set is handle-wide
+                           and fixed at create.  RLFC_EINVAL if < 0, or > 0 in slab mode.                               */
+  const rlfc_sensor *sensors;
+                        /* n_sensors entries, copied and validated before any device call: RLFC_EINVAL for NULL with
+                           n_sensors > 0, a field outside RLFC_SENSOR_P .. RLFC_SENSOR_UY or a non-finite coordinate.     */
 } rlfc_config;
 
 void rlfc_default_config(rlfc_config *cfg);
@@ -181,6 +200,18 @@ int  rlfc_env_restore(rlfc_env *env, const int *env_ids, const int *slots, int n
    written or of another parameter set is skipped and sets flags bit 1 of the destination. */
 int  rlfc_env_snapshot_device(rlfc_env *env, const int *d_env_ids, const int *d_slots, int n);
 int  rlfc_env_restore_device(rlfc_env *env, const int *d_env_ids, const int *d_slots, int n, int keep_accumulators);
+
+/* The sensors (rlfc_config.sensors) of every environment, out[n_envs][n_sensors].  Each environment's sensors hold the
+   sample of its most recent solver step, taken from the state the next step starts from -- the u and p rlfc_env_get_fields
+   returns -- so right after any call sensor == Field.linear of rlfc_env_get_fields(e).  An environment that takes no part
+   in a solver step keeps its values: after rlfc_env_step an environment holds the sample of the step that completed its
+   observation window (its sensor observation), one whose episode is over keeps its last one.  rlfc_env_reset and
+   rlfc_env_reset_params leave sensors alone (the next step overwrites them); snapshots carry them with the state.
+   HOST memory, synchronises the handle's stream.  RLFC_EINVAL for a handle created without sensors. */
+int  rlfc_env_get_sensors(rlfc_env *env, float *out);
+/* Same into DEVICE memory: one device-to-device copy on the handle's stream, no sync.  Enqueued after
+   rlfc_env_step_device, it gives a GPU-resident policy its observation without the host. */
+int  rlfc_env_get_sensors_device(rlfc_env *env, float *d_out);
 
 /* One solver step (AFCCylinder.update2) without the draw() accumulation.  HOST pointers.
      actions [n_envs][2] (NULL = keep current xi); force [n_envs][2] raw (fx, fy) = -pressForce;

@@ -194,18 +194,19 @@ HostLevel coarsen(const HostLevel& F) {
   return C;
 }
 
-// Field.linear Field.pde:175-190 index/fraction part for a btype-0 field
-Sample resolve_sample(int n, int m, float x0, float y0) {
+}  // namespace
+
+Sample resolve_sample(int n, int m, float x0, float y0, int btype) {
   Sample sp;
   float x = fmin2(fmax2(0.5f, x0), n - 1.5f);
+  if (btype == 1) x += 0.5f;
   int i = (int)x; if (i > n - 2) i = n - 2;
   float y = fmin2(fmax2(0.5f, y0), m - 1.5f);
+  if (btype == 2) y += 0.5f;
   int j = (int)y; if (j > m - 2) j = m - 2;
   sp.i = i; sp.j = j; sp.s = x - i; sp.t = y - j;
   return sp;
 }
-
-}  // namespace
 
 int build_geometry(const rlfc_config& cfg, Geometry& g, std::string& err, bool hierarchy) {
   if (cfg.resolution < 2 || cfg.x_lengths < 1 || cfg.y_lengths < 1 || cfg.re <= 0) {
@@ -316,7 +317,7 @@ int build_geometry(const rlfc_config& cfg, Geometry& g, std::string& err, bool h
   for (int e = 0; e < kCircleVerts; e++) {
     const Edge& o = main_cyl.edge[e];
     ForceEdge fe;
-    fe.at = resolve_sample(n, m, o.cx, o.cy);
+    fe.at = resolve_sample(n, m, o.cx, o.cy, 0);
     fe.l = o.l; fe.nx = o.nx; fe.ny = o.ny;
     g.force_edges.push_back(fe);
   }
@@ -329,7 +330,7 @@ int build_geometry(const rlfc_config& cfg, Geometry& g, std::string& err, bool h
     for (int i = 0; i < RLFC_NUM_PROBES; i++) {
       float xp = fcos((float)i / RLFC_NUM_PROBES * kPi * 2) * res / 2 + cx;
       float yp = fsin((float)i / RLFC_NUM_PROBES * kPi * 2) * res / 2 + cy;
-      g.probes.push_back(resolve_sample(n, m, xp, yp));
+      g.probes.push_back(resolve_sample(n, m, xp, yp, 0));
     }
   }
   return RLFC_OK;

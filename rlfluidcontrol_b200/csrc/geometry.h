@@ -29,6 +29,10 @@ struct Sample {
   float s, t;
 };
 
+// Field.linear's index/fraction part (Field.pde:175-190) for a field of the given btype (0 = p, 1 = u.x, 2 = u.y): the
+// point clamped to [0.5, n-1.5] x [0.5, m-1.5], shifted by +0.5 in x (btype 1) or y (btype 2), truncated and capped at n-2 / m-2
+Sample resolve_sample(int n, int m, float x0, float y0, int btype);
+
 struct ForceEdge {    // one polygon edge of body 0: OrthoNormal {l, nx, ny, cen}
   Sample at;
   float l, nx, ny;

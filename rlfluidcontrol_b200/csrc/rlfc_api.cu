@@ -53,6 +53,7 @@ struct rlfc_env {
   int* d_skip = nullptr;                   // [B] mask of launch_poisson_rebuild* outside a step (1 = keep)
   SnapSlots snap{};                        // rlfc_config.n_snapshots slots (snap.S = 0: none)
   int *snap_env = nullptr, *snap_slot = nullptr;   // [max(B, S)] the pairs of a host snapshot / restore call
+  SensorSet sens{};                        // rlfc_config.sensors of the whole batch (sens.n = 0: none)
   int device = 0;
   cudaStream_t stream = nullptr;
   bool own_stream = false;
@@ -77,6 +78,7 @@ struct rlfc_env {
     int e0 = 0, B = 0;
     SolverParams sp{};                       // view of the batch arrays restricted to [e0, e0 + B); lev[0].x = pressure buffer A
     SolverParams spB{};                      // same view with lev[0].x = pressure buffer B (p ping-pongs A -> B -> A per half step)
+    SensorSet sens{};                        // the view's sensors (out at e0 * n)
     float *uAx = nullptr, *uAy = nullptr, *uBx = nullptr, *uBy = nullptr, *uCx = nullptr, *uCy = nullptr;
     cudaStream_t st = nullptr;               // group 0 runs on the handle's stream
     cudaEvent_t done = nullptr;
@@ -374,7 +376,8 @@ int snapshot_enqueue(rlfc_env* E, const int* d_env, const int* d_slot, int n, in
   const bool rebuild = restore && sp.adaptive;
   if (rebuild) CU(cudaMemsetAsync(E->d_skip, 1, sp.B * sizeof(int), E->stream));   // nonzero = keep; the copy clears
   E->run("k_snapshot_copy", 0, [&] {
-    return launch_snapshot_copy(sp, E->snap, E->uAx, E->uAy, d_env, d_slot, n, restore, keep, rebuild ? E->d_skip : nullptr, E->stream);
+    return launch_snapshot_copy(sp, E->snap, E->sens, E->uAx, E->uAy, d_env, d_slot, n, restore, keep, rebuild ? E->d_skip : nullptr,
+                                E->stream);
   });
   if (rebuild) {
     E->run("k_poisson_rebuild0", 0, [&] { return launch_poisson_rebuild0(sp, E->d_skip, E->stream); });
@@ -519,6 +522,8 @@ int solver_step_eager(rlfc_env* E, Group& G, int accumulate) {
   if ((rc = project_eager(E, G, G.uCx, G.uCy, 1))) return rc;
   if (!sp.fast_bc)
     E->run("k_heun", 6, [&] { return launch_heun(sp, G.uCx, G.uCy, G.uBx, G.uBy, G.uAx, G.uAy, st); }, st);
+  // (before k_force, which freezes an environment at the end of its window: this step's sample is its observation)
+  if (G.sens.n > 0) E->run("k_sensors", 0, [&] { return launch_sensors(sp, G.sens, G.uAx, G.uAy, st); }, st);
   E->run("k_force", 0, [&] { return launch_force(sp, accumulate, st); }, st);
   CU(cudaGetLastError());
   return RLFC_OK;
@@ -594,6 +599,7 @@ int build_step_graph(rlfc_env* E, Group& G, int accumulate) {
   if (!rc) rc = capture_half_step(E, G, st, G.uBx, G.uBy, G.uAx, G.uAy, G.uCx, G.uCy, 1, &n_outer);
   if (!rc) {
     if (!G.sp.fast_bc) n_outer += launch_heun(G.sp, G.uCx, G.uCy, G.uBx, G.uBy, G.uAx, G.uAy, st);
+    n_outer += launch_sensors(G.sp, G.sens, G.uAx, G.uAy, st);   // (nothing without sensors; before k_force, see solver_step_eager)
     n_outer += launch_force(G.sp, accumulate, st);
   }
   cudaGraph_t graph = nullptr;
@@ -848,6 +854,18 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
   if (cfg->n_snapshots < 0) return fail(RLFC_EINVAL, "n_snapshots must be >= 0");
   if (cfg->n_snapshots > 0 && cfg->n_devices > 1)
     return fail(RLFC_EINVAL, "n_snapshots is not available in slab mode (n_devices > 1)");
+  if (cfg->n_sensors < 0) return fail(RLFC_EINVAL, "n_sensors must be >= 0");
+  if (cfg->n_sensors > 0) {
+    if (!cfg->sensors) return fail(RLFC_EINVAL, "sensors is NULL with n_sensors > 0");
+    if (cfg->n_devices > 1) return fail(RLFC_EINVAL, "n_sensors is not available in slab mode (n_devices > 1)");
+    for (int k = 0; k < cfg->n_sensors; k++) {
+      const rlfc_sensor& s = cfg->sensors[k];
+      if (s.field < RLFC_SENSOR_P || s.field > RLFC_SENSOR_UY)
+        return fail(RLFC_EINVAL, "sensors[" + std::to_string(k) + "]: field must be 0 (p), 1 (u.x) or 2 (u.y)");
+      if (!std::isfinite(s.x) || !std::isfinite(s.y))
+        return fail(RLFC_EINVAL, "sensors[" + std::to_string(k) + "]: coordinates must be finite");
+    }
+  }
   // per-environment parameters: every set validated and its geometry built before any device call
   std::vector<EnvGeometry> env_geo;
   std::vector<int> env_set;
@@ -865,6 +883,7 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
   E->cfg.init_bdim_path = nullptr;
   E->env_mode = cfg->env_params != nullptr;
   E->cfg.env_params = nullptr;              // (copied into E->params below)
+  E->cfg.sensors = nullptr;                 // (resolved into E->sens below)
   int rc = RLFC_OK;
   auto bail = [&](int code) { rlfc_env_destroy(E); return code; };
 
@@ -1148,6 +1167,18 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
     if (sp.nforce > 64 || sp.nprobe > 64) return bail(fail(RLFC_EINVAL, "too many force/probe points"));
     TRY(upload_vec(E, fp, &sp.force_pts));
     TRY(upload_vec(E, pp, &sp.probe_pts));
+    // sensors: resolved once to their cell and fractions (Field.linear with the field's btype = the sensor's field code)
+    std::vector<SensorPt> sv;
+    for (int k = 0; k < cfg->n_sensors; k++) {
+      const rlfc_sensor& s = cfg->sensors[k];
+      const Sample a = resolve_sample(g.n, g.m, s.x, s.y, s.field);
+      sv.push_back({a.i, a.j, a.s, a.t, s.field});
+    }
+    E->sens.n = (int)sv.size();
+    if (E->sens.n > 0) {
+      TRY(upload_vec(E, sv, &E->sens.pts));
+      TRY(E->dmalloc(&E->sens.out, (size_t)B * E->sens.n));
+    }
   }
   // per-env fields
   const size_t S = sp.stride * B;
@@ -1193,6 +1224,7 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
     s.S = cfg->n_snapshots;
     TRY(E->dmalloc(&s.ux, sp.stride * s.S)); TRY(E->dmalloc(&s.uy, sp.stride * s.S)); TRY(E->dmalloc(&s.p, sp.stride * s.S));
     TRY(E->dmalloc(&s.rec, (size_t)kSnapWords * s.S)); TRY(E->dmalloc(&s.hdr, (size_t)kSnapHdr * s.S));
+    if (E->sens.n > 0) TRY(E->dmalloc(&s.sens, (size_t)E->sens.n * s.S));
     TRY(E->dmalloc(&s.env_par, (size_t)5 * B)); TRY(E->dmalloc(&s.refused, B));
     TRY(E->dmalloc(&E->snap_env, std::max(B, s.S))); TRY(E->dmalloc(&E->snap_slot, std::max(B, s.S)));
     TRY(upload_snapshot_params(E));
@@ -1302,6 +1334,8 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
     v.sc.callLearn += e0; v.sc.Cd += e0; v.sc.Cl += e0; v.sc.obs += 2 * e0; v.sc.active += e0; v.sc.iters += 2 * e0;
     v.sc.frozen += e0; v.sc.non_finite += e0;
     v.sc.psum += e0; v.sc.any_active += g;
+    G.sens = E->sens;
+    if (G.sens.out) G.sens.out += (size_t)e0 * G.sens.n;
     if (v.xs_recs) {
       v.xs_ctot += (size_t)e0 * v.xs_nchunks;
       v.xs_cflag += (size_t)e0 * v.xs_nchunks; v.xs_epoch += e0;
@@ -1320,7 +1354,7 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
     else if (cudaStreamCreateWithFlags(&G.st, cudaStreamNonBlocking) != cudaSuccess) return bail(fail(RLFC_ECUDA, "cudaStreamCreate failed"));
     if (cudaEventCreateWithFlags(&G.done, cudaEventDisableTiming) != cudaSuccess) return bail(fail(RLFC_ECUDA, "cudaEventCreate failed"));
   }
-  E->whole.e0 = 0; E->whole.B = B; E->whole.sp = sp; E->whole.st = E->stream;
+  E->whole.e0 = 0; E->whole.B = B; E->whole.sp = sp; E->whole.sens = E->sens; E->whole.st = E->stream;
   for (int l = 0; l < sp.chain_levels; l++) {
     ChainLevel& ch = E->whole.sp.lev[l].ch;
     ch.ticket = E->chain_tickets + (size_t)n_groups * kMaxLevels + l;
@@ -1693,6 +1727,23 @@ int rlfc_env_restore_device(rlfc_env* E, const int* d_env_ids, const int* d_slot
   if (rc) return rc;
   CU(cudaSetDevice(E->device));
   return snapshot_enqueue(E, d_env_ids, d_slots, n, 1, keep_accumulators != 0);
+}
+
+int rlfc_env_get_sensors(rlfc_env* E, float* out) {
+  if (!E || !out) return fail(RLFC_EINVAL, "null argument");
+  if (!E->sens.n) return fail(RLFC_EINVAL, "the handle has no sensors (rlfc_config.n_sensors = 0)");
+  CU(cudaSetDevice(E->device));
+  CU(cudaMemcpyAsync(out, E->sens.out, (size_t)E->sp.B * E->sens.n * sizeof(float), cudaMemcpyDeviceToHost, E->stream));
+  CU(cudaStreamSynchronize(E->stream));
+  return RLFC_OK;
+}
+
+int rlfc_env_get_sensors_device(rlfc_env* E, float* d_out) {
+  if (!E || !d_out) return fail(RLFC_EINVAL, "null argument");
+  if (!E->sens.n) return fail(RLFC_EINVAL, "the handle has no sensors (rlfc_config.n_sensors = 0)");
+  CU(cudaSetDevice(E->device));
+  CU(cudaMemcpyAsync(d_out, E->sens.out, (size_t)E->sp.B * E->sens.n * sizeof(float), cudaMemcpyDeviceToDevice, E->stream));
+  return RLFC_OK;
 }
 
 int rlfc_env_check_cfl(rlfc_env* E, float* dt) {

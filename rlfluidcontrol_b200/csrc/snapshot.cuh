@@ -5,7 +5,7 @@
 // fields (u.x, u.y of the step-start buffer A, p = lev[0].x, the MG initial guess) and the scalar record of snap_word.
 // The slot layout is solver.h SnapSlots.  One kernel serves both directions: grid (chunks, pairs), each pair moves three
 // contiguous blocks of n*P floats (16-byte accesses; stride is a multiple of 32 floats, so every block starts 128-byte
-// aligned), and the first chunk of a pair also moves the scalar record.
+// aligned), and the first chunk of a pair also moves the scalar record and the sensors.
 #pragma once
 #include "solver.h"
 
@@ -23,6 +23,7 @@ struct SnapArgs {
   size_t stride4;                              // level-0 per-environment stride in float4
   int nv;                                      // float4 of one field that are copied (n*P/4)
   int B, nprobe;
+  SensorSet sens;                              // the environments' sensors (sens.n = 0: none)
   const int *env, *slot;
   int n, restore, keep;
   int* skip;
@@ -101,13 +102,20 @@ __global__ void __launch_bounds__(kSnapThreads) k_snapshot_copy(const __grid_con
       }
       if (!a.restore && w < kSnapHdr) a.s.hdr[(size_t)w * S + s] = w == 0 ? 1u : a.s.env_par[(size_t)(w - 1) * B + e];
     }
+    if (blockIdx.x == 0)
+      for (int k2 = threadIdx.x; k2 < a.sens.n; k2 += kSnapThreads) {
+        float* x = a.sens.out + (size_t)e * a.sens.n + k2;
+        float* r = a.s.sens + (size_t)s * a.sens.n + k2;
+        if (a.restore) *x = *r;
+        else *r = *x;
+      }
   }
 }
 
 }  // namespace
 
-int launch_snapshot_copy(const SolverParams& q, const SnapSlots& s, float* ux, float* uy, const int* d_env, const int* d_slot,
-                         int n, int restore, int keep_accumulators, int* skip, cudaStream_t st) {
+int launch_snapshot_copy(const SolverParams& q, const SnapSlots& s, const SensorSet& sens, float* ux, float* uy, const int* d_env,
+                         const int* d_slot, int n, int restore, int keep_accumulators, int* skip, cudaStream_t st) {
   if (n <= 0) return 0;
   SnapArgs a{};
   a.s = s;
@@ -119,6 +127,7 @@ int launch_snapshot_copy(const SolverParams& q, const SnapSlots& s, float* ux, f
   a.nv = q.n * q.P / 4;
   a.B = q.B;
   a.nprobe = q.nprobe;
+  a.sens = sens;
   a.env = d_env;
   a.slot = d_slot;
   a.n = n;

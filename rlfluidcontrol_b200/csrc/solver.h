@@ -67,6 +67,7 @@ struct BandFace {           // a face where the BDIM blend differs from the iden
 };
 
 struct SamplePt { int i, j; float s, t; };
+struct SensorPt { int i, j; float s, t; int field; };   // a sample point of field 0 = p, 1 = u.x, 2 = u.y (rlfc_sensor)
 struct ForcePt { int i, j; float s, t, l, nx, ny; };
 
 // Per-env scalar state (struct of arrays on the device)
@@ -166,16 +167,26 @@ struct SolverParams {
   const int   *env_nband_x, *env_nband_y;   // [B] band faces of each environment (<= nband_x / nband_y)
 };
 
+// Flow sensors (rlfc_config.sensors) of a view of the batch; n = 0: none, nothing is launched for them.  Kept out of
+// SolverParams: growing that struct by even 8 bytes changes the register allocation of k_resid_down0<true> (-Xptxas -v).
+struct SensorSet {
+  const SensorPt* pts;      // [n] resolved sample points
+  int n;
+  float* out;               // [B][n] the sample of each environment's last solver step (k_sensors)
+};
+
 // Snapshot slots (rlfc_config.n_snapshots; snapshot.cuh).  Slot s holds one environment's state: u.x, u.y (step-start
 // buffer A) and p (lev[0].x) at s * stride in the level-0 pitched layout, the scalar record rec[w * S + s] (word w of
 // snap_word in snapshot.cuh) and the header hdr[w * S + s]: w = 0 written (0 = never), w = 1 .. 5 the bits of the
-// (re, dR, gR, theta, t_step) tuple of the environment it was taken from.
+// (re, dR, gR, theta, t_step) tuple of the environment it was taken from.  With sensors, slot s also holds the
+// environment's n sensor values at sens + s * n (SensorSet).
 constexpr int kSnapWords = 48;
 constexpr int kSnapHdr = 6;
 struct SnapSlots {
   int S;                    // slots (0 = none allocated)
   float *ux, *uy, *p;       // [S] fields at s * stride
   unsigned *rec;            // [kSnapWords][S]
+  float *sens;              // [S][n] sensors (nullptr without sensors)
   unsigned *hdr;            // [kSnapHdr][S]
   unsigned *env_par;        // [5][B] each environment's parameter tuple (bits), what a restore compares the header with
   int *refused;             // [B] 1 = the last restore into the environment was skipped (rlfc_env_get_flags bit 1)
@@ -238,6 +249,9 @@ int launch_heun(const SolverParams& P, const float* ucx, const float* ucy, const
                 float* uax, float* uay, cudaStream_t st);
 // force + probes + time advance; accumulate != 0 applies the clientCFD.draw() accumulation
 int launch_force(const SolverParams& P, int accumulate, cudaStream_t st);
+// flow sensors: s.out[e][k] = Field.linear of sensor k's field (u.x = ux, u.y = uy, p = P.lev[0].x) for every environment
+// not frozen.  A step runs it after the corrector's last kernel and before launch_force, which may freeze the environment
+int launch_sensors(const SolverParams& P, const SensorSet& s, const float* ux, const float* uy, cudaStream_t st);
 // BDIM.checkCFL of every environment's current velocity: d_dt[B] = min(1/(max(|ux|+|uy|) + 3 nu), 1)
 int launch_check_cfl(const SolverParams& P, const float* ux, const float* uy, float* d_dt, cudaStream_t st);
 // adaptive mode, start of a solver step: sc.dt[e] = BDIM.checkCFL of u for every environment not frozen (frozen ones keep theirs)
@@ -258,8 +272,9 @@ int launch_emit_obs(const SolverParams& P, const float* d_actions, float* d_obs,
 // environment d_env[k].  A pair with an entry out of range is skipped; of pairs with the same destination the last wins;
 // a restore from an unwritten slot or a slot of another parameter tuple is skipped and sets refused[e] (else clears it).
 // keep_accumulators = 1: a restore leaves callLearn, Cd, Cl and obs as they are.  skip != nullptr: a restore writes
-// skip[e] = 0 for every environment it restored (the mask of a following launch_poisson_rebuild*).
-int launch_snapshot_copy(const SolverParams& P, const SnapSlots& s, float* ux, float* uy, const int* d_env, const int* d_slot,
-                         int n, int restore, int keep_accumulators, int* skip, cudaStream_t st);
+// skip[e] = 0 for every environment it restored (the mask of a following launch_poisson_rebuild*).  The environments' sensors
+// `sens` move with the state (sens.n = 0: none).
+int launch_snapshot_copy(const SolverParams& P, const SnapSlots& s, const SensorSet& sens, float* ux, float* uy, const int* d_env,
+                         const int* d_slot, int n, int restore, int keep_accumulators, int* skip, cudaStream_t st);
 
 }  // namespace rlfc

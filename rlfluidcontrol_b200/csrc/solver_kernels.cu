@@ -16,6 +16,7 @@
 //   k_project_shift p += -sum(p)/N, velocity correction by grad p        VectorField.pde:136-139
 //   k_bc          u.setBC after the projection                          VectorField.pde:140
 //   k_heun        u = (u + us) * 0.5                                     BDIM.pde:95-96
+//   k_sensors     Field.linear of p / u.x / u.y at the user's points     Field.pde:175-190
 //   k_force       pressForce + probes + time + draw() accumulation       Body.pde:296-303, SaveScalar.pde:61-72, clientCFD.pde:39-47
 #include "solver.h"
 #include "smooth_rows.cuh"
@@ -1350,6 +1351,18 @@ k_force(const __grid_constant__ SolverParams q, int accumulate) {
   }
 }
 
+// flow sensors: thread (blockIdx.x * 128 + threadIdx.x) samples one sensor of environment blockIdx.y (Field.linear of its
+// field; the btype shift is resolved on the host)
+__global__ void __launch_bounds__(128)
+k_sensors(const SensorSet ss, const float* __restrict__ p, const float* __restrict__ ux, const float* __restrict__ uy,
+          const int* __restrict__ frozen, size_t stride, int P) {
+  const int e = blockIdx.y, k = blockIdx.x * blockDim.x + threadIdx.x;
+  if (k >= ss.n || frozen[e]) return;
+  const SensorPt s = ss.pts[k];
+  const float* a = (s.field == 0 ? p : s.field == 1 ? ux : uy) + (size_t)e * stride;
+  ss.out[(size_t)e * ss.n + k] = sample_linear(a, P, s.i, s.j, s.s, s.t);
+}
+
 // Start of a call.  mode 0 (single solver steps): xi = act where given, every env runs.  mode 1 (RL step): the reference
 // changes xi only when callAction returns, i.e. right after an observation was emitted (clientCFD.pde:44-54): an env
 // that has not reached its first callLearn boundary yet (t <= initTime after a reset, or mid-window after an episode
@@ -1890,6 +1903,12 @@ int launch_heun(const SolverParams& q, const float* ucx, const float* ucy, const
                 float* uax, float* uay, cudaStream_t st) {
   dim3 blk(32, 8);
   k_heun<<<grid2d(q.m, q.n, q.B, blk), blk, 0, st>>>(ucx, ucy, ubx, uby, uax, uay, q.n, q.m, q.P, q.stride, q.sc.frozen, q.slab_rank, q.slab_n);
+  return 1;
+}
+
+int launch_sensors(const SolverParams& q, const SensorSet& s, const float* ux, const float* uy, cudaStream_t st) {
+  if (s.n <= 0) return 0;
+  k_sensors<<<dim3((s.n + 127) / 128, q.B), 128, 0, st>>>(s, q.lev[0].x, ux, uy, q.sc.frozen, q.stride, q.P);
   return 1;
 }
 

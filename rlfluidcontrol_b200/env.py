@@ -30,6 +30,14 @@ class EnvParams(C.Structure):
 ENV_PARAM_KEYS = tuple(name for name, _ in EnvParams._fields_)
 
 
+class Sensor(C.Structure):
+    """rlfc_sensor: Field.linear of one field at one point (grid coordinates, one unit = one cell)."""
+    _fields_ = [("field", C.c_int), ("x", C.c_float), ("y", C.c_float)]
+
+
+SENSOR_FIELDS = {"p": 0, "ux": 1, "uy": 2}   # RLFC_SENSOR_P, _UX, _UY
+
+
 class Config(C.Structure):
     _fields_ = [
         ("resolution", C.c_int), ("x_lengths", C.c_int), ("y_lengths", C.c_int), ("re", C.c_int),
@@ -39,6 +47,7 @@ class Config(C.Structure):
         ("mg_max_iters", C.c_int), ("init_bdim_path", C.c_char_p), ("stream", C.c_void_p),
         ("n_groups", C.c_int), ("n_devices", C.c_int), ("adaptive_dt", C.c_int),
         ("env_params", C.POINTER(EnvParams)), ("n_snapshots", C.c_int),
+        ("n_sensors", C.c_int), ("sensors", C.POINTER(Sensor)),
     ]
 
 
@@ -93,6 +102,8 @@ def load_library():
     L.rlfc_env_restore.argtypes = [vp, ip, ip, C.c_int, C.c_int]
     L.rlfc_env_snapshot_device.argtypes = [vp, vp, vp, C.c_int]
     L.rlfc_env_restore_device.argtypes = [vp, vp, vp, C.c_int, C.c_int]
+    L.rlfc_env_get_sensors.argtypes = [vp, fp]
+    L.rlfc_env_get_sensors_device.argtypes = [vp, vp]
     L.rlfc_env_field_sum.argtypes = [vp, fp]
     L.rlfc_env_field_sum_stats.argtypes = [vp, ip]
     L.rlfc_env_get_static.argtypes = [vp, C.c_char_p, C.c_int, fp, ip, ip]
@@ -138,12 +149,25 @@ def _env_params_array(params, cfg):
     return arr
 
 
+def _sensor_array(sensors):
+    """A sequence of (field, x, y) with field "p", "ux" or "uy" -> rlfc_sensor[n]."""
+    sensors = list(sensors)
+    arr = (Sensor * len(sensors))()
+    for i, (field, x, y) in enumerate(sensors):
+        if field not in SENSOR_FIELDS:
+            raise ValueError(f"sensor {i}: unknown field {field!r} (expected one of {sorted(SENSOR_FIELDS)})")
+        arr[i].field, arr[i].x, arr[i].y = SENSOR_FIELDS[field], float(x), float(y)
+    return arr
+
+
 class AFCCylinderBatch:
     """A batch of AFCCylinder environments on one GPU."""
 
-    def __init__(self, n_envs=1, init_state="default", device=-1, stream=None, env_params=None, **overrides):
+    def __init__(self, n_envs=1, init_state="default", device=-1, stream=None, env_params=None, sensors=None, **overrides):
         """env_params: None (every environment uses the scalar config's re, dR, gR, theta, t_step), or n_envs entries, dicts
-        or a structured array, each environment's own constructor arguments (missing keys: the scalar config's)."""
+        or a structured array, each environment's own constructor arguments (missing keys: the scalar config's).
+        sensors: None, or a sequence of (field, x, y), field "p", "ux" or "uy", (x, y) in grid coordinates: the flow
+        sampled in every environment after each of its solver steps (`sensors()`)."""
         self._L = load_library()
         cfg = Config()
         self._L.rlfc_default_config(C.byref(cfg))
@@ -164,6 +188,11 @@ class AFCCylinderBatch:
             if len(self._env_params) != cfg.n_envs:
                 raise ValueError(f"env_params has {len(self._env_params)} entries for {cfg.n_envs} environments")
             cfg.env_params = C.cast(self._env_params, C.POINTER(EnvParams))
+        if sensors is not None:
+            self._sensors = _sensor_array(sensors)
+            cfg.n_sensors = len(self._sensors)
+            cfg.sensors = C.cast(self._sensors, C.POINTER(Sensor))
+        self.n_sensors = cfg.n_sensors
         self.cfg = cfg
         h = C.c_void_p()
         rc = self._L.rlfc_env_create(C.byref(cfg), C.byref(h))
@@ -271,6 +300,18 @@ class AFCCylinderBatch:
         restore from an unwritten slot or one of another parameter set is skipped and sets flags() bit 1."""
         self._check(self._L.rlfc_env_restore_device(self._h, C.c_void_p(d_env_ids), C.c_void_p(d_slots), int(n),
                                                     int(keep_accumulators)), "rlfc_env_restore_device")
+
+    def sensors(self):
+        """(n_envs, n_sensors) float32: each environment's sensors, sampled after its most recent solver step from the
+        state `get_fields` returns.  `step(a)` followed by `sensors()` gives the sensor observation of each environment."""
+        out = np.empty((self.n_envs, self.n_sensors), np.float32)
+        self._check(self._L.rlfc_env_get_sensors(self._h, _fp(out)), "rlfc_env_get_sensors")
+        return out
+
+    def sensors_device(self, d_out):
+        """sensors() into a device float32 buffer of n_envs * n_sensors (data_ptr() int), asynchronous on the handle's
+        stream: after `step_device` it gives a GPU-resident policy its observation without the host."""
+        self._check(self._L.rlfc_env_get_sensors_device(self._h, C.c_void_p(d_out)), "rlfc_env_get_sensors_device")
 
     @staticmethod
     def _pairs(env_ids, slots):
