@@ -118,6 +118,16 @@ typedef struct {
   const rlfc_sensor *sensors;
                         /* n_sensors entries, copied and validated before any device call: RLFC_EINVAL for NULL with
                            n_sensors > 0, a field outside RLFC_SENSOR_P .. RLFC_SENSOR_UY or a non-finite coordinate.     */
+  int   n_param_sets;   /* 0 (default) = no parameter library: nothing is allocated or launched for it.  > 0 = the number of
+                           entries of `param_sets`, a library of constructor arguments that rlfc_env_reset_sets(_device)
+                           switches environments to on the device.  Puts the handle in per-environment mode: without
+                           env_params it is a handle created with env_params = n_envs copies of the scalar config's set.
+                           About 3.25 MB of device memory per distinct set at the default grid.                        */
+  const rlfc_env_params *param_sets;
+                        /* n_param_sets entries, copied, validated (as env_params) and their geometries built at create,
+                           before any device call.  RLFC_EINVAL for n_param_sets < 0, NULL with n_param_sets > 0, an
+                           invalid entry (the message names param_sets[k]), slab mode, or a grid with chained or wavefront
+                           levels.                                                                                     */
 } rlfc_config;
 
 void rlfc_default_config(rlfc_config *cfg);
@@ -138,8 +148,23 @@ int  rlfc_env_reset(rlfc_env *env, const int *env_ids, int n, int reset_accumula
 int  rlfc_env_reset_params(rlfc_env *env, const int *env_ids, int n, const rlfc_env_params *params,
                            int reset_accumulators);
 /* params[n_envs]: each environment's constructor arguments (the scalar config's for every environment of a handle
-   created without env_params). */
+   created without env_params), as the environments hold them now, including sets switched by rlfc_env_reset_sets_device. */
 int  rlfc_env_get_params(rlfc_env *env, rlfc_env_params *params);
+
+/* setUpNewSim into the parameter library (rlfc_config.param_sets), handles with a library only.  Environment env_ids[k]
+   becomes what rlfc_env_reset_params({env_ids[k]}, {param_sets[sets[k]]}, reset_accumulators) makes it -- the set's
+   geometry, nu, dR*D, dt = t_step*resolution and Poisson hierarchy, u and p from the init state, t = 0, xi = 0, BDIM.t from
+   the checkpoint, force = 0, the frozen and non-finite flags cleared, with reset_accumulators callLearn = substeps and
+   Cd = Cl = obs = 0 -- bit for bit, without building anything on the host.  Sensors, probes, MG iteration counts and flags
+   bit 1 stay as they are (as with rlfc_env_reset).  A later rlfc_env_reset keeps the set; rlfc_env_reset_params puts the
+   environment back on its own geometry slot.
+   HOST arrays, synchronous on return, all or nothing: RLFC_EINVAL (and nothing changes) for a handle without a library, an
+   id or set out of range, or an environment listed twice. */
+int  rlfc_env_reset_sets(rlfc_env *env, const int *env_ids, const int *sets, int n, int reset_accumulators);
+/* Same with DEVICE int arrays of length n, asynchronous on the handle's stream.  Defined for every input: a pair with an
+   entry out of range is skipped (a negative set is the way to skip one, e.g. sets = where(done, draw, -1)); of pairs with
+   the same environment the last in-range pair wins. */
+int  rlfc_env_reset_sets_device(rlfc_env *env, const int *d_env_ids, const int *d_sets, int n, int reset_accumulators);
 
 /* One RL step for every environment, with the cadence of clientCFD.draw() (clientCFD.pde:35-55).  All pointers are
    HOST memory.

@@ -54,6 +54,12 @@ struct rlfc_env {
   SnapSlots snap{};                        // rlfc_config.n_snapshots slots (snap.S = 0: none)
   int *snap_env = nullptr, *snap_slot = nullptr;   // [max(B, S)] the pairs of a host snapshot / restore call
   SensorSet sens{};                        // rlfc_config.sensors of the whole batch (sens.n = 0: none)
+  // parameter library (rlfc_config.param_sets; lib.L = 0: none)
+  ParamLib lib{};
+  std::vector<rlfc_env_params> lib_params; // [L] the sets as given
+  std::vector<LibSet> h_lib;               // [L] host copy of lib.sets
+  std::vector<int> h_env_set;              // [B] host copy of lib.env_set as of the last sync_env_sets
+  int *set_env = nullptr, *set_ids = nullptr;   // [B] the pairs of a host rlfc_env_reset_sets call
   int device = 0;
   cudaStream_t stream = nullptr;
   bool own_stream = false;
@@ -251,13 +257,14 @@ struct EnvGeometry {
 
 // Validates the parameter sets p[0 .. n-1] for the grid of `cfg` and builds their geometries (without the hierarchy, which
 // the device builds): equal sets once, on a few threads.  set_of[k] = the entry of `out` that p[k] uses.  Touches no device.
+// Messages name the entry as table[k].
 int build_env_geometries(const rlfc_config& cfg, const rlfc_env_params* p, int n, std::vector<EnvGeometry>& out,
-                         std::vector<int>& set_of, std::string& err) {
+                         std::vector<int>& set_of, std::string& err, const char* table = "env_params") {
   std::vector<int> uniq;                   // index into p of the first occurrence of each distinct set
   set_of.assign(n, 0);
   for (int k = 0; k < n; k++) {
     const rlfc_env_params& q = p[k];
-    const std::string at = "env_params[" + std::to_string(k) + "]: ";
+    const std::string at = std::string(table) + "[" + std::to_string(k) + "]: ";
     if (q.re < 1) { err = at + "re must be >= 1"; return RLFC_EINVAL; }
     if (!(q.dR > 0 && q.dR <= 1)) { err = at + "dR must be in (0, 1]"; return RLFC_EINVAL; }
     if (!(q.gR >= 0) || !std::isfinite(q.gR)) { err = at + "gR must be finite and >= 0"; return RLFC_EINVAL; }
@@ -302,28 +309,36 @@ int build_env_geometries(const rlfc_config& cfg, const rlfc_env_params* p, int n
   for (auto& x : th) x.join();
   for (size_t u = 0; u < uniq.size(); u++)
     if (rc[u]) {
-      err = "env_params[" + std::to_string(uniq[u]) + "]: " + msg[u];
+      err = std::string(table) + "[" + std::to_string(uniq[u]) + "]: " + msg[u];
       return RLFC_EINVAL;
     }
   return RLFC_OK;
 }
 
-// environment e's parameters: its geometry into slot e (del, the body-velocity basis, the band lists) and the host copies of
-// its scalars; the caller uploads the per-environment arrays and rebuilds the hierarchy
-int upload_env_geometry(rlfc_env* E, int e, const rlfc_env_params& p, const EnvGeometry& G) {
+// a geometry into geometry slot `slot` (del, the body-velocity basis, the band lists)
+int upload_slot_geometry(rlfc_env* E, int slot, const EnvGeometry& G) {
   SolverParams& sp = E->sp;
   const Geometry& g = G.g;
   const std::vector<float>* src[10] = {&g.del_x, &g.del_y, &g.w1_x, &g.w2_x, &g.ry1_x, &g.ry2_x, &g.w1_y, &g.w2_y, &g.rx1_y, &g.rx2_y};
   const float* dst[10] = {sp.del_x, sp.del_y, sp.w1_x, sp.w2_x, sp.ry1_x, sp.ry2_x, sp.w1_y, sp.w2_y, sp.rx1_y, sp.rx2_y};
   for (int f = 0; f < 10; f++)
-    CU(cudaMemcpy2DAsync(const_cast<float*>(dst[f]) + (size_t)e * sp.stride, sp.P * sizeof(float), src[f]->data(),
+    CU(cudaMemcpy2DAsync(const_cast<float*>(dst[f]) + (size_t)slot * sp.stride, sp.P * sizeof(float), src[f]->data(),
                          g.m * sizeof(float), g.m * sizeof(float), g.n, cudaMemcpyHostToDevice, E->stream));
   if (!G.bx.empty())
-    CU(cudaMemcpyAsync(const_cast<BandFace*>(sp.band_x) + (size_t)e * sp.nband_x, G.bx.data(), G.bx.size() * sizeof(BandFace),
+    CU(cudaMemcpyAsync(const_cast<BandFace*>(sp.band_x) + (size_t)slot * sp.nband_x, G.bx.data(), G.bx.size() * sizeof(BandFace),
                        cudaMemcpyHostToDevice, E->stream));
   if (!G.by.empty())
-    CU(cudaMemcpyAsync(const_cast<BandFace*>(sp.band_y) + (size_t)e * sp.nband_y, G.by.data(), G.by.size() * sizeof(BandFace),
+    CU(cudaMemcpyAsync(const_cast<BandFace*>(sp.band_y) + (size_t)slot * sp.nband_y, G.by.data(), G.by.size() * sizeof(BandFace),
                        cudaMemcpyHostToDevice, E->stream));
+  return RLFC_OK;
+}
+
+// environment e's parameters: its geometry into slot e and the host copies of its scalars; the caller uploads the
+// per-environment arrays and rebuilds the hierarchy
+int upload_env_geometry(rlfc_env* E, int e, const rlfc_env_params& p, const EnvGeometry& G) {
+  const Geometry& g = G.g;
+  int rc = upload_slot_geometry(E, e, G);
+  if (rc) return rc;
   E->params[e] = p;
   E->dt0[e] = g.dt;
   E->h_nu[e] = g.nu;
@@ -341,7 +356,66 @@ int upload_env_scalars(rlfc_env* E) {
   CU(cudaMemcpyAsync(const_cast<float*>(sp.env_dRD), E->h_dRD.data(), B * sizeof(float), cudaMemcpyHostToDevice, E->stream));
   CU(cudaMemcpyAsync(const_cast<int*>(sp.env_nband_x), E->h_nbx.data(), B * sizeof(int), cudaMemcpyHostToDevice, E->stream));
   CU(cudaMemcpyAsync(const_cast<int*>(sp.env_nband_y), E->h_nby.data(), B * sizeof(int), cudaMemcpyHostToDevice, E->stream));
+  if (E->lib.L) {   // (env_slot is written at create otherwise; with a library the device changes it too)
+    std::vector<int> slot(B);
+    for (int e = 0; e < (int)B; e++) slot[e] = E->h_env_set[e] < 0 ? e : E->h_lib[E->h_env_set[e]].slot;
+    CU(cudaMemcpyAsync(const_cast<int*>(sp.env_slot), slot.data(), B * sizeof(int), cudaMemcpyHostToDevice, E->stream));
+    CU(cudaMemcpyAsync(E->lib.env_set, E->h_env_set.data(), B * sizeof(int), cudaMemcpyHostToDevice, E->stream));
+  }
   CU(cudaStreamSynchronize(E->stream));
+  return RLFC_OK;
+}
+
+// ---- parameter library (rlfc_config.param_sets) ----
+
+// The host copies of what an environment holds (params, dt0, h_nu, h_dRD, h_nbx, h_nby) go stale once the device switches
+// it to a library set.  Host entry points that read them call this first: it synchronises the handle's stream, reads
+// lib.env_set back and refreshes the copies of the environments that hold a library set.  (An environment back on its own
+// slot got its copies from rlfc_env_reset_params, which put it there.)  Without a library it does nothing.
+int sync_env_sets(rlfc_env* E) {
+  if (!E->lib.L) return RLFC_OK;
+  const int B = E->sp.B;
+  CU(cudaMemcpyAsync(E->h_env_set.data(), E->lib.env_set, B * sizeof(int), cudaMemcpyDeviceToHost, E->stream));
+  CU(cudaStreamSynchronize(E->stream));
+  for (int e = 0; e < B; e++) {
+    const int s = E->h_env_set[e];
+    if (s < 0) continue;
+    const LibSet& L = E->h_lib[s];
+    E->params[e] = E->lib_params[s];
+    E->dt0[e] = L.dt0;
+    E->h_nu[e] = L.nu; E->h_dRD[e] = L.dRD;
+    E->h_nbx[e] = L.nbx; E->h_nby[e] = L.nby;
+  }
+  return RLFC_OK;
+}
+
+// environment e's geometry slot per the host copies (after sync_env_sets)
+int slot_of(const rlfc_env* E, int e) {
+  if (!E->env_mode) return 0;
+  return E->lib.L && E->h_env_set[e] >= 0 ? E->h_lib[E->h_env_set[e]].slot : e;
+}
+
+// the one reset path of both variants: n pairs in device memory, enqueued on the handle's stream, then the Poisson
+// hierarchies of the environments reset, from their new del and dt (fixed and adaptive dt alike)
+int reset_sets_enqueue(rlfc_env* E, const int* d_env, const int* d_set, int n, int reset_accumulators) {
+  if (n <= 0) return RLFC_OK;
+  SolverParams& sp = E->whole.sp;
+  CU(cudaMemsetAsync(E->d_skip, 1, sp.B * sizeof(int), E->stream));   // nonzero = keep; the reset clears
+  E->run("k_reset_sets", 0, [&] {
+    return launch_reset_sets(sp, E->lib, E->snap, E->init_ux, E->init_uy, E->init_p, E->init_t, E->uAx, E->uAy, d_env, d_set, n,
+                             reset_accumulators, E->d_skip, E->stream);
+  });
+  E->run("k_poisson_rebuild0", 0, [&] { return launch_poisson_rebuild0(sp, E->d_skip, E->stream); });
+  E->run("k_poisson_rebuild_coarse", 0, [&] { return launch_poisson_rebuild_coarse(sp, E->d_skip, E->stream); });
+  CU(cudaGetLastError());
+  return RLFC_OK;
+}
+
+int reset_sets_check_handle(rlfc_env* E, int n, bool have_ptrs) {
+  if (!E) return fail(RLFC_EINVAL, "null handle");
+  if (!E->lib.L) return fail(RLFC_EINVAL, "the handle has no parameter library (rlfc_config.n_param_sets = 0)");
+  if (n < 0) return fail(RLFC_EINVAL, "bad pair count");
+  if (n > 0 && !have_ptrs) return fail(RLFC_EINVAL, "null argument");
   return RLFC_OK;
 }
 
@@ -408,6 +482,7 @@ int snapshot_host(rlfc_env* E, const int* env_ids, const int* slots, int n, int 
     if (seen[dst]++) return fail(RLFC_EINVAL, std::string(restore ? "env id " : "slot ") + std::to_string(dst) + " listed twice");
   }
   CU(cudaSetDevice(E->device));
+  if (restore && n > 0 && (rc = sync_env_sets(E))) return rc;   // (params[e]: the set the destination holds now)
   if (restore && n > 0) {
     // device snapshots write slots the host never sees: read the headers back
     std::vector<unsigned> hdr((size_t)kSnapHdr * S);
@@ -874,6 +949,22 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
     std::string err;
     if (build_env_geometries(*cfg, cfg->env_params, cfg->n_envs, env_geo, env_set, err)) return fail(RLFC_EINVAL, err);
   }
+  // parameter library: the same, for its entries
+  std::vector<EnvGeometry> lib_geo;
+  std::vector<int> lib_set;
+  if (cfg->n_param_sets < 0) return fail(RLFC_EINVAL, "n_param_sets must be >= 0");
+  if (cfg->n_param_sets > 0) {
+    if (!cfg->param_sets) return fail(RLFC_EINVAL, "param_sets is NULL with n_param_sets > 0");
+    if (cfg->n_devices > 1) return fail(RLFC_EINVAL, "param_sets is not available in slab mode (n_devices > 1)");
+    std::string err;
+    if (build_env_geometries(*cfg, cfg->param_sets, cfg->n_param_sets, lib_geo, lib_set, err, "param_sets"))
+      return fail(RLFC_EINVAL, err);
+    if (!cfg->env_params) {   // every environment on the scalar config's set, in its own slot (as env_params would give)
+      const rlfc_env_params p0 = params_of(*cfg);
+      std::vector<rlfc_env_params> own(cfg->n_envs, p0);
+      if (build_env_geometries(*cfg, own.data(), cfg->n_envs, env_geo, env_set, err)) return fail(RLFC_EINVAL, err);
+    }
+  }
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
     return fail(RLFC_ENODEV, "no CUDA device available (rlfc has no CPU fallback)");
@@ -881,8 +972,9 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
   E->cfg = *cfg;
   if (cfg->init_bdim_path) E->init_path = cfg->init_bdim_path;
   E->cfg.init_bdim_path = nullptr;
-  E->env_mode = cfg->env_params != nullptr;
+  E->env_mode = cfg->env_params != nullptr || cfg->n_param_sets > 0;
   E->cfg.env_params = nullptr;              // (copied into E->params below)
+  E->cfg.param_sets = nullptr;              // (copied into E->lib_params below)
   E->cfg.sensors = nullptr;                 // (resolved into E->sens below)
   int rc = RLFC_OK;
   auto bail = [&](int code) { rlfc_env_destroy(E); return code; };
@@ -960,12 +1052,14 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
     TRY(upload_static(E, g.c_x, g.n, g.m, sp.P, &sp.c_x));
     TRY(upload_static(E, g.c_y, g.n, g.m, sp.P, &sp.c_y));
   }
+  // geometry slots: one per environment, then one per distinct library set
+  const int nslots = B + (int)lib_geo.size();
   if (env_mode) {
     // one geometry slot per environment: del and the body-velocity basis at e * stride (filled by upload_env_geometry)
     const float** slot[10] = {&sp.del_x, &sp.del_y, &sp.w1_x, &sp.w2_x, &sp.ry1_x, &sp.ry2_x, &sp.w1_y, &sp.w2_y, &sp.rx1_y, &sp.rx2_y};
     for (const float** f : slot) {
       float* d = nullptr;
-      TRY(E->dmalloc(&d, sp.stride * B));
+      TRY(E->dmalloc(&d, sp.stride * nslots));
       *f = d;
     }
   } else {
@@ -1087,7 +1181,7 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
   }
   if (per_env) {
     // the per-environment hierarchy exists for the row-pipeline and single-warp smoothers only
-    const std::string what = adaptive ? "adaptive_dt" : "env_params";
+    const std::string what = adaptive ? "adaptive_dt" : cfg->env_params ? "env_params" : "param_sets";
     if (sp.chain_levels > 0)
       return bail(fail(RLFC_EINVAL, what + " is not available with the chained strip smoother (a level too wide for the "
                                            "row pipeline, or RLFC_SMOOTHER=chain)"));
@@ -1123,8 +1217,8 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
     if (const char* ev = std::getenv("RLFC_FAST_BC")) sp.fast_bc = sp.fast_bc && std::atoi(ev) != 0;
     if (env_mode) {
       BandFace* d = nullptr;
-      TRY(E->dmalloc(&d, (size_t)sp.nband_x * B)); sp.band_x = d;
-      TRY(E->dmalloc(&d, (size_t)sp.nband_y * B)); sp.band_y = d;
+      TRY(E->dmalloc(&d, (size_t)sp.nband_x * nslots)); sp.band_x = d;
+      TRY(E->dmalloc(&d, (size_t)sp.nband_y * nslots)); sp.band_y = d;
     } else {
       TRY(upload_vec(E, bx, &sp.band_x));
       TRY(upload_vec(E, by, &sp.band_y));
@@ -1141,10 +1235,32 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
     if (env_mode) {
       for (int e = 0; e < B; e++) {
         slot[e] = e;
-        TRY(upload_env_geometry(E, e, cfg->env_params[e], env_geo[env_set[e]]));
+        TRY(upload_env_geometry(E, e, cfg->env_params ? cfg->env_params[e] : params_of(E->cfg), env_geo[env_set[e]]));
       }
+      // the library: set s in slot B + (its first equal set's index among the distinct ones)
+      for (size_t u = 0; u < lib_geo.size(); u++) TRY(upload_slot_geometry(E, B + (int)u, lib_geo[u]));
       if (cudaStreamSynchronize(E->stream) != cudaSuccess) return bail(fail(RLFC_ECUDA, "geometry upload failed"));
+      E->lib_params.assign(cfg->param_sets, cfg->param_sets + cfg->n_param_sets);
+      for (int k = 0; k < cfg->n_param_sets; k++) {
+        const EnvGeometry& G = lib_geo[lib_set[k]];
+        LibSet L{};
+        L.slot = B + lib_set[k];
+        L.nbx = (int)G.bx.size(); L.nby = (int)G.by.size();
+        L.nu = G.g.nu; L.dRD = G.g.dR * G.g.D; L.dt0 = G.g.dt;
+        param_bits(cfg->param_sets[k], L.bits);
+        E->h_lib.push_back(L);
+      }
       env_geo.clear();
+      lib_geo.clear();
+    }
+    if (!E->h_lib.empty()) {
+      E->lib.L = (int)E->h_lib.size();
+      TRY(upload_vec(E, E->h_lib, &E->lib.sets));
+      TRY(E->dmalloc(&E->lib.env_set, B, false));
+      TRY(E->dmalloc(&E->set_env, B)); TRY(E->dmalloc(&E->set_ids, B));
+      E->h_env_set.assign(B, -1);
+      if (cudaMemcpyAsync(E->lib.env_set, E->h_env_set.data(), B * sizeof(int), cudaMemcpyHostToDevice, E->stream) != cudaSuccess)
+        return bail(fail(RLFC_ECUDA, "library table upload failed"));
     }
     int* d = nullptr;
     TRY(E->dmalloc(&d, B)); sp.env_slot = d;
@@ -1445,6 +1561,7 @@ int rlfc_env_reset(rlfc_env* E, const int* env_ids, int n, int reset_accumulator
     if (env_ids[k] < 0 || env_ids[k] >= sp.B) return fail(RLFC_EINVAL, "env id out of range");
   CU(cudaSetDevice(E->device));
   int rc;
+  if ((rc = sync_env_sets(E))) return rc;   // (dt0: the set each environment holds now)
   if ((rc = broadcast_field(E, E->uAx, E->init_ux, env_ids, n))) return rc;
   if ((rc = broadcast_field(E, E->uAy, E->init_uy, env_ids, n))) return rc;
   if ((rc = broadcast_field(E, sp.lev[0].x, E->init_p, env_ids, n))) return rc;
@@ -1471,7 +1588,7 @@ int rlfc_env_reset(rlfc_env* E, const int* env_ids, int n, int reset_accumulator
 
 int rlfc_env_reset_params(rlfc_env* E, const int* env_ids, int n, const rlfc_env_params* params, int reset_accumulators) {
   if (!E) return fail(RLFC_EINVAL, "null handle");
-  if (!E->env_mode) return fail(RLFC_EINVAL, "rlfc_env_reset_params needs a handle created with env_params");
+  if (!E->env_mode) return fail(RLFC_EINVAL, "rlfc_env_reset_params needs a handle created with env_params or param_sets");
   const int B = E->sp.B;
   if (n < 0 || n > B) return fail(RLFC_EINVAL, "bad env count");
   if (n > 0 && (!env_ids || !params)) return fail(RLFC_EINVAL, "null argument");
@@ -1489,8 +1606,11 @@ int rlfc_env_reset_params(rlfc_env* E, const int* env_ids, int n, const rlfc_env
   }
   CU(cudaSetDevice(E->device));
   int rc;
-  for (int k = 0; k < n; k++)
+  if ((rc = sync_env_sets(E))) return rc;   // (the others' host copies, which upload_env_scalars writes back)
+  for (int k = 0; k < n; k++) {
     if ((rc = upload_env_geometry(E, env_ids[k], params[k], geo[set[k]]))) return rc;
+    if (E->lib.L) E->h_env_set[env_ids[k]] = -1;   // back on its own slot
+  }
   if ((rc = upload_env_scalars(E))) return rc;
   if ((rc = upload_snapshot_params(E))) return rc;
   if ((rc = rlfc_env_reset(E, env_ids, n, reset_accumulators))) return rc;   // (sc.dt = the new t_step*resolution)
@@ -1507,6 +1627,9 @@ int rlfc_env_reset_params(rlfc_env* E, const int* env_ids, int n, const rlfc_env
 
 int rlfc_env_get_params(rlfc_env* E, rlfc_env_params* params) {
   if (!E || !params) return fail(RLFC_EINVAL, "null argument");
+  CU(cudaSetDevice(E->device));
+  int rc = sync_env_sets(E);
+  if (rc) return rc;
   std::copy(E->params.begin(), E->params.end(), params);
   return RLFC_OK;
 }
@@ -1545,6 +1668,7 @@ int rlfc_env_step(rlfc_env* E, const float* actions, float* obs, float* reward, 
   const float init_time = sp.init_time > 0 ? sp.init_time : 0;
   float dt_min = sp.dt;
   if (sp.per_env) dt_min = *std::min_element(E->dt0.begin(), E->dt0.end());
+  for (const LibSet& L : E->h_lib) dt_min = std::min(dt_min, L.dt0);   // (a bound over own and library sets: no sync)
   int max_rounds = sp.per_env ? 3 + (int)(init_time / (dt_min / sp.resolution)) / sp.substeps
                               : 3 + (int)(init_time / sp.dt_over_res) / sp.substeps;
   std::vector<float> h_dt(sp.adaptive ? B : 0);
@@ -1660,6 +1784,8 @@ int rlfc_env_load_bdim(rlfc_env* E, int e, const char* path) {
     // adaptive mode: any positive dt; it becomes the environment's current dt
     if (!(dt > 0) || !std::isfinite(dt)) return fail(RLFC_EIO, "checkpoint dt " + std::to_string(dt) + " is not a positive number");
   } else {
+    CU(cudaSetDevice(E->device));
+    if ((rc = sync_env_sets(E))) return rc;
     const float fixed = E->dt0[e];   // the environment's t_step*resolution (the handle's without env_params)
     if (dt != fixed && !(std::fabs(dt - fixed) <= 1e-6f * fixed))
       return fail(RLFC_EIO, "checkpoint dt " + std::to_string(dt) + " does not match the environment's " + std::to_string(fixed));
@@ -1727,6 +1853,34 @@ int rlfc_env_restore_device(rlfc_env* E, const int* d_env_ids, const int* d_slot
   if (rc) return rc;
   CU(cudaSetDevice(E->device));
   return snapshot_enqueue(E, d_env_ids, d_slots, n, 1, keep_accumulators != 0);
+}
+
+int rlfc_env_reset_sets(rlfc_env* E, const int* env_ids, const int* sets, int n, int reset_accumulators) {
+  int rc = reset_sets_check_handle(E, n, env_ids && sets);
+  if (rc) return rc;
+  const int B = E->sp.B;
+  if (n > B) return fail(RLFC_EINVAL, "bad pair count");
+  std::vector<char> seen(B, 0);
+  for (int k = 0; k < n; k++) {
+    if (env_ids[k] < 0 || env_ids[k] >= B) return fail(RLFC_EINVAL, "env id " + std::to_string(env_ids[k]) + " out of range");
+    if (sets[k] < 0 || sets[k] >= E->lib.L) return fail(RLFC_EINVAL, "set " + std::to_string(sets[k]) + " out of range");
+    if (seen[env_ids[k]]++) return fail(RLFC_EINVAL, "env id " + std::to_string(env_ids[k]) + " listed twice");
+  }
+  CU(cudaSetDevice(E->device));
+  if (n > 0) {
+    CU(cudaMemcpyAsync(E->set_env, env_ids, n * sizeof(int), cudaMemcpyHostToDevice, E->stream));
+    CU(cudaMemcpyAsync(E->set_ids, sets, n * sizeof(int), cudaMemcpyHostToDevice, E->stream));
+  }
+  if ((rc = reset_sets_enqueue(E, E->set_env, E->set_ids, n, reset_accumulators != 0))) return rc;
+  CU(cudaStreamSynchronize(E->stream));
+  return RLFC_OK;
+}
+
+int rlfc_env_reset_sets_device(rlfc_env* E, const int* d_env_ids, const int* d_sets, int n, int reset_accumulators) {
+  int rc = reset_sets_check_handle(E, n, d_env_ids && d_sets);
+  if (rc) return rc;
+  CU(cudaSetDevice(E->device));
+  return reset_sets_enqueue(E, d_env_ids, d_sets, n, reset_accumulators != 0);
 }
 
 int rlfc_env_get_sensors(rlfc_env* E, float* out) {
@@ -1845,11 +1999,13 @@ int rlfc_env_get_coeffs(rlfc_env* E, int e, const char* name, int level, float* 
   if (!out) return RLFC_OK;
   const float* src = (nm == "lower.x" || nm == "c.x") ? L.lx : (nm == "lower.y" || nm == "c.y") ? L.ly : nm == "inv" ? L.inv : L.diag;
   size_t off = (size_t)e * L.stride;
-  if (nm == "del.x" || nm == "del.y") {   // the environment's geometry slot
-    src = nm == "del.x" ? E->sp.del_x : E->sp.del_y;
-    off = E->env_mode ? (size_t)e * E->sp.stride : 0;
-  }
   CU(cudaSetDevice(E->device));
+  if (nm == "del.x" || nm == "del.y") {   // the environment's geometry slot
+    int rc = sync_env_sets(E);
+    if (rc) return rc;
+    src = nm == "del.x" ? E->sp.del_x : E->sp.del_y;
+    off = (size_t)slot_of(E, e) * E->sp.stride;
+  }
   CU(cudaMemcpy2DAsync(out, L.m * sizeof(float), src + off, L.P * sizeof(float), L.m * sizeof(float), L.n,
                        cudaMemcpyDeviceToHost, E->stream));
   CU(cudaStreamSynchronize(E->stream));

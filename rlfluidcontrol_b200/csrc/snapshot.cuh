@@ -52,21 +52,40 @@ __device__ __forceinline__ unsigned* snap_word(const EnvScalars& sc, int nprobe,
   return f ? reinterpret_cast<unsigned*>(f) : reinterpret_cast<unsigned*>(i);
 }
 
+// Pair k of the device arrays (x[k], y[k]) applies when x[k] is in [0, nx), y[k] in [0, ny) (a negative entry is the way
+// to skip a pair) and no later pair in range has the same destination (x if dst_x, else y): of pairs with the same
+// destination the last one wins.  Called by every thread of the CTA (one __syncthreads_or); the result is CTA-uniform.
+__device__ __forceinline__ bool pair_applies(const int* x, const int* y, int k, int n, int nx, int ny, bool dst_x) {
+  const int xk = x[k], yk = y[k];
+  if (xk < 0 || xk >= nx || yk < 0 || yk >= ny) return false;
+  const int dst = dst_x ? xk : yk;
+  int later = 0;
+  for (int k2 = k + 1 + (int)threadIdx.x; k2 < n; k2 += kSnapThreads) {
+    const int x2 = x[k2], y2 = y[k2];
+    if (x2 >= 0 && x2 < nx && y2 >= 0 && y2 < ny && (dst_x ? x2 : y2) == dst) later = 1;
+  }
+  return !__syncthreads_or(later);
+}
+
+// chunk c of one field: kSnapThreads * kSnapVec float4 of nv, streamed (the copy is read once)
+__device__ __forceinline__ void copy_chunk(const float4* __restrict__ src, float4* __restrict__ dst, int c, int nv) {
+  const int i0 = c * kSnapThreads * kSnapVec + (int)threadIdx.x;
+  float4 v[kSnapVec];
+#pragma unroll
+  for (int u = 0; u < kSnapVec; u++)
+    if (i0 + u * kSnapThreads < nv) v[u] = __ldcs(src + i0 + u * kSnapThreads);
+#pragma unroll
+  for (int u = 0; u < kSnapVec; u++)
+    if (i0 + u * kSnapThreads < nv) dst[i0 + u * kSnapThreads] = v[u];
+}
+
 __global__ void __launch_bounds__(kSnapThreads) k_snapshot_copy(const __grid_constant__ SnapArgs a) {
   const int S = a.s.S, B = a.B;
   const int cpf = (a.nv + kSnapThreads * kSnapVec - 1) / (kSnapThreads * kSnapVec);   // chunks per field
   const int f = blockIdx.x / cpf, c = blockIdx.x - f * cpf;
   for (int k = blockIdx.y; k < a.n; k += gridDim.y) {
+    if (!pair_applies(a.env, a.slot, k, a.n, B, S, a.restore)) continue;
     const int e = a.env[k], s = a.slot[k];
-    if (e < 0 || e >= B || s < 0 || s >= S) continue;        // a negative entry is the way to skip a pair
-    // of pairs with the same destination the last one wins: this pair applies only if no later pair in range has it
-    const int dst = a.restore ? e : s;
-    int later = 0;
-    for (int k2 = k + 1 + (int)threadIdx.x; k2 < a.n; k2 += kSnapThreads) {
-      const int e2 = a.env[k2], s2 = a.slot[k2];
-      if (e2 >= 0 && e2 < B && s2 >= 0 && s2 < S && (a.restore ? e2 : s2) == dst) later = 1;
-    }
-    if (__syncthreads_or(later)) continue;
     if (a.restore) {
       // only a written slot of the destination's own parameter tuple (whose geometry and fixed-dt hierarchy it has); no
       // short circuit, so that the eleven loads are independent and issue together
@@ -84,14 +103,7 @@ __global__ void __launch_bounds__(kSnapThreads) k_snapshot_copy(const __grid_con
     float4* sf = reinterpret_cast<float4*>(f == 0 ? a.s.ux : f == 1 ? a.s.uy : a.s.p) + (size_t)s * a.stride4;
     const float4* __restrict__ src = a.restore ? sf : ef;
     float4* __restrict__ dstp = a.restore ? ef : sf;
-    const int i0 = c * kSnapThreads * kSnapVec + (int)threadIdx.x;
-    float4 v[kSnapVec];
-#pragma unroll
-    for (int u = 0; u < kSnapVec; u++)
-      if (i0 + u * kSnapThreads < a.nv) v[u] = __ldcs(src + i0 + u * kSnapThreads);
-#pragma unroll
-    for (int u = 0; u < kSnapVec; u++)
-      if (i0 + u * kSnapThreads < a.nv) dstp[i0 + u * kSnapThreads] = v[u];
+    copy_chunk(src, dstp, c, a.nv);
     if (blockIdx.x == 0 && threadIdx.x < kSnapWords) {
       const int w = threadIdx.x;
       unsigned* x = snap_word(a.sc, a.nprobe, e, w);

@@ -192,6 +192,21 @@ struct SnapSlots {
   int *refused;             // [B] 1 = the last restore into the environment was skipped (rlfc_env_get_flags bit 1)
 };
 
+// Parameter library (rlfc_config.param_sets; param_sets.cuh).  Set s's geometry lives in geometry slot sets[s].slot >= B
+// (equal sets share one); the rest of what an environment of set s holds per environment is in its LibSet.  Kept out of
+// SolverParams for the reason SensorSet is.
+struct LibSet {
+  int slot;                 // geometry slot: del_x .. rx2_y at slot * stride, band lists at slot * nband_x / nband_y
+  int nbx, nby;             // band faces (env_nband_x / env_nband_y)
+  float nu, dRD, dt0;       // D/Re, dR*D, t_step*resolution
+  unsigned bits[5];         // the (re, dR, gR, theta, t_step) tuple's bits (SnapSlots::env_par)
+};
+struct ParamLib {
+  int L;                    // sets (0 = no library: nothing allocated)
+  const LibSet* sets;       // [L]
+  int* env_set;             // [B] the set each environment holds, -1 = its own slot (env_params / rlfc_env_reset_params)
+};
+
 #ifdef __CUDACC__
 // true = block `blk` of `nblk` (a kernel's row-block or strip index) belongs to another device
 __device__ __forceinline__ bool slab_skip(unsigned blk, unsigned nblk, int rank, int n) {
@@ -276,5 +291,14 @@ int launch_emit_obs(const SolverParams& P, const float* d_actions, float* d_obs,
 // `sens` move with the state (sens.n = 0: none).
 int launch_snapshot_copy(const SolverParams& P, const SnapSlots& s, const SensorSet& sens, float* ux, float* uy, const int* d_env,
                          const int* d_slot, int n, int restore, int keep_accumulators, int* skip, cudaStream_t st);
+// Parameter-library reset of n (environment, set) pairs, device arrays d_env[n], d_set[n] (P: the whole batch, per_env):
+// environment d_env[k] takes library set d_set[k] (env_slot, env_set, env_nu, env_dRD, env_nband_x/y, sc.dt = dt0, and
+// with snapshots snap.env_par), the init fields init_ux / init_uy / init_p (one environment, pitched) into ux, uy and
+// P.lev[0].x, and the reset scalars of rlfc_env_reset (flow_t = init_t; reset_accumulators: callLearn = substeps, Cd = Cl =
+// obs = 0).  Pairs out of range are skipped, of pairs with the same environment the last wins, and skip[e] = 0 is written
+// for every environment reset (the mask of the following launch_poisson_rebuild*).
+int launch_reset_sets(const SolverParams& P, const ParamLib& lib, const SnapSlots& snap, const float* init_ux,
+                      const float* init_uy, const float* init_p, float init_t, float* ux, float* uy, const int* d_env,
+                      const int* d_set, int n, int reset_accumulators, int* skip, cudaStream_t st);
 
 }  // namespace rlfc

@@ -1956,3 +1956,4 @@ int launch_emit_obs(const SolverParams& q, const float* d_actions, float* d_obs,
 }  // namespace rlfc
 
 #include "snapshot.cuh"
+#include "param_sets.cuh"

@@ -48,6 +48,7 @@ class Config(C.Structure):
         ("n_groups", C.c_int), ("n_devices", C.c_int), ("adaptive_dt", C.c_int),
         ("env_params", C.POINTER(EnvParams)), ("n_snapshots", C.c_int),
         ("n_sensors", C.c_int), ("sensors", C.POINTER(Sensor)),
+        ("n_param_sets", C.c_int), ("param_sets", C.POINTER(EnvParams)),
     ]
 
 
@@ -82,6 +83,8 @@ def load_library():
     L.rlfc_env_reset.argtypes = [vp, ip, C.c_int, C.c_int]
     L.rlfc_env_reset_params.argtypes = [vp, ip, C.c_int, C.POINTER(EnvParams), C.c_int]
     L.rlfc_env_get_params.argtypes = [vp, C.POINTER(EnvParams)]
+    L.rlfc_env_reset_sets.argtypes = [vp, ip, ip, C.c_int, C.c_int]
+    L.rlfc_env_reset_sets_device.argtypes = [vp, vp, vp, C.c_int, C.c_int]
     L.rlfc_env_step.argtypes = [vp, fp, fp, fp, ip]
     L.rlfc_env_step_device.argtypes = [vp, vp, vp, vp, vp]
     L.rlfc_env_substep.argtypes = [vp, fp, fp, fp]
@@ -163,11 +166,14 @@ def _sensor_array(sensors):
 class AFCCylinderBatch:
     """A batch of AFCCylinder environments on one GPU."""
 
-    def __init__(self, n_envs=1, init_state="default", device=-1, stream=None, env_params=None, sensors=None, **overrides):
+    def __init__(self, n_envs=1, init_state="default", device=-1, stream=None, env_params=None, sensors=None, param_sets=None,
+                 **overrides):
         """env_params: None (every environment uses the scalar config's re, dR, gR, theta, t_step), or n_envs entries, dicts
         or a structured array, each environment's own constructor arguments (missing keys: the scalar config's).
         sensors: None, or a sequence of (field, x, y), field "p", "ux" or "uy", (x, y) in grid coordinates: the flow
-        sampled in every environment after each of its solver steps (`sensors()`)."""
+        sampled in every environment after each of its solver steps (`sensors()`).
+        param_sets: None, or a library of constructor arguments given like env_params (any number of entries), built at
+        create; `reset_sets` / `reset_sets_device` switch environments to its entries on the device."""
         self._L = load_library()
         cfg = Config()
         self._L.rlfc_default_config(C.byref(cfg))
@@ -188,11 +194,16 @@ class AFCCylinderBatch:
             if len(self._env_params) != cfg.n_envs:
                 raise ValueError(f"env_params has {len(self._env_params)} entries for {cfg.n_envs} environments")
             cfg.env_params = C.cast(self._env_params, C.POINTER(EnvParams))
+        if param_sets is not None:
+            self._param_sets = _env_params_array(param_sets, cfg)
+            cfg.n_param_sets = len(self._param_sets)
+            cfg.param_sets = C.cast(self._param_sets, C.POINTER(EnvParams))
         if sensors is not None:
             self._sensors = _sensor_array(sensors)
             cfg.n_sensors = len(self._sensors)
             cfg.sensors = C.cast(self._sensors, C.POINTER(Sensor))
         self.n_sensors = cfg.n_sensors
+        self.n_param_sets = cfg.n_param_sets
         self.cfg = cfg
         h = C.c_void_p()
         rc = self._L.rlfc_env_create(C.byref(cfg), C.byref(h))
@@ -245,6 +256,21 @@ class AFCCylinderBatch:
             ids = np.ascontiguousarray(env_ids, dtype=np.int32)
             rc = self._L.rlfc_env_reset(self._h, ids.ctypes.data_as(C.POINTER(C.c_int)), len(ids), int(reset_accumulators))
         self._check(rc, "rlfc_env_reset")
+
+    def reset_sets(self, env_ids, sets, reset_accumulators=False):
+        """setUpNewSim into the parameter library: environment env_ids[k] takes param_sets[sets[k]] with its geometry and
+        Poisson hierarchy, bit for bit what `reset([e], params=[param_sets[s]])` gives, without building anything on the
+        host.  All or nothing: an id or set out of range or an environment listed twice raises and changes nothing."""
+        ids, st = self._pairs(env_ids, sets, "sets")
+        self._check(self._L.rlfc_env_reset_sets(self._h, _ip(ids), _ip(st), len(ids), int(reset_accumulators)),
+                    "rlfc_env_reset_sets")
+
+    def reset_sets_device(self, d_env_ids, d_sets, n, reset_accumulators=False):
+        """reset_sets() with device int32 arrays of length n (data_ptr() ints), asynchronous on the handle's stream:
+        reset_sets_device(arange(B), where(done, draw, -1), B) gives the finished environments new parameter sets without
+        the host.  Pairs with an entry out of range (e.g. -1) are skipped; of pairs with the same environment the last wins."""
+        self._check(self._L.rlfc_env_reset_sets_device(self._h, C.c_void_p(d_env_ids), C.c_void_p(d_sets), int(n),
+                                                       int(reset_accumulators)), "rlfc_env_reset_sets_device")
 
     def params(self):
         """Each environment's constructor arguments: a structured array with the fields re, dR, gR, theta, t_step."""
@@ -314,11 +340,11 @@ class AFCCylinderBatch:
         self._check(self._L.rlfc_env_get_sensors_device(self._h, C.c_void_p(d_out)), "rlfc_env_get_sensors_device")
 
     @staticmethod
-    def _pairs(env_ids, slots):
+    def _pairs(env_ids, slots, what="slots"):
         ids = np.ascontiguousarray(env_ids, dtype=np.int32).reshape(-1)
         sl = np.ascontiguousarray(slots, dtype=np.int32).reshape(-1)
         if len(ids) != len(sl):
-            raise ValueError(f"{len(ids)} environment ids for {len(sl)} slots")
+            raise ValueError(f"{len(ids)} environment ids for {len(sl)} {what}")
         return ids, sl
 
     def update2(self, actions=None, want_probes=False):
