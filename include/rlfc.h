@@ -40,7 +40,11 @@ extern "C" {
 #define RLFC_ECUDA    -3   /* CUDA runtime error (message in rlfc_last_error)                */
 #define RLFC_EIO      -4   /* checkpoint file could not be read / written / parsed           */
 #define RLFC_ENOMEM   -5
-#define RLFC_EGRID    -6   /* grid not MG-divisible (MG.pde:99-106 would exit())             */
+#define RLFC_EGRID    -6   /* a grid the reference's multigrid cannot run: level 0 (x_lengths*resolution by
+                              y_lengths*resolution cells) must be even in both directions, because MG.prolongate
+                              and MG.increment (MG.pde:94-97,139-152) would write past the coarse correction, and a
+                              coarse level that is not divisible must have a side <= 9 (incl. ghosts), because
+                              MG.divisible (MG.pde:99-106) would exit()                                          */
 #define RLFC_ENOTCONV -7   /* reserved                                                       */
 
 #define RLFC_NUM_PROBES 32 /* SaveScalar numTheta, clientCFD.pde:102                         */

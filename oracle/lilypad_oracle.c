@@ -818,8 +818,24 @@ static void build_hierarchy(ora_env *e) {
   e->hier[nl].n = 0;
 }
 
+/* Grids the reference cannot run, decided from the level sizes alone (n, m incl. ghosts):
+   - an odd level 0: MG.prolongate (MG.pde:139-152) builds an even-sized correction from the coarse level and
+     MG.increment (MG.pde:94-97) adds it over the whole fine field, past the correction's end;
+   - a coarse level that is not divisible while both sides are > 9: MG.divisible (MG.pde:101-104) calls exit(). */
+static int grid_runnable(int n, int m) {
+  if ((n - 2) % 2 != 0 || (m - 2) % 2 != 0) return 0;
+  for (;;) {
+    n = (n - 2) / 2 + 2;                          /* MG.restrict MG.pde:108-122 */
+    m = (m - 2) / 2 + 2;
+    int divisible = (n - 2) % 2 == 0 && (m - 2) % 2 == 0 && n > 4 && m > 4;
+    if (divisible) continue;
+    return !(n > 9 && m > 9);
+  }
+}
+
 /* AFCCylinder ctor AFCCylinder.pde:11-42 + BDIM ctor BDIM.pde:41-71 (without resume) */
 ora_env *ora_env_new(const ora_config *cfg) {
+  if (!grid_runnable(cfg->xLengths * cfg->resolution + 2, cfg->yLengths * cfg->resolution + 2)) return NULL;
   ora_env *e = (ora_env *)calloc(1, sizeof(ora_env));
   e->cfg = *cfg;
   const int resolution = cfg->resolution;

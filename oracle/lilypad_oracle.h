@@ -114,7 +114,10 @@ typedef struct {
 } ora_config;
 
 ora_config ora_default_config(void);                                      /* clientCFD.pde:9,14,94-96 */
-ora_env *ora_env_new(const ora_config *cfg);                              /* AFCCylinder.pde:11-42 (no resume) */
+/* AFCCylinder.pde:11-42 (no resume).  NULL for a grid the reference cannot run: an odd level 0 (MG.prolongate /
+   MG.increment, MG.pde:94-97,139-152, would write past the coarse correction) or a non-divisible coarse level with
+   both sides > 9 (MG.divisible, MG.pde:101-104, would exit()). */
+ora_env *ora_env_new(const ora_config *cfg);
 void     ora_env_free(ora_env *e);
 int      ora_env_n(const ora_env *e);   /* array dims incl. ghosts */
 int      ora_env_m(const ora_env *e);

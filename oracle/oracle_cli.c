@@ -40,6 +40,7 @@ int main(int argc, char **argv) {
     if (argc >= 5) cfg.literal = atoi(argv[4]);
     FILE *trace = argc >= 6 ? fopen(argv[5], "w") : NULL;
     ora_env *e = ora_env_new(&cfg);
+    if (!e) { fprintf(stderr, "the reference cannot run this grid\n"); return 1; }
     if (strcmp(argv[2], "uniform")) {
       int n, m; float t, dt, *ux, *uy, *p;
       int rc = ora_read_bdimb(argv[2], &n, &m, &t, &dt, &ux, &uy, &p);

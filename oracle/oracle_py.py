@@ -249,6 +249,9 @@ class OracleEnv:
             setattr(cfg, k, v)
         self.cfg = cfg
         self._e = L.ora_env_new(C.byref(cfg))
+        if not self._e:
+            raise ValueError(f"the reference cannot run the grid resolution={cfg.resolution}, xLengths={cfg.xLengths}, "
+                             f"yLengths={cfg.yLengths} (MG.pde:94-104,139-152)")
         self.n, self.m = L.ora_env_n(self._e), L.ora_env_m(self._e)
         self._drv = L.ora_driver_new()
 

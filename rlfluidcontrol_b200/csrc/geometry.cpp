@@ -15,6 +15,9 @@ namespace {
 constexpr float kPi = 3.1415927f;     // PConstants.PI
 constexpr float kTwoPi = 6.2831855f;  // PConstants.TWO_PI
 constexpr int kCircleVerts = 40;      // EllipseBody.m, Body.pde:384
+// MG.divisible's message before its exit() (MG.pde:101-104)
+constexpr const char* kMgExitMessage =
+    "MultiGrid requires the size in each direction be a large factor of two (2^p) times a small number (N=1..9)";
 
 inline float fsin(float x) { return (float)std::sin((double)x); }
 inline float fcos(float x) { return (float)std::cos((double)x); }
@@ -215,6 +218,20 @@ int build_geometry(const rlfc_config& cfg, Geometry& g, std::string& err, bool h
   }
   const int nc = cfg.x_lengths * cfg.resolution, mc = cfg.y_lengths * cfg.resolution;   // AFCCylinder.pde:12-13
   const int n = nc + 2, m = mc + 2;                                                     // BDIM.pde:42
+  if (nc % 2 != 0 || mc % 2 != 0) {
+    // the finest level always restricts (MG.pde:70-72): MG.prolongate (MG.pde:139-152) then builds an even-sized
+    // correction and MG.increment (MG.pde:94-97) adds it over the whole odd-sized fine field, past its end.  The coarse
+    // levels' MG.divisible (MG.pde:101-104) runs first, inside vCycle: where it would exit(), report that instead.
+    err = "level 0 must have an even number of cells in each direction (" + std::to_string(nc) + "x" + std::to_string(mc) +
+          "): MG.prolongate / MG.increment cannot correct an odd grid";
+    for (int cn = n, cm = m;;) {
+      cn = (cn - 2) / 2 + 2; cm = (cm - 2) / 2 + 2;                                     // MG.pde:108-122
+      if ((cn - 2) % 2 == 0 && (cm - 2) % 2 == 0 && cn > 4 && cm > 4) continue;
+      if (cn > 9 && cm > 9) err = kMgExitMessage;
+      break;
+    }
+    return RLFC_EGRID;
+  }
   g.n = n; g.m = m;
   g.resolution = cfg.resolution;
   g.D = (float)cfg.resolution;                                                          // AFCCylinder.pde:27
@@ -294,7 +311,7 @@ int build_geometry(const rlfc_config& cfg, Geometry& g, std::string& err, bool h
       if ((F.n - 2) < 2 || (F.m - 2) < 2) { err = "grid too small for multigrid"; return RLFC_EGRID; }
     } else if (!divisible) {
       if (F.n > 9 && F.m > 9) {
-        err = "MultiGrid requires the size in each direction be a large factor of two (2^p) times a small number (N=1..9)";
+        err = kMgExitMessage;
         return RLFC_EGRID;   // MG.pde:101-104 would exit()
       }
       break;

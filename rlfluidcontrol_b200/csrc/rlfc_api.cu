@@ -1308,10 +1308,10 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
   if (const char* ev = std::getenv("RLFC_TINY")) sp.tiny = std::atoi(ev) != 0;
   sp.resid_march = 1;
   if (const char* ev = std::getenv("RLFC_RESID")) sp.resid_march = std::strcmp(ev, "tile") != 0;
-  // (odd level-0 sizes cannot pair rows / columns for the restriction: MG.divisible rules them out anyway; a batch of fewer
-  // than ~8 Mi cells does not give the marching kernel enough warps -- one 2048x1024 domain: 38 vs 31 us)
-  if ((((g.n - 2) | (g.m - 2)) & 1) || (long long)B * (g.n - 2) * (g.m - 2) < (8ll << 20)) sp.resid_march = 0;
-  if (const char* ev = std::getenv("RLFC_RESID")) if (std::strcmp(ev, "march") == 0 && !(((g.n - 2) | (g.m - 2)) & 1)) sp.resid_march = 1;
+  // (the kernel pairs level-0 rows / columns for the restriction, which build_geometry's even level 0 guarantees; a batch of
+  // fewer than ~8 Mi cells does not give the marching kernel enough warps -- one 2048x1024 domain: 38 vs 31 us)
+  if ((long long)B * (g.n - 2) * (g.m - 2) < (8ll << 20)) sp.resid_march = 0;
+  if (const char* ev = std::getenv("RLFC_RESID")) if (std::strcmp(ev, "march") == 0) sp.resid_march = 1;
   // slab mode keeps the tile kernel: the marching kernel bulk-copies its rows (cp.async.bulk), which here would read
   // other devices' memory through the shared address range, a combination that has not been run on several devices
   if (slab) sp.resid_march = 0;

@@ -157,7 +157,11 @@ def test_reset_and_field_roundtrip(rlfc, init_state, tmp_path):
             env.load_bdim(0, bad)
 
 
-@pytest.mark.parametrize("resolution,xl,yl", [(16, 16, 8), (8, 16, 8), (12, 8, 4), (24, 8, 4)])
+# (resolution, x_lengths, y_lengths) besides the default (24, 16, 8); tests/test_gpu_shapes.py holds the ragged ones
+OTHER_GRIDS = [(16, 16, 8), (8, 16, 8), (12, 8, 4), (24, 8, 4)]
+
+
+@pytest.mark.parametrize("resolution,xl,yl", OTHER_GRIDS)
 def test_other_grids(rlfc, oracle, resolution, xl, yl):
     """Other AFCCylinder grids (different columns-per-lane of the row smoother, different MG depths): impulsive
     start, non-zero actions, every float equal to the oracle's."""
