@@ -152,7 +152,8 @@ int  rlfc_env_reset(rlfc_env *env, const int *env_ids, int n, int reset_accumula
 int  rlfc_env_reset_params(rlfc_env *env, const int *env_ids, int n, const rlfc_env_params *params,
                            int reset_accumulators);
 /* params[n_envs]: each environment's constructor arguments (the scalar config's for every environment of a handle
-   created without env_params), as the environments hold them now, including sets switched by rlfc_env_reset_sets_device. */
+   created without env_params), as the environments hold them now, including sets switched by rlfc_env_reset_sets_device
+   and rlfc_env_reset_params_device. */
 int  rlfc_env_get_params(rlfc_env *env, rlfc_env_params *params);
 
 /* setUpNewSim into the parameter library (rlfc_config.param_sets), handles with a library only.  Environment env_ids[k]
@@ -169,6 +170,20 @@ int  rlfc_env_reset_sets(rlfc_env *env, const int *env_ids, const int *sets, int
    entry out of range is skipped (a negative set is the way to skip one, e.g. sets = where(done, draw, -1)); of pairs with
    the same environment the last in-range pair wins. */
 int  rlfc_env_reset_sets_device(rlfc_env *env, const int *d_env_ids, const int *d_sets, int n, int reset_accumulators);
+
+/* setUpNewSim with arbitrary constructor arguments, built on the device: per-environment handles only (env_params or
+   param_sets; else RLFC_EINVAL).  d_env_ids[n] and d_params[n] are DEVICE arrays (rlfc_env_params packed, 20 bytes
+   each); asynchronous on the handle's stream.  An applied pair (e, p) makes environment e bit for bit what
+   rlfc_env_reset_params({e}, {p}, reset_accumulators) makes it: p's geometry in e's own slot, nu, dR*D, dt =
+   t_step*resolution, the Poisson hierarchy, the init state and the reset scalars.  An environment that held a library set
+   goes back to its own slot.  Sensors, probes, MG iteration counts and flags bit 1 stay as they are.
+   Defined for every input: a pair whose id is out of range is skipped (ids = where(done, arange(n_envs), -1) skips the
+   others); of pairs with the same environment the last in-range pair wins.  If the winning pair's set is invalid -- the
+   rules of rlfc_env_params, or |theta| > 6.2831855f (2 pi, the range over which the device reproduces the host's sin and
+   cos; rlfc_env_reset_params accepts any finite theta) -- the environment is left completely unchanged and its flags bit 2
+   is set; a device parameter reset that applies clears it.  RLFC_EINVAL for n < 0 or a NULL array with n > 0. */
+int  rlfc_env_reset_params_device(rlfc_env *env, const int *d_env_ids, const rlfc_env_params *d_params, int n,
+                                  int reset_accumulators);
 
 /* One RL step for every environment, with the cadence of clientCFD.draw() (clientCFD.pde:35-55).  All pointers are
    HOST memory.
@@ -205,7 +220,8 @@ int  rlfc_env_running(rlfc_env *env, int *n_running);
 /* Per-environment health flags, flags[n_envs]: bit 0 = a non-finite force was produced since the last reset (the
    environment has diverged; SURVEY section 5 failure detection).  Bit 1 = the last restore aimed at the environment was
    skipped because its slot was never written or holds a state of another parameter set (rlfc_env_restore_device; a restore
-   that applies clears it).  Synchronises the handle's stream. */
+   that applies clears it).  Bit 2 = the last device parameter reset aimed at the environment was refused because its set
+   is invalid (rlfc_env_reset_params_device; one that applies clears it).  Synchronises the handle's stream. */
 int  rlfc_env_get_flags(rlfc_env *env, int *flags);
 
 /* Snapshots of complete environment states in the handle's rlfc_config.n_snapshots device slots (ALE cloneState /

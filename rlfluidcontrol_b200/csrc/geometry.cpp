@@ -199,6 +199,14 @@ HostLevel coarsen(const HostLevel& F) {
 
 }  // namespace
 
+void circle_vertex_factors(float cos_th[40], float sin_th[40]) {
+  for (int i = 0; i < kCircleVerts; i++) {
+    const float th = -kTwoPi * i / ((float)kCircleVerts);   // as Cylinder's constructor
+    cos_th[i] = fcos(th);
+    sin_th[i] = fsin(th);
+  }
+}
+
 Sample resolve_sample(int n, int m, float x0, float y0, int btype) {
   Sample sp;
   float x = fmin2(fmax2(0.5f, x0), n - 1.5f);

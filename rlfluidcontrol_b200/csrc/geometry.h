@@ -58,6 +58,10 @@ struct Geometry {
 // builds.
 int build_geometry(const rlfc_config& cfg, Geometry& g, std::string& err, bool hierarchy = true);
 
+// The factors cos(th_i), sin(th_i) of the 40 polygon vertex angles th_i = -TWO_PI*i/40 of every body, as build_geometry
+// takes them (the device geometry builder, geometry_device.cuh, reads this table instead of evaluating them).
+void circle_vertex_factors(float cos_th[40], float sin_th[40]);
+
 // Checkpoint IO (BDIM.write / BDIM.resume text format BDIM.pde:226-251, and the .bdimb binary form).
 int read_checkpoint(const std::string& path, int n, int m, float& t, float& dt,
                     std::vector<float>& ux, std::vector<float>& uy, std::vector<float>& p, std::string& err);

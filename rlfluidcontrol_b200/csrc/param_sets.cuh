@@ -29,6 +29,22 @@ struct ResetSetsArgs {
   int* skip;
 };
 
+// rlfc_env_reset's scalars of environment e, with dt = the set's t_step*resolution
+__device__ __forceinline__ void reset_scalars(const EnvScalars& sc, int e, float init_t, float dt0, int reset_acc, int substeps) {
+  sc.xi[2 * e] = 0.f; sc.xi[2 * e + 1] = 0.f;
+  sc.t[e] = 0.f;
+  sc.flow_t[e] = init_t;                                 // BDIM.resume: t = stuff[0]
+  sc.force[2 * e] = 0.f; sc.force[2 * e + 1] = 0.f;
+  sc.frozen[e] = 0;
+  sc.non_finite[e] = 0;
+  sc.dt[e] = dt0;                                        // t_step*resolution
+  if (reset_acc) {
+    sc.callLearn[e] = substeps;
+    sc.Cd[e] = 0.f; sc.Cl[e] = 0.f;
+    sc.obs[2 * e] = 0.f; sc.obs[2 * e + 1] = 0.f;
+  }
+}
+
 __global__ void __launch_bounds__(kSnapThreads) k_reset_sets(const __grid_constant__ ResetSetsArgs a) {
   const int cpf = (a.nv + kSnapThreads * kSnapVec - 1) / (kSnapThreads * kSnapVec);   // chunks per field
   const int f = blockIdx.x / cpf, c = blockIdx.x - f * cpf;
@@ -48,19 +64,7 @@ __global__ void __launch_bounds__(kSnapThreads) k_reset_sets(const __grid_consta
       a.env_nby[e] = L.nby;
       if (a.env_par)
         for (int w = 0; w < 5; w++) a.env_par[(size_t)w * a.B + e] = L.bits[w];
-      // rlfc_env_reset's scalars
-      a.sc.xi[2 * e] = 0.f; a.sc.xi[2 * e + 1] = 0.f;
-      a.sc.t[e] = 0.f;
-      a.sc.flow_t[e] = a.init_t;                             // BDIM.resume: t = stuff[0]
-      a.sc.force[2 * e] = 0.f; a.sc.force[2 * e + 1] = 0.f;
-      a.sc.frozen[e] = 0;
-      a.sc.non_finite[e] = 0;
-      a.sc.dt[e] = L.dt0;                                    // t_step*resolution
-      if (a.reset_acc) {
-        a.sc.callLearn[e] = a.substeps;
-        a.sc.Cd[e] = 0.f; a.sc.Cl[e] = 0.f;
-        a.sc.obs[2 * e] = 0.f; a.sc.obs[2 * e + 1] = 0.f;
-      }
+      reset_scalars(a.sc, e, a.init_t, L.dt0, a.reset_acc, a.substeps);
       a.skip[e] = 0;
     }
   }

@@ -60,6 +60,10 @@ struct rlfc_env {
   std::vector<LibSet> h_lib;               // [L] host copy of lib.sets
   std::vector<int> h_env_set;              // [B] host copy of lib.env_set as of the last sync_env_sets
   int *set_env = nullptr, *set_ids = nullptr;   // [B] the pairs of a host rlfc_env_reset_sets call
+  // device parameter resets (rlfc_env_reset_params_device; per-environment handles)
+  ParamReset pr{};
+  CircleFactors circle{};                  // the 40 polygon vertex factors the device builder reads
+  bool par_pending = false;                // a device parameter reset was enqueued since the last sync_env_sets
   int device = 0;
   cudaStream_t stream = nullptr;
   bool own_stream = false;
@@ -356,6 +360,8 @@ int upload_env_scalars(rlfc_env* E) {
   CU(cudaMemcpyAsync(const_cast<float*>(sp.env_dRD), E->h_dRD.data(), B * sizeof(float), cudaMemcpyHostToDevice, E->stream));
   CU(cudaMemcpyAsync(const_cast<int*>(sp.env_nband_x), E->h_nbx.data(), B * sizeof(int), cudaMemcpyHostToDevice, E->stream));
   CU(cudaMemcpyAsync(const_cast<int*>(sp.env_nband_y), E->h_nby.data(), B * sizeof(int), cudaMemcpyHostToDevice, E->stream));
+  if (E->pr.params)
+    CU(cudaMemcpyAsync(E->pr.params, E->params.data(), B * sizeof(rlfc_env_params), cudaMemcpyHostToDevice, E->stream));
   if (E->lib.L) {   // (env_slot is written at create otherwise; with a library the device changes it too)
     std::vector<int> slot(B);
     for (int e = 0; e < (int)B; e++) slot[e] = E->h_env_set[e] < 0 ? e : E->h_lib[E->h_env_set[e]].slot;
@@ -369,23 +375,41 @@ int upload_env_scalars(rlfc_env* E) {
 // ---- parameter library (rlfc_config.param_sets) ----
 
 // The host copies of what an environment holds (params, dt0, h_nu, h_dRD, h_nbx, h_nby) go stale once the device switches
-// it to a library set.  Host entry points that read them call this first: it synchronises the handle's stream, reads
-// lib.env_set back and refreshes the copies of the environments that hold a library set.  (An environment back on its own
-// slot got its copies from rlfc_env_reset_params, which put it there.)  Without a library it does nothing.
+// it to a library set or builds it a new set (rlfc_env_reset_params_device).  Host entry points that read them call this
+// first: it synchronises the handle's stream, reads lib.env_set back and refreshes the copies of the environments that
+// hold a library set; after a device parameter reset it also reads back the set and band counts each environment holds on
+// its own slot.  (Otherwise an environment on its own slot got its copies from rlfc_env_reset_params, which put it there.)
+// Without a library and without a device parameter reset since the last call it does nothing.
 int sync_env_sets(rlfc_env* E) {
-  if (!E->lib.L) return RLFC_OK;
+  if (!E->lib.L && !E->par_pending) return RLFC_OK;
   const int B = E->sp.B;
-  CU(cudaMemcpyAsync(E->h_env_set.data(), E->lib.env_set, B * sizeof(int), cudaMemcpyDeviceToHost, E->stream));
+  std::vector<rlfc_env_params> own(E->par_pending ? B : 0);
+  std::vector<int> nbx(own.size()), nby(own.size());
+  if (E->lib.L) CU(cudaMemcpyAsync(E->h_env_set.data(), E->lib.env_set, B * sizeof(int), cudaMemcpyDeviceToHost, E->stream));
+  if (E->par_pending) {
+    CU(cudaMemcpyAsync(own.data(), E->pr.params, B * sizeof(rlfc_env_params), cudaMemcpyDeviceToHost, E->stream));
+    CU(cudaMemcpyAsync(nbx.data(), E->sp.env_nband_x, B * sizeof(int), cudaMemcpyDeviceToHost, E->stream));
+    CU(cudaMemcpyAsync(nby.data(), E->sp.env_nband_y, B * sizeof(int), cudaMemcpyDeviceToHost, E->stream));
+  }
   CU(cudaStreamSynchronize(E->stream));
   for (int e = 0; e < B; e++) {
-    const int s = E->h_env_set[e];
-    if (s < 0) continue;
-    const LibSet& L = E->h_lib[s];
-    E->params[e] = E->lib_params[s];
-    E->dt0[e] = L.dt0;
-    E->h_nu[e] = L.nu; E->h_dRD[e] = L.dRD;
-    E->h_nbx[e] = L.nbx; E->h_nby[e] = L.nby;
+    const int s = E->lib.L ? E->h_env_set[e] : -1;
+    if (s >= 0) {
+      const LibSet& L = E->h_lib[s];
+      E->params[e] = E->lib_params[s];
+      E->dt0[e] = L.dt0;
+      E->h_nu[e] = L.nu; E->h_dRD[e] = L.dRD;
+      E->h_nbx[e] = L.nbx; E->h_nby[e] = L.nby;
+    } else if (E->par_pending) {   // what build_geometry makes of the set (geometry.cpp)
+      const rlfc_env_params& p = own[e];
+      const float D = (float)E->cfg.resolution;
+      E->params[e] = p;
+      E->dt0[e] = p.t_step * E->cfg.resolution;
+      E->h_nu[e] = D / p.re; E->h_dRD[e] = p.dR * D;
+      E->h_nbx[e] = nbx[e]; E->h_nby[e] = nby[e];
+    }
   }
+  E->par_pending = false;
   return RLFC_OK;
 }
 
@@ -1270,6 +1294,10 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
     float* f = nullptr;
     TRY(E->dmalloc(&f, B)); sp.env_nu = f;
     TRY(E->dmalloc(&f, B)); sp.env_dRD = f;
+    if (env_mode) {   // rlfc_env_reset_params_device
+      TRY(E->dmalloc(&E->pr.params, B)); TRY(E->dmalloc(&E->pr.status, B)); TRY(E->dmalloc(&E->pr.refused, B));
+      circle_vertex_factors(E->circle.c, E->circle.s);
+    }
     if (cudaMemcpyAsync(d = const_cast<int*>(sp.env_slot), slot.data(), B * sizeof(int), cudaMemcpyHostToDevice, E->stream) != cudaSuccess)
       return bail(fail(RLFC_ECUDA, "slot table upload failed"));
     TRY(upload_env_scalars(E));
@@ -1666,6 +1694,10 @@ int rlfc_env_step(rlfc_env* E, const float* actions, float* obs, float* reward, 
   // (adaptive mode: the bound follows the smallest dt any environment has taken in the rounds so far)
   // (per-environment mode: the smallest t_step*resolution to start with)
   const float init_time = sp.init_time > 0 ? sp.init_time : 0;
+  if (E->par_pending) {   // (dt0 after a device parameter reset)
+    int rc = sync_env_sets(E);
+    if (rc) return rc;
+  }
   float dt_min = sp.dt;
   if (sp.per_env) dt_min = *std::min_element(E->dt0.begin(), E->dt0.end());
   for (const LibSet& L : E->h_lib) dt_min = std::min(dt_min, L.dt0);   // (a bound over own and library sets: no sync)
@@ -1825,11 +1857,14 @@ int rlfc_env_running(rlfc_env* E, int* n_running) {
 int rlfc_env_get_flags(rlfc_env* E, int* flags) {
   if (!E || !flags) return fail(RLFC_EINVAL, "null argument");
   CU(cudaSetDevice(E->device));
-  std::vector<int> refused(E->snap.S ? E->sp.B : 0);
+  std::vector<int> refused(E->snap.S ? E->sp.B : 0), par_refused(E->pr.refused ? E->sp.B : 0);
   CU(cudaMemcpyAsync(E->h_done, E->sp.sc.non_finite, E->sp.B * sizeof(int), cudaMemcpyDeviceToHost, E->stream));
   if (E->snap.S) CU(cudaMemcpyAsync(refused.data(), E->snap.refused, E->sp.B * sizeof(int), cudaMemcpyDeviceToHost, E->stream));
+  if (E->pr.refused)
+    CU(cudaMemcpyAsync(par_refused.data(), E->pr.refused, E->sp.B * sizeof(int), cudaMemcpyDeviceToHost, E->stream));
   CU(cudaStreamSynchronize(E->stream));
-  for (int e = 0; e < E->sp.B; e++) flags[e] = (E->h_done[e] ? 1 : 0) | (E->snap.S && refused[e] ? 2 : 0);
+  for (int e = 0; e < E->sp.B; e++)
+    flags[e] = (E->h_done[e] ? 1 : 0) | (E->snap.S && refused[e] ? 2 : 0) | (E->pr.refused && par_refused[e] ? 4 : 0);
   return RLFC_OK;
 }
 
@@ -1881,6 +1916,29 @@ int rlfc_env_reset_sets_device(rlfc_env* E, const int* d_env_ids, const int* d_s
   if (rc) return rc;
   CU(cudaSetDevice(E->device));
   return reset_sets_enqueue(E, d_env_ids, d_sets, n, reset_accumulators != 0);
+}
+
+int rlfc_env_reset_params_device(rlfc_env* E, const int* d_env_ids, const rlfc_env_params* d_params, int n,
+                                 int reset_accumulators) {
+  if (!E) return fail(RLFC_EINVAL, "null handle");
+  if (!E->env_mode)
+    return fail(RLFC_EINVAL, "rlfc_env_reset_params_device needs a handle created with env_params or param_sets");
+  if (n < 0) return fail(RLFC_EINVAL, "bad pair count");
+  if (n > 0 && (!d_env_ids || !d_params)) return fail(RLFC_EINVAL, "null argument");
+  if (n == 0) return RLFC_OK;
+  CU(cudaSetDevice(E->device));
+  SolverParams& sp = E->whole.sp;
+  CU(cudaMemsetAsync(E->d_skip, 1, sp.B * sizeof(int), E->stream));   // nonzero = keep; the reset clears
+  E->run("k_param_geometry+k_reset_params", 0, [&] {
+    return launch_reset_params(sp, E->lib, E->snap, E->pr, E->circle, E->cfg.x_lengths * E->cfg.resolution,
+                               E->cfg.y_lengths * E->cfg.resolution, sp.nband_x, E->init_ux, E->init_uy, E->init_p, E->init_t,
+                               E->uAx, E->uAy, d_env_ids, d_params, n, reset_accumulators != 0, E->d_skip, E->stream);
+  });
+  E->run("k_poisson_rebuild0", 0, [&] { return launch_poisson_rebuild0(sp, E->d_skip, E->stream); });
+  E->run("k_poisson_rebuild_coarse", 0, [&] { return launch_poisson_rebuild_coarse(sp, E->d_skip, E->stream); });
+  CU(cudaGetLastError());
+  E->par_pending = true;
+  return RLFC_OK;
 }
 
 int rlfc_env_get_sensors(rlfc_env* E, float* out) {

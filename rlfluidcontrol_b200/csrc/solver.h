@@ -13,6 +13,8 @@
 #include <cstddef>
 #include <cstdint>
 
+#include "../../include/rlfc.h"
+
 namespace rlfc {
 
 constexpr int kMaxLevels = 16;
@@ -207,6 +209,18 @@ struct ParamLib {
   int* env_set;             // [B] the set each environment holds, -1 = its own slot (env_params / rlfc_env_reset_params)
 };
 
+// Device parameter resets (rlfc_env_reset_params_device; geometry_device.cuh) of a per-environment handle.  Kept out of
+// SolverParams for the reason SensorSet is.
+struct ParamReset {
+  rlfc_env_params* params;  // [B] the set each environment holds on its own slot (what the host copies are refreshed from)
+  int* status;              // [B] outcome for the winning pair of the last call: 1 = applied, 2 = refused
+  int* refused;             // [B] 1 = the last device parameter reset aimed at the environment was refused (flags bit 2)
+};
+// The factors of the 40 polygon vertex angles (geometry.h circle_vertex_factors), passed by value.
+struct CircleFactors {
+  float c[40], s[40];
+};
+
 #ifdef __CUDACC__
 // true = block `blk` of `nblk` (a kernel's row-block or strip index) belongs to another device
 __device__ __forceinline__ bool slab_skip(unsigned blk, unsigned nblk, int rank, int n) {
@@ -300,5 +314,16 @@ int launch_snapshot_copy(const SolverParams& P, const SnapSlots& s, const Sensor
 int launch_reset_sets(const SolverParams& P, const ParamLib& lib, const SnapSlots& snap, const float* init_ux,
                       const float* init_uy, const float* init_p, float init_t, float* ux, float* uy, const int* d_env,
                       const int* d_set, int n, int reset_accumulators, int* skip, cudaStream_t st);
+// Device parameter reset of n (environment, parameter set) pairs, device arrays d_env[n], d_par[n] (P: the whole batch,
+// per_env; two launches): the winning pair of each environment (pairs out of range are skipped, the last in-range pair per
+// environment wins) is validated as build_env_geometries validates a set, plus |theta| <= 2 pi.  An applied pair builds the
+// set's geometry into the environment's own slot (del, the body-velocity basis, the band lists, as build_geometry and
+// band_lists make them), points the environment at it (env_slot, lib.env_set = -1, env_nu, env_dRD, env_nband_x/y,
+// pr.params, snap.env_par) and does what launch_reset_sets does with dt = t_step*resolution; a refused pair changes
+// nothing but pr.refused[e] = 1.  cap = the slots' band capacity (nband_x == nband_y).
+int launch_reset_params(const SolverParams& P, const ParamLib& lib, const SnapSlots& snap, const ParamReset& pr,
+                        const CircleFactors& cf, int nc, int mc, int cap, const float* init_ux, const float* init_uy,
+                        const float* init_p, float init_t, float* ux, float* uy, const int* d_env,
+                        const rlfc_env_params* d_par, int n, int reset_accumulators, int* skip, cudaStream_t st);
 
 }  // namespace rlfc

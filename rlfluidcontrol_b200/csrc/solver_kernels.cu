@@ -1957,3 +1957,4 @@ int launch_emit_obs(const SolverParams& q, const float* d_actions, float* d_obs,
 
 #include "snapshot.cuh"
 #include "param_sets.cuh"
+#include "geometry_device.cuh"

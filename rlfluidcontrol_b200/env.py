@@ -85,6 +85,7 @@ def load_library():
     L.rlfc_env_get_params.argtypes = [vp, C.POINTER(EnvParams)]
     L.rlfc_env_reset_sets.argtypes = [vp, ip, ip, C.c_int, C.c_int]
     L.rlfc_env_reset_sets_device.argtypes = [vp, vp, vp, C.c_int, C.c_int]
+    L.rlfc_env_reset_params_device.argtypes = [vp, vp, vp, C.c_int, C.c_int]
     L.rlfc_env_step.argtypes = [vp, fp, fp, fp, ip]
     L.rlfc_env_step_device.argtypes = [vp, vp, vp, vp, vp]
     L.rlfc_env_substep.argtypes = [vp, fp, fp, fp]
@@ -272,6 +273,15 @@ class AFCCylinderBatch:
         self._check(self._L.rlfc_env_reset_sets_device(self._h, C.c_void_p(d_env_ids), C.c_void_p(d_sets), int(n),
                                                        int(reset_accumulators)), "rlfc_env_reset_sets_device")
 
+    def reset_params_device(self, d_env_ids, d_params, n, reset_accumulators=False):
+        """reset(params=...) with the parameter sets built on the device: device arrays of length n (data_ptr() ints),
+        int32 environment ids and packed rlfc_env_params (20 bytes each: int32 re, float32 dR, gR, theta, t_step, e.g. an
+        (n, 5) int32 tensor torch.stack([re.int(), dR.view(torch.int32), ...], 1)), asynchronous on the handle's stream.
+        Pairs whose id is out of range (e.g. -1) are skipped; of pairs with the same environment the last wins.  An
+        invalid set, or |theta| > 2 pi, leaves its environment unchanged and sets flags() bit 2."""
+        self._check(self._L.rlfc_env_reset_params_device(self._h, C.c_void_p(d_env_ids), C.c_void_p(d_params), int(n),
+                                                         int(reset_accumulators)), "rlfc_env_reset_params_device")
+
     def params(self):
         """Each environment's constructor arguments: a structured array with the fields re, dR, gR, theta, t_step."""
         arr = (EnvParams * self.n_envs)()
@@ -417,7 +427,8 @@ class AFCCylinderBatch:
 
     def flags(self):
         """Per-environment health flags (bit 0: a non-finite force was produced since the last reset; bit 1: the last
-        restore aimed at the environment was skipped, its slot unwritten or of another parameter set)."""
+        restore aimed at the environment was skipped, its slot unwritten or of another parameter set; bit 2: the last
+        device parameter reset aimed at the environment was refused, its set invalid)."""
         f = np.empty(self.n_envs, np.int32)
         self._check(self._L.rlfc_env_get_flags(self._h, f.ctypes.data_as(C.POINTER(C.c_int))), "rlfc_env_get_flags")
         return f
