@@ -96,7 +96,8 @@ struct rlfc_env {
     long long graph_launches = 0;            // kernel nodes of one replay outside the MG loops' WHILE bodies
   };
   std::vector<Group> groups;
-  Group whole;                               // the entire batch on the handle's stream (eager / profiled path)
+  Group whole;                               // the entire batch on the handle's stream (eager / profiled path; slab mode:
+                                             // the whole domain as device 0 sees it alone)
   // Slab mode (cfg.n_devices > 1, BASELINE config 5): one domain advanced by several devices over one shared address
   // range (vmm.h); every device runs the same kernel sequence on its row blocks / strips, a barrier between kernels
   struct SlabDev {
@@ -107,7 +108,6 @@ struct rlfc_env {
     void* local[2] = {nullptr, nullptr};     // cudaMalloc'd on this device: ticket counters, barrier epoch
   };
   std::vector<SlabDev> slab;
-  SolverParams solo{}, soloB{};              // the whole domain as ONE device sees it (kernels that run on device 0 only)
   VmmPool vmm;
   bool home_only = false;                    // dmalloc: keep the next allocations on device 0 (data only it touches)
   long long slab_barriers = 0;
@@ -531,186 +531,272 @@ int snapshot_host(rlfc_env* E, const int* env_ids, const int* slots, int n, int 
   return RLFC_OK;
 }
 
-// ---- one MG-projected half step on velocity buffer U (BDIM.updateUP tail + VectorField.project) ----
-// The floats-per-interior-cell figures are each kernel's ALGORITHMIC traffic per env (SURVEY 8d
-// convention: per-env arrays only, one read per input and one write per output).
-// Level-0 residual flow of one MG iteration: down0 reads r and writes the smoothed residual to the `d`
-// buffer, up0 updates it in place, smooth0 consumes it and writes the new residual back to r.
+// ---- one solver step (AFCCylinder.update2, AFCCylinder.pde:45-61), written once for every path ----
+// solver_step lists the kernels of one step in launch order and hands each to a sink, which launches it eagerly (EagerSink:
+// RLFC_NO_GRAPH, rlfc_env_set_profiling), captures it into a group's step graph (CaptureSink) or launches it on every device
+// of a slab-mode handle (SlabSink).  The floats-per-interior-cell figures are each kernel's ALGORITHMIC traffic per env
+// (SURVEY 8d convention: per-env arrays only, one read per input and one write per output).
 using Group = rlfc_env::Group;
+using SlabDev = rlfc_env::SlabDev;
 
-// eager path: every kernel individually launched (optionally event-timed); the data-dependent loop exit
-// (MG.pde:34) costs one 4-byte readback per iteration
-int project_eager(rlfc_env* E, Group& G, float* Ux, float* Uy, int which) {
-  SolverParams& sp = G.sp;
-  SolverParams& sb = G.spB;
-  cudaStream_t st = G.st;
+enum View : bool { kA = false, kB = true };      // the view a kernel takes: pressure buffer A (sp) or B (spB) at lev[0].x
+enum Place : bool { kEach = false, kSolo = true };   // slab mode: every device on its own rows / strips, or device 0 alone
+struct StepKernel {
+  const char* name;         // profile name (rlfc_env_get_profile)
+  double fpc;               // floats per interior cell
+  View view;
+  Place place;
+};
+
+enum { kDown, kUp, kSweeps, kIncr };
+// profile name of one kernel of a chained level l; the levels from 4 on share one name
+const char* chain_name(int piece, int l) {
+  static const char* const nm[4][5] = {
+      {"k_chain_down_L0", "k_chain_down_L1", "k_chain_down_L2", "k_chain_down_L3", "k_chain_down_L4+"},
+      {"k_chain_up_L0", "k_chain_up_L1", "k_chain_up_L2", "k_chain_up_L3", "k_chain_up_L4+"},
+      {"k_chain_sweeps_L0", "k_chain_sweeps_L1", "k_chain_sweeps_L2", "k_chain_sweeps_L3", "k_chain_sweeps_L4+"},
+      {"k_chain_incr_L0", "k_chain_incr_L1", "k_chain_incr_L2", "k_chain_incr_L3", "k_chain_incr_L4+"}};
+  return nm[piece][std::min(l, 4)];
+}
+
+// One MG-projected half step on velocity buffer U (BDIM.updateUP tail + VectorField.project); which = 1: the corrector.
+// Level-0 residual flow of one MG iteration: down0 reads r and writes the smoothed residual to the `d` buffer, up0 updates
+// it in place, smooth0 consumes it and writes the new residual back to r.
+template <class Sink>
+int project(Sink& S, const Group& G, float* Ux, float* Uy, int which) {
+  const SolverParams& sp = G.sp;
   float* r = sp.lev[0].r;
   float* rs = sp.lev[0].d;
   float* pA = sp.lev[0].x;
-  float* pB = sb.lev[0].x;
+  float* pB = G.spB.lev[0].x;
+  const int nch = sp.chain_levels;   // levels 0 .. nch-1 chained (grid-wide kernels); the one-CTA kernel takes the rest
+  // below level 0's restriction: the chained levels' restrictions, the coarse levels, the chained levels' corrections and
+  // smooth(4) top down; then level 0's
+  auto vcycle = [&] {
+    for (int l = 1; l < nch; l++) {
+      S.run({chain_name(kDown, l), 0, kB, kEach}, [&](auto& v, auto st) { return launch_chain_down(v, l, st); });
+      S.sync();
+    }
+    S.run({nch ? "k_mg_coarse_cta" : "k_mg_coarse", 0.5, kB, kSolo}, [&](auto& v, auto st) { return launch_coarse_cta(v, st); });
+    S.sync();
+    for (int l = nch - 1; l >= 0; l--) {
+      S.run({chain_name(kUp, l), l ? 0 : 4.25, kB, kEach}, [&](auto& v, auto st) { return launch_chain_up(v, l, l ? nullptr : rs, st); });
+      S.sync();
+      S.run({chain_name(kSweeps, l), l ? 0 : 3.0, kB, kEach}, [&](auto& v, auto st) { return launch_chain_sweeps(v, l, st); });
+      S.sync();
+      S.run({chain_name(kIncr, l), l ? 0 : 4.0, kB, kEach},
+            [&](auto& v, auto st) { return launch_chain_incr(v, l, l ? nullptr : r, l ? 0 : which, st); });
+      S.sync();
+    }
+    if (!nch) {
+      S.run({"k_mg_up0", 4.25, kB, kEach}, [&](auto& v, auto st) { return launch_mg_up0(v, rs, st); });
+      S.run({"k_smooth0", 4, kB, kEach}, [&](auto& v, auto st) { return launch_smooth0(v, rs, r, which, st); });
+    }
+  };
+  int rc = S.mg_loop(
+      [&] {   // the first iteration (MG.pde:32-35 is a do-while in effect: iter < itmx holds on entry)
+        S.run({"k_resid_down0", 5.25, kA, kEach},
+              [&](auto& v, auto st) { return launch_resid_down0(v, Ux, Uy, pA, pB, rs, which, st); });
+        S.sync();
+        vcycle();
+      },
+      [&] {   // a further iteration (the row smoother has left the residual skewed)
+        if (!nch && !sp.lev[0].wave) S.run({"k_unskew_r", 2, kB, kEach}, [&](auto& v, auto st) { return launch_unskew_r(v, r, st); });
+        S.run({"k_mg_down0", 4.25, kB, kEach}, [&](auto& v, auto st) { return launch_mg_down0(v, r, rs, st); });
+        S.sync();
+        vcycle();
+      });
+  if (rc) return rc;
+  // Field.sum (a serial float chain over the whole field): segment summaries (tables, then the serial pass), or the plain chain
+  if (sp.xs_recs) {
+    S.run({"k_xsum_tables", 1, kB, kSolo}, [&](auto& v, auto st) { return launch_psum_tables(v, st); });
+    S.run({"k_xsum_pass", 0, kB, kSolo}, [&](auto& v, auto st) { return launch_psum_pass(v, st); });
+  } else {
+    S.run({"k_psum", 1, kB, kSolo}, [&](auto& v, auto st) { return launch_psum(v, st); });
+  }
+  S.sync();
+  if (which == 1 && sp.fast_bc) {
+    // corrector: Heun average fused into the projection and the boundary-condition kernels (BDIM.pde:95-96)
+    S.run({"k_project_shift_heun", 8, kA, kEach},
+          [&](auto& v, auto st) { return launch_project_shift_heun(v, pB, pA, Ux, Uy, G.uBx, G.uBy, G.uAx, G.uAy, st); });
+    S.sync();
+    S.run({"k_bc_heun", 0, kA, kSolo}, [&](auto& v, auto st) { return launch_bc_heun(v, Ux, Uy, G.uBx, G.uBy, G.uAx, G.uAy, st); });
+  } else {
+    S.run({"k_project_shift", 6, kA, kEach}, [&](auto& v, auto st) { return launch_project_shift(v, pB, pA, Ux, Uy, st); });
+    S.sync();
+    S.run({"k_bc", 0, kA, kSolo}, [&](auto& v, auto st) { return launch_bc(v, Ux, Uy, st); });
+  }
+  S.sync();
+  return RLFC_OK;
+}
+
+// AFCCylinder.update2 for view G.  Sink: run(StepKernel, launch(view, stream) -> launches), sync() (slab mode: a barrier
+// of all devices between dependent kernels; the other sinks ignore it) and mg_loop(first iteration, further iteration).
+template <class Sink>
+int solver_step(Sink& S, const Group& G, int accumulate) {
+  const SolverParams& sp = G.sp;
+  int rc;
+  S.sync();   // (slab mode: whatever device 0 enqueued since the last step -- actions, resets, field uploads -- is visible to all)
+  if (sp.adaptive) {
+    // AFCCylinder.update (AFCCylinder.pde:63-84): dt = flow.checkCFL(), then the Poisson hierarchy of c = del*dt, on the
+    // device (dt never goes to the host).  (Slab mode has neither adaptive dt nor sensors.)
+    S.run({"k_check_cfl", 2, kA, kSolo}, [&](auto& v, auto st) { return launch_step_cfl(v, G.uAx, G.uAy, st); });
+    S.run({"k_poisson_rebuild0", 0, kA, kSolo}, [&](auto& v, auto st) { return launch_poisson_rebuild0(v, v.sc.frozen, st); });
+    S.run({"k_poisson_rebuild_coarse", 0, kA, kSolo},
+          [&](auto& v, auto st) { return launch_poisson_rebuild_coarse(v, v.sc.frozen, st); });
+  }
+  // which = 0, predictor BDIM.update(): u0 = u (buffer A), F = AdvDif(u) -> B, updateUP
+  // which = 1, corrector BDIM.update2(): us = u (B), F = AdvDif(u; + u0) -> C, updateUP, u = (u + us)/2 -> A
+  for (int which = 0; which < 2; which++) {
+    float* sx = which ? G.uBx : G.uAx;
+    float* sy = which ? G.uBy : G.uAy;
+    float* dx = which ? G.uCx : G.uBx;
+    float* dy = which ? G.uCy : G.uBy;
+    S.run({"k_advdif", 5, kA, kEach}, [&](auto& v, auto st) { return launch_advdif(v, sx, sy, G.uAx, G.uAy, dx, dy, st); });
+    S.sync();
+    S.run({"k_band_bc", 0, kA, kSolo}, [&](auto& v, auto st) { return launch_band_bc(v, dx, dy, st); });
+    S.sync();
+    if ((rc = project(S, G, dx, dy, which))) return rc;
+  }
+  if (!sp.fast_bc) {
+    S.run({"k_heun", 6, kA, kEach}, [&](auto& v, auto st) { return launch_heun(v, G.uCx, G.uCy, G.uBx, G.uBy, G.uAx, G.uAy, st); });
+    S.sync();
+  }
+  // (before k_force, which freezes an environment at the end of its window: this step's sample is its observation)
+  if (G.sens.n > 0) S.run({"k_sensors", 0, kA, kSolo}, [&](auto& v, auto st) { return launch_sensors(v, G.sens, G.uAx, G.uAy, st); });
+  S.run({"k_force", 0, kA, kSolo}, [&](auto& v, auto st) { return launch_force(v, accumulate, st); });
+  S.sync();
+  return RLFC_OK;
+}
+
+// the MG loop driven from the host (eager and slab paths): the data-dependent loop exit (MG.pde:34) costs one 4-byte
+// readback of any_active per iteration, on device 0's stream `st`
+template <class First, class Body>
+int polled_mg_loop(rlfc_env* E, const SolverParams& sp, cudaStream_t st, First& first, Body& body) {
   for (int it = 0; it < sp.mg_max_iters; it++) {
+    cudaSetDevice(E->device);   // (slab mode: the iteration's kernels leave another device current)
     CU(cudaMemsetAsync(sp.sc.any_active, 0, sizeof(int), st));
-    if (it == 0)
-      E->run("k_resid_down0", 5.25, [&] { return launch_resid_down0(sp, Ux, Uy, pA, pB, rs, which, st); }, st);
-    else {
-      // (the row smoother has left the residual skewed)
-      E->run("k_unskew_r", 2, [&] { return launch_unskew_r(sb, r, st); }, st);
-      E->run("k_mg_down0", 4.25, [&] { return launch_mg_down0(sb, r, rs, st); }, st);
-    }
-    if (sp.chain_levels > 0 && E->profiling) {   // per-kernel timing of the chained levels
-      const int first = std::max(1, sp.chain_levels);
-      static const char* nm[4][4] = {{"k_chain_down_L1", "k_chain_up_L1", "k_chain_sweeps_L1", "k_chain_incr_L1"},
-                                     {"k_chain_down_L2", "k_chain_up_L2", "k_chain_sweeps_L2", "k_chain_incr_L2"},
-                                     {"k_chain_down_L3", "k_chain_up_L3", "k_chain_sweeps_L3", "k_chain_incr_L3"},
-                                     {"k_chain_down_L4+", "k_chain_up_L4+", "k_chain_sweeps_L4+", "k_chain_incr_L4+"}};
-      for (int l = 1; l < first; l++) E->run(nm[std::min(l, 4) - 1][0], 0, [&] { return launch_chain_down(sb, l, st); }, st);
-      E->run("k_mg_coarse_cta", 0.5, [&] { return launch_coarse_cta(sb, st); }, st);
-      for (int l = first - 1; l >= 1; l--) {
-        E->run(nm[std::min(l, 4) - 1][1], 0, [&] { return launch_chain_up(sb, l, nullptr, st); }, st);
-        E->run(nm[std::min(l, 4) - 1][2], 0, [&] { return launch_chain_sweeps(sb, l, st); }, st);
-        E->run(nm[std::min(l, 4) - 1][3], 0, [&] { return launch_chain_incr(sb, l, nullptr, 0, st); }, st);
-      }
-      E->run("k_chain_up_L0", 4.25, [&] { return launch_chain_up(sb, 0, rs, st); }, st);
-      E->run("k_chain_sweeps_L0", 3, [&] { return launch_chain_sweeps(sb, 0, st); }, st);
-      E->run("k_chain_incr_L0", 4, [&] { return launch_chain_incr(sb, 0, r, which, st); }, st);
-    } else {
-    E->run("k_mg_coarse", 0.5, [&] { return launch_mg_coarse(sb, st); }, st);
-    E->run("k_mg_up0", 4.25, [&] { return launch_mg_up0(sb, rs, st); }, st);
-    E->run("k_smooth0", 4, [&] { return launch_smooth0(sb, rs, r, which, st); }, st);
-    }
+    if (it == 0) first();
+    else body();
     E->mg_iter_launch_rounds++;
+    cudaSetDevice(E->device);
     CU(cudaMemcpyAsync(E->h_any, sp.sc.any_active, sizeof(int), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));
     if (!*E->h_any) break;
   }
-  if (E->profiling && sb.xs_recs) {
-    E->run("k_xsum_tables", 1, [&] { return launch_psum_tables(sb, st); }, st);
-    E->run("k_xsum_pass", 0, [&] { return launch_psum_pass(sb, st); }, st);
-  } else {
-    E->run("k_psum", 1, [&] { return launch_psum(sb, st); }, st);
+  return RLFC_OK;
+}
+
+// eager path: every kernel launched on its own on the view's stream, event-timed when profiling
+struct EagerSink {
+  rlfc_env* E;
+  const Group& G;
+  template <class F>
+  void run(const StepKernel& k, F&& launch) {
+    E->run(k.name, k.fpc, [&] { return launch(k.view == kB ? G.spB : G.sp, G.st); }, G.st);
   }
-  if (which == 1 && sp.fast_bc) {
-    // corrector: Heun average fused into the projection and the boundary-condition kernels (BDIM.pde:95-96)
-    E->run("k_project_shift_heun", 8, [&] { return launch_project_shift_heun(sp, pB, pA, Ux, Uy, G.uBx, G.uBy, G.uAx, G.uAy, st); }, st);
-    E->run("k_bc_heun", 0, [&] { return launch_bc_heun(sp, Ux, Uy, G.uBx, G.uBy, G.uAx, G.uAy, st); }, st);
+  void sync() {}
+  template <class First, class Body>
+  int mg_loop(First&& first, Body&& body) { return polled_mg_loop(E, G.sp, G.st, first, body); }
+};
+
+// graph path: one CUDA graph per group = one solver step; each MGsolver loop is a WHILE conditional node whose body is one
+// further iteration and whose condition is written on the device (k_loopcond), so no host round trip remains
+struct CaptureSink {
+  rlfc_env* E;
+  const Group& G;
+  cudaStream_t st;          // the stream being captured: the group's, or aux_stream while a WHILE body is recorded
+  long long launches = 0;   // kernel nodes outside the WHILE bodies (Group::graph_launches)
+  template <class F>
+  void run(const StepKernel& k, F&& launch) {
+    launches += launch(k.view == kB ? G.spB : G.sp, st);
+  }
+  void sync() {}
+  template <class First, class Body>
+  int mg_loop(First&& first, Body&& body) {
+    first();
+    cudaStreamCaptureStatus status;
+    cudaGraph_t graph;
+    const cudaGraphNode_t* deps;
+    size_t ndeps;
+    CU(cudaStreamGetCaptureInfo(st, &status, nullptr, &graph, &deps, &ndeps));
+    cudaGraphConditionalHandle handle;
+    CU(cudaGraphConditionalHandleCreate(&handle, graph, 0, cudaGraphCondAssignDefault));
+    // the condition is written by a kernel ahead of the node and again at the end of every body pass
+    auto loopcond = [&] { return launch_loopcond(G.spB, (unsigned long long)handle, st); };
+    launches += loopcond();
+    CU(cudaStreamGetCaptureInfo(st, &status, nullptr, &graph, &deps, &ndeps));
+    cudaGraphNodeParams np{};
+    np.type = cudaGraphNodeTypeConditional;
+    np.conditional.handle = handle;
+    np.conditional.type = cudaGraphCondTypeWhile;
+    np.conditional.size = 1;
+    cudaGraphNode_t cond;
+    CU(cudaGraphAddNode(&cond, graph, deps, ndeps, &np));
+    CU(cudaStreamBeginCaptureToGraph(E->aux_stream, np.conditional.phGraph_out[0], nullptr, nullptr, 0,
+                                     cudaStreamCaptureModeThreadLocal));
+    const cudaStream_t outer = st;
+    const long long outer_launches = launches;
+    st = E->aux_stream;
+    body();
+    loopcond();
+    st = outer;
+    launches = outer_launches;
+    CU(cudaStreamEndCapture(E->aux_stream, nullptr));
+    CU(cudaStreamUpdateCaptureDependencies(st, &cond, 1, cudaStreamSetCaptureDependencies));
     return RLFC_OK;
   }
-  E->run("k_project_shift", 6, [&] { return launch_project_shift(sp, pB, pA, Ux, Uy, st); }, st);
-  E->run("k_bc", 0, [&] { return launch_bc(sp, Ux, Uy, st); }, st);
-  return RLFC_OK;
-}
-
-// AFCCylinder.update2 for one group, eager
-int solver_step_eager(rlfc_env* E, Group& G, int accumulate) {
-  SolverParams& sp = G.sp;
-  cudaStream_t st = G.st;
-  int rc;
-  if (sp.adaptive) {
-    // AFCCylinder.update (AFCCylinder.pde:63-84): dt = flow.checkCFL(), then the Poisson hierarchy of c = del*dt
-    E->run("k_check_cfl", 2, [&] { return launch_step_cfl(sp, G.uAx, G.uAy, st); }, st);
-    E->run("k_poisson_rebuild0", 0, [&] { return launch_poisson_rebuild0(sp, sp.sc.frozen, st); }, st);
-    E->run("k_poisson_rebuild_coarse", 0, [&] { return launch_poisson_rebuild_coarse(sp, sp.sc.frozen, st); }, st);
-  }
-  // predictor BDIM.update(): u0 = u (buffer A), F = AdvDif(u) -> B, updateUP
-  E->run("k_advdif", 5, [&] { return launch_advdif(sp, G.uAx, G.uAy, G.uAx, G.uAy, G.uBx, G.uBy, st); }, st);
-  E->run("k_band_bc", 0, [&] { return launch_band_bc(sp, G.uBx, G.uBy, st); }, st);
-  if ((rc = project_eager(E, G, G.uBx, G.uBy, 0))) return rc;
-  // corrector BDIM.update2(): us = u (B), F = AdvDif(u; + u0) -> C, updateUP, u = (u + us)/2 -> A
-  E->run("k_advdif", 5, [&] { return launch_advdif(sp, G.uBx, G.uBy, G.uAx, G.uAy, G.uCx, G.uCy, st); }, st);
-  E->run("k_band_bc", 0, [&] { return launch_band_bc(sp, G.uCx, G.uCy, st); }, st);
-  if ((rc = project_eager(E, G, G.uCx, G.uCy, 1))) return rc;
-  if (!sp.fast_bc)
-    E->run("k_heun", 6, [&] { return launch_heun(sp, G.uCx, G.uCy, G.uBx, G.uBy, G.uAx, G.uAy, st); }, st);
-  // (before k_force, which freezes an environment at the end of its window: this step's sample is its observation)
-  if (G.sens.n > 0) E->run("k_sensors", 0, [&] { return launch_sensors(sp, G.sens, G.uAx, G.uAy, st); }, st);
-  E->run("k_force", 0, [&] { return launch_force(sp, accumulate, st); }, st);
-  CU(cudaGetLastError());
-  return RLFC_OK;
-}
-
-// graph path: one CUDA graph per group = one solver step; each MGsolver loop is a WHILE conditional node whose
-// body is one iteration and whose condition is written on the device (k_loopcond), so no host round trip remains
-int capture_half_step(rlfc_env* E, Group& G, cudaStream_t st, const float* sx, const float* sy, const float* u0x,
-                      const float* u0y, float* dx, float* dy, int which, long long* n_outer) {
-  SolverParams& sp = G.sp;
-  SolverParams& sb = G.spB;
-  float* r = sp.lev[0].r;
-  float* rs = sp.lev[0].d;
-  float* pA = sp.lev[0].x;
-  float* pB = sb.lev[0].x;
-  *n_outer += launch_advdif(sp, sx, sy, u0x, u0y, dx, dy, st);
-  *n_outer += launch_band_bc(sp, dx, dy, st);
-  // first MG iteration (MG.pde:32-35 is a do-while in effect: iter < itmx holds on entry)
-  *n_outer += launch_resid_down0(sp, dx, dy, pA, pB, rs, which, st);
-  *n_outer += launch_mg_coarse(sb, st);
-  *n_outer += launch_mg_up0(sb, rs, st);
-  *n_outer += launch_smooth0(sb, rs, r, which, st);
-  // ---- WHILE node: further iterations while any environment is still unconverged (rare) ----
-  cudaStreamCaptureStatus status;
-  cudaGraph_t graph;
-  const cudaGraphNode_t* deps;
-  size_t ndeps;
-  CU(cudaStreamGetCaptureInfo(st, &status, nullptr, &graph, &deps, &ndeps));
-  cudaGraphConditionalHandle handle;
-  CU(cudaGraphConditionalHandleCreate(&handle, graph, 0, cudaGraphCondAssignDefault));
-  // the condition is written by a kernel ahead of the node and again at the end of every body pass
-  *n_outer += launch_loopcond(sb, (unsigned long long)handle, st);
-  CU(cudaStreamGetCaptureInfo(st, &status, nullptr, &graph, &deps, &ndeps));
-  cudaGraphNodeParams np{};
-  np.type = cudaGraphNodeTypeConditional;
-  np.conditional.handle = handle;
-  np.conditional.type = cudaGraphCondTypeWhile;
-  np.conditional.size = 1;
-  cudaGraphNode_t cond;
-  CU(cudaGraphAddNode(&cond, graph, deps, ndeps, &np));
-  cudaGraph_t body = np.conditional.phGraph_out[0];
-  CU(cudaStreamBeginCaptureToGraph(E->aux_stream, body, nullptr, nullptr, 0, cudaStreamCaptureModeThreadLocal));
-  launch_unskew_r(sb, r, E->aux_stream);
-  launch_mg_down0(sb, r, rs, E->aux_stream);
-  launch_mg_coarse(sb, E->aux_stream);
-  launch_mg_up0(sb, rs, E->aux_stream);
-  launch_smooth0(sb, rs, r, which, E->aux_stream);
-  launch_loopcond(sb, (unsigned long long)handle, E->aux_stream);
-  CU(cudaStreamEndCapture(E->aux_stream, nullptr));
-  CU(cudaStreamUpdateCaptureDependencies(st, &cond, 1, cudaStreamSetCaptureDependencies));
-  // ---- projection tail ----
-  *n_outer += launch_psum(sb, st);
-  if (which == 1 && sp.fast_bc) {   // corrector: Heun average fused in (BDIM.pde:95-96); sx, sy = us, u0x, u0y = step-start buffer
-    *n_outer += launch_project_shift_heun(sp, pB, pA, dx, dy, sx, sy, const_cast<float*>(u0x), const_cast<float*>(u0y), st);
-    *n_outer += launch_bc_heun(sp, dx, dy, sx, sy, const_cast<float*>(u0x), const_cast<float*>(u0y), st);
-  } else {
-    *n_outer += launch_project_shift(sp, pB, pA, dx, dy, st);
-    *n_outer += launch_bc(sp, dx, dy, st);
-  }
-  return RLFC_OK;
-}
+};
 
 int build_step_graph(rlfc_env* E, Group& G, int accumulate) {
-  cudaStream_t st = G.st;
-  long long n_outer = 0;
-  CU(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
-  if (G.sp.adaptive) {   // dt = flow.checkCFL() and the hierarchy of c = del*dt, on the device (dt never goes to the host)
-    n_outer += launch_step_cfl(G.sp, G.uAx, G.uAy, st);
-    n_outer += launch_poisson_rebuild0(G.sp, G.sp.sc.frozen, st);
-    n_outer += launch_poisson_rebuild_coarse(G.sp, G.sp.sc.frozen, st);
-  }
-  int rc = capture_half_step(E, G, st, G.uAx, G.uAy, G.uAx, G.uAy, G.uBx, G.uBy, 0, &n_outer);
-  if (!rc) rc = capture_half_step(E, G, st, G.uBx, G.uBy, G.uAx, G.uAy, G.uCx, G.uCy, 1, &n_outer);
-  if (!rc) {
-    if (!G.sp.fast_bc) n_outer += launch_heun(G.sp, G.uCx, G.uCy, G.uBx, G.uBy, G.uAx, G.uAy, st);
-    n_outer += launch_sensors(G.sp, G.sens, G.uAx, G.uAy, st);   // (nothing without sensors; before k_force, see solver_step_eager)
-    n_outer += launch_force(G.sp, accumulate, st);
-  }
+  CaptureSink S{E, G, G.st};
+  CU(cudaStreamBeginCapture(G.st, cudaStreamCaptureModeThreadLocal));
+  const int rc = solver_step(S, G, accumulate);
   cudaGraph_t graph = nullptr;
-  cudaError_t ce = cudaStreamEndCapture(st, &graph);
+  cudaError_t ce = cudaStreamEndCapture(G.st, &graph);
   if (rc) { if (graph) cudaGraphDestroy(graph); return rc; }
   if (ce != cudaSuccess) return fail(RLFC_ECUDA, std::string("cudaStreamEndCapture: ") + cudaGetErrorString(ce));
   ce = cudaGraphInstantiate(&G.step_graph[accumulate], graph, 0);
   cudaGraphDestroy(graph);
   if (ce != cudaSuccess) return fail(RLFC_ECUDA, std::string("cudaGraphInstantiate: ") + cudaGetErrorString(ce));
-  G.graph_launches = n_outer;
+  G.graph_launches = S.launches;
   return RLFC_OK;
 }
+
+// Slab mode: one solver step of ONE domain on several devices, eager launches.  Grid-wide kernels are launched with their
+// full grid on every device (blocks of other devices' rows / strips exit at once); kernels that are one CTA per environment
+// (setBC, the coarsest levels, Field.sum, the force read-out) run on device 0; a barrier separates dependent kernels.  Halo
+// operands and the few remote results travel as ordinary loads and stores through the shared address range; the
+// Gauss-Seidel sweeps cross device boundaries strip to strip through the tagged edge arrays (smooth_chain3.cuh).
+struct SlabSink {
+  rlfc_env* E;
+  // launch(D) on every device D, event-timed on device 0 when profiling
+  template <class F>
+  void each(const char* name, double fpc, F&& launch) {
+    for (size_t d = 0; d < E->slab.size(); d++) {
+      SlabDev& D = E->slab[d];
+      cudaSetDevice(D.device);
+      if (d == 0) E->run(name, fpc, [&] { return launch(D); }, D.st);
+      else E->launches += launch(D);
+    }
+  }
+  template <class F>
+  void run(const StepKernel& k, F&& launch) {
+    if (k.place == kEach) {
+      each(k.name, k.fpc, [&](SlabDev& D) { return launch(k.view == kB ? D.spB : D.sp, D.st); });
+      return;
+    }
+    const Group& W = E->whole;   // the whole domain as device 0 sees it alone (W.st = device 0's stream)
+    cudaSetDevice(E->device);
+    E->run(k.name, k.fpc, [&] { return launch(k.view == kB ? W.spB : W.sp, W.st); }, W.st);
+  }
+  void sync() {
+    each("k_slab_barrier", 0, [](SlabDev& D) { return launch_slab_barrier(D.bar, D.st); });
+    E->slab_barriers++;
+  }
+  template <class First, class Body>
+  int mg_loop(First&& first, Body&& body) { return polled_mg_loop(E, E->whole.sp, E->whole.st, first, body); }
+};
 
 // fork the group streams off the handle's stream / join them back
 int fork_groups(rlfc_env* E) {
@@ -727,131 +813,24 @@ int join_groups(rlfc_env* E) {
   return RLFC_OK;
 }
 
-// ---- slab mode: one solver step (AFCCylinder.update2) of ONE domain on several devices, eager launches ----
-// Grid-wide kernels are launched with their full grid on every device (blocks of other devices' rows / strips exit at
-// once); kernels that are one CTA per environment (setBC, the coarsest levels, Field.sum, the force read-out) run on
-// device 0; a barrier separates dependent kernels.  Halo operands and the few remote results travel as ordinary
-// loads and stores through the shared address range; the Gauss-Seidel sweeps cross device boundaries strip to strip
-// through the tagged edge arrays (smooth_chain3.cuh).
-using SlabDev = rlfc_env::SlabDev;
-
-template <typename F>
-void slab_all(rlfc_env* E, const char* name, double fpc, F&& launch) {
-  for (size_t d = 0; d < E->slab.size(); d++) {
-    SlabDev& D = E->slab[d];
-    cudaSetDevice(D.device);
-    if (d == 0) E->run(name, fpc, [&] { return launch(D); }, D.st);
-    else E->launches += launch(D);
-  }
-}
-template <typename F>
-void slab_first(rlfc_env* E, const char* name, double fpc, F&& launch) {
-  SlabDev& D = E->slab[0];
-  cudaSetDevice(D.device);
-  E->run(name, fpc, [&] { return launch(D); }, D.st);
-}
-void slab_barrier(rlfc_env* E) {
-  slab_all(E, "k_slab_barrier", 0, [&](SlabDev& D) { return launch_slab_barrier(D.bar, D.st); });
-  E->slab_barriers++;
-}
-
-int slab_project(rlfc_env* E, float* Ux, float* Uy, int which) {
-  const SolverParams& s0 = E->slab[0].sp;
-  float* r = s0.lev[0].r;
-  float* rs = s0.lev[0].d;
-  float* pA = s0.lev[0].x;
-  float* pB = E->slab[0].spB.lev[0].x;
-  const int first = std::max(1, s0.chain_levels);
-  static const char* nm[4][4] = {{"k_chain_down_L1", "k_chain_up_L1", "k_chain_sweeps_L1", "k_chain_incr_L1"},
-                                 {"k_chain_down_L2", "k_chain_up_L2", "k_chain_sweeps_L2", "k_chain_incr_L2"},
-                                 {"k_chain_down_L3", "k_chain_up_L3", "k_chain_sweeps_L3", "k_chain_incr_L3"},
-                                 {"k_chain_down_L4+", "k_chain_up_L4+", "k_chain_sweeps_L4+", "k_chain_incr_L4+"}};
-  for (int it = 0; it < s0.mg_max_iters; it++) {
-    cudaSetDevice(E->slab[0].device);
-    CU(cudaMemsetAsync(s0.sc.any_active, 0, sizeof(int), E->slab[0].st));
-    if (it == 0) slab_all(E, "k_resid_down0", 5.25, [&](SlabDev& D) { return launch_resid_down0(D.sp, Ux, Uy, pA, pB, rs, which, D.st); });
-    else slab_all(E, "k_mg_down0", 4.25, [&](SlabDev& D) { return launch_mg_down0(D.spB, r, rs, D.st); });
-    slab_barrier(E);
-    for (int l = 1; l < first; l++) {
-      slab_all(E, nm[std::min(l, 4) - 1][0], 0, [&](SlabDev& D) { return launch_chain_down(D.spB, l, D.st); });
-      slab_barrier(E);
-    }
-    slab_first(E, "k_mg_coarse_cta", 0.5, [&](SlabDev& D) { return launch_coarse_cta(E->soloB, D.st); });
-    slab_barrier(E);
-    for (int l = first - 1; l >= 0; l--) {
-      const int k = std::min(std::max(l, 1), 4) - 1;
-      slab_all(E, l ? nm[k][1] : "k_chain_up_L0", l ? 0 : 4.25, [&](SlabDev& D) { return launch_chain_up(D.spB, l, l ? nullptr : rs, D.st); });
-      slab_barrier(E);
-      slab_all(E, l ? nm[k][2] : "k_chain_sweeps_L0", l ? 0 : 3, [&](SlabDev& D) { return launch_chain_sweeps(D.spB, l, D.st); });
-      slab_barrier(E);
-      slab_all(E, l ? nm[k][3] : "k_chain_incr_L0", l ? 0 : 4, [&](SlabDev& D) { return launch_chain_incr(D.spB, l, l ? nullptr : r, l ? 0 : which, D.st); });
-      slab_barrier(E);
-    }
-    E->mg_iter_launch_rounds++;
-    cudaSetDevice(E->slab[0].device);
-    CU(cudaMemcpyAsync(E->h_any, s0.sc.any_active, sizeof(int), cudaMemcpyDeviceToHost, E->slab[0].st));
-    CU(cudaStreamSynchronize(E->slab[0].st));
-    if (!*E->h_any) break;
-  }
-  // projection tail: Field.sum on device 0 (a serial float chain over the whole field), then the grid-wide correction
-  if (E->soloB.xs_recs) {
-    slab_first(E, "k_xsum_tables", 1, [&](SlabDev& D) { return launch_psum_tables(E->soloB, D.st); });
-    slab_first(E, "k_xsum_pass", 0, [&](SlabDev& D) { return launch_psum_pass(E->soloB, D.st); });
-  } else {
-    slab_first(E, "k_psum", 1, [&](SlabDev& D) { return launch_psum(E->soloB, D.st); });
-  }
-  slab_barrier(E);
-  if (which == 1 && s0.fast_bc) {
-    Group& G = E->whole;
-    slab_all(E, "k_project_shift_heun", 8, [&](SlabDev& D) { return launch_project_shift_heun(D.sp, pB, pA, Ux, Uy, G.uBx, G.uBy, G.uAx, G.uAy, D.st); });
-    slab_barrier(E);
-    slab_first(E, "k_bc_heun", 0, [&](SlabDev& D) { return launch_bc_heun(E->solo, Ux, Uy, G.uBx, G.uBy, G.uAx, G.uAy, D.st); });
-    slab_barrier(E);
-    return RLFC_OK;
-  }
-  slab_all(E, "k_project_shift", 6, [&](SlabDev& D) { return launch_project_shift(D.sp, pB, pA, Ux, Uy, D.st); });
-  slab_barrier(E);
-  slab_first(E, "k_bc", 0, [&](SlabDev& D) { return launch_bc(E->solo, Ux, Uy, D.st); });
-  slab_barrier(E);
-  return RLFC_OK;
-}
-
-int slab_step(rlfc_env* E, int accumulate) {
-  Group& G = E->whole;
-  int rc;
-  slab_barrier(E);   // (whatever device 0 enqueued since the last step -- actions, resets, field uploads -- is visible to all)
-  slab_all(E, "k_advdif", 5, [&](SlabDev& D) { return launch_advdif(D.sp, G.uAx, G.uAy, G.uAx, G.uAy, G.uBx, G.uBy, D.st); });
-  slab_barrier(E);
-  slab_first(E, "k_band_bc", 0, [&](SlabDev& D) { return launch_band_bc(E->solo, G.uBx, G.uBy, D.st); });
-  slab_barrier(E);
-  if ((rc = slab_project(E, G.uBx, G.uBy, 0))) return rc;
-  slab_all(E, "k_advdif", 5, [&](SlabDev& D) { return launch_advdif(D.sp, G.uBx, G.uBy, G.uAx, G.uAy, G.uCx, G.uCy, D.st); });
-  slab_barrier(E);
-  slab_first(E, "k_band_bc", 0, [&](SlabDev& D) { return launch_band_bc(E->solo, G.uCx, G.uCy, D.st); });
-  slab_barrier(E);
-  if ((rc = slab_project(E, G.uCx, G.uCy, 1))) return rc;
-  if (!E->slab[0].sp.fast_bc) {
-    slab_all(E, "k_heun", 6, [&](SlabDev& D) { return launch_heun(D.sp, G.uCx, G.uCy, G.uBx, G.uBy, G.uAx, G.uAy, D.st); });
-    slab_barrier(E);
-  }
-  slab_first(E, "k_force", 0, [&](SlabDev& D) { return launch_force(E->solo, accumulate, D.st); });
-  slab_barrier(E);
-  cudaSetDevice(E->slab[0].device);
-  CU(cudaGetLastError());
-  return RLFC_OK;
-}
-
 // `nsteps` solver steps (AFCCylinder.update2) for the whole batch
 int solver_steps(rlfc_env* E, int nsteps, int accumulate) {
   int rc;
   if (!E->slab.empty()) {
-    for (int s = 0; s < nsteps; s++)
-      if ((rc = slab_step(E, accumulate))) return rc;
+    SlabSink S{E};
+    for (int s = 0; s < nsteps; s++) {
+      if ((rc = solver_step(S, E->whole, accumulate))) return rc;
+      cudaSetDevice(E->device);
+      CU(cudaGetLastError());
+    }
     return RLFC_OK;
   }
   if (!E->use_graph || E->profiling) {
-    for (int s = 0; s < nsteps; s++)
-      if ((rc = solver_step_eager(E, E->whole, accumulate))) return rc;
+    EagerSink S{E, E->whole};
+    for (int s = 0; s < nsteps; s++) {
+      if ((rc = solver_step(S, E->whole, accumulate))) return rc;
+      CU(cudaGetLastError());
+    }
     return RLFC_OK;
   }
   if ((rc = fork_groups(E))) return rc;
@@ -865,6 +844,61 @@ int solver_steps(rlfc_env* E, int nsteps, int accumulate) {
   if ((rc = join_groups(E))) return rc;
   CU(cudaGetLastError());
   return RLFC_OK;
+}
+
+// G = the view of environments [e0, e0 + n) of the batch arrays (E->sp): sp, spB (lev[0].x = pressure buffer B), sensors
+// and velocity buffers.  `row` selects the view's own ticket counters, launch tags and any_active word.
+void make_view(const rlfc_env* E, int e0, int n, int row, Group& G) {
+  const SolverParams& sp = E->sp;
+  G.e0 = e0; G.B = n;
+  G.sp = sp;
+  SolverParams& v = G.sp;
+  v.B = n;
+  for (int l = 0; l < v.nlevels; l++) {
+    const size_t o = (size_t)e0 * v.lev[l].stride;
+    v.lev[l].r += o; v.lev[l].x += o; v.lev[l].d += o;
+    if (v.lev[l].w) v.lev[l].w += o;
+    if (v.per_env) {
+      v.lev[l].lx += o; v.lev[l].ly += o; v.lev[l].inv += o; v.lev[l].diag += o;
+      if (v.lev[l].rt.T) { v.lev[l].rt.T += (size_t)e0 * v.lev[l].rt.entries * v.lev[l].rt.K * 32; v.lev[l].rt.copies = n; }
+    }
+  }
+  if (v.per_env) {
+    v.c_x = v.lev[0].lx; v.c_y = v.lev[0].ly; v.sc.dt += e0;
+    v.env_slot += e0; v.env_nu += e0; v.env_dRD += e0; v.env_nband_x += e0; v.env_nband_y += e0;
+  }
+  for (int l = 0; l < v.chain_levels; l++) {
+    ChainLevel& ch = v.lev[l].ch;
+    ch.rsk += (size_t)e0 * ch.sk_stride;
+    for (int gsw = 0; gsw < 5; gsw++) ch.dsk[gsw] += (size_t)e0 * ch.sk_stride;
+    ch.edge += (size_t)e0 * ch.NS * ch.TE;
+    ch.ticket = E->chain_tickets + (size_t)row * kMaxLevels + l;
+    ch.tag_hi = (unsigned)(row + 1) << 26;
+  }
+  if (v.chain_levels > 0) { v.rr_chain += (size_t)e0 * v.rr_chain_n; v.rr_count += e0; }
+  v.band_tmp += (size_t)e0 * (v.nband_x + v.nband_y);
+  v.rsk += (size_t)e0 * v.rsk_stride;
+  v.sc.flow_t += e0;
+  v.sc.xi += 2 * e0; v.sc.t += e0; v.sc.force += 2 * e0; v.sc.probes += (size_t)e0 * RLFC_NUM_PROBES;
+  v.sc.callLearn += e0; v.sc.Cd += e0; v.sc.Cl += e0; v.sc.obs += 2 * e0; v.sc.active += e0; v.sc.iters += 2 * e0;
+  v.sc.frozen += e0; v.sc.non_finite += e0;
+  v.sc.psum += e0; v.sc.any_active += row;
+  if (v.xs_recs) {
+    v.xs_ctot += (size_t)e0 * v.xs_nchunks;
+    v.xs_cflag += (size_t)e0 * v.xs_nchunks; v.xs_epoch += e0;
+    v.xs_recs += (size_t)e0 * v.xs_nbatches * 192;
+    if (v.xs_blk) {
+      v.xs_blk += (size_t)e0 * ((v.xs_nbatches + 31) / 32) * 256;
+      if (v.xs_corr) { v.xs_pred += (size_t)e0 * v.xs_nbatches; v.xs_inc += (size_t)e0 * v.xs_nbatches; v.xs_corr += (size_t)e0 * v.xs_nbatches; }
+    }
+  }
+  v.xs_stats += 8 * e0;
+  G.spB = v;
+  G.spB.lev[0].x = E->pB + (size_t)e0 * sp.stride;
+  G.sens = E->sens;
+  if (G.sens.out) G.sens.out += (size_t)e0 * G.sens.n;
+  const size_t o = (size_t)e0 * sp.stride;
+  G.uAx = E->uAx + o; G.uAy = E->uAy + o; G.uBx = E->uBx + o; G.uBy = E->uBy + o; G.uCx = E->uCx + o; G.uCy = E->uCy + o;
 }
 
 int load_initial_state(rlfc_env* E) {
@@ -1415,7 +1449,7 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
     }
     E->home_only = false;
   }
-  TRY(E->dmalloc(&sp.sc.any_active, n_groups));
+  TRY(E->dmalloc(&sp.sc.any_active, n_groups + 1));   // one word per view of the batch: the groups and the whole batch
   if (sp.chain_levels > 0) {
     sp.rr_chain_n = chain_incr_blocks(g.n - 2, sp.lev[0].ch.NS);
     TRY(E->dmalloc(&sp.rr_chain, (size_t)sp.rr_chain_n * B));
@@ -1439,71 +1473,20 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
       !hostalloc((void**)&E->h_done, B * sizeof(int)) || !hostalloc((void**)&E->h_any, sizeof(int)))
     return bail(fail(RLFC_ENOMEM, "cudaMallocHost failed"));
 
-  // environment groups (contiguous), streams, events
+  // views of the batch: the environment groups (contiguous, each on its own stream; group 0 on the handle's), then the
+  // whole batch on the handle's stream
   if ((rc = configure_kernels(sp))) return bail(fail(RLFC_ECUDA, "kernel attribute configuration failed"));
   E->groups.resize(n_groups);
   for (int g = 0; g < n_groups; g++) {
-    rlfc_env::Group& G = E->groups[g];
+    Group& G = E->groups[g];
     const int e0 = (int)((long long)B * g / n_groups), e1 = (int)((long long)B * (g + 1) / n_groups);
-    G.e0 = e0; G.B = e1 - e0;
-    G.sp = sp;
-    SolverParams& v = G.sp;
-    v.B = G.B;
-    for (int l = 0; l < v.nlevels; l++) {
-      const size_t o = (size_t)e0 * v.lev[l].stride;
-      v.lev[l].r += o; v.lev[l].x += o; v.lev[l].d += o;
-      if (v.lev[l].w) v.lev[l].w += o;
-      if (v.per_env) {
-        v.lev[l].lx += o; v.lev[l].ly += o; v.lev[l].inv += o; v.lev[l].diag += o;
-        if (v.lev[l].rt.T) { v.lev[l].rt.T += (size_t)e0 * v.lev[l].rt.entries * v.lev[l].rt.K * 32; v.lev[l].rt.copies = G.B; }
-      }
-    }
-    if (v.per_env) {
-      v.c_x = v.lev[0].lx; v.c_y = v.lev[0].ly; v.sc.dt += e0;
-      v.env_slot += e0; v.env_nu += e0; v.env_dRD += e0; v.env_nband_x += e0; v.env_nband_y += e0;
-    }
-    for (int l = 0; l < v.chain_levels; l++) {
-      ChainLevel& ch = v.lev[l].ch;
-      ch.rsk += (size_t)e0 * ch.sk_stride;
-      for (int gsw = 0; gsw < 5; gsw++) ch.dsk[gsw] += (size_t)e0 * ch.sk_stride;
-      ch.edge += (size_t)e0 * ch.NS * ch.TE;
-      ch.ticket = E->chain_tickets + (size_t)g * kMaxLevels + l;
-      ch.tag_hi = (unsigned)(g + 1) << 26;
-    }
-    if (v.chain_levels > 0) { v.rr_chain += (size_t)e0 * v.rr_chain_n; v.rr_count += e0; }
-    v.band_tmp += (size_t)e0 * (v.nband_x + v.nband_y);
-    v.rsk += (size_t)e0 * v.rsk_stride;
-    v.sc.flow_t += e0;
-    v.sc.xi += 2 * e0; v.sc.t += e0; v.sc.force += 2 * e0; v.sc.probes += (size_t)e0 * RLFC_NUM_PROBES;
-    v.sc.callLearn += e0; v.sc.Cd += e0; v.sc.Cl += e0; v.sc.obs += 2 * e0; v.sc.active += e0; v.sc.iters += 2 * e0;
-    v.sc.frozen += e0; v.sc.non_finite += e0;
-    v.sc.psum += e0; v.sc.any_active += g;
-    G.sens = E->sens;
-    if (G.sens.out) G.sens.out += (size_t)e0 * G.sens.n;
-    if (v.xs_recs) {
-      v.xs_ctot += (size_t)e0 * v.xs_nchunks;
-      v.xs_cflag += (size_t)e0 * v.xs_nchunks; v.xs_epoch += e0;
-      v.xs_recs += (size_t)e0 * v.xs_nbatches * 192;
-      if (v.xs_blk) {
-        v.xs_blk += (size_t)e0 * ((v.xs_nbatches + 31) / 32) * 256;
-        if (v.xs_corr) { v.xs_pred += (size_t)e0 * v.xs_nbatches; v.xs_inc += (size_t)e0 * v.xs_nbatches; v.xs_corr += (size_t)e0 * v.xs_nbatches; }
-      }
-    }
-    v.xs_stats += 8 * e0;
-    const size_t o = (size_t)e0 * sp.stride;
-    G.uAx = E->uAx + o; G.uAy = E->uAy + o; G.uBx = E->uBx + o; G.uBy = E->uBy + o; G.uCx = E->uCx + o; G.uCy = E->uCy + o;
-    G.spB = G.sp;
-    G.spB.lev[0].x = E->pB + (size_t)e0 * sp.stride;
+    make_view(E, e0, e1 - e0, g, G);
     if (g == 0) G.st = E->stream;
     else if (cudaStreamCreateWithFlags(&G.st, cudaStreamNonBlocking) != cudaSuccess) return bail(fail(RLFC_ECUDA, "cudaStreamCreate failed"));
     if (cudaEventCreateWithFlags(&G.done, cudaEventDisableTiming) != cudaSuccess) return bail(fail(RLFC_ECUDA, "cudaEventCreate failed"));
   }
-  E->whole.e0 = 0; E->whole.B = B; E->whole.sp = sp; E->whole.sens = E->sens; E->whole.st = E->stream;
-  for (int l = 0; l < sp.chain_levels; l++) {
-    ChainLevel& ch = E->whole.sp.lev[l].ch;
-    ch.ticket = E->chain_tickets + (size_t)n_groups * kMaxLevels + l;
-    ch.tag_hi = (unsigned)(n_groups + 1) << 26;
-  }
+  make_view(E, 0, B, n_groups, E->whole);
+  E->whole.st = E->stream;
   if (sp.chain_levels > 0) {
     // every counter starts at one full launch's worth of tickets, so that launch serials (the tags) start at 1 and
     // never equal the 0 the arrays are initialised with
@@ -1517,9 +1500,6 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
         cudaStreamSynchronize(E->stream) != cudaSuccess)
       return bail(fail(RLFC_ECUDA, "ticket initialisation failed"));
   }
-  E->whole.spB = E->whole.sp; E->whole.spB.lev[0].x = E->pB;
-  E->whole.uAx = E->uAx; E->whole.uAy = E->uAy; E->whole.uBx = E->uBx; E->whole.uBy = E->uBy;
-  E->whole.uCx = E->uCx; E->whole.uCy = E->uCy;
   if (slab) {
     // per-device views: the same arrays (one address range), each device its row blocks / strips, its own streams,
     // ticket counters and barrier epoch in its own memory
@@ -1530,7 +1510,6 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
     if ((rc = E->dmalloc(&bar_count, 1))) return bail(rc);
     E->home_only = false;
     if (cudaStreamSynchronize(E->stream) != cudaSuccess) return bail(fail(RLFC_ECUDA, "initialisation failed"));
-    E->solo = E->whole.sp; E->soloB = E->whole.spB;
     E->slab.resize(nd);
     for (int d = 0; d < nd; d++) {
       rlfc_env::SlabDev& D = E->slab[d];

@@ -254,16 +254,16 @@ int launch_project_shift_heun(const SolverParams& P, const float* p_in, float* p
                               const float* usy, float* uox, float* uoy, cudaStream_t st);
 int launch_bc_heun(const SolverParams& P, float* ux, float* uy, const float* usx, const float* usy, float* uox, float* uoy,
                    cudaStream_t st);
-// one MG iteration (V-cycle + smooth(4)) on active envs = down0, coarse, up0, smooth0;
-// r_in/r_out are the level-0 ping-pong residual buffers
+// one MG iteration (V-cycle + smooth(4)) on active envs = down0, the chained levels' down passes, the one-CTA coarse kernel
+// (levels max(1, chain_levels) ..), the chained levels' up / sweeps / incr top down, then level 0's up0 and smooth0 unless
+// level 0 is chained; r_in/r_out are the level-0 ping-pong residual buffers
 int launch_mg_down0(const SolverParams& P, const float* r_in, float* r_out, cudaStream_t st);
-int launch_mg_coarse(const SolverParams& P, cudaStream_t st);
-// the pieces launch_mg_coarse / launch_mg_up0 / launch_smooth0 are made of when levels use the chained strip smoother
 int launch_chain_down(const SolverParams& P, int level, cudaStream_t st);
 int launch_coarse_cta(const SolverParams& P, cudaStream_t st);
 int launch_chain_up(const SolverParams& P, int level, const float* r, cudaStream_t st);
 int launch_chain_sweeps(const SolverParams& P, int level, cudaStream_t st);
 int launch_chain_incr(const SolverParams& P, int level, float* r_out, int which, cudaStream_t st);
+// level 0 row-smoothed or wavefront-smoothed (not chained)
 int launch_mg_up0(const SolverParams& P, float* r, cudaStream_t st);
 // rows smoother only: plain level-0 residual <- skewed residual (needed before a further MG iteration's down0)
 int launch_unskew_r(const SolverParams& P, float* r, cudaStream_t st);

@@ -1771,7 +1771,7 @@ int configure_kernels(const SolverParams& q) {
   return (e3 == cudaSuccess && e4 == cudaSuccess) ? 0 : -1;
 }
 
-// chained strip smoother (smooth_chain.cuh): the pieces of one level, individually launchable (profiling) ...
+// chained strip smoother (smooth_chain.cuh): the kernels of one level
 int launch_chain_sweeps(const SolverParams& q, int l, cudaStream_t st) {
   const ChainLevel& ch = q.lev[l].ch;
   if (ch.ns_loc > 0) {
@@ -1811,24 +1811,8 @@ int chain_incr_blocks(int ni, int NS) {
   return ((runs + kChIncWarps - 1) / kChIncWarps) * NS;
 }
 
-// ... and as the composites the step graph captures
-int launch_mg_coarse(const SolverParams& q, cudaStream_t st) {
-  // wide levels run as grid-wide kernels around the one-CTA-per-environment kernel of the small levels
-  int nl = 0;
-  const int first = max(1, q.chain_levels);
-  for (int l = 1; l < first; l++) nl += launch_chain_down(q, l, st);
-  nl += launch_coarse_cta(q, st);
-  for (int l = first - 1; l >= 1; l--) {
-    nl += launch_chain_up(q, l, nullptr, st);
-    nl += launch_chain_sweeps(q, l, st);
-    nl += launch_chain_incr(q, l, nullptr, 0, st);
-  }
-  return nl;
-}
-
 int launch_mg_up0(const SolverParams& q, float* r, cudaStream_t st) {
   dim3 blk(32, 8);
-  if (q.lev[0].ch.on) return launch_chain_up(q, 0, r, st);
   if (!q.lev[0].wave) {
     if (q.per_env) k_mg_up0_blk<true><<<dim3((q.n - 2 + kUpRows - 1) / kUpRows, q.B), 256, up0_smem(q), st>>>(q, r);
     else k_mg_up0_blk<false><<<dim3((q.n - 2 + kUpRows - 1) / kUpRows, q.B), 256, up0_smem(q), st>>>(q, r);
@@ -1845,7 +1829,6 @@ int launch_unskew_r(const SolverParams& q, float* r, cudaStream_t st) {
 }
 
 int launch_smooth0(const SolverParams& q, const float* r_in, float* r_out, int which, cudaStream_t st) {
-  if (q.lev[0].ch.on) return launch_chain_sweeps(q, 0, st) + launch_chain_incr(q, 0, r_out, which, st);
   if (q.lev[0].wave) {
     k_smooth0_wave<<<q.B, 1024, 0, st>>>(q, r_in, r_out, which);
     return 1;
