@@ -30,6 +30,8 @@
 #ifndef RLFC_H
 #define RLFC_H
 
+#include <stddef.h>
+
 #ifdef __cplusplus
 extern "C" {
 #endif
@@ -221,7 +223,9 @@ int  rlfc_env_running(rlfc_env *env, int *n_running);
    environment has diverged; SURVEY section 5 failure detection).  Bit 1 = the last restore aimed at the environment was
    skipped because its slot was never written or holds a state of another parameter set (rlfc_env_restore_device; a restore
    that applies clears it).  Bit 2 = the last device parameter reset aimed at the environment was refused because its set
-   is invalid (rlfc_env_reset_params_device; one that applies clears it).  Synchronises the handle's stream. */
+   is invalid (rlfc_env_reset_params_device; one that applies clears it).  Bit 3 = the last device import aimed at the
+   environment was refused because its record failed a check (rlfc_env_import_device; one that applies clears it).
+   Synchronises the handle's stream. */
 int  rlfc_env_get_flags(rlfc_env *env, int *flags);
 
 /* Snapshots of complete environment states in the handle's rlfc_config.n_snapshots device slots (ALE cloneState /
@@ -245,6 +249,67 @@ int  rlfc_env_restore(rlfc_env *env, const int *env_ids, const int *slots, int n
    written or of another parameter set is skipped and sets flags bit 1 of the destination. */
 int  rlfc_env_snapshot_device(rlfc_env *env, const int *d_env_ids, const int *d_slots, int n);
 int  rlfc_env_restore_device(rlfc_env *env, const int *d_env_ids, const int *d_slots, int n, int keep_accumulators);
+
+/* State records: one environment's complete state -- what a snapshot slot holds -- as bytes that any handle of the same
+   grid can import, on any device and in any process.  The library only turns states into bytes and back on the handle's
+   device; moving the bytes (files, torch.distributed, peer copies) is the caller's.  Not available in slab mode (RLFC_EINVAL).
+
+   Format (version 1).  Little-endian; u32 / i32 / f32 words unless noted; n, m = rows and columns incl. ghosts
+   (x_lengths*resolution + 2, y_lengths*resolution + 2); K = the exporting handle's n_sensors.
+     offset  bytes  field
+     0       8      magic "RLFCSTAT"
+     8       8      u64 checksum of bytes [16, length) (below)
+     16      4      version = RLFC_RECORD_VERSION
+     20      4      adaptive_dt of the exporting handle (0 / 1)
+     24      8      u64 length of the record in bytes = 272 + 16 K + 12 n m
+     32      20     resolution, x_lengths, y_lengths, n, m (i32)
+     52      20     re, dR, gR, theta, t_step: the environment's parameter tuple, as bits (re i32, the rest f32)
+     72      4      probes (RLFC_NUM_PROBES)
+     76      4      K
+     80      192    the scalar record, 48 words: xi[2], t, BDIM.t, dt, force[2], probes[32] (f32), callLearn (i32), Cd, Cl,
+                    obs[2] (f32), frozen, non_finite (i32), MG iterations[2] (i32)
+     272     12 K   the exporting handle's sensor table, rlfc_sensor[K] (field i32, x f32, y f32)
+     272+12K 4 K    the environment's sensor values (f32)
+     272+16K 4 n m  u.x (step-start velocity), reference layout a[i][j] as rlfc_env_get_fields returns it
+     ...     4 n m  u.y
+     ...     4 n m  p (also the initial guess of the next pressure solve)
+   Checksum: with w_i the u32 word at byte offset 4 i, the sum mod 2^64 over i = 4 .. length/4 - 1 of mix(i << 32 | w_i),
+   where mix is MurmurHash3's 64-bit finalizer: x ^= x >> 33; x *= 0xff51afd7ed558ccd; x ^= x >> 33;
+   x *= 0xc4ceb9fe1a85ec53; x ^= x >> 33.  mix is a bijection, so any change of one word (any single flipped bit) changes
+   the sum; the terms are independent, so the sum is computed in parallel in any order.
+   What a snapshot slot leaves out a record leaves out too: the geometry and Poisson hierarchy (rebuilt from the tuple and
+   dt), the pressure buffer B, the velocity buffers B and C, and the Field.sum tables, which every step writes before reading.
+
+   An import of record r into environment e checks, in this order: magic and version, length (as above, and equal to the
+   size of the records of the call), grid (resolution, x_lengths, y_lengths, n, m, probes equal to the handle's), checksum,
+   tuple (bitwise equal to e's own), and dt (a fixed-dt handle requires e's own fixed dt bit for bit; an adaptive handle
+   accepts any finite dt > 0, which becomes e's current dt).  An applied import makes e continue bit-identically to the
+   exporting environment, through every entry point; in adaptive mode it rebuilds e's Poisson hierarchy.  keep_accumulators
+   has rlfc_env_restore's meaning.  Sensor values are imported only when the record's sensor table is byte-equal to the
+   handle's; otherwise e keeps its own (the next step overwrites them, as after rlfc_env_reset). */
+#define RLFC_RECORD_VERSION      1
+#define RLFC_RECORD_HEADER_BYTES 80
+/* Bytes of one record of cfg's grid and n_sensors, without a device.  RLFC_EINVAL for a NULL argument or a grid that is
+   not positive or n_sensors < 0. */
+int  rlfc_record_bytes(const rlfc_config *cfg, size_t *bytes);
+/* The checksum above of the `bytes` bytes at `record` (bytes a multiple of 4); what the header's checksum field holds. */
+unsigned long long rlfc_record_checksum(const void *record, size_t bytes);
+/* Environment env_ids[k] -> record k of host_buf (n consecutive records of rlfc_record_bytes each).  Synchronous on return.
+   RLFC_EINVAL for an id out of range (nothing is written). */
+int  rlfc_env_export(rlfc_env *env, const int *env_ids, int n, void *host_buf);
+/* Record k of host_buf -> environment env_ids[k].  The records are consecutive and all as long as record 0.  Synchronous, all
+   or nothing: every record is checked before anything changes, and RLFC_EINVAL (nothing changes) for an id out of range, a
+   destination listed twice or a record that fails a check; rlfc_last_error names the record and the check. */
+int  rlfc_env_import(rlfc_env *env, const int *env_ids, int n, const void *host_buf, int keep_accumulators);
+/* Same with DEVICE arrays, asynchronous on the handle's stream, defined for every input.  Export: d_buf (16-byte aligned)
+   receives n records of rlfc_record_bytes each; a pair whose id is out of range writes a record with a zero header, which
+   every import refuses.  Import: d_buf (16-byte aligned) holds n records of record_bytes each (RLFC_EINVAL if that is not the
+   size of a record of the handle's grid); a pair whose id is out of range is skipped, and of pairs with the same destination
+   the last in-range pair wins.  A winning record that fails a check leaves its environment completely unchanged and sets
+   its flags bit 3; an import that applies clears it. */
+int  rlfc_env_export_device(rlfc_env *env, const int *d_env_ids, int n, void *d_buf);
+int  rlfc_env_import_device(rlfc_env *env, const int *d_env_ids, int n, const void *d_buf, size_t record_bytes,
+                            int keep_accumulators);
 
 /* The sensors (rlfc_config.sensors) of every environment, out[n_envs][n_sensors].  Each environment's sensors hold the
    sample of its most recent solver step, taken from the state the next step starts from -- the u and p rlfc_env_get_fields

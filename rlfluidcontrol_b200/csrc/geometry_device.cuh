@@ -155,7 +155,7 @@ struct ResetParamsArgs {
   BandFace *band_x, *band_y;                   // slot s at s*cap
   int *env_slot, *env_nbx, *env_nby;
   float *env_nu, *env_dRD;
-  unsigned* env_par;                           // [5][B] snapshot parameter tuples (nullptr without snapshots)
+  unsigned* env_par;                           // [5][B] parameter tuples (nullptr without snapshots or records)
   const float4 *iux, *iuy, *ip;                // the init state (one environment)
   float4 *ux, *uy, *p;                         // the environments' fields (batch base)
   size_t stride, stride4;                      // level-0 per-environment stride in floats / float4
@@ -405,7 +405,7 @@ int launch_reset_params(const SolverParams& q, const ParamLib& lib, const SnapSl
   a.env_nby = const_cast<int*>(q.env_nband_y);
   a.env_nu = const_cast<float*>(q.env_nu);
   a.env_dRD = const_cast<float*>(q.env_dRD);
-  a.env_par = snap.S ? snap.env_par : nullptr;
+  a.env_par = snap.env_par;
   a.iux = reinterpret_cast<const float4*>(init_ux);
   a.iuy = reinterpret_cast<const float4*>(init_uy);
   a.ip = reinterpret_cast<const float4*>(init_p);

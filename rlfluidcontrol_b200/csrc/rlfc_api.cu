@@ -54,6 +54,13 @@ struct rlfc_env {
   SnapSlots snap{};                        // rlfc_config.n_snapshots slots (snap.S = 0: none)
   int *snap_env = nullptr, *snap_slot = nullptr;   // [max(B, S)] the pairs of a host snapshot / restore call
   SensorSet sens{};                        // rlfc_config.sensors of the whole batch (sens.n = 0: none)
+  std::vector<rlfc_sensor> sensor_table;   // rlfc_config.sensors as given (what a record's sensor table holds)
+  // state records (records.cuh): nothing is allocated before the first record call (rec.refused = nullptr until then)
+  RecordBufs rec{};
+  std::vector<void*> rec_bufs;             // rec's growing scratch, its id buffer and the host calls' staging buffer
+  size_t rec_pairs = 0, rec_partials = 0, rec_id_cap = 0, rec_stage_bytes = 0;
+  int* rec_ids = nullptr;                  // [rec_pairs] the ids of a host export / import call
+  unsigned char* rec_stage = nullptr;      // the records of a host export / import call
   // parameter library (rlfc_config.param_sets; lib.L = 0: none)
   ParamLib lib{};
   std::vector<rlfc_env_params> lib_params; // [L] the sets as given
@@ -451,9 +458,9 @@ void param_bits(const rlfc_env_params& p, unsigned out[5]) {
   std::memcpy(&out[3], &p.theta, 4); std::memcpy(&out[4], &p.t_step, 4);
 }
 
-// E->params -> snap.env_par (what a restore compares a slot's header with)
+// E->params -> snap.env_par (what a restore compares a slot's header with, and what a record's header holds)
 int upload_snapshot_params(rlfc_env* E) {
-  if (!E->snap.S) return RLFC_OK;
+  if (!E->snap.env_par) return RLFC_OK;
   const int B = (int)E->params.size();
   std::vector<unsigned> bits((size_t)5 * B);
   for (int e = 0; e < B; e++) {
@@ -528,6 +535,139 @@ int snapshot_host(rlfc_env* E, const int* env_ids, const int* slots, int n, int 
   }
   if ((rc = snapshot_enqueue(E, E->snap_env, E->snap_slot, n, restore, keep))) return rc;
   CU(cudaStreamSynchronize(E->stream));
+  return RLFC_OK;
+}
+
+// ---- state records (rlfc.h "State records"; records.cuh) ----
+
+const char* record_check_name(int v) {
+  switch (v) {
+    case kRecMagic: return "magic (not a state record)";
+    case kRecVersion: return "version (not RLFC_RECORD_VERSION)";
+    case kRecLength: return "length (does not match its header, or not the size of the call's records)";
+    case kRecGrid: return "grid (resolution, x_lengths, y_lengths, n, m or probes differ from the handle's)";
+    case kRecChecksum: return "checksum (the record is corrupted)";
+    case kRecTuple: return "parameter tuple (differs from the destination's)";
+    case kRecDt: return "dt (not the destination's fixed dt, or not a finite dt > 0)";
+    default: return "?";
+  }
+}
+
+int records_check_handle(rlfc_env* E, int n, bool have_ptrs) {
+  if (!E) return fail(RLFC_EINVAL, "null handle");
+  if (!E->slab.empty()) return fail(RLFC_EINVAL, "state records are not available in slab mode (n_devices > 1)");
+  if (n < 0) return fail(RLFC_EINVAL, "bad pair count");
+  if (n > 0 && !have_ptrs) return fail(RLFC_EINVAL, "null argument");
+  return RLFC_OK;
+}
+
+// a device buffer of at least `need` T (contents kept only when it does not grow; zeroed when it does)
+template <typename T>
+int rec_grow(rlfc_env* E, T** p, size_t& cap, size_t need) {
+  if (need <= cap) return RLFC_OK;
+  if (*p) {   // (cudaFree waits for the device: no enqueued launch still reads the old buffer)
+    E->rec_bufs.erase(std::find(E->rec_bufs.begin(), E->rec_bufs.end(), (void*)*p));
+    CU(cudaFree(*p));
+    *p = nullptr;
+    cap = 0;
+  }
+  void* q = nullptr;
+  cudaError_t e = cudaMalloc(&q, need * sizeof(T));
+  if (e != cudaSuccess) return fail(RLFC_ENOMEM, std::string("cudaMalloc: ") + cudaGetErrorString(e));
+  E->rec_bufs.push_back(q);
+  CU(cudaMemsetAsync(q, 0, need * sizeof(T), E->stream));
+  *p = (T*)q;
+  cap = need;
+  return RLFC_OK;
+}
+
+// what a record call of n pairs of `bytes`-long records needs: on the first call the parameter tuples (snap.env_par, kept
+// current by every later device reset), the refusal flags and the sensor table; the per-pair scratch
+int records_prepare(rlfc_env* E, int n, size_t bytes) {
+  int rc;
+  if (!E->rec.refused) {
+    const int B = E->sp.B;
+    if (!E->snap.env_par) {
+      if ((rc = sync_env_sets(E))) return rc;
+      if ((rc = E->dmalloc(&E->snap.env_par, (size_t)5 * B))) return rc;
+      if ((rc = upload_snapshot_params(E))) return rc;
+    }
+    if ((rc = E->dmalloc(&E->rec.refused, B))) return rc;
+    if (!E->sensor_table.empty()) {
+      const rlfc_sensor* t = nullptr;
+      if ((rc = upload_vec(E, E->sensor_table, &t))) return rc;
+      E->rec.sensors = t;
+    }
+    E->rec.env_par = E->snap.env_par;
+    E->rec.grid[0] = E->cfg.resolution; E->rec.grid[1] = E->cfg.x_lengths; E->rec.grid[2] = E->cfg.y_lengths;
+  }
+  size_t cap = E->rec_pairs;
+  if ((rc = rec_grow(E, &E->rec.ticket, cap, (size_t)n))) return rc;
+  cap = E->rec_pairs;
+  if ((rc = rec_grow(E, &E->rec.hcode, cap, (size_t)n))) return rc;
+  cap = E->rec_pairs;
+  if ((rc = rec_grow(E, &E->rec.verdict, cap, (size_t)n))) return rc;
+  E->rec_pairs = std::max(E->rec_pairs, (size_t)n);
+  return rec_grow(E, &E->rec.partial, E->rec_partials, (size_t)n * record_chunks(E->sp.n, E->sp.m, bytes));
+}
+
+size_t own_record_bytes(const rlfc_env* E) { return record_bytes(E->sp.n, E->sp.m, E->sens.n); }
+
+int record_export_enqueue(rlfc_env* E, const int* d_ids, int n, void* d_buf) {
+  if (n <= 0) return RLFC_OK;
+  int rc = records_prepare(E, n, own_record_bytes(E));
+  if (rc) return rc;
+  SolverParams& sp = E->whole.sp;
+  E->run("k_export", 0, [&] { return launch_record_export(sp, E->sens, E->rec, E->uAx, E->uAy, d_ids, n, d_buf, E->stream); });
+  CU(cudaGetLastError());
+  return RLFC_OK;
+}
+
+// the check pass (verdicts only); the host variant reads the verdicts before it applies
+int record_check_enqueue(rlfc_env* E, const int* d_ids, int n, const void* d_buf, size_t bytes) {
+  int rc = records_prepare(E, n, bytes);
+  if (rc) return rc;
+  SolverParams& sp = E->whole.sp;
+  E->run("k_import_check", 0, [&] {
+    return launch_record_import(sp, E->sens, E->rec, E->uAx, E->uAy, d_ids, n, d_buf, bytes, 1, 0, nullptr, E->stream);
+  });
+  CU(cudaGetLastError());
+  return RLFC_OK;
+}
+
+// the apply pass; in adaptive mode then the Poisson hierarchy of exactly the environments imported (restore's skip mask)
+int record_apply_enqueue(rlfc_env* E, const int* d_ids, int n, const void* d_buf, size_t bytes, int keep) {
+  SolverParams& sp = E->whole.sp;
+  const bool rebuild = sp.adaptive;
+  if (rebuild) CU(cudaMemsetAsync(E->d_skip, 1, sp.B * sizeof(int), E->stream));   // nonzero = keep; the import clears
+  E->run("k_import", 0, [&] {
+    return launch_record_import(sp, E->sens, E->rec, E->uAx, E->uAy, d_ids, n, d_buf, bytes, 0, keep,
+                                rebuild ? E->d_skip : nullptr, E->stream);
+  });
+  if (rebuild) {
+    E->run("k_poisson_rebuild0", 0, [&] { return launch_poisson_rebuild0(sp, E->d_skip, E->stream); });
+    E->run("k_poisson_rebuild_coarse", 0, [&] { return launch_poisson_rebuild_coarse(sp, E->d_skip, E->stream); });
+  }
+  CU(cudaGetLastError());
+  return RLFC_OK;
+}
+
+// host ids: in range and (import) no destination twice
+int record_host_ids(rlfc_env* E, const int* ids, int n, bool import) {
+  const int B = E->sp.B;
+  std::vector<char> seen(B, 0);
+  for (int k = 0; k < n; k++) {
+    if (ids[k] < 0 || ids[k] >= B) return fail(RLFC_EINVAL, "env id " + std::to_string(ids[k]) + " out of range");
+    if (import && seen[ids[k]]++) return fail(RLFC_EINVAL, "env id " + std::to_string(ids[k]) + " listed twice");
+  }
+  return RLFC_OK;
+}
+
+int record_stage(rlfc_env* E, const int* ids, int n, size_t bytes) {
+  int rc = rec_grow(E, &E->rec_ids, E->rec_id_cap, (size_t)n);
+  if (rc) return rc;
+  if ((rc = rec_grow(E, &E->rec_stage, E->rec_stage_bytes, (size_t)n * bytes))) return rc;
+  CU(cudaMemcpyAsync(E->rec_ids, ids, n * sizeof(int), cudaMemcpyHostToDevice, E->stream));
   return RLFC_OK;
 }
 
@@ -967,6 +1107,7 @@ void rlfc_env_destroy(rlfc_env* E) {
   if (E->aux_stream) cudaStreamDestroy(E->aux_stream);
   if (E->fork_ev) cudaEventDestroy(E->fork_ev);
   for (void* p : E->allocs) cudaFree(p);
+  for (void* p : E->rec_bufs) cudaFree(p);
   for (void* p : {(void*)E->h_actions, (void*)E->h_obs, (void*)E->h_reward, (void*)E->h_force, (void*)E->h_probes,
                   (void*)E->h_done, (void*)E->h_any})
     if (p) cudaFreeHost(p);
@@ -1033,6 +1174,7 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
   E->env_mode = cfg->env_params != nullptr || cfg->n_param_sets > 0;
   E->cfg.env_params = nullptr;              // (copied into E->params below)
   E->cfg.param_sets = nullptr;              // (copied into E->lib_params below)
+  if (cfg->n_sensors > 0 && cfg->sensors) E->sensor_table.assign(cfg->sensors, cfg->sensors + cfg->n_sensors);
   E->cfg.sensors = nullptr;                 // (resolved into E->sens below)
   int rc = RLFC_OK;
   auto bail = [&](int code) { rlfc_env_destroy(E); return code; };
@@ -1836,14 +1978,18 @@ int rlfc_env_running(rlfc_env* E, int* n_running) {
 int rlfc_env_get_flags(rlfc_env* E, int* flags) {
   if (!E || !flags) return fail(RLFC_EINVAL, "null argument");
   CU(cudaSetDevice(E->device));
-  std::vector<int> refused(E->snap.S ? E->sp.B : 0), par_refused(E->pr.refused ? E->sp.B : 0);
+  std::vector<int> refused(E->snap.S ? E->sp.B : 0), par_refused(E->pr.refused ? E->sp.B : 0),
+      rec_refused(E->rec.refused ? E->sp.B : 0);
   CU(cudaMemcpyAsync(E->h_done, E->sp.sc.non_finite, E->sp.B * sizeof(int), cudaMemcpyDeviceToHost, E->stream));
   if (E->snap.S) CU(cudaMemcpyAsync(refused.data(), E->snap.refused, E->sp.B * sizeof(int), cudaMemcpyDeviceToHost, E->stream));
   if (E->pr.refused)
     CU(cudaMemcpyAsync(par_refused.data(), E->pr.refused, E->sp.B * sizeof(int), cudaMemcpyDeviceToHost, E->stream));
+  if (E->rec.refused)
+    CU(cudaMemcpyAsync(rec_refused.data(), E->rec.refused, E->sp.B * sizeof(int), cudaMemcpyDeviceToHost, E->stream));
   CU(cudaStreamSynchronize(E->stream));
   for (int e = 0; e < E->sp.B; e++)
-    flags[e] = (E->h_done[e] ? 1 : 0) | (E->snap.S && refused[e] ? 2 : 0) | (E->pr.refused && par_refused[e] ? 4 : 0);
+    flags[e] = (E->h_done[e] ? 1 : 0) | (E->snap.S && refused[e] ? 2 : 0) | (E->pr.refused && par_refused[e] ? 4 : 0) |
+               (E->rec.refused && rec_refused[e] ? 8 : 0);
   return RLFC_OK;
 }
 
@@ -1918,6 +2064,91 @@ int rlfc_env_reset_params_device(rlfc_env* E, const int* d_env_ids, const rlfc_e
   CU(cudaGetLastError());
   E->par_pending = true;
   return RLFC_OK;
+}
+
+int rlfc_record_bytes(const rlfc_config* cfg, size_t* bytes) {
+  if (!cfg || !bytes) return fail(RLFC_EINVAL, "null argument");
+  if (cfg->resolution < 1 || cfg->x_lengths < 1 || cfg->y_lengths < 1) return fail(RLFC_EINVAL, "the grid must be positive");
+  if (cfg->n_sensors < 0) return fail(RLFC_EINVAL, "n_sensors must be >= 0");
+  *bytes = record_bytes(cfg->x_lengths * cfg->resolution + 2, cfg->y_lengths * cfg->resolution + 2, cfg->n_sensors);
+  return RLFC_OK;
+}
+
+unsigned long long rlfc_record_checksum(const void* record, size_t bytes) {
+  const unsigned char* r = static_cast<const unsigned char*>(record);
+  unsigned long long sum = 0;
+  for (size_t w = 4; w < bytes / 4; w++) {
+    unsigned x;
+    std::memcpy(&x, r + 4 * w, 4);
+    sum += record_mix(w, x);
+  }
+  return sum;
+}
+
+int rlfc_env_export(rlfc_env* E, const int* env_ids, int n, void* host_buf) {
+  int rc = records_check_handle(E, n, env_ids && host_buf);
+  if (rc || n == 0) return rc;
+  if ((rc = record_host_ids(E, env_ids, n, false))) return rc;
+  CU(cudaSetDevice(E->device));
+  const size_t bytes = own_record_bytes(E);
+  if ((rc = records_prepare(E, n, bytes)) || (rc = record_stage(E, env_ids, n, bytes))) return rc;
+  if ((rc = record_export_enqueue(E, E->rec_ids, n, E->rec_stage))) return rc;
+  CU(cudaMemcpyAsync(host_buf, E->rec_stage, (size_t)n * bytes, cudaMemcpyDeviceToHost, E->stream));
+  CU(cudaStreamSynchronize(E->stream));
+  return RLFC_OK;
+}
+
+int rlfc_env_import(rlfc_env* E, const int* env_ids, int n, const void* host_buf, int keep_accumulators) {
+  int rc = records_check_handle(E, n, env_ids && host_buf);
+  if (rc || n == 0) return rc;
+  if ((rc = record_host_ids(E, env_ids, n, true))) return rc;
+  // record 0's header gives the size of every record of the call: checked here before any of them is read
+  unsigned w[RLFC_RECORD_HEADER_BYTES / 4];
+  std::memcpy(w, host_buf, sizeof(w));
+  const unsigned long long len = w[6] | (unsigned long long)w[7] << 32;
+  int v = kRecApply;
+  if (std::memcmp(w, "RLFCSTAT", 8)) v = kRecMagic;
+  else if (w[4] != RLFC_RECORD_VERSION) v = kRecVersion;
+  else if (w[11] > 0xffffu || w[12] > 0xffffu || len != record_bytes((int)w[11], (int)w[12], 0) + 16ull * w[19]) v = kRecLength;
+  else if ((int)w[8] != E->cfg.resolution || (int)w[9] != E->cfg.x_lengths || (int)w[10] != E->cfg.y_lengths ||
+           (int)w[11] != E->sp.n || (int)w[12] != E->sp.m || (int)w[18] != E->sp.nprobe) v = kRecGrid;
+  if (v) return fail(RLFC_EINVAL, std::string("record 0: ") + record_check_name(v));
+  CU(cudaSetDevice(E->device));
+  if ((rc = records_prepare(E, n, len)) || (rc = record_stage(E, env_ids, n, len))) return rc;
+  CU(cudaMemcpyAsync(E->rec_stage, host_buf, (size_t)n * len, cudaMemcpyHostToDevice, E->stream));
+  if ((rc = record_check_enqueue(E, E->rec_ids, n, E->rec_stage, len))) return rc;
+  std::vector<int> verdict(n);
+  CU(cudaMemcpyAsync(verdict.data(), E->rec.verdict, n * sizeof(int), cudaMemcpyDeviceToHost, E->stream));
+  CU(cudaStreamSynchronize(E->stream));
+  for (int k = 0; k < n; k++)
+    if (verdict[k])
+      return fail(RLFC_EINVAL, "record " + std::to_string(k) + " (env id " + std::to_string(env_ids[k]) + "): " +
+                                   record_check_name(verdict[k]));
+  if ((rc = record_apply_enqueue(E, E->rec_ids, n, E->rec_stage, len, keep_accumulators != 0))) return rc;
+  CU(cudaStreamSynchronize(E->stream));
+  return RLFC_OK;
+}
+
+int rlfc_env_export_device(rlfc_env* E, const int* d_env_ids, int n, void* d_buf) {
+  int rc = records_check_handle(E, n, d_env_ids && d_buf);
+  if (rc) return rc;
+  if (reinterpret_cast<uintptr_t>(d_buf) % 16) return fail(RLFC_EINVAL, "the record buffer must be 16-byte aligned");
+  CU(cudaSetDevice(E->device));
+  return record_export_enqueue(E, d_env_ids, n, d_buf);
+}
+
+int rlfc_env_import_device(rlfc_env* E, const int* d_env_ids, int n, const void* d_buf, size_t record_bytes_,
+                           int keep_accumulators) {
+  int rc = records_check_handle(E, n, d_env_ids && d_buf);
+  if (rc) return rc;
+  if (reinterpret_cast<uintptr_t>(d_buf) % 16) return fail(RLFC_EINVAL, "the record buffer must be 16-byte aligned");
+  const size_t base = record_bytes(E->sp.n, E->sp.m, 0);
+  if (record_bytes_ < base || (record_bytes_ - base) % 16 || (record_bytes_ - base) / 16 > (1u << 24))
+    return fail(RLFC_EINVAL, "record_bytes " + std::to_string(record_bytes_) + " is not the size of a record of the handle's grid");
+  if (n == 0) return RLFC_OK;
+  CU(cudaSetDevice(E->device));
+  if ((rc = record_check_enqueue(E, d_env_ids, n, d_buf, record_bytes_))) return rc;
+  return record_apply_enqueue(E, d_env_ids, n, d_buf, record_bytes_, keep_accumulators != 0);
 }
 
 int rlfc_env_get_sensors(rlfc_env* E, float* out) {

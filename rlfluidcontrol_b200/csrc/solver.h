@@ -194,6 +194,35 @@ struct SnapSlots {
   int *refused;             // [B] 1 = the last restore into the environment was skipped (rlfc_env_get_flags bit 1)
 };
 
+// State records (rlfc.h "State records"; records.cuh).  Allocated by the first record call of a handle, kept out of
+// SolverParams for the reason SensorSet is.
+struct RecordBufs {
+  const unsigned *env_par;  // [5][B] each environment's parameter tuple (bits): SnapSlots::env_par
+  const rlfc_sensor *sensors;   // [n_sensors] the sensor table as given at create (nullptr without sensors)
+  int *refused;             // [B] 1 = the last device import aimed at the environment was refused (rlfc_env_get_flags bit 3)
+  unsigned long long *partial;  // [pairs][chunks] partial checksums
+  unsigned *ticket;         // [pairs] CTAs of a pair done (zero between launches)
+  int *hcode, *verdict;     // [pairs] header verdict, final verdict (RecordCheck, kRecSkip)
+  int grid[3];              // resolution, x_lengths, y_lengths
+};
+// The checks of an import, in the order they are made; the verdict of a pair is the first that fails (0: apply)
+enum RecordCheck { kRecSkip = -1, kRecApply = 0, kRecMagic, kRecVersion, kRecLength, kRecGrid, kRecChecksum, kRecTuple, kRecDt };
+// the checksum term of word value x at word index w of a record: MurmurHash3's 64-bit finalizer of (w << 32 | x), a
+// bijection, so that changing any one word changes the sum mod 2^64
+__host__ __device__ inline unsigned long long record_mix(unsigned long long w, unsigned x) {
+  unsigned long long h = w << 32 | x;
+  h ^= h >> 33;
+  h *= 0xff51afd7ed558ccdull;
+  h ^= h >> 33;
+  h *= 0xc4ceb9fe1a85ec53ull;
+  h ^= h >> 33;
+  return h;
+}
+// bytes of a record of an n x m grid (incl. ghosts) with K sensors
+__host__ __device__ inline size_t record_bytes(int n, int m, int K) {
+  return RLFC_RECORD_HEADER_BYTES + 4 * kSnapWords + 16 * (size_t)K + 12 * (size_t)n * m;
+}
+
 // Parameter library (rlfc_config.param_sets; param_sets.cuh).  Set s's geometry lives in geometry slot sets[s].slot >= B
 // (equal sets share one); the rest of what an environment of set s holds per environment is in its LibSet.  Kept out of
 // SolverParams for the reason SensorSet is.
@@ -325,5 +354,17 @@ int launch_reset_params(const SolverParams& P, const ParamLib& lib, const SnapSl
                         const CircleFactors& cf, int nc, int mc, int cap, const float* init_ux, const float* init_uy,
                         const float* init_p, float init_t, float* ux, float* uy, const int* d_env,
                         const rlfc_env_params* d_par, int n, int reset_accumulators, int* skip, cudaStream_t st);
+
+// State records (records.cuh): record_chunks = the partial checksums per pair a launch of bytes-long records needs.
+// Export writes record k (record_bytes(P.n, P.m, sens.n) bytes at rec + k * that) of environment d_ids[k], a record with a
+// zero header for an id out of range.  Import with check = 1 writes rb.verdict (the winning pair of each destination is
+// checked, the others skipped) and nothing else; check = 0 then applies the pairs whose verdict is 0, writes rb.refused of
+// every winning pair and skip[e] = 0 of those applied.
+int record_chunks(int n, int m, size_t bytes);
+int launch_record_export(const SolverParams& P, const SensorSet& sens, const RecordBufs& rb, float* ux, float* uy,
+                         const int* d_ids, int n, void* rec, cudaStream_t st);
+int launch_record_import(const SolverParams& P, const SensorSet& sens, const RecordBufs& rb, float* ux, float* uy,
+                         const int* d_ids, int n, const void* rec, size_t bytes, int check, int keep_accumulators, int* skip,
+                         cudaStream_t st);
 
 }  // namespace rlfc

@@ -1939,5 +1939,6 @@ int launch_emit_obs(const SolverParams& q, const float* d_actions, float* d_obs,
 }  // namespace rlfc
 
 #include "snapshot.cuh"
+#include "records.cuh"
 #include "param_sets.cuh"
 #include "geometry_device.cuh"

@@ -106,6 +106,13 @@ def load_library():
     L.rlfc_env_restore.argtypes = [vp, ip, ip, C.c_int, C.c_int]
     L.rlfc_env_snapshot_device.argtypes = [vp, vp, vp, C.c_int]
     L.rlfc_env_restore_device.argtypes = [vp, vp, vp, C.c_int, C.c_int]
+    L.rlfc_record_bytes.argtypes = [C.POINTER(Config), C.POINTER(C.c_size_t)]
+    L.rlfc_record_checksum.argtypes = [vp, C.c_size_t]
+    L.rlfc_record_checksum.restype = C.c_ulonglong
+    L.rlfc_env_export.argtypes = [vp, ip, C.c_int, vp]
+    L.rlfc_env_import.argtypes = [vp, ip, C.c_int, vp, C.c_int]
+    L.rlfc_env_export_device.argtypes = [vp, vp, C.c_int, vp]
+    L.rlfc_env_import_device.argtypes = [vp, vp, C.c_int, vp, C.c_size_t, C.c_int]
     L.rlfc_env_get_sensors.argtypes = [vp, fp]
     L.rlfc_env_get_sensors_device.argtypes = [vp, vp]
     L.rlfc_env_field_sum.argtypes = [vp, fp]
@@ -337,6 +344,45 @@ class AFCCylinderBatch:
         self._check(self._L.rlfc_env_restore_device(self._h, C.c_void_p(d_env_ids), C.c_void_p(d_slots), int(n),
                                                     int(keep_accumulators)), "rlfc_env_restore_device")
 
+    @property
+    def record_bytes(self):
+        """Bytes of one state record of this handle (rlfc_record_bytes)."""
+        n = C.c_size_t()
+        self._check(self._L.rlfc_record_bytes(C.byref(self.cfg), C.byref(n)), "rlfc_record_bytes")
+        return n.value
+
+    def export_states(self, env_ids):
+        """The complete states of environments env_ids as len(env_ids) consecutive state records (include/rlfc.h "State
+        records"; `records.parse_record` reads one).  Any handle of the same grid imports them, on any device or process."""
+        ids = np.ascontiguousarray(env_ids, dtype=np.int32).reshape(-1)
+        out = bytearray(len(ids) * self.record_bytes)
+        buf = (C.c_char * len(out)).from_buffer(out) if out else None
+        self._check(self._L.rlfc_env_export(self._h, _ip(ids), len(ids), buf), "rlfc_env_export")
+        return bytes(out)
+
+    def import_states(self, env_ids, records, keep_accumulators=False):
+        """Record k of `records` (bytes of consecutive equal-size records) -> environment env_ids[k]; all or nothing: a
+        record that fails a check raises RlfcError naming it, and nothing changes.  keep_accumulators: as in restore()."""
+        ids = np.ascontiguousarray(env_ids, dtype=np.int32).reshape(-1)
+        data = np.frombuffer(memoryview(records).cast("B"), np.uint8)
+        if len(ids) and data.size < len(ids) * 16:
+            raise ValueError(f"{data.size} bytes cannot hold {len(ids)} records")
+        self._check(self._L.rlfc_env_import(self._h, _ip(ids), len(ids), data.ctypes.data if data.size else None,
+                                            int(keep_accumulators)), "rlfc_env_import")
+
+    def export_states_device(self, d_env_ids, n, d_records):
+        """export_states() into a 16-byte aligned device buffer of n * record_bytes (data_ptr() ints), asynchronous on the
+        handle's stream.  A pair whose id is out of range writes a record every import refuses."""
+        self._check(self._L.rlfc_env_export_device(self._h, C.c_void_p(d_env_ids), int(n), C.c_void_p(d_records)),
+                    "rlfc_env_export_device")
+
+    def import_states_device(self, d_env_ids, n, d_records, record_bytes, keep_accumulators=False):
+        """import_states() from a device buffer of n records of record_bytes each, asynchronous.  Ids out of range are
+        skipped, the last in-range pair per environment wins; a record that fails a check leaves its environment
+        unchanged and sets flags() bit 3."""
+        self._check(self._L.rlfc_env_import_device(self._h, C.c_void_p(d_env_ids), int(n), C.c_void_p(d_records),
+                                                   int(record_bytes), int(keep_accumulators)), "rlfc_env_import_device")
+
     def sensors(self):
         """(n_envs, n_sensors) float32: each environment's sensors, sampled after its most recent solver step from the
         state `get_fields` returns.  `step(a)` followed by `sensors()` gives the sensor observation of each environment."""
@@ -428,7 +474,8 @@ class AFCCylinderBatch:
     def flags(self):
         """Per-environment health flags (bit 0: a non-finite force was produced since the last reset; bit 1: the last
         restore aimed at the environment was skipped, its slot unwritten or of another parameter set; bit 2: the last
-        device parameter reset aimed at the environment was refused, its set invalid)."""
+        device parameter reset aimed at the environment was refused, its set invalid; bit 3: the last device import aimed
+        at the environment was refused, its record failing a check)."""
         f = np.empty(self.n_envs, np.int32)
         self._check(self._L.rlfc_env_get_flags(self._h, f.ctypes.data_as(C.POINTER(C.c_int))), "rlfc_env_get_flags")
         return f
