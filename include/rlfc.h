@@ -134,6 +134,11 @@ typedef struct {
                            before any device call.  RLFC_EINVAL for n_param_sets < 0, NULL with n_param_sets > 0, an
                            invalid entry (the message names param_sets[k]), slab mode, or a grid with chained or wavefront
                            levels.                                                                                     */
+  int   stats_every;    /* 0 (default) = no flow statistics: nothing is allocated or launched for them.  k >= 1 = every
+                           environment accumulates flow statistics (rlfc_env_get_stats below) from a sample after every
+                           k-th solver step it takes part in, counted since its statistics were last reset.  56 bytes per
+                           pitched cell of device memory, 4.3 MB per environment at the default grid.  RLFC_EINVAL if < 0,
+                           or > 0 in slab mode.                                                                        */
 } rlfc_config;
 
 void rlfc_default_config(rlfc_config *cfg);
@@ -322,6 +327,43 @@ int  rlfc_env_get_sensors(rlfc_env *env, float *out);
 /* Same into DEVICE memory: one device-to-device copy on the handle's stream, no sync.  Enqueued after
    rlfc_env_step_device, it gives a GPU-resident policy its observation without the host. */
 int  rlfc_env_get_sensors_device(rlfc_env *env, float *d_out);
+
+/* Flow statistics (rlfc_config.stats_every = k >= 1): running sums from which the mean flow, the RMS of its fluctuations and
+   the Reynolds shear stress of each environment follow.  Each environment holds RLFC_NUM_STATS float64 sums per cell of the
+   reference layout n x m (ghosts included, as rlfc_env_get_fields returns it) and a sample count:
+     RLFC_STAT_UX, _UY, _P        sum of (double)x for x = u.x, u.y, p
+     RLFC_STAT_UXUX, _UYUY, _PP   sum of (double)x * (double)x
+     RLFC_STAT_UV                 sum of (double)ucc * (double)vcc on interior cells (1 <= i <= n-2, 1 <= j <= m-2), where
+                                  ucc = (u.x[i][j] + u.x[i+1][j]) * 0.5f and vcc = (u.y[i][j] + u.y[i][j+1]) * 0.5f in float;
+                                  zero on the ghost cells
+   The product of two floats is exact in double, so every term is rounded once, when it is added; the terms of a cell are
+   added in step order, so the sums are reproducible bit for bit and equal to the same sums taken on the host.
+   A sample is the state the next solver step starts from -- the u and p rlfc_env_get_fields returns, what sensors read.  An
+   environment takes part in a solver step as it does for sensors: one frozen at the start of the step (waiting at the end of
+   its observation window, or past episode_time) takes no sample and does not advance its step counter.  A sample is taken
+   after every k-th step an environment takes part in since its statistics were last reset.  In adaptive mode a sample counts
+   once whatever the dt of its step: the statistics are per step, not time-weighted.
+   Statistics are analysis, not state: rlfc_env_reset, _reset_params, _reset_sets, _reset_params_device, _restore, _import
+   and their device variants leave them as they are, and snapshot slots and state records do not carry them. */
+#define RLFC_NUM_STATS  7
+#define RLFC_STAT_UX    0
+#define RLFC_STAT_UY    1
+#define RLFC_STAT_P     2
+#define RLFC_STAT_UXUX  3
+#define RLFC_STAT_UYUY  4
+#define RLFC_STAT_PP    5
+#define RLFC_STAT_UV    6
+/* Environment e's sample count and, unless sums is NULL, its sums, sums[RLFC_NUM_STATS][n][m].  HOST memory, synchronises the
+   handle's stream.  RLFC_EINVAL for a handle created without statistics, an e out of range or a NULL count. */
+int  rlfc_env_get_stats(rlfc_env *env, int e, long long *count, double *sums);
+/* Start new statistics for environments env_ids[0 .. n-1] (NULL = all): their sums, sample counts and step counters become 0,
+   so the next sample is taken k steps later.  HOST array, synchronous on return, all or nothing: RLFC_EINVAL (and nothing
+   changes) for a handle without statistics or an id out of range. */
+int  rlfc_env_stats_reset(rlfc_env *env, const int *env_ids, int n);
+/* Same with a DEVICE int array of length n, asynchronous on the handle's stream.  An id out of range is skipped, so
+   ids = where(done, arange(n_envs), -1) starts new statistics for the finished episodes without the host.  RLFC_EINVAL for a
+   handle without statistics, n < 0 or a NULL array with n > 0. */
+int  rlfc_env_stats_reset_device(rlfc_env *env, const int *d_env_ids, int n);
 
 /* One solver step (AFCCylinder.update2) without the draw() accumulation.  HOST pointers.
      actions [n_envs][2] (NULL = keep current xi); force [n_envs][2] raw (fx, fy) = -pressForce;

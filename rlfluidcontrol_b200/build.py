@@ -15,7 +15,7 @@ CSRC = PKG / "csrc"
 LIB = PKG / "librlfc.so"
 SOURCES = ["rlfc_api.cu", "solver_kernels.cu", "geometry.cpp", "vmm.cpp"]
 HEADERS = ["solver.h", "geometry.h", "vmm.h", "smooth_rows.cuh", "smooth_wave.cuh", "smooth_chain.cuh", "smooth_chain3.cuh", "smooth_tiny.cuh", "exact_sum.cuh",
-           "exact_sum_kernels.cuh", "snapshot.cuh", "records.cuh", "param_sets.cuh", "geometry_device.cuh",
+           "exact_sum_kernels.cuh", "snapshot.cuh", "records.cuh", "param_sets.cuh", "geometry_device.cuh", "flow_stats.cuh",
            "../../include/rlfc.h"]
 
 NVCC_FLAGS = [

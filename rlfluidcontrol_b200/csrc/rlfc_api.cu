@@ -55,6 +55,7 @@ struct rlfc_env {
   int *snap_env = nullptr, *snap_slot = nullptr;   // [max(B, S)] the pairs of a host snapshot / restore call
   SensorSet sens{};                        // rlfc_config.sensors of the whole batch (sens.n = 0: none)
   std::vector<rlfc_sensor> sensor_table;   // rlfc_config.sensors as given (what a record's sensor table holds)
+  FlowStats fs{};                          // rlfc_config.stats_every of the whole batch (fs.every = 0: none)
   // state records (records.cuh): nothing is allocated before the first record call (rec.refused = nullptr until then)
   RecordBufs rec{};
   std::vector<void*> rec_bufs;             // rec's growing scratch, its id buffer and the host calls' staging buffer
@@ -96,6 +97,7 @@ struct rlfc_env {
     SolverParams sp{};                       // view of the batch arrays restricted to [e0, e0 + B); lev[0].x = pressure buffer A
     SolverParams spB{};                      // same view with lev[0].x = pressure buffer B (p ping-pongs A -> B -> A per half step)
     SensorSet sens{};                        // the view's sensors (out at e0 * n)
+    FlowStats fs{};                          // the view's flow statistics (at environment e0)
     float *uAx = nullptr, *uAy = nullptr, *uBx = nullptr, *uBy = nullptr, *uCx = nullptr, *uCy = nullptr;
     cudaStream_t st = nullptr;               // group 0 runs on the handle's stream
     cudaEvent_t done = nullptr;
@@ -804,6 +806,11 @@ int solver_step(Sink& S, const Group& G, int accumulate) {
   }
   // (before k_force, which freezes an environment at the end of its window: this step's sample is its observation)
   if (G.sens.n > 0) S.run({"k_sensors", 0, kA, kSolo}, [&](auto& v, auto st) { return launch_sensors(v, G.sens, G.uAx, G.uAy, st); });
+  if (G.fs.every > 0) {
+    // a sampled step reads 3 floats and reads and writes 7 doubles on every cell of the n x m layout: 124 B per cell
+    const double fpc = 31.0 * sp.n * sp.m / ((double)(sp.n - 2) * (sp.m - 2));
+    S.run({"k_flow_stats", fpc, kA, kSolo}, [&](auto& v, auto st) { return launch_flow_stats(v, G.fs, G.uAx, G.uAy, st); });
+  }
   S.run({"k_force", 0, kA, kSolo}, [&](auto& v, auto st) { return launch_force(v, accumulate, st); });
   S.sync();
   return RLFC_OK;
@@ -1037,6 +1044,11 @@ void make_view(const rlfc_env* E, int e0, int n, int row, Group& G) {
   G.spB.lev[0].x = E->pB + (size_t)e0 * sp.stride;
   G.sens = E->sens;
   if (G.sens.out) G.sens.out += (size_t)e0 * G.sens.n;
+  G.fs = E->fs;
+  if (G.fs.every > 0) {
+    G.fs.sums += (size_t)e0 * kNumStats * sp.stride;
+    G.fs.count += e0; G.fs.step += e0; G.fs.ticket += e0;
+  }
   const size_t o = (size_t)e0 * sp.stride;
   G.uAx = E->uAx + o; G.uAy = E->uAy + o; G.uBx = E->uBx + o; G.uBy = E->uBy + o; G.uCx = E->uCx + o; G.uCy = E->uCy + o;
 }
@@ -1140,6 +1152,9 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
         return fail(RLFC_EINVAL, "sensors[" + std::to_string(k) + "]: coordinates must be finite");
     }
   }
+  if (cfg->stats_every < 0) return fail(RLFC_EINVAL, "stats_every must be >= 0");
+  if (cfg->stats_every > 0 && cfg->n_devices > 1)
+    return fail(RLFC_EINVAL, "stats_every is not available in slab mode (n_devices > 1)");
   // per-environment parameters: every set validated and its geometry built before any device call
   std::vector<EnvGeometry> env_geo;
   std::vector<int> env_set;
@@ -1506,6 +1521,12 @@ int rlfc_env_create(const rlfc_config* cfg, rlfc_env** out) {
   TRY(E->dmalloc(&E->uBx, S)); TRY(E->dmalloc(&E->uBy, S));
   TRY(E->dmalloc(&E->uCx, S)); TRY(E->dmalloc(&E->uCy, S));
   TRY(E->dmalloc(&E->init_ux, sp.stride)); TRY(E->dmalloc(&E->init_uy, sp.stride)); TRY(E->dmalloc(&E->init_p, sp.stride));
+  if (cfg->stats_every > 0) {   // flow statistics (solver.h FlowStats), all zero: no samples yet
+    FlowStats& f = E->fs;
+    f.every = cfg->stats_every;
+    TRY(E->dmalloc(&f.sums, (size_t)kNumStats * sp.stride * B));
+    TRY(E->dmalloc(&f.count, B)); TRY(E->dmalloc(&f.step, B)); TRY(E->dmalloc(&f.ticket, B));
+  }
   // per-env scalars
   sp.rr_blocks = 0;
   sp.tiny = 1;
@@ -2149,6 +2170,58 @@ int rlfc_env_import_device(rlfc_env* E, const int* d_env_ids, int n, const void*
   CU(cudaSetDevice(E->device));
   if ((rc = record_check_enqueue(E, d_env_ids, n, d_buf, record_bytes_))) return rc;
   return record_apply_enqueue(E, d_env_ids, n, d_buf, record_bytes_, keep_accumulators != 0);
+}
+
+int rlfc_env_get_stats(rlfc_env* E, int e, long long* count, double* sums) {
+  if (!E || !count) return fail(RLFC_EINVAL, "null argument");
+  if (!E->fs.every) return fail(RLFC_EINVAL, "the handle has no flow statistics (rlfc_config.stats_every = 0)");
+  const SolverParams& sp = E->sp;
+  if (e < 0 || e >= sp.B) return fail(RLFC_EINVAL, "env id " + std::to_string(e) + " out of range");
+  CU(cudaSetDevice(E->device));
+  CU(cudaMemcpyAsync(count, E->fs.count + e, sizeof(long long), cudaMemcpyDeviceToHost, E->stream));
+  for (int s = 0; sums && s < kNumStats; s++)
+    CU(cudaMemcpy2DAsync(sums + (size_t)s * sp.n * sp.m, sp.m * sizeof(double), E->fs.sums + ((size_t)e * kNumStats + s) * sp.stride,
+                         sp.P * sizeof(double), sp.m * sizeof(double), sp.n, cudaMemcpyDeviceToHost, E->stream));
+  CU(cudaStreamSynchronize(E->stream));
+  return RLFC_OK;
+}
+
+int rlfc_env_stats_reset(rlfc_env* E, const int* env_ids, int n) {
+  if (!E) return fail(RLFC_EINVAL, "null handle");
+  if (!E->fs.every) return fail(RLFC_EINVAL, "the handle has no flow statistics (rlfc_config.stats_every = 0)");
+  const int B = E->sp.B;
+  if (!env_ids) n = B;
+  if (n < 0) return fail(RLFC_EINVAL, "bad env count");
+  for (int k = 0; env_ids && k < n; k++)
+    if (env_ids[k] < 0 || env_ids[k] >= B) return fail(RLFC_EINVAL, "env id " + std::to_string(env_ids[k]) + " out of range");
+  CU(cudaSetDevice(E->device));
+  const FlowStats& f = E->fs;
+  const size_t per_env = (size_t)kNumStats * E->sp.stride;
+  if (!env_ids) {
+    CU(cudaMemsetAsync(f.sums, 0, per_env * B * sizeof(double), E->stream));
+    CU(cudaMemsetAsync(f.count, 0, B * sizeof(long long), E->stream));
+    CU(cudaMemsetAsync(f.step, 0, B * sizeof(int), E->stream));
+  }
+  for (int k = 0; env_ids && k < n; k++) {
+    const int e = env_ids[k];
+    CU(cudaMemsetAsync(f.sums + e * per_env, 0, per_env * sizeof(double), E->stream));
+    CU(cudaMemsetAsync(f.count + e, 0, sizeof(long long), E->stream));
+    CU(cudaMemsetAsync(f.step + e, 0, sizeof(int), E->stream));
+  }
+  CU(cudaStreamSynchronize(E->stream));
+  return RLFC_OK;
+}
+
+int rlfc_env_stats_reset_device(rlfc_env* E, const int* d_env_ids, int n) {
+  if (!E) return fail(RLFC_EINVAL, "null handle");
+  if (!E->fs.every) return fail(RLFC_EINVAL, "the handle has no flow statistics (rlfc_config.stats_every = 0)");
+  if (n < 0) return fail(RLFC_EINVAL, "bad env count");
+  if (n > 0 && !d_env_ids) return fail(RLFC_EINVAL, "null argument");
+  if (n == 0) return RLFC_OK;
+  CU(cudaSetDevice(E->device));
+  E->run("k_stats_reset", 0, [&] { return launch_stats_reset(E->sp, E->fs, d_env_ids, n, E->stream); });
+  CU(cudaGetLastError());
+  return RLFC_OK;
 }
 
 int rlfc_env_get_sensors(rlfc_env* E, float* out) {

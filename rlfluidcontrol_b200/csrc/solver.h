@@ -177,6 +177,17 @@ struct SensorSet {
   float* out;               // [B][n] the sample of each environment's last solver step (k_sensors)
 };
 
+// Flow statistics (rlfc_config.stats_every; flow_stats.cuh) of a view of the batch, pointers at the view's environment e0;
+// every = 0: none, nothing is allocated or launched for them.  Kept out of SolverParams for the reason SensorSet is.
+constexpr int kNumStats = RLFC_NUM_STATS;
+struct FlowStats {
+  int every;                // a sample after every `every`-th solver step an environment takes part in
+  double* sums;             // [B][kNumStats][stride] the running sums in the level-0 pitched layout, sum s of e at (e*7 + s)*stride
+  long long* count;         // [B] samples taken
+  int* step;                // [B] solver steps taken part in since the last sample (or the last statistics reset)
+  unsigned* ticket;         // [B] CTAs of the running launch that have read `step` (zero between launches)
+};
+
 // Snapshot slots (rlfc_config.n_snapshots; snapshot.cuh).  Slot s holds one environment's state: u.x, u.y (step-start
 // buffer A) and p (lev[0].x) at s * stride in the level-0 pitched layout, the scalar record rec[w * S + s] (word w of
 // snap_word in snapshot.cuh) and the header hdr[w * S + s]: w = 0 written (0 = never), w = 1 .. 5 the bits of the
@@ -310,6 +321,11 @@ int launch_force(const SolverParams& P, int accumulate, cudaStream_t st);
 // flow sensors: s.out[e][k] = Field.linear of sensor k's field (u.x = ux, u.y = uy, p = P.lev[0].x) for every environment
 // not frozen.  A step runs it after the corrector's last kernel and before launch_force, which may freeze the environment
 int launch_sensors(const SolverParams& P, const SensorSet& s, const float* ux, const float* uy, cudaStream_t st);
+// flow statistics: every environment not frozen advances its step counter, and on every f.every-th step adds u.x = ux, u.y = uy,
+// p = P.lev[0].x to its sums (rlfc.h "Flow statistics").  A step runs it right after launch_sensors, for the same reason
+int launch_flow_stats(const SolverParams& P, const FlowStats& f, const float* ux, const float* uy, cudaStream_t st);
+// zero the sums, count and step counter of environments d_ids[0 .. n-1] (device array; ids out of range are skipped)
+int launch_stats_reset(const SolverParams& P, const FlowStats& f, const int* d_ids, int n, cudaStream_t st);
 // BDIM.checkCFL of every environment's current velocity: d_dt[B] = min(1/(max(|ux|+|uy|) + 3 nu), 1)
 int launch_check_cfl(const SolverParams& P, const float* ux, const float* uy, float* d_dt, cudaStream_t st);
 // adaptive mode, start of a solver step: sc.dt[e] = BDIM.checkCFL of u for every environment not frozen (frozen ones keep theirs)

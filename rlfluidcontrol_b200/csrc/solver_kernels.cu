@@ -17,6 +17,7 @@
 //   k_bc          u.setBC after the projection                          VectorField.pde:140
 //   k_heun        u = (u + us) * 0.5                                     BDIM.pde:95-96
 //   k_sensors     Field.linear of p / u.x / u.y at the user's points     Field.pde:175-190
+//   k_flow_stats  running float64 sums of u.x, u.y, p, their squares and ucc*vcc (flow_stats.cuh)
 //   k_force       pressForce + probes + time + draw() accumulation       Body.pde:296-303, SaveScalar.pde:61-72, clientCFD.pde:39-47
 #include "solver.h"
 #include "smooth_rows.cuh"
@@ -1942,3 +1943,4 @@ int launch_emit_obs(const SolverParams& q, const float* d_actions, float* d_obs,
 #include "records.cuh"
 #include "param_sets.cuh"
 #include "geometry_device.cuh"
+#include "flow_stats.cuh"

@@ -16,6 +16,8 @@ _PKG = Path(__file__).resolve().parent
 # RLFC_LIBRARY selects another build of the same library (e.g. an instrumented one made by tools/); never a fallback
 _LIB_PATH = Path(os.environ["RLFC_LIBRARY"]).resolve() if os.environ.get("RLFC_LIBRARY") else _PKG / "librlfc.so"
 NUM_PROBES = 32
+# rlfc.h "Flow statistics": the sums of rlfc_env_get_stats, in this order (RLFC_STAT_UX .. RLFC_STAT_UV)
+STAT_NAMES = ("ux", "uy", "p", "uxux", "uyuy", "pp", "uv")
 
 
 class RlfcError(RuntimeError):
@@ -49,6 +51,7 @@ class Config(C.Structure):
         ("env_params", C.POINTER(EnvParams)), ("n_snapshots", C.c_int),
         ("n_sensors", C.c_int), ("sensors", C.POINTER(Sensor)),
         ("n_param_sets", C.c_int), ("param_sets", C.POINTER(EnvParams)),
+        ("stats_every", C.c_int),
     ]
 
 
@@ -115,6 +118,9 @@ def load_library():
     L.rlfc_env_import_device.argtypes = [vp, vp, C.c_int, vp, C.c_size_t, C.c_int]
     L.rlfc_env_get_sensors.argtypes = [vp, fp]
     L.rlfc_env_get_sensors_device.argtypes = [vp, vp]
+    L.rlfc_env_get_stats.argtypes = [vp, C.c_int, C.POINTER(C.c_longlong), C.POINTER(C.c_double)]
+    L.rlfc_env_stats_reset.argtypes = [vp, ip, C.c_int]
+    L.rlfc_env_stats_reset_device.argtypes = [vp, vp, C.c_int]
     L.rlfc_env_field_sum.argtypes = [vp, fp]
     L.rlfc_env_field_sum_stats.argtypes = [vp, ip]
     L.rlfc_env_get_static.argtypes = [vp, C.c_char_p, C.c_int, fp, ip, ip]
@@ -171,6 +177,29 @@ def _sensor_array(sensors):
     return arr
 
 
+def flow_stats_from_sums(count, sums):
+    """The flow statistics of one environment from its sample count and sums[7, n, m] (`AFCCylinderBatch.stats_sums`), in
+    float64: the means of ux, uy and p; their variances sum(x^2)/N - mean^2; and uv_cov = sum(ucc*vcc)/N - mean(ucc)*mean(vcc)
+    on the interior cells (zero on the ghost cells), the cell-centred means taken from the face means as ucc and vcc are from
+    the faces: mean(ucc)[i][j] = (mean(ux)[i][j] + mean(ux)[i+1][j]) / 2, mean(vcc)[i][j] = (mean(uy)[i][j] + mean(uy)[i][j+1]) / 2.
+    Returns a dict of (n, m) arrays and the count."""
+    if count <= 0:
+        raise ValueError("no samples: the statistics were reset and no sampled step has run since")
+    S = np.asarray(sums, np.float64)
+    N = float(count)
+    mean = {k: S[i] / N for i, k in enumerate(("ux", "uy", "p"))}
+    out = dict(count=int(count))
+    for i, k in enumerate(("ux", "uy", "p")):
+        out[f"mean_{k}"] = mean[k]
+        out[f"var_{k}"] = S[3 + i] / N - mean[k] * mean[k]
+    cov = np.zeros_like(S[6])
+    ucc = (mean["ux"][1:-1, 1:-1] + mean["ux"][2:, 1:-1]) * 0.5
+    vcc = (mean["uy"][1:-1, 1:-1] + mean["uy"][1:-1, 2:]) * 0.5
+    cov[1:-1, 1:-1] = S[6][1:-1, 1:-1] / N - ucc * vcc
+    out["uv_cov"] = cov
+    return out
+
+
 class AFCCylinderBatch:
     """A batch of AFCCylinder environments on one GPU."""
 
@@ -181,7 +210,9 @@ class AFCCylinderBatch:
         sensors: None, or a sequence of (field, x, y), field "p", "ux" or "uy", (x, y) in grid coordinates: the flow
         sampled in every environment after each of its solver steps (`sensors()`).
         param_sets: None, or a library of constructor arguments given like env_params (any number of entries), built at
-        create; `reset_sets` / `reset_sets_device` switch environments to its entries on the device."""
+        create; `reset_sets` / `reset_sets_device` switch environments to its entries on the device.
+        stats_every (a config keyword): 0 (default) = no flow statistics; k >= 1 = every environment accumulates the sums of
+        `stats_sums` / `flow_stats` from a sample after every k-th solver step it takes part in."""
         self._L = load_library()
         cfg = Config()
         self._L.rlfc_default_config(C.byref(cfg))
@@ -394,6 +425,35 @@ class AFCCylinderBatch:
         """sensors() into a device float32 buffer of n_envs * n_sensors (data_ptr() int), asynchronous on the handle's
         stream: after `step_device` it gives a GPU-resident policy its observation without the host."""
         self._check(self._L.rlfc_env_get_sensors_device(self._h, C.c_void_p(d_out)), "rlfc_env_get_sensors_device")
+
+    def stats_sums(self, e):
+        """(count, sums[7, n, m] float64) of environment e's flow statistics (rlfc.h "Flow statistics"; the sums in the
+        order of STAT_NAMES).  Synchronises the handle's stream."""
+        count = C.c_longlong()
+        sums = np.empty((len(STAT_NAMES), self.n, self.m), np.float64)
+        self._check(self._L.rlfc_env_get_stats(self._h, int(e), C.byref(count), sums.ctypes.data_as(C.POINTER(C.c_double))),
+                    "rlfc_env_get_stats")
+        return count.value, sums
+
+    def flow_stats(self, e):
+        """Environment e's mean flow, variances and Reynolds shear stress from its sums (`flow_stats_from_sums`).  Samples
+        are per step: in adaptive mode they are not weighted by dt."""
+        return flow_stats_from_sums(*self.stats_sums(e))
+
+    def stats_reset(self, env_ids=None):
+        """Start new statistics for the listed environments (None = all); the next sample comes stats_every steps later.
+        All or nothing: an id out of range raises and changes nothing."""
+        if env_ids is None:
+            rc = self._L.rlfc_env_stats_reset(self._h, None, self.n_envs)
+        else:
+            ids = np.ascontiguousarray(env_ids, dtype=np.int32).reshape(-1)
+            rc = self._L.rlfc_env_stats_reset(self._h, _ip(ids), len(ids))
+        self._check(rc, "rlfc_env_stats_reset")
+
+    def stats_reset_device(self, d_env_ids, n):
+        """stats_reset() with a device int32 array of length n (data_ptr() int), asynchronous on the handle's stream: ids out
+        of range are skipped, so stats_reset_device(where(done, arange(B), -1), B) restarts the finished episodes' statistics."""
+        self._check(self._L.rlfc_env_stats_reset_device(self._h, C.c_void_p(d_env_ids), int(n)), "rlfc_env_stats_reset_device")
 
     @staticmethod
     def _pairs(env_ids, slots, what="slots"):
